@@ -58,8 +58,8 @@ int launch_aggregate_normalize(const void* E, int e_dtype, int64_t n_src, int64_
 
 // Arguments of the list-merge kernel (topk_merge.cu).
 //  * public use (hgr_topk_merge / SIMT path): `P` lists of length KL == K per row, all valid.
-//  * tcgen05 path: `use_sched` -- row tile mt owns sched.parts(mt) * wpq lists of length KL (the per-warp
-//    partial lists of each CTA segment).  When KL < K the lists are SPECULATIVE (narrower than K); the merge
+//  * tcgen05 path: `use_sched` -- row tile mt owns sched.parts(mt) lists of length KL (the partial lists of
+//    each worker segment).  When KL < K the lists are SPECULATIVE (narrower than K); the merge
 //    certifies every row (a full list whose last entry still beats the merged K-th value may hide candidates)
 //    and re-scans uncertified rows exactly on the CUDA cores, for which it needs X / bank.
 // Row-block scatter of the final lists: rows [g * block_rows, (g + 1) * block_rows) go to val[g] / idx[g] (each a
@@ -83,7 +83,7 @@ struct MergeArgs {
   int64_t P, B;
   int KL, K;
   int64_t part_stride;      // elements between consecutive lists (0 -> B * KL)
-  int use_sched, wpq;
+  int use_sched;
   Sched sched;
   const int32_t* col_id;
   int32_t id_base;

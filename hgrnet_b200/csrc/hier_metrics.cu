@@ -15,6 +15,7 @@
 // smallest position j in `cols` wins; a masked column holds exactly -1.0f, so when no in-level value exceeds -1 the
 // first position holding -1 wins -- `first_out[l]` is the first position whose column is NOT at level l.
 #include "common.cuh"
+#include "topk_list.cuh"
 
 namespace hgr {
 namespace {
@@ -146,9 +147,9 @@ hier_metrics_kernel(const float* __restrict__ logits, int64_t ldl, const int32_t
 }
 
 // Second half of the FUSED path (hgr_hier_metrics_fused): the per-level in-level maxima come from the GEMM epilogue
-// (score_pair.cu, kEpiLevel) as (order key << 32 | ~sorted bank row) words; one thread per image row decodes them, maps
-// the sorted bank row back to its position in `train_index`, and applies the same rules as the kernel above: the -1
-// fill (first_out), first position among equal values, chain matching and counting.
+// (score_pair.cu, kEpiLevel) as winner words (topk_list.cuh: order key << 32 | ~sorted bank row); one thread per image
+// row decodes them, maps the sorted bank row back to its position in `train_index`, and applies the same rules as the
+// kernel above: the -1 fill (first_out), first position among equal values, chain matching and counting.
 __global__ void __launch_bounds__(128)
 hier_finish_kernel(unsigned long long* __restrict__ lvl_best, int64_t B, int64_t M, int n_levels,
                    const int32_t* __restrict__ sorted_to_pos, const int32_t* __restrict__ first_out,
@@ -166,9 +167,8 @@ hier_finish_kernel(unsigned long long* __restrict__ lvl_best, int64_t B, int64_t
     lvl_best[row * n_levels + lane] = 0ull;     // the workspace is handed back zeroed: the next call needs no memset
     const int32_t fo = first_out[lane];
     if (w != 0ull) {
-      const uint32_t k = static_cast<uint32_t>(w >> 32);
-      v = __uint_as_float((k & 0x80000000u) ? (k & 0x7FFFFFFFu) : ~k);
-      j = sorted_to_pos[~static_cast<uint32_t>(w)];
+      v = winner_value(w);
+      j = sorted_to_pos[winner_item(w)];
     }
     node = j;
     if (fo >= 0 && fo < M && better(-1.0f, fo, v, j)) node = fo;   // the masked array holds -1 at every out-of-level position

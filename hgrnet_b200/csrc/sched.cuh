@@ -75,31 +75,19 @@ struct TileWalker {
   int64_t C;
   bool first;
   int seq;
-  int rem_first;
-  int full_units;   // units of a full sub-tile (sub-tile width / 16)
-  __host__ __device__ TileWalker(const Sched& s, int cta, int64_t C_, int rem_first_ = 1, int sub_n = kSubN)
-      : u(s.unit_begin(cta)), u_end(s.unit_begin(cta + 1)), U(s.U), C(C_), first(true), seq(0),
-        rem_first(rem_first_), full_units(sub_n / kUnit) {}
-  // Sub-tiles of a segment in ascending column order; the REMAINDER (segment length mod 256 columns) comes
-  // first: a narrow sub-tile costs almost a full one on the tensor pipe (the A operand is re-streamed for
-  // every sub-tile), so it is best spent while the epilogue has nothing to drain yet, and its short epilogue
-  // frees the first accumulator buffer long before the third sub-tile needs it.
+  __host__ __device__ TileWalker(const Sched& s, int cta, int64_t C_)
+      : u(s.unit_begin(cta)), u_end(s.unit_begin(cta + 1)), U(s.U), C(C_), first(true), seq(0) {}
+  // Sub-tiles of a segment in ascending column order: full 256-column sub-tiles first, the REMAINDER (segment length
+  // mod 256 columns) last -- its short epilogue is then the exposed tail of the worker.
   __host__ __device__ bool next(SubTile& t) {
     if (u >= u_end) return false;
     const int mt = static_cast<int>(u / U);
     int uu = static_cast<int>(u - static_cast<int64_t>(mt) * U);
-    const int kFull = full_units;
+    constexpr int kFull = kSubN / kUnit;
     int64_t seg = U - uu;                          // units left in this segment
     if (u_end - u < seg) seg = u_end - u;
-    int nu;
-    if (first) {
-      const int rem = static_cast<int>(seg % kFull);
-      nu = (rem != 0 && rem_first) ? rem : (seg < kFull ? static_cast<int>(seg) : kFull);
-      seq = 0;
-    } else {
-      nu = seg < kFull ? static_cast<int>(seg) : kFull;
-      ++seq;
-    }
+    const int nu = seg < kFull ? static_cast<int>(seg) : kFull;
+    seq = first ? 0 : seq + 1;
     t.seq = seq;
     t.mt = mt;
     t.col0 = uu * kUnit;

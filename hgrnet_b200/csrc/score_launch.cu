@@ -105,27 +105,26 @@ int common_setup(const __nv_bfloat16* X, const __nv_bfloat16* bank, int64_t B, i
   p->B = B;
   p->C = C;
   p->num_k_blocks = static_cast<int>((D + kBlockK - 1) / kBlockK);
-  p->rem_first = 0;   // remainder sub-tile last: its short epilogue is the exposed tail of the worker
   return HGR_OK;
 }
 
 // ---- list-width policy -------------------------------------------------------------------
 // With bank rows in random order, each of a row's true top-K members falls into a given list with probability
-// `share` = the fraction of the row's columns that list streams (the largest one: a worker's chunk of the schedule,
-// halved when two epilogue warps alternate its chunks).  A list of KL < K entries cannot be certified when it
-// receives KL or more of them: probability <= C(K, KL) * share^KL.  A repair re-scans that list's column range with
-// ONE warp of the merge kernel: measured ~0.6 us per bank row of 1024 elements (a 590-column range of cfg 2:
-// 0.36 ms; a 4,700-column range of cfg 5: 2.8 ms), and the whole call waits for it.
+// `share` = the fraction of the row's columns that list streams (the largest one: a worker's chunk of the schedule).
+// A list of KL < K entries cannot be certified when it receives KL or more of them: probability <= C(K, KL) *
+// share^KL.  A repair re-scans that list's column range with ONE warp of the merge kernel: measured ~0.6 us per bank
+// row of 1024 elements (a 590-column range of cfg 2: 0.36 ms; a 4,700-column range of cfg 5: 2.8 ms), and the whole
+// call waits for it.
 double overflow_bound(int K, int KL, double share) {
   double c = 1.0;
   for (int i = 0; i < KL; ++i) c = c * (K - i) / (i + 1);
   return c * std::pow(share, KL);
 }
 
-double max_list_share(const Sched& s, int wpq) {
+double max_list_share(const Sched& s) {
   const double chunk = static_cast<double>((s.T + s.G - 1) / s.G);   // units per worker
   const double share = chunk / static_cast<double>(s.U);
-  return (share > 1.0 ? 1.0 : share) / wpq;
+  return share > 1.0 ? 1.0 : share;
 }
 
 // Speculate only while the EXPECTED repair time per call stays below 1.5 % of the call's estimated duration (main
@@ -207,7 +206,7 @@ void umma_plan(int64_t B, int64_t C, int64_t D, int K, int32_t* plan) {
   plan[1] = s.MT;
   plan[2] = s.U;
   plan[3] = s.P;
-  plan[4] = pick_list_len(K, B, C, D, s.P, max_list_share(s, 1), true);
+  plan[4] = pick_list_len(K, B, C, D, s.P, max_list_share(s), true);
   plan[5] = 1;
   plan[6] = pair_ring_depth(B);
   plan[7] = static_cast<int32_t>((s.T + s.G - 1) / s.G * kUnit);
@@ -251,7 +250,7 @@ int launch_score_topk_umma(const __nv_bfloat16* X, const __nv_bfloat16* bank, co
   } else {
     const bool global_cert = variant == kVarProd && C_total > 0 && scatter != nullptr && scatter->emit_bound != 0;
     const int KL = global_cert ? pick_list_len_global(K, B, C, D, C_total, p.sched)
-                               : pick_list_len(K, B, C, D, p.sched.P, max_list_share(p.sched, 1), variant == kVarProd);
+                               : pick_list_len(K, B, C, D, p.sched.P, max_list_share(p.sched), variant == kVarProd);
     p.KL = KL;
     p.part_val = reinterpret_cast<float*>(static_cast<uint8_t*>(ws) + kWsHeaderBytes);
     p.part_idx = reinterpret_cast<int32_t*>(p.part_val + static_cast<size_t>(p.sched.P) * B * KL);
@@ -270,7 +269,6 @@ int launch_score_topk_umma(const __nv_bfloat16* X, const __nv_bfloat16* bank, co
   m.B = B;
   m.K = K;
   m.use_sched = 1;
-  m.wpq = 1;
   m.sched = p.sched;
   m.col_id = col_id;
   m.id_base = id_base;

@@ -40,25 +40,17 @@ constexpr int kSkSelectTo = 24; // a mid-stream selection leaves 20..24 entries
 constexpr int kSkThreads = 128; // epilogue threads per CTA (queue entries of one thread are kSkThreads * 8 bytes apart)
 constexpr uint32_t kSkStride = kSkThreads * 8;
 constexpr int kSkQueueBytes = (kSkQueue + 1) * kSkThreads * 8;   // + one dud slot per row (branch-free appends)
-constexpr uint32_t kKeyNegInf = 0x007FFFFFu;   // order key of -inf; smaller keys are (negative) NaN patterns
+constexpr uint32_t kKeyNegInf = 0x007FFFFFu;   // order key (topk_list.cuh) of -inf; smaller keys are (negative) NaN patterns
 
-// monotone map fp32 -> uint32 (larger float <=> larger key) and back
-__device__ __forceinline__ uint32_t okey(float v) {
-  const uint32_t b = __float_as_uint(v);
-  return b ^ (static_cast<uint32_t>(static_cast<int32_t>(b) >> 31) | 0x80000000u);
-}
-__device__ __forceinline__ float okey_inv(uint32_t k) {
-  return __uint_as_float((k & 0x80000000u) ? (k & 0x7FFFFFFFu) : ~k);
-}
 // Filter threshold for "key(x) >= k": the largest float below the value of key k (x > result).  -inf when k is not
 // above -inf.  A result of +-0 is replaced by the smallest negative float: the float compare treats -0 == +0, which
 // would otherwise drop a +0 that the key order keeps (looser is always valid).
 __device__ __forceinline__ float below_key(uint32_t k) {
   if (k <= kKeyNegInf) return -INFINITY;
-  const float f = okey_inv(k - 1);
+  const float f = order_key_value(k - 1);
   return f == 0.0f ? __uint_as_float(0x80000001u) : f;
 }
-__device__ __forceinline__ float below(float tau) { return below_key(okey(tau)); }
+__device__ __forceinline__ float below(float tau) { return below_key(order_key(tau)); }
 
 // Column classes are a function of the ABSOLUTE bank row: class(col) = (col & 31) % 10, so that the warm-up pass (which
 // sees whole chunks) and the per-entry publishing (which sees single columns) agree.  A chunk starts at a multiple of
@@ -134,7 +126,7 @@ struct FloorSlots {
     if (row == nullptr) return;
 #pragma unroll
     for (int g = 0; g < kSkGroups; ++g) {
-      const uint32_t k = okey(sk.hi[g]);
+      const uint32_t k = order_key(sk.hi[g]);
       if (k > kKeyNegInf) red_max(g, k);
     }
   }
@@ -233,7 +225,7 @@ __device__ __forceinline__ void sk_publish_new(SkQueue& q, const FloorSlots& fs,
 #pragma unroll
     for (int i = 0; i < 2; ++i)
       if (e0 + i < n && fs.row != nullptr && __uint_as_float(xb[i]) > floor)
-        fs.red_max(sk_class(static_cast<int>(col[i])), okey(__uint_as_float(xb[i])));
+        fs.red_max(sk_class(static_cast<int>(col[i])), order_key(__uint_as_float(xb[i])));
   }
   q.pub = q.wr;
 }
@@ -263,7 +255,7 @@ static __device__ __noinline__ SkState sk_select_impl(uint32_t q_base, uint32_t 
   const bool act = cnt > limit;
   uint32_t key[kSkQueue];
 #pragma unroll
-  for (int e = 0; e < kSkQueue; ++e) key[e] = okey(ptx::ld_shared_f32(q_base + e * kSkStride));
+  for (int e = 0; e < kSkQueue; ++e) key[e] = order_key(ptx::ld_shared_f32(q_base + e * kSkStride));
   uint32_t lo = 0xFFFFFFFFu, hi = 0u;
 #pragma unroll
   for (int e = 0; e < kSkQueue; ++e) {
@@ -310,7 +302,7 @@ static __device__ __noinline__ SkState sk_select_impl(uint32_t q_base, uint32_t 
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
       ptx::st_shared_v2(w, xb[i], col[i]);
-      const uint32_t k = okey(__uint_as_float(xb[i]));
+      const uint32_t k = order_key(__uint_as_float(xb[i]));
       bool keep = e0 + i < cnt;
       if (act) {
         const bool tied = k == lo;
@@ -331,7 +323,7 @@ static __device__ __noinline__ SkState sk_select_impl(uint32_t q_base, uint32_t 
     const float f = below_key(lo);
     out.in = fmaxf(out.in, f);
     out.keep = fmaxf(out.keep, f);
-    if (ties) out.in = fmaxf(out.in, okey_inv(lo));
+    if (ties) out.in = fmaxf(out.in, order_key_value(lo));
   }
   return out;
 }

@@ -11,6 +11,24 @@
 
 namespace hgr {
 
+// Order key: monotone map fp32 -> uint32 (larger float <=> larger key, -0 below +0) and back.  Lists that leave a
+// register or meet in an atomic carry it instead of the float: as the key alone (floor words), or packed into a
+// WINNER WORD key << 32 | ~item, whose unsigned order is (value desc, item asc) -- the order above.
+__device__ __forceinline__ uint32_t order_key(float v) {
+  const uint32_t b = __float_as_uint(v);
+  return b ^ (static_cast<uint32_t>(static_cast<int32_t>(b) >> 31) | 0x80000000u);
+}
+__device__ __forceinline__ float order_key_value(uint32_t k) {
+  return __uint_as_float((k & 0x80000000u) ? (k & 0x7FFFFFFFu) : ~k);
+}
+__device__ __forceinline__ unsigned long long winner_word(uint32_t key, uint32_t item) {
+  return (static_cast<unsigned long long>(key) << 32) | static_cast<uint32_t>(~item);
+}
+__device__ __forceinline__ float winner_value(unsigned long long w) {
+  return order_key_value(static_cast<uint32_t>(w >> 32));
+}
+__device__ __forceinline__ int32_t winner_item(unsigned long long w) { return static_cast<int32_t>(~static_cast<uint32_t>(w)); }
+
 template <int KL>
 struct SortedList {
   float v[KL];
@@ -24,24 +42,6 @@ struct SortedList {
     }
   }
   __device__ __forceinline__ float thr() const { return v[KL - 1]; }
-
-  // Insert into a list whose slots >= S are known to be empty (-inf): touches S slots only.  Used to seed the
-  // list from the first columns of a segment at a fraction of the cost of full-depth inserts.
-  template <int S>
-  __device__ __forceinline__ void insert_prefix(float x, int32_t id) {
-    static_assert(S >= 1 && S <= KL, "prefix length");
-#pragma unroll
-    for (int j = S - 1; j >= 1; --j) {
-      const bool above = x > v[j - 1];
-      const bool here = x > v[j];
-      v[j] = above ? v[j - 1] : (here ? x : v[j]);
-      i[j] = above ? i[j - 1] : (here ? id : i[j]);
-    }
-    if (x > v[0]) {
-      v[0] = x;
-      i[0] = id;
-    }
-  }
 
   // pre-condition: x > thr().  Fully unrolled, branch-free (predicated selects).
   __device__ __forceinline__ void insert(float x, int32_t id) {

@@ -24,15 +24,6 @@ namespace {
 
 constexpr int kMergeWarps = 4;
 
-// monotone map fp32 -> uint32 (larger float <=> larger key) and back
-__device__ __forceinline__ uint32_t f32_order_key(float v) {
-  const uint32_t b = __float_as_uint(v);
-  return (b & 0x80000000u) ? ~b : (b | 0x80000000u);
-}
-__device__ __forceinline__ float f32_from_order_key(uint32_t k) {
-  return __uint_as_float((k & 0x80000000u) ? (k & 0x7FFFFFFFu) : ~k);
-}
-
 constexpr int kDoubtWords = 10;  // bit per list, up to 320 lists per row
 
 // Exact repair of a row whose speculative lists could not all be certified.  Only the column ranges of the
@@ -49,7 +40,7 @@ struct RepairArgs {
   const void* X;
   const void* bank;
   Sched sched;
-  int KL, wpq, D8;
+  int KL, D8;
 };
 __device__ __noinline__ void repair_row(const RepairArgs a, int64_t row, int lane, int cnt, const uint32_t* dmask,
                                         SortedList<HGR_TOPK_MAX>& full) {
@@ -58,17 +49,11 @@ __device__ __noinline__ void repair_row(const RepairArgs a, int64_t row, int lan
   const int64_t pstride = a.pstride;
   const int32_t mt = static_cast<int32_t>(row / a.sched.rows);
   const int32_t w0 = a.sched.first_cta(mt);
-  const int workers = cnt / a.wpq;
-  for (int wi = 0; wi < workers; ++wi) {
-    bool doubtful = false;
-    for (int m = 0; m < a.wpq; ++m) {
-      const int p = wi * a.wpq + m;
-      doubtful |= (dmask[p >> 5] >> (p & 31)) & 1u;
-    }
-    if (doubtful) {
+  for (int p = 0; p < cnt; ++p) {   // list p of the row = worker w0 + p
+    if ((dmask[p >> 5] >> (p & 31)) & 1u) {
       // the worker's chunk of flattened units, clipped to this row tile -> bank rows [c0, c1)
       const int64_t t0 = static_cast<int64_t>(mt) * a.sched.U;
-      int64_t u0 = a.sched.unit_begin(w0 + wi) - t0, u1 = a.sched.unit_begin(w0 + wi + 1) - t0;
+      int64_t u0 = a.sched.unit_begin(w0 + p) - t0, u1 = a.sched.unit_begin(w0 + p + 1) - t0;
       u0 = u0 < 0 ? 0 : u0;
       u1 = u1 > a.sched.U ? a.sched.U : u1;
       int64_t c0 = u0 * kUnit, c1 = u1 * kUnit;
@@ -77,14 +62,11 @@ __device__ __noinline__ void repair_row(const RepairArgs a, int64_t row, int lan
         scan_row_range_lanes<HGR_TOPK_MAX>(reinterpret_cast<const uint4*>(a.X) + row * a.D8,
                                            reinterpret_cast<const uint4*>(a.bank), c0, c1, a.D8, lane, full);
     } else {
-      for (int m = 0; m < a.wpq; ++m) {
-        const int p = wi * a.wpq + m;
-        for (int k = 0; k < KL; ++k) {
-          const int64_t g = p * pstride + row * KL + k;
-          const int32_t it = a.part_idx[g];
-          const float v = a.part_val[g];
-          if (it >= 0 && v > full.thr()) full.insert(v, it);
-        }
+      for (int k = 0; k < KL; ++k) {
+        const int64_t g = p * pstride + row * KL + k;
+        const int32_t it = a.part_idx[g];
+        const float v = a.part_val[g];
+        if (it >= 0 && v > full.thr()) full.insert(v, it);
       }
     }
   }
@@ -146,7 +128,6 @@ __device__ __noinline__ Cand repair_cold(const MergeArgs* a, int64_t row, int la
     ra.bank = a->bank;
     ra.sched = a->sched;
     ra.KL = a->KL;
-    ra.wpq = a->wpq;
     ra.D8 = a->D8;
     repair_row(ra, row, lane, cnt, dmask, full);
   }
@@ -161,6 +142,38 @@ __device__ __noinline__ Cand repair_cold(const MergeArgs* a, int64_t row, int la
     }
   }
   return c;
+}
+
+// Lists of a row: P, or -- for the scoring kernel's own lists -- one per worker of the row's tile.
+__device__ __forceinline__ int row_lists(const MergeArgs& a, int64_t row) {
+  return a.use_sched ? a.sched.parts(static_cast<int32_t>(row / a.sched.rows)) : static_cast<int>(a.P);
+}
+
+// Hit@k counters of the block's rows (s_hits) into the global ones, one atomic per cut-off.  `tid` = threadIdx.x, read
+// by the kernel, where it keeps the range its launch bounds give it (read in here, it loses it: more spills).
+__device__ __forceinline__ void flush_hits(const MergeArgs& a, const int* s_hits, int tid) {
+  __syncthreads();
+  if (a.hits && tid < HGR_NUM_HITS && s_hits[tid] != 0)
+    atomicAdd(reinterpret_cast<unsigned long long*>(a.hits) + tid, static_cast<unsigned long long>(s_hits[tid]));
+}
+
+// The ksel <= 32 winners of a row, compacted into win[0, ksel) as winner words in any order: lane r < ksel gets rank r
+// (ranked by counting -- the words are distinct).
+__device__ __forceinline__ void rank_winners(unsigned long long* win, int ksel, int lane, float& my_v, int32_t& my_i) {
+  __syncwarp();
+  unsigned long long mine = 0;
+  int rank = 0;
+  if (lane < ksel) {
+    mine = win[lane];
+    for (int j = 0; j < ksel; ++j) rank += win[j] > mine;
+  }
+  __syncwarp();
+  if (lane < ksel) win[rank] = mine;
+  __syncwarp();
+  if (lane < ksel) {
+    my_v = winner_value(win[lane]);
+    my_i = winner_item(win[lane]);
+  }
 }
 
 // Tail shared by both merge kernels.  Lane r holds rank r of the merged list (my_v, my_i = bank row or -1).
@@ -246,8 +259,7 @@ topk_merge_kernel(const __grid_constant__ MergeArgs a) {
   for (int r = 0; r < kMergeWarps; ++r) {
     const int64_t row = row0 + r;
     if (row >= a.B) break;
-    int cnt = slots;
-    if (a.use_sched) cnt = a.sched.parts(static_cast<int32_t>(row / a.sched.rows)) * a.wpq;
+    const int cnt = row_lists(a, row);
     const int n = cnt * KL;
     for (int e = threadIdx.x; e < n; e += kMergeWarps * 32) {
       const int p = e / KL, k = e - p * KL;
@@ -260,8 +272,7 @@ topk_merge_kernel(const __grid_constant__ MergeArgs a) {
 
   const int64_t row = row0 + warp;
   if (row < a.B) {
-    int cnt = slots;
-    if (a.use_sched) cnt = a.sched.parts(static_cast<int32_t>(row / a.sched.rows)) * a.wpq;
+    const int cnt = row_lists(a, row);
     const float* lv = s_val + warp * slots * KL;
     const int32_t* li = s_idx + warp * slots * KL;
 
@@ -293,7 +304,7 @@ topk_merge_kernel(const __grid_constant__ MergeArgs a) {
       const int32_t lbi = bi;
       // warp arg-max with two REDUX instructions: max of an order-preserving integer image of the value, then
       // the smallest item among the lanes that hold that value
-      const uint32_t lkey = f32_order_key(lbv);
+      const uint32_t lkey = order_key(lbv);
       const uint32_t mkey = __reduce_max_sync(0xffffffffu, lkey);
       const uint32_t mitem =
           __reduce_min_sync(0xffffffffu, (lkey == mkey && lbi >= 0) ? static_cast<uint32_t>(lbi) : 0xFFFFFFFFu);
@@ -301,7 +312,7 @@ topk_merge_kernel(const __grid_constant__ MergeArgs a) {
         kth = -INFINITY;
         break;
       }
-      bv = f32_from_order_key(mkey);
+      bv = order_key_value(mkey);
       bi = static_cast<int32_t>(mitem);
       kth = bv;
       // the lowest lane holding the winner advances that list
@@ -343,10 +354,7 @@ topk_merge_kernel(const __grid_constant__ MergeArgs a) {
     }
     finish_row(a, row, lane, my_v, my_i, doubt, s_dmask[warp], cnt, s_hits, tailmax);
   }
-  __syncthreads();
-  if (a.hits && threadIdx.x < HGR_NUM_HITS && s_hits[threadIdx.x] != 0)
-    atomicAdd(reinterpret_cast<unsigned long long*>(a.hits) + threadIdx.x,
-              static_cast<unsigned long long>(s_hits[threadIdx.x]));
+  flush_hits(a, s_hits, threadIdx.x);
 }
 
 // ---- selection merge (few candidates per row) -----------------------------------------------------------------
@@ -371,8 +379,7 @@ topk_select_kernel(const __grid_constant__ MergeArgs a) {
   const int64_t row = static_cast<int64_t>(blockIdx.x) * kMergeWarps + warp;
   const int64_t pstride = a.part_stride > 0 ? a.part_stride : a.B * KL;
   if (row < a.B) {
-    int cnt = static_cast<int>(a.P);
-    if (a.use_sched) cnt = a.sched.parts(static_cast<int32_t>(row / a.sched.rows)) * a.wpq;
+    const int cnt = row_lists(a, row);
     const int N = cnt * KL;
 
     uint32_t key[NPL];   // 0 = empty slot; larger key <=> larger value
@@ -393,7 +400,7 @@ topk_select_kernel(const __grid_constant__ MergeArgs a) {
 #pragma unroll
     for (int s = 0; s < NPL; ++s) {
       const bool ok = (lane + 32 * s < N) && item[s] >= 0;
-      key[s] = ok ? f32_order_key(val[s]) : 0u;
+      key[s] = ok ? order_key(val[s]) : 0u;
       item[s] = ok ? item[s] : -1;
       tail[s] = ok && tail[s];
     }
@@ -461,32 +468,15 @@ topk_select_kernel(const __grid_constant__ MergeArgs a) {
         if (sel[s]) {
           const int pos = base + __popc(b & ((1u << lane) - 1u));
           if (pos < 32)
-            s_win[warp][pos] = (static_cast<unsigned long long>(key[s]) << 32) | static_cast<uint32_t>(~item[s]);
+            s_win[warp][pos] = winner_word(key[s], static_cast<uint32_t>(item[s]));
         }
         base += __popc(b);
       }
-      __syncwarp();
-      unsigned long long mine = 0;
-      int rank = 0;
-      if (lane < ksel) {
-        mine = s_win[warp][lane];
-        for (int j = 0; j < ksel; ++j) rank += s_win[warp][j] > mine;
-      }
-      __syncwarp();
-      if (lane < ksel) s_win[warp][rank] = mine;
-      __syncwarp();
-      if (lane < ksel) {
-        const unsigned long long w = s_win[warp][lane];
-        my_v = f32_from_order_key(static_cast<uint32_t>(w >> 32));
-        my_i = static_cast<int32_t>(~static_cast<uint32_t>(w));
-      }
+      rank_winners(s_win[warp], ksel, lane, my_v, my_i);
     }
     finish_row(a, row, lane, my_v, my_i, doubt, s_dmask[warp], cnt, s_hits, tailmax);
   }
-  __syncthreads();
-  if (a.hits && threadIdx.x < HGR_NUM_HITS && s_hits[threadIdx.x] != 0)
-    atomicAdd(reinterpret_cast<unsigned long long*>(a.hits) + threadIdx.x,
-              static_cast<unsigned long long>(s_hits[threadIdx.x]));
+  flush_hits(a, s_hits, threadIdx.x);
 }
 
 // ---- ranking merge (very few candidates per row) ------------------------------------------------------------------
@@ -514,8 +504,7 @@ topk_rank_kernel(const __grid_constant__ MergeArgs a) {
   const int64_t row = static_cast<int64_t>(blockIdx.x) * kMergeWarps + warp;
   const int64_t pstride = a.part_stride > 0 ? a.part_stride : a.B * KL;
   if (row < a.B) {
-    int cnt = static_cast<int>(a.P);
-    if (a.use_sched) cnt = a.sched.parts(static_cast<int32_t>(row / a.sched.rows)) * a.wpq;
+    const int cnt = row_lists(a, row);
     const int N = cnt * KL;
 
     unsigned long long w[NPL];   // 0 = empty slot
@@ -537,7 +526,7 @@ topk_rank_kernel(const __grid_constant__ MergeArgs a) {
 #pragma unroll
     for (int s = 0; s < NPL; ++s) {
       const bool ok = (lane + 32 * s < N) && item[s] >= 0;
-      w[s] = ok ? (static_cast<unsigned long long>(f32_order_key(val[s])) << 32) | static_cast<uint32_t>(~item[s]) : 0ull;
+      w[s] = ok ? winner_word(order_key(val[s]), static_cast<uint32_t>(item[s])) : 0ull;
       tail[s] = ok && lk[s] == KL - 1;
       if (tail[s]) tailmax = fmaxf(tailmax, val[s]);
       nvalid += ok;
@@ -573,8 +562,8 @@ topk_rank_kernel(const __grid_constant__ MergeArgs a) {
     if (ksel > 0) {
       if (lane < ksel) {
         const unsigned long long x = s_win[warp][lane];
-        my_v = f32_from_order_key(static_cast<uint32_t>(x >> 32));
-        my_i = static_cast<int32_t>(~static_cast<uint32_t>(x));
+        my_v = winner_value(x);
+        my_i = winner_item(x);
       }
       const uint32_t T = static_cast<uint32_t>(s_win[warp][ksel - 1] >> 32);   // key of the K-th winner
 #pragma unroll
@@ -587,10 +576,7 @@ topk_rank_kernel(const __grid_constant__ MergeArgs a) {
     }
     finish_row(a, row, lane, my_v, my_i, doubt, s_dmask[warp], cnt, s_hits, tailmax);
   }
-  __syncthreads();
-  if (a.hits && threadIdx.x < HGR_NUM_HITS && s_hits[threadIdx.x] != 0)
-    atomicAdd(reinterpret_cast<unsigned long long*>(a.hits) + threadIdx.x,
-              static_cast<unsigned long long>(s_hits[threadIdx.x]));
+  flush_hits(a, s_hits, threadIdx.x);
 }
 
 // ---- candidate-list merge (floor-sketch epilogue) ---------------------------------------------------------------
@@ -610,8 +596,7 @@ topk_merge_counts_kernel(const __grid_constant__ MergeArgs a) {
   const int64_t row = static_cast<int64_t>(blockIdx.x) * kMergeWarps + warp;
   uint2* cand = reinterpret_cast<uint2*>(smem_raw) + static_cast<size_t>(warp) * a.P * cap;
   if (row < a.B) {
-    int lists = static_cast<int>(a.P);
-    if (a.use_sched) lists = a.sched.parts(static_cast<int32_t>(row / a.sched.rows));
+    const int lists = row_lists(a, row);
     int N = 0;
     for (int l0 = 0; l0 < lists; l0 += 32) {
       const int l = l0 + lane;
@@ -634,7 +619,7 @@ topk_merge_counts_kernel(const __grid_constant__ MergeArgs a) {
     // keys of this lane's entries: lane, lane + 32, ...
     uint32_t kmax = 0, kmin = 0xFFFFFFFFu;
     for (int e = lane; e < N; e += 32) {
-      const uint32_t k = f32_order_key(__uint_as_float(cand[e].x));
+      const uint32_t k = order_key(__uint_as_float(cand[e].x));
       cand[e].x = k;   // keep the key: the value is recovered from it
       kmax = k > kmax ? k : kmax;
       kmin = k < kmin ? k : kmin;
@@ -678,7 +663,7 @@ topk_merge_counts_kernel(const __grid_constant__ MergeArgs a) {
         const unsigned b = __ballot_sync(0xffffffffu, sel);
         if (sel) {
           const int pos = base + __popc(b & ((1u << lane) - 1u));
-          if (pos < 32) s_win[warp][pos] = (static_cast<unsigned long long>(cand[e].x) << 32) | static_cast<uint32_t>(~cand[e].y);
+          if (pos < 32) s_win[warp][pos] = winner_word(cand[e].x, cand[e].y);
         }
         base += __popc(b);
       }
@@ -687,33 +672,16 @@ topk_merge_counts_kernel(const __grid_constant__ MergeArgs a) {
         for (int e = lane; e < N; e += 32)
           if (cand[e].x == T && (!tie_any || cand[e].y > tie_floor) && cand[e].y < best) best = cand[e].y;
         best = __reduce_min_sync(0xffffffffu, best);
-        if (lane == 0 && base < 32) s_win[warp][base] = (static_cast<unsigned long long>(T) << 32) | static_cast<uint32_t>(~best);
+        if (lane == 0 && base < 32) s_win[warp][base] = winner_word(T, best);
         ++base;
         tie_floor = best;
         tie_any = true;
       }
-      __syncwarp();
-      unsigned long long mine = 0;
-      int rank = 0;
-      if (lane < ksel) {
-        mine = s_win[warp][lane];
-        for (int j = 0; j < ksel; ++j) rank += s_win[warp][j] > mine;
-      }
-      __syncwarp();
-      if (lane < ksel) s_win[warp][rank] = mine;
-      __syncwarp();
-      if (lane < ksel) {
-        const unsigned long long w = s_win[warp][lane];
-        my_v = f32_from_order_key(static_cast<uint32_t>(w >> 32));
-        my_i = static_cast<int32_t>(~static_cast<uint32_t>(w));
-      }
+      rank_winners(s_win[warp], ksel, lane, my_v, my_i);
     }
     finish_row(a, row, lane, my_v, my_i, false, nullptr, 0, s_hits);
   }
-  __syncthreads();
-  if (a.hits && threadIdx.x < HGR_NUM_HITS && s_hits[threadIdx.x] != 0)
-    atomicAdd(reinterpret_cast<unsigned long long*>(a.hits) + threadIdx.x,
-              static_cast<unsigned long long>(s_hits[threadIdx.x]));
+  flush_hits(a, s_hits, threadIdx.x);
 }
 
 // ---- cross-GPU sequencing of the peer-memory exchange ---------------------------------------------------------
@@ -802,7 +770,7 @@ int launch_topk_merge(const MergeArgs& args, cudaStream_t stream) {
     return set_error(HGR_ERR_UNSUPPORTED, "topk merge: %lld lists per row exceed 320", (long long)args.P);
   if (args.K > HGR_TOPK_MAX || args.KL < 1)
     return set_error(HGR_ERR_UNSUPPORTED, "topk merge: K = %d / KL = %d unsupported", args.K, args.KL);
-  if (args.KL < args.K && (args.X == nullptr || args.bank == nullptr || !args.use_sched || args.wpq < 1))
+  if (args.KL < args.K && (args.X == nullptr || args.bank == nullptr || !args.use_sched))
     return set_error(HGR_ERR_BAD_ARG, "topk merge: speculative lists need X / bank / the schedule for the exact repair");
   const int blocks = static_cast<int>((args.B + kMergeWarps - 1) / kMergeWarps);
   const int64_t cand = args.P * args.KL;  // candidates per row (upper bound)

@@ -40,7 +40,6 @@ struct Params {
   int64_t ldo;
   unsigned int* stats; // [0] = rows re-scanned by the merge kernel of this call (reset here)
   unsigned long long* timeline;  // optional [CTA][24] %globaltimer stamps (HGR_TIMELINE=1), else nullptr
-  int rem_first;       // sub-tile order inside a segment: remainder first (1) or last (0)
   int stages;          // operand ring depth of the CTA-pair kernel (set by its launcher)
   // floor-sketch epilogue (sketch_epi.cuh); stats[1] = launch epoch of the workspace, stats[2] = finished CTAs
   // per-level arg-max epilogue (kEpiLevel, row f1: TOR / POR without the dense logits): the bank rows are sorted by
@@ -142,22 +141,22 @@ __device__ __forceinline__ float warmup_floor_pairs(uint32_t taddr, int nvalid) 
 // to a per-thread queue, the TMEM buffer is handed back to the MMA warp at once, and only then is the queue
 // drained into the list -- in lock-step over one dense batch per sub-tile, while the tensor core already works
 // two sub-tiles ahead.  The epilogue leaves the critical path of the MMAs entirely.
-template <int NTHR, int DEPTH>
+constexpr int kDeferQueue = 64;                   // queue entries per thread (+1 dud slot)
+constexpr uint32_t kDeferStride = 128 * 8;        // one entry of each of the CTA's 128 epilogue threads
 struct CandQueue {
-  uint32_t base;  // shared-space byte address of entry 0 of this thread; entries are NTHR * 8 bytes apart
+  uint32_t base;  // shared-space byte address of entry 0 of this thread; entries are kDeferStride bytes apart
   uint32_t wr;    // next free entry
   __device__ __forceinline__ void init(uint32_t b) { base = wr = b; }
-  __device__ __forceinline__ uint32_t limit() const { return base + DEPTH * NTHR * 8; }  // the dud slot
-  __device__ __forceinline__ int count() const { return static_cast<int>((wr - base) / (NTHR * 8)); }
+  __device__ __forceinline__ uint32_t limit() const { return base + kDeferQueue * kDeferStride; }  // the dud slot
+  __device__ __forceinline__ int count() const { return static_cast<int>((wr - base) / kDeferStride); }
 };
 
 // Branch-free append: every value is stored at the write cursor, the cursor only advances for survivors (the
 // next store overwrites a non-survivor) and saturates at the last slot, which therefore only ever holds duds.
 // (Inline-asm stores inside an `if` would be compiled as 32 divergent branches per chunk.)  The queue has
-// DEPTH + 1 entries per thread.  Returns false when some lane of the warp ran out of slots: the caller then
+// kDeferQueue + 1 entries per thread.  Returns false when some lane of the warp ran out of slots: the caller then
 // rewinds, drains and appends the same chunk again.
-template <int NTHR, int DEPTH>
-__device__ __forceinline__ bool cand_append_chunk(CandQueue<NTHR, DEPTH>& q, const uint32_t (&r)[kChunk], int nv,
+__device__ __forceinline__ bool cand_append_chunk(CandQueue& q, const uint32_t (&r)[kChunk], int nv,
                                                   int col_chunk, float thr) {
   uint32_t wr = q.wr;
   const uint32_t lim = q.limit();
@@ -165,7 +164,7 @@ __device__ __forceinline__ bool cand_append_chunk(CandQueue<NTHR, DEPTH>& q, con
   for (int j = 0; j < kChunk; ++j) {
     const bool pass = (__uint_as_float(r[j]) > thr) && (nv >= kChunk || j < nv);  // ragged tail: drop columns >= C
     ptx::st_shared_v2(wr, r[j], static_cast<uint32_t>(col_chunk + j));
-    wr += pass ? NTHR * 8 : 0;
+    wr += pass ? kDeferStride : 0;
     wr = wr < lim ? wr : lim;
   }
   q.wr = wr;
@@ -173,9 +172,9 @@ __device__ __forceinline__ bool cand_append_chunk(CandQueue<NTHR, DEPTH>& q, con
 }
 
 // Same without the per-value saturation (one op less on the cursor's dependency chain): the caller guarantees
-// room for a whole chunk (count <= DEPTH - 32 in every lane).
-template <bool FULL, int NTHR, int DEPTH>
-__device__ __forceinline__ void cand_append_chunk_roomy(CandQueue<NTHR, DEPTH>& q, const uint32_t (&r)[kChunk],
+// room for a whole chunk (count <= kDeferQueue - 32 in every lane).
+template <bool FULL>
+__device__ __forceinline__ void cand_append_chunk_roomy(CandQueue& q, const uint32_t (&r)[kChunk],
                                                         int nv, int col_chunk, float thr) {
   uint32_t wr = q.wr;
   // store-all / advance-on-pass: every value is written at the cursor and the next store overwrites a
@@ -185,24 +184,24 @@ __device__ __forceinline__ void cand_append_chunk_roomy(CandQueue<NTHR, DEPTH>& 
   for (int j = 0; j < kChunk; ++j) {
     const bool pass = (__uint_as_float(r[j]) > thr) && (FULL || j < nv);
     ptx::st_shared_v2(wr, r[j], static_cast<uint32_t>(col_chunk + j));
-    wr += pass ? NTHR * 8 : 0;
+    wr += pass ? kDeferStride : 0;
   }
   q.wr = wr;
 }
 
-template <int KL, int NTHR, int DEPTH>
-__device__ __forceinline__ void cand_drain(SortedList<KL>& list, CandQueue<NTHR, DEPTH>& q) {
+template <int KL>
+__device__ __forceinline__ void cand_drain(SortedList<KL>& list, CandQueue& q) {
   const int cnt = q.count();
   const int maxc = __reduce_max_sync(0xffffffffu, cnt);
   uint32_t rd = q.base;
   // the next entry is fetched while the current one is inserted (one warp per scheduler: nothing else would hide
-  // the shared-memory latency); reading one entry past a lane's count stays inside its DEPTH + 1 slots
+  // the shared-memory latency); reading one entry past a lane's count stays inside its kDeferQueue + 1 slots
   uint32_t xb, col;
   ptx::ld_shared_v2(rd, xb, col);
   for (int e = 0; e < maxc; ++e) {
     const float x = e < cnt ? __uint_as_float(xb) : -INFINITY;
     const int32_t c = static_cast<int32_t>(col);
-    rd += NTHR * 8;
+    rd += kDeferStride;
     ptx::ld_shared_v2(rd, xb, col);
     if (x > list.thr()) list.insert(x, c);
   }
