@@ -20,6 +20,7 @@ HGR_IMPL_TCGEN05_EXACT, HGR_IMPL_TCGEN05_NULL, HGR_IMPL_TCGEN05_SKETCH = 4, 5, 1
 HGR_IMPL_FLAG_NO_MERGE = 0x100
 HGR_NUM_HITS = 5
 HGR_TOPK_MAX = 32
+HGR_HIER_MAX_CHAIN = 32
 HIT_CUTS = (1, 2, 5, 10, 20)  # main.py:120
 
 # every symbol include/hgr_b200.h declares: name -> (restype, argtypes)
@@ -64,6 +65,9 @@ SIGNATURES = {
     "hgr_hier_metrics_fused": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int64, c_void_p, c_int, c_void_p, c_void_p,
                                        c_void_p, c_void_p, c_int, c_void_p, c_size_t, c_void_p, c_void_p, c_void_p,
                                        c_void_p]),
+    "hgr_hier_metrics_fused_rows": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int64, c_void_p, c_int, c_void_p,
+                                            c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t,
+                                            c_void_p, c_void_p, c_void_p, c_void_p]),
     "hgr_masked_ce_workspace_bytes": (c_size_t, [c_int64, c_int64, c_int64]),
     "hgr_om_backward_workspace_bytes": (c_size_t, [c_int64, c_int64, c_int64]),
     "hgr_om_backward": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int64, c_int64, c_void_p, c_void_p, c_void_p,

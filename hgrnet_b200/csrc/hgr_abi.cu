@@ -495,6 +495,37 @@ int hgr_hier_metrics_fused(const void* X, const void* bank_sorted, int64_t B, in
   return launch_hier_finish(best, B, M, n_levels, sorted_to_pos, first_out, chain, chain_level, L, lvl_idx, top1, counts, s);
 }
 
+int hgr_hier_metrics_fused_rows(const void* X, const void* bank_sorted, int64_t B, int64_t M, int64_t D,
+                                const int32_t* level_end, int n_levels, const int32_t* sorted_to_pos,
+                                const int32_t* first_out, const int32_t* targets, int64_t n_nodes,
+                                const int32_t* chain_ptr, const int32_t* chain_pos, const int32_t* chain_level,
+                                void* workspace, size_t workspace_bytes, int32_t* lvl_idx, int32_t* top1,
+                                int64_t* counts, void* stream) {
+  HGR_CHECK_ARG(B >= 0 && M > 0 && M <= (int64_t(1) << 31) - 512, "hgr_hier_metrics_fused_rows: bad sizes B=%lld M=%lld",
+                (long long)B, (long long)M);
+  HGR_CHECK_ARG(D > 0 && D % 8 == 0, "hgr_hier_metrics_fused_rows: D = %lld must be a positive multiple of 8", (long long)D);
+  HGR_CHECK_ARG(n_nodes > 0 && n_nodes < (int64_t(1) << 31) - 1, "hgr_hier_metrics_fused_rows: n_nodes = %lld",
+                (long long)n_nodes);
+  HGR_CHECK_ARG(n_levels >= 1 && n_levels <= 32, "hgr_hier_metrics_fused_rows: %d levels outside [1, 32]", n_levels);
+  if (B == 0) return HGR_OK;
+  HGR_CHECK_ARG(X && bank_sorted && level_end && sorted_to_pos && first_out && targets && chain_ptr && chain_pos &&
+                    chain_level && counts && workspace,
+                "hgr_hier_metrics_fused_rows: null pointer");
+  HGR_CHECK_ARG(aligned16(X) && aligned16(bank_sorted) && aligned16(workspace),
+                "hgr_hier_metrics_fused_rows: X / bank / workspace must be 16-byte aligned");
+  HGR_CHECK_ARG(workspace_bytes >= static_cast<size_t>(B) * n_levels * 8, "hgr_hier_metrics_fused_rows: workspace %zu < %zu bytes",
+                workspace_bytes, static_cast<size_t>(B) * n_levels * 8);
+  if (!umma_supported(B, M, D, 1))
+    return set_error(HGR_ERR_UNSUPPORTED, "hgr_hier_metrics_fused_rows: shape not supported by the tcgen05 kernel");
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  unsigned long long* best = static_cast<unsigned long long*>(workspace);
+  const int rc = launch_level_argmax_umma(static_cast<const __nv_bfloat16*>(X), static_cast<const __nv_bfloat16*>(bank_sorted), B, M,
+                                          D, level_end, n_levels, best, s);
+  if (rc != HGR_OK) return rc;
+  return launch_hier_finish_rows(best, B, M, n_levels, sorted_to_pos, first_out, targets, n_nodes, chain_ptr, chain_pos,
+                                 chain_level, lvl_idx, top1, counts, s);
+}
+
 size_t hgr_masked_ce_workspace_bytes(int64_t B, int64_t U, int64_t T) { return masked_ce_workspace_bytes(B, U, T) + 16; }
 
 int hgr_masked_ce(const float* logits, int64_t ldl, int64_t B, int64_t U, const int32_t* set_ptr, const int32_t* set_col,

@@ -14,6 +14,9 @@
 // Tie rule = first position (what an arg-max over the masked array returns on the CPU): among equal values the
 // smallest position j in `cols` wins; a masked column holds exactly -1.0f, so when no in-level value exceeds -1 the
 // first position holding -1 wins -- `first_out[l]` is the first position whose column is NOT at level l.
+//
+// The fused paths (hgr_hier_metrics_fused / _rows) apply the same rules to per-level winners taken in the GEMM
+// epilogue; the _rows variant matches every row against the chain of its own label (batches that mix classes).
 #include "common.cuh"
 #include "topk_list.cuh"
 
@@ -146,19 +149,25 @@ hier_metrics_kernel(const float* __restrict__ logits, int64_t ldl, const int32_t
   }
 }
 
-// Second half of the FUSED path (hgr_hier_metrics_fused): the per-level in-level maxima come from the GEMM epilogue
-// (score_pair.cu, kEpiLevel) as winner words (topk_list.cuh: order key << 32 | ~sorted bank row); one thread per image
-// row decodes them, maps the sorted bank row back to its position in `train_index`, and applies the same rules as the
-// kernel above: the -1 fill (first_out), first position among equal values, chain matching and counting.
-__global__ void __launch_bounds__(128)
-hier_finish_kernel(unsigned long long* __restrict__ lvl_best, int64_t B, int64_t M, int n_levels,
-                   const int32_t* __restrict__ sorted_to_pos, const int32_t* __restrict__ first_out,
-                   const int32_t* __restrict__ chain, const int32_t* __restrict__ chain_level, int L,
-                   int32_t* __restrict__ lvl_idx, int32_t* __restrict__ top1, unsigned long long* counts) {
-  // one WARP per image row, lane = level (n_levels <= 32): every load of a row is issued at once
-  const int lane = threadIdx.x & 31;
-  const int64_t row = (static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
-  if (row >= B) return;
+// Second half of the FUSED paths: the per-level in-level maxima come from the GEMM epilogue (score_pair.cu, kEpiLevel)
+// as winner words (topk_list.cuh: order key << 32 | ~sorted bank row).  `finish_row` is run by one WARP per image row,
+// lane = level (n_levels <= 32), so every load of a row is issued at once: it decodes the winners, maps the sorted bank
+// row back to its position in `train_index`, and applies the same rules as the kernel above -- the -1 fill (first_out),
+// first position among equal values, chain matching.  It returns the row's counts (warp-uniform) and hands its words of
+// the workspace back zeroed, so the next call needs no memset.  L == 0 decodes the row and counts nothing.
+// kMaxChain: the longest chain the caller passes (<= 64).  At 32 the chain is matched in ONE group of 32 whatever L is,
+// so the warp votes sit under no branch on L (a per-row L from memory would otherwise make the compiler assume
+// divergence there and spill).
+struct RowCounts {
+  unsigned long long tor, point, edge;
+};
+
+template <int kMaxChain>
+__device__ __forceinline__ RowCounts finish_row(unsigned long long* __restrict__ lvl_best, int64_t row, int lane,
+                                                int64_t M, int n_levels, const int32_t* __restrict__ sorted_to_pos,
+                                                const int32_t* __restrict__ first_out, const int32_t* __restrict__ chain,
+                                                const int32_t* __restrict__ chain_level, int L,
+                                                int32_t* __restrict__ lvl_idx, int32_t* __restrict__ top1) {
   float v = -INFINITY;          // in-level maximum of my level (before the -1 rule)
   int32_t j = 0x7FFFFFFF;       // its position in train_index
   int32_t node = 0;             // winner of my level after the -1 rule
@@ -190,26 +199,89 @@ hier_finish_kernel(unsigned long long* __restrict__ lvl_best, int64_t B, int64_t
   const int32_t t1 = bj == 0x7FFFFFFF ? -1 : bj;
   if (top1 && lane == 0) top1[row] = t1;
   // chain matching: lane k takes chain entries k, k + 32 (L <= 64); match[k] needs the winner of level chain_level[k]
-  unsigned long long tor = 0, point = 0, edge = 0;
+  RowCounts c{0, 0, 0};
   bool carry = false;           // match[k0 - 1] of the previous group of 32
-  for (int k0 = 0; k0 < L; k0 += 32) {
+  const int k_end = kMaxChain <= 32 ? 32 : L;
+  for (int k0 = 0; k0 < k_end; k0 += 32) {
     const int k = k0 + lane;
     const int32_t p = k < L ? chain[k] : -2;
     const int cl = k < L ? chain_level[k] : -1;
     const int32_t win = __shfl_sync(0xffffffffu, node, cl >= 0 && cl < 32 ? cl : 0);
     const bool m = k < L && cl >= 0 && cl < n_levels && win == p;
     const unsigned mm = __ballot_sync(0xffffffffu, m);
-    tor += __popc(__ballot_sync(0xffffffffu, k < L && t1 == p));
-    point += __popc(mm);
-    edge += __popc(mm & ((mm << 1) | (carry ? 1u : 0u)));   // match[k] and match[k - 1]
+    c.tor += __popc(__ballot_sync(0xffffffffu, k < L && t1 == p));
+    c.point += __popc(mm);
+    c.edge += __popc(mm & ((mm << 1) | (carry ? 1u : 0u)));   // match[k] and match[k - 1]
     carry = (mm >> 31) & 1u;
   }
-  if (L == 1) edge = point;
+  if (L == 1) c.edge = c.point;
+  return c;
+}
+
+// hgr_hier_metrics_fused: one chain for the whole batch, three counters.
+__global__ void __launch_bounds__(128)
+hier_finish_kernel(unsigned long long* __restrict__ lvl_best, int64_t B, int64_t M, int n_levels,
+                   const int32_t* __restrict__ sorted_to_pos, const int32_t* __restrict__ first_out,
+                   const int32_t* __restrict__ chain, const int32_t* __restrict__ chain_level, int L,
+                   int32_t* __restrict__ lvl_idx, int32_t* __restrict__ top1, unsigned long long* counts) {
+  const int lane = threadIdx.x & 31;
+  const int64_t row = (static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
+  if (row >= B) return;
+  const RowCounts c = finish_row<64>(lvl_best, row, lane, M, n_levels, sorted_to_pos, first_out, chain, chain_level, L,
+                                     lvl_idx, top1);
   if (lane == 0) {
-    if (tor) atomicAdd(counts + 0, tor);
-    if (point) atomicAdd(counts + 1, point);
-    if (edge) atomicAdd(counts + 2, edge);
+    if (c.tor) atomicAdd(counts + 0, c.tor);
+    if (c.point) atomicAdd(counts + 1, c.point);
+    if (c.edge) atomicAdd(counts + 2, c.edge);
   }
+}
+
+// hgr_hier_metrics_fused_rows: every row is matched against the chain of its own label, looked up in the chain table
+// (CSR over all nodes).  Counters are kept per chain length L ({rows, TOR hits, points, edges} in bin L), so they stay
+// integer and exact; the reference's per-batch divisions by L - 1 and L follow on the host.  A block first reduces its
+// rows into a shared histogram: in a single-label batch every row would otherwise hit the same four global words.
+constexpr int kRowsPerBlock = 8;
+constexpr int kHistWords = (HGR_HIER_MAX_CHAIN + 1) * 4;
+
+__global__ void __launch_bounds__(kRowsPerBlock * 32)
+hier_finish_rows_kernel(unsigned long long* __restrict__ lvl_best, int64_t B, int64_t M, int n_levels,
+                        const int32_t* __restrict__ sorted_to_pos, const int32_t* __restrict__ first_out,
+                        const int32_t* __restrict__ targets, int64_t n_nodes, const int32_t* __restrict__ chain_ptr,
+                        const int32_t* __restrict__ chain_pos, const int32_t* __restrict__ chain_level,
+                        int32_t* __restrict__ lvl_idx, int32_t* __restrict__ top1, unsigned long long* counts) {
+  __shared__ unsigned int s_cnt[kHistWords];      // <= kRowsPerBlock * HGR_HIER_MAX_CHAIN per word: 32 bits suffice
+  for (int i = threadIdx.x; i < kHistWords; i += blockDim.x) s_cnt[i] = 0u;
+  __syncthreads();
+  const int lane = threadIdx.x & 31;
+  const int64_t row = static_cast<int64_t>(blockIdx.x) * kRowsPerBlock + (threadIdx.x >> 5);
+  if (row < B) {                                            // warp-uniform
+    // the row's chain; a target outside [0, n_nodes) or a chain length outside [1, HGR_HIER_MAX_CHAIN] is skipped
+    // (decoded, so that lvl_idx / top1 are written and the workspace is zeroed, but counted nowhere)
+    int32_t c0 = 0;
+    int L = 0;
+    if (lane == 0) {
+      const int32_t t = targets[row];
+      if (t >= 0 && t < n_nodes) {
+        c0 = chain_ptr[t];
+        L = chain_ptr[t + 1] - c0;
+        if (L < 1 || L > HGR_HIER_MAX_CHAIN) L = 0;
+      }
+    }
+    c0 = __shfl_sync(0xffffffffu, c0, 0);
+    L = __shfl_sync(0xffffffffu, L, 0);
+    const RowCounts c = finish_row<HGR_HIER_MAX_CHAIN>(lvl_best, row, lane, M, n_levels, sorted_to_pos, first_out,
+                                                       chain_pos + c0, chain_level + c0, L, lvl_idx, top1);
+    if (lane == 0 && L > 0) {
+      unsigned int* bin = s_cnt + 4 * L;
+      atomicAdd(bin + 0, 1u);
+      if (c.tor) atomicAdd(bin + 1, static_cast<unsigned int>(c.tor));
+      if (c.point) atomicAdd(bin + 2, static_cast<unsigned int>(c.point));
+      if (c.edge) atomicAdd(bin + 3, static_cast<unsigned int>(c.edge));
+    }
+  }
+  __syncthreads();
+  for (int i = threadIdx.x; i < kHistWords; i += blockDim.x)
+    if (s_cnt[i]) atomicAdd(counts + i, static_cast<unsigned long long>(s_cnt[i]));
 }
 
 }  // namespace
@@ -222,6 +294,20 @@ int launch_hier_finish(unsigned long long* lvl_best, int64_t B, int64_t M, int n
   const int blocks = static_cast<int>((B + 3) / 4);     // one warp per image row
   hier_finish_kernel<<<blocks, 128, 0, stream>>>(lvl_best, B, M, n_levels, sorted_to_pos, first_out, chain, chain_level, L,
                                                  lvl_idx, top1, reinterpret_cast<unsigned long long*>(counts));
+  HGR_CHECK_LAUNCH();
+  return HGR_OK;
+}
+
+int launch_hier_finish_rows(unsigned long long* lvl_best, int64_t B, int64_t M, int n_levels, const int32_t* sorted_to_pos,
+                            const int32_t* first_out, const int32_t* targets, int64_t n_nodes, const int32_t* chain_ptr,
+                            const int32_t* chain_pos, const int32_t* chain_level, int32_t* lvl_idx, int32_t* top1,
+                            int64_t* counts, cudaStream_t stream) {
+  if (n_levels < 1 || n_levels > kMaxLevels)
+    return set_error(HGR_ERR_UNSUPPORTED, "hgr_hier_metrics_fused_rows: %d levels outside [1, %d]", n_levels, kMaxLevels);
+  const int blocks = static_cast<int>((B + kRowsPerBlock - 1) / kRowsPerBlock);     // one warp per image row
+  hier_finish_rows_kernel<<<blocks, kRowsPerBlock * 32, 0, stream>>>(
+      lvl_best, B, M, n_levels, sorted_to_pos, first_out, targets, n_nodes, chain_ptr, chain_pos, chain_level, lvl_idx,
+      top1, reinterpret_cast<unsigned long long*>(counts));
   HGR_CHECK_LAUNCH();
   return HGR_OK;
 }

@@ -12,8 +12,10 @@ Output format: ``count_acc`` (utils.py:135-146) and the log files of main.py:205
 from __future__ import annotations
 
 import copy
-from typing import Iterable, Optional
+import itertools
+from typing import Iterable, Optional, Sequence, Tuple
 
+import numpy as np
 import torch
 
 from . import ops
@@ -33,18 +35,59 @@ def count_acc(hits_dict, num_tot):
     return out_str, acc_dict
 
 
+def chain_table(c2p: Sequence[Sequence[int]], depth: np.ndarray, train_ids: Sequence[int]
+                ) -> Tuple[np.ndarray, np.ndarray, np.ndarray]:
+    """The chain table of ``hgr_hier_metrics_fused_rows``: a CSR over all nodes whose row n is the reference's label
+    chain ``c2p[n] + [n]`` (main.py:152).  Returns int32 ``(chain_ptr [N + 1], chain_pos, chain_level)``: per entry the
+    node's position in ``train_ids`` (the last one if it repeats, -1 if it is not a train class) and its depth."""
+    n = len(c2p)
+    lens = np.fromiter((len(c) + 1 for c in c2p), dtype=np.int64, count=n)
+    chain_ptr = np.zeros(n + 1, dtype=np.int64)
+    np.cumsum(lens, out=chain_ptr[1:])
+    nodes = np.fromiter(itertools.chain.from_iterable((*c, i) for i, c in enumerate(c2p)), dtype=np.int64,
+                        count=int(chain_ptr[-1]))
+    pos_of = np.full(n, -1, dtype=np.int64)
+    train = np.asarray(train_ids, dtype=np.int64)
+    pos_of[train] = np.arange(train.size)                # repeated ids: the last assignment stays, as in a dict
+    return (chain_ptr.astype(np.int32), pos_of[nodes].astype(np.int32),
+            np.asarray(depth, dtype=np.int64)[nodes].astype(np.int32))
+
+
+_TOTALS_DIV = {}
+
+
+def hier_totals(counts: torch.Tensor) -> torch.Tensor:
+    """Per-chain-length counters (``ops.new_hier_counts``: bin L = {rows, TOR hits, points, edges}) -> float64 ``[4]``
+    ``(rows, hits, point, path)`` on the counters' device: the sums the reference adds to ``path_all_count``,
+    ``hits_all``, ``point_all`` and ``path_all`` (main.py:158-191), with ``point = sum_L points_L / L`` and
+    ``path = sum_L edges_L / max(L - 1, 1)``.  No host synchronisation."""
+    div = _TOTALS_DIV.get(counts.device)
+    if div is None or div.shape[0] != counts.shape[0]:
+        L = torch.arange(counts.shape[0], dtype=torch.float64)
+        one = torch.ones_like(L)
+        div = torch.stack([one, one, L.clamp(min=1), (L - 1).clamp(min=1)], 1).to(counts.device)
+        _TOTALS_DIV[counts.device] = div
+    return (counts.double() / div).sum(0)
+
+
 class HierMetrics:
     """TOR / POR accumulators (main.py:123-127,152-191).  One fused pass per batch (``hgr_hier_metrics``): per-level
     arg-max over the train columns, chain matching and counting on the device; the per-batch divisions by the chain
-    length stay device-side float ops, nothing is copied to the host before the ratios are printed."""
+    length stay device-side float ops, nothing is copied to the host before the ratios are printed.
+
+    ``update`` / ``update_fused`` score a single-label batch against one label (the reference's ``targets[0]``);
+    ``update_rows`` scores every row against its own label and needs no host work per batch."""
 
     def __init__(self, model):
         self.model = model
         dev = model.device
-        self.hits_all = torch.zeros((), dtype=torch.float64, device=dev)
-        self.path_all = torch.zeros((), dtype=torch.float64, device=dev)
-        self.point_all = torch.zeros((), dtype=torch.float64, device=dev)
-        self.path_all_count = 0
+        # (rows counted by update_rows, hits, point, path) -- the order of hier_totals: update_rows folds a batch in with
+        # one add
+        self._acc = torch.zeros(4, dtype=torch.float64, device=dev)
+        self.hits_all = self._acc[1]
+        self.point_all = self._acc[2]
+        self.path_all = self._acc[3]
+        self._rows_host = 0                   # rows of update / update_fused (the batch size is known on the host)
         depth = torch.from_numpy(model.hierarchy.depth).to(torch.int64)
         self.n_levels = int(depth.max()) + 1 if depth.numel() else 1
         # Only the TRAIN columns enter TOR / POR (main.py:143,155,174): the dense logits are taken against the train
@@ -68,6 +111,36 @@ class HierMetrics:
         self._level_end = torch.cumsum(torch.bincount(dt, minlength=self.n_levels), 0).tolist()
         self._bank_sorted = None      # built on first use from model.bank_train (update_classifier must have run)
         self._bank_version = None
+        self._train_ids = train.tolist()
+        self._chains = None           # chain table of update_rows, built on first use
+        self._counts = None
+
+    @property
+    def path_all_count(self) -> int:
+        """Rows scored so far (synchronises when ``update_rows`` has run)."""
+        return self._rows_host + int(self._acc[0])
+
+    def sorted_bank(self) -> torch.Tensor:
+        """The train rows of the bank sorted by level; re-sorted when ``model.bank_train`` was refreshed (new tensor or
+        in-place update)."""
+        bank = self.model.bank_train
+        stamp = (bank.data_ptr(), bank._version)
+        if self._bank_sorted is None or self._bank_version != stamp:
+            self._bank_sorted = bank[self._sorted_to_pos.long()].contiguous()
+            self._bank_version = stamp
+        return self._bank_sorted
+
+    def rows_args(self) -> dict:
+        """Every argument of ``ops.hier_metrics_fused_rows`` except the batch (``x_norm``, ``targets``) and the
+        counters.  Device tensors; the chain table is built on the first call."""
+        if self._chains is None:
+            m = self.model
+            dev = self._first_out.device
+            self._chains = tuple(torch.from_numpy(a).to(dev)
+                                 for a in chain_table(m.c2p, m.hierarchy.depth, self._train_ids))
+        chain_ptr, chain_pos, chain_level = self._chains
+        return dict(bank_sorted=self.sorted_bank(), level_end=self._level_end, sorted_to_pos=self._sorted_to_pos,
+                    first_out=self._first_out, chain_ptr=chain_ptr, chain_pos=chain_pos, chain_level=chain_level)
 
     def update(self, logits_train: torch.Tensor, target: int):
         """``logits_train`` [B, M]: cosine logits against ``model.bank_train`` (column j = node train_index[j])."""
@@ -84,17 +157,13 @@ class HierMetrics:
         self.hits_all += c[0]                                               # main.py:158-160
         self.path_all += c[2] if L == 1 else c[2] / (L - 1)                 # main.py:179-190
         self.point_all += c[1] / L                                          # main.py:191
-        self.path_all_count += B
+        self._rows_host += B
 
     def update_fused(self, x_norm: torch.Tensor, target: int):
         """``update`` without the dense logits: ``x_norm`` [B, D] bf16 normalised image features; the per-level arg-max
         over the train classes runs in the epilogue of the GEMM against the level-sorted train bank."""
         m = self.model
-        bank = m.bank_train
-        stamp = (bank.data_ptr(), bank._version)       # a refreshed bank (new tensor or in-place update) is re-sorted
-        if self._bank_sorted is None or self._bank_version != stamp:
-            self._bank_sorted = bank[self._sorted_to_pos.long()].contiguous()
-            self._bank_version = stamp
+        bank_sorted = self.sorted_bank()
         B = x_norm.shape[0]
         parents = list(m.c2p[target]) + [target]
         L = len(parents)
@@ -102,13 +171,24 @@ class HierMetrics:
         chain = torch.tensor([self._pos_of.get(p, -1) for p in parents], dtype=torch.int32).to(dev, non_blocking=True)
         chain_level = torch.tensor([len(m.c2p[p]) for p in parents], dtype=torch.int32).to(dev, non_blocking=True)
         counts = torch.zeros(3, dtype=torch.int64, device=dev)
-        ops.hier_metrics_fused(x_norm, self._bank_sorted, self._level_end, self._sorted_to_pos, self._first_out, chain,
+        ops.hier_metrics_fused(x_norm, bank_sorted, self._level_end, self._sorted_to_pos, self._first_out, chain,
                                chain_level, counts)
         c = counts.double()
         self.hits_all += c[0]
         self.path_all += c[2] if L == 1 else c[2] / (L - 1)
         self.point_all += c[1] / L
-        self.path_all_count += B
+        self._rows_host += B
+
+    def update_rows(self, x_norm: torch.Tensor, targets: torch.Tensor):
+        """``update_fused`` with one label per row: row i is scored against the chain of node ``targets[i]``, so a
+        batch may mix classes; for a single-label batch it adds what ``update_fused`` adds.  Rows whose target lies
+        outside ``[0, n_nodes)`` are skipped (padding).  No host work per batch and no synchronisation."""
+        if self._counts is None:
+            self._counts = ops.new_hier_counts(x_norm.device)
+        else:
+            self._counts.zero_()
+        ops.hier_metrics_fused_rows(x_norm, targets=targets.to(torch.int32), counts=self._counts, **self.rows_args())
+        self._acc += hier_totals(self._counts)
 
     def ratios(self, num_sample):
         return (float(self.hits_all) / num_sample * 100.0, float(self.path_all) / self.path_all_count * 100.0,

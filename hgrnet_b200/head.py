@@ -242,11 +242,19 @@ class tree_model(nn.Module):
         return ops.score_topk(x, self.bank_test, col_id=self._test_index_i32, targets=t, K=K, hits=hits)
 
     def make_eval_stream(self, batch: int, slots: int = 4, streams: int = 2, feat_dtype=torch.float32, K: int = 20,
-                         banks=None, host_io: bool = True):
-        """CUDA-graph replayed eval step over pre-computed image features (hgrnet_b200.stream.EvalStream)."""
+                         banks=None, host_io: bool = True, hier_metrics: bool = False):
+        """CUDA-graph replayed eval step over pre-computed image features (hgrnet_b200.stream.EvalStream).
+
+        ``hier_metrics=True`` adds TOR / POR (``EvalStream.hier_ratios``), every row scored against its own label.  The
+        stream keeps the device pointers of ``bank_test`` and of the level-sorted ``bank_train`` taken now: after
+        ``update_classifier`` refreshes the banks, build a new stream."""
         from .stream import EvalStream
+        hier = None
+        if hier_metrics:
+            from .evaluate import HierMetrics
+            hier = HierMetrics(self)
         return EvalStream(self.bank_test, col_id=self._test_index_i32, batch=batch, feat_dtype=feat_dtype, K=K,
-                          slots=slots, streams=streams, banks=banks, host_io=host_io)
+                          slots=slots, streams=streams, banks=banks, host_io=host_io, hier=hier)
 
     # ------------------------------------------------------------------ training step
     def _schedule(self, training_method, target):

@@ -13,7 +13,7 @@ import torch
 from . import _cabi
 from ._cabi import (HGR_IMPL_AUTO, HGR_IMPL_SIMT, HGR_IMPL_TCGEN05,  # noqa: F401
                     HGR_IMPL_TCGEN05_EXACT, HGR_IMPL_TCGEN05_NULL, HGR_IMPL_TCGEN05_SKETCH,
-                    HGR_NUM_HITS)
+                    HGR_HIER_MAX_CHAIN, HGR_NUM_HITS)
 
 _DTYPE_CODE = {torch.float32: _cabi.HGR_F32, torch.bfloat16: _cabi.HGR_BF16, torch.float16: _cabi.HGR_F16}
 _workspaces = {}
@@ -394,6 +394,19 @@ def hier_metrics(logits: torch.Tensor, cols: Optional[torch.Tensor], level: torc
                                      _ptr(top1), _ptr(counts), _stream()))
 
 
+def _hier_workspace(nbytes: int, device) -> torch.Tensor:
+    """Per-stream scratch of the fused TOR / POR calls: zero when allocated, handed back zeroed by every call (the
+    scoring kernel's workspace on the same stream keeps header words, so this is a separate buffer)."""
+    key = ("hier", device.index, _stream())
+    ws = _workspaces.get(key)
+    if ws is None or ws.numel() < nbytes:
+        if ws is not None:
+            _retired.append(ws)
+        ws = torch.zeros(max(nbytes, 1 << 16), dtype=torch.uint8, device=device)
+        _workspaces[key] = ws
+    return ws
+
+
 def hier_metrics_fused(x_norm: torch.Tensor, bank_sorted: torch.Tensor, level_end, sorted_to_pos: torch.Tensor,
                        first_out: torch.Tensor, chain: torch.Tensor, chain_level: torch.Tensor, counts: torch.Tensor,
                        lvl_idx: Optional[torch.Tensor] = None, top1: Optional[torch.Tensor] = None) -> None:
@@ -415,17 +428,57 @@ def hier_metrics_fused(x_norm: torch.Tensor, bank_sorted: torch.Tensor, level_en
     if sorted_to_pos.numel() != M or first_out.numel() != n_levels or chain.numel() != chain_level.numel():
         raise ValueError("hier_metrics_fused: inconsistent sizes")
     ends = (ctypes.c_int32 * n_levels)(*[int(e) for e in level_end])
-    # its own scratch (zeroed by every call): the scoring kernel's workspace on this stream keeps header words
-    key = ("hier", x_norm.device.index, _stream())
-    ws = _workspaces.get(key)
-    if ws is None or ws.numel() < B * n_levels * 8:
-        if ws is not None:
-            _retired.append(ws)
-        ws = torch.zeros(max(B * n_levels * 8, 1 << 16), dtype=torch.uint8, device=x_norm.device)
-        _workspaces[key] = ws
+    ws = _hier_workspace(B * n_levels * 8, x_norm.device)
     _cabi.check(lib.hgr_hier_metrics_fused(_ptr(x_norm), _ptr(bank_sorted), B, M, D, ends, n_levels, _ptr(sorted_to_pos),
                                            _ptr(first_out), _ptr(chain), _ptr(chain_level), chain.numel(), _ptr(ws),
                                            ws.numel(), _ptr(lvl_idx), _ptr(top1), _ptr(counts), _stream()))
+
+
+def new_hier_counts(device) -> torch.Tensor:
+    """Zeroed per-chain-length counters of ``hier_metrics_fused_rows``: int64 ``[HGR_HIER_MAX_CHAIN + 1, 4]``, bin L =
+    ``{rows, TOR hits, points, edges}`` of the rows whose label chain has L entries."""
+    return torch.zeros((HGR_HIER_MAX_CHAIN + 1, 4), dtype=torch.int64, device=device)
+
+
+def hier_metrics_fused_rows(x_norm: torch.Tensor, bank_sorted: torch.Tensor, level_end, sorted_to_pos: torch.Tensor,
+                            first_out: torch.Tensor, targets: torch.Tensor, chain_ptr: torch.Tensor,
+                            chain_pos: torch.Tensor, chain_level: torch.Tensor, counts: torch.Tensor,
+                            lvl_idx: Optional[torch.Tensor] = None, top1: Optional[torch.Tensor] = None) -> None:
+    """``hier_metrics_fused`` with one label per row: row i is matched against the chain of node ``targets[i]``, read
+    from the chain table ``chain_ptr [n_nodes + 1]`` / ``chain_pos`` / ``chain_level`` (``evaluate.chain_table``).
+    ``counts`` (``new_hier_counts``) is incremented per chain length; rows whose target is outside ``[0, n_nodes)`` are
+    counted nowhere.  No host work depends on the batch's contents, so the call can be captured in a CUDA graph.  See
+    ``hgr_hier_metrics_fused_rows`` in the header."""
+    import ctypes
+    lib = _cabi.load()
+    x_norm = _require(x_norm, "x_norm", torch.bfloat16)
+    bank_sorted = _require(bank_sorted, "bank_sorted", torch.bfloat16)
+    sorted_to_pos = _require(sorted_to_pos, "sorted_to_pos", torch.int32)
+    first_out = _require(first_out, "first_out", torch.int32)
+    targets = _require(targets, "targets", torch.int32)
+    chain_ptr = _require(chain_ptr, "chain_ptr", torch.int32)
+    chain_pos = _require(chain_pos, "chain_pos", torch.int32)
+    chain_level = _require(chain_level, "chain_level", torch.int32)
+    if not counts.is_cuda:
+        raise ValueError("counts must be a CUDA tensor: hgrnet_b200 has no CPU path")
+    if counts.dtype != torch.int64 or counts.numel() != (HGR_HIER_MAX_CHAIN + 1) * 4 or not counts.is_contiguous():
+        raise ValueError("counts must be a contiguous int64 [%d, 4] tensor (new_hier_counts)" % (HGR_HIER_MAX_CHAIN + 1))
+    B, D = x_norm.shape
+    M = bank_sorted.shape[0]
+    n_levels = len(level_end)
+    n_nodes = chain_ptr.numel() - 1
+    if sorted_to_pos.numel() != M or first_out.numel() != n_levels or targets.numel() != B \
+            or chain_pos.numel() != chain_level.numel():
+        raise ValueError("hier_metrics_fused_rows: inconsistent sizes")
+    for name, t, shape in (("lvl_idx", lvl_idx, (B, n_levels)), ("top1", top1, (B,))):
+        if t is not None and (t.dtype != torch.int32 or tuple(t.shape) != shape or not t.is_contiguous() or not t.is_cuda):
+            raise ValueError("%s must be a contiguous CUDA int32 %s tensor" % (name, list(shape)))
+    ends = (ctypes.c_int32 * n_levels)(*[int(e) for e in level_end])
+    ws = _hier_workspace(B * n_levels * 8, x_norm.device)
+    _cabi.check(lib.hgr_hier_metrics_fused_rows(_ptr(x_norm), _ptr(bank_sorted), B, M, D, ends, n_levels,
+                                                _ptr(sorted_to_pos), _ptr(first_out), _ptr(targets), n_nodes,
+                                                _ptr(chain_ptr), _ptr(chain_pos), _ptr(chain_level), _ptr(ws), ws.numel(),
+                                                _ptr(lvl_idx), _ptr(top1), _ptr(counts), _stream()))
 
 
 def masked_ce(logits: torch.Tensor, set_ptr: torch.Tensor, set_col: torch.Tensor, label_pos: torch.Tensor,

@@ -16,6 +16,13 @@ are independent), so the copy of batch i+1 and the small kernels of neighbouring
 the GEMM of batch i and CTAs of the next GEMM start as soon as SMs drain.  Results (top-K values /
 node ids) stay in the slot's device buffers; the Hit@{1,2,5,10,20} counters accumulate on the
 device (atomics commute) and are mirrored to pinned host memory every step.
+
+With ``hier`` (an ``evaluate.HierMetrics``) each graph also runs the hierarchical metrics TOR / POR
+(main.py:143,152-191) on the slot's per-row labels after the scoring call
+(``ops.hier_metrics_fused_rows``: per-level arg-max in the epilogue of a GEMM against the level-sorted train bank, then
+per-row chain matching).  Its per-chain-length counters share one device buffer with the hit counters, so a step still
+makes one D2H copy.  The level-sorted train bank, like ``bank``, is taken when the stream is built: after a bank
+refresh, build a new stream.
 """
 from __future__ import annotations
 
@@ -24,15 +31,18 @@ from typing import Optional
 import torch
 
 from . import ops
+from ._cabi import HGR_HIER_MAX_CHAIN
 
 
 class EvalStream:
     def __init__(self, bank: torch.Tensor, col_id: Optional[torch.Tensor] = None, id_base: int = 0, *, batch: int,
                  feat_dtype=torch.float32, K: int = 20, slots: int = 4, streams: int = 2, banks=None,
-                 host_io: bool = True):
+                 host_io: bool = True, hier=None):
         """``bank`` [C, D] bf16 on the device.  ``banks``: optional list of bank tensors to rotate over per slot
         (benchmarks use it to keep the working set larger than L2).  ``host_io=False`` skips the H2D / D2H nodes
-        (features are then written straight into ``dev_feats`` / ``dev_labels``)."""
+        (features are then written straight into ``dev_feats`` / ``dev_labels``).  ``hier``: optional
+        ``evaluate.HierMetrics`` of the model; when given, every step also counts TOR / POR (``hier_ratios``).  Labels
+        are node ids; a label outside the hierarchy (e.g. -1 padding) is counted by neither metric."""
         self.device = bank.device
         self.K = K
         self.B = batch
@@ -51,11 +61,18 @@ class EvalStream:
 
         self.dev_pack = [torch.zeros(nbytes, dtype=torch.uint8, device=self.device) for _ in range(slots)]
         self.dev_feats, self.dev_labels = map(list, zip(*[views(p) for p in self.dev_pack]))
+        # hit counters, then (with hier) the per-chain-length TOR / POR counters: one buffer, one D2H copy per step
+        self.hier = hier
+        self._hier_args = hier.rows_args() if hier is not None else None
+        n_counters = ops.HGR_NUM_HITS + (0 if hier is None else (HGR_HIER_MAX_CHAIN + 1) * 4)
         if host_io:
             self.host_pack = [torch.zeros(nbytes, dtype=torch.uint8).pin_memory() for _ in range(slots)]
             self.host_feats, self.host_labels = map(list, zip(*[views(p) for p in self.host_pack]))
-            self.host_hits = torch.zeros(ops.HGR_NUM_HITS, dtype=torch.int64).pin_memory()
-        self.hits = ops.new_hits(self.device)
+            self.host_counters = torch.zeros(n_counters, dtype=torch.int64).pin_memory()
+            self.host_hits = self.host_counters[:ops.HGR_NUM_HITS]
+        self.counters = torch.zeros(n_counters, dtype=torch.int64, device=self.device)
+        self.hits = self.counters[:ops.HGR_NUM_HITS]
+        self.hier_counts = self.counters[ops.HGR_NUM_HITS:].view(HGR_HIER_MAX_CHAIN + 1, 4) if hier is not None else None
         self.val = [None] * slots
         self.idx = [None] * slots
         self.streams = [torch.cuda.Stream(device=self.device) for _ in range(max(1, min(streams, slots)))]
@@ -73,8 +90,10 @@ class EvalStream:
         self.val[s], self.idx[s] = ops.score_topk(x, self.banks[s % len(self.banks)], col_id=self.col_id,
                                                   id_base=self.id_base, targets=self.dev_labels[s], K=self.K,
                                                   hits=self.hits)                    # clip_tree.py:331 + main.py:136-147
+        if self._hier_args is not None:                                              # main.py:143,152-191
+            ops.hier_metrics_fused_rows(x, targets=self.dev_labels[s], counts=self.hier_counts, **self._hier_args)
         if self.host_io:
-            self.host_hits.copy_(self.hits, non_blocking=True)
+            self.host_counters.copy_(self.counters, non_blocking=True)
 
     def _capture(self):
         cur = torch.cuda.current_stream(self.device)
@@ -86,7 +105,7 @@ class EvalStream:
                 self._body(s)                             # warm-up: workspace allocation, lazy module loading
         for st in self.streams:
             st.synchronize()
-        self.hits.zero_()
+        self.counters.zero_()
         torch.cuda.synchronize(self.device)
         for s in range(self.slots):
             st = self._stream_of(s)
@@ -126,3 +145,15 @@ class EvalStream:
         # (the per-step D2H copies of several streams land in the same 40 bytes in no particular order: read the
         # counters once more now that every stream is idle)
         return self.hits.tolist()
+
+    def hier_ratios(self):
+        """``(hit_ratio, path_ratio, point_ratio)`` in percent -- the TOR / POR of the reference's ``test()`` line -- over
+        the rows scored so far whose label lies in the hierarchy (synchronises).  Needs ``hier``."""
+        if self.hier is None:
+            raise RuntimeError("EvalStream was built without hier metrics (pass hier=HierMetrics(model))")
+        from .evaluate import hier_totals
+        self.synchronize()
+        rows, hits, point, path = hier_totals(self.hier_counts).tolist()
+        if rows == 0:
+            return 0.0, 0.0, 0.0
+        return hits / rows * 100.0, path / rows * 100.0, point / rows * 100.0

@@ -302,6 +302,31 @@ int hgr_hier_metrics_fused(const void* X, const void* bank_sorted, int64_t B, in
                            void* stream);
 
 /*
+ * hgr_hier_metrics_fused for batches that mix labels: every row is matched against the chain of ITS OWN label.  For a
+ * single-label batch this is exactly the reference's metric, whose per-batch edge / (L-1) and point / L are sums of
+ * per-row terms.  Needs no host work per batch and no memset, so it can be captured in a CUDA graph.
+ *
+ *  X, bank_sorted, B, M, D, level_end, n_levels, sorted_to_pos, first_out, workspace, lvl_idx, top1:
+ *               as hgr_hier_metrics_fused (lvl_idx / top1 do not depend on the labels; both optional)
+ *  targets      [B] int32 node id of each row's label
+ *  chain table  CSR over all n_nodes nodes, built once per model: the chain of node n is c2p[n] + [n], entries
+ *               [chain_ptr[n], chain_ptr[n+1]); per entry chain_pos = its position in train_index (-1: not a train
+ *               class) and chain_level = its depth.  chain_ptr [n_nodes + 1] int32, chain_pos / chain_level int32.
+ *  counts       [HGR_HIER_MAX_CHAIN + 1][4] int64, INCREMENTED: bin L (chain length) holds {rows, TOR hits, points,
+ *               edges} of the rows whose chain has L entries (bin 0 stays zero).  The reference's totals follow on the
+ *               host: hits = sum_L tor_L, path = sum_L edges_L / max(L-1, 1), point = sum_L points_L / L.
+ * A row whose target lies outside [0, n_nodes), or whose chain length lies outside [1, HGR_HIER_MAX_CHAIN], is counted
+ * nowhere (its lvl_idx / top1 are still written): callers pad a fixed-shape batch with target -1.
+ */
+#define HGR_HIER_MAX_CHAIN 32 /* = the 32-level limit of the per-level arg-max epilogue */
+int hgr_hier_metrics_fused_rows(const void* X, const void* bank_sorted, int64_t B, int64_t M, int64_t D,
+                                const int32_t* level_end, int n_levels, const int32_t* sorted_to_pos,
+                                const int32_t* first_out, const int32_t* targets, int64_t n_nodes,
+                                const int32_t* chain_ptr, const int32_t* chain_pos, const int32_t* chain_level,
+                                void* workspace, size_t workspace_bytes, int32_t* lvl_idx, int32_t* top1,
+                                int64_t* counts, void* stream);
+
+/*
  * Fused masked cross-entropy of the OM training step over T sampled class sets
  * (model/clip_tree.py:241-277 with nn.CrossEntropyLoss, :49,:275).
  *
