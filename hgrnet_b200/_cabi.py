@@ -68,7 +68,12 @@ SIGNATURES = {
     "hgr_hier_metrics_fused_rows": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int64, c_void_p, c_int, c_void_p,
                                             c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t,
                                             c_void_p, c_void_p, c_void_p, c_void_p]),
-    "hgr_masked_ce_workspace_bytes": (c_size_t, [c_int64, c_int64, c_int64]),
+    "hgr_hier_level_scatter": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int64, c_void_p, c_int, c_int64, c_void_p,
+                                       c_size_t, c_int64, c_int, c_void_p, c_void_p]),
+    "hgr_hier_finish_rows_gathered": (c_int, [c_void_p, c_int, c_int64, c_int64, c_int64, c_int, c_void_p, c_void_p,
+                                              c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                              c_void_p]),
+    "hgr_masked_ce_workspace_bytes":(c_size_t, [c_int64, c_int64, c_int64]),
     "hgr_om_backward_workspace_bytes": (c_size_t, [c_int64, c_int64, c_int64]),
     "hgr_om_backward": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int64, c_int64, c_void_p, c_void_p, c_void_p,
                                 c_void_p, c_float, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),

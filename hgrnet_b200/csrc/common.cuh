@@ -147,6 +147,14 @@ int launch_hier_finish_rows(unsigned long long* lvl_best, int64_t B, int64_t M, 
                             const int32_t* first_out, const int32_t* targets, int64_t n_nodes, const int32_t* chain_ptr,
                             const int32_t* chain_pos, const int32_t* chain_level, int32_t* lvl_idx, int32_t* top1,
                             int64_t* counts, cudaStream_t stream);
+// class-sharded TOR / POR (hgr_hier_level_scatter / hgr_hier_finish_rows_gathered)
+int launch_hier_push(unsigned long long* lvl_best, int64_t B, int n_levels, int64_t row_base, int64_t block_rows,
+                     int n_blocks, unsigned long long* const* dst, cudaStream_t stream);
+int launch_hier_finish_gathered(const unsigned long long* parts, int n_parts, int64_t part_stride, int64_t B, int64_t M,
+                                int n_levels, const int32_t* sorted_to_pos, const int32_t* first_out,
+                                const int32_t* targets, int64_t n_nodes, const int32_t* chain_ptr,
+                                const int32_t* chain_pos, const int32_t* chain_level, int32_t* lvl_idx, int32_t* top1,
+                                int64_t* counts, cudaStream_t stream);
 int launch_hier_metrics(const float* logits, int64_t ldl, int64_t B, const int32_t* cols, int64_t M,
                         const int8_t* level, int n_levels, const int32_t* first_out, const int32_t* chain,
                         const int32_t* chain_level, int L, int32_t* lvl_idx, int32_t* top1, int64_t* counts,

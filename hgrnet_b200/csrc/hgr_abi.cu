@@ -526,6 +526,65 @@ int hgr_hier_metrics_fused_rows(const void* X, const void* bank_sorted, int64_t 
                                  chain_level, lvl_idx, top1, counts, s);
 }
 
+int hgr_hier_level_scatter(const void* X, const void* bank_shard, int64_t B, int64_t M_r, int64_t D,
+                           const int32_t* level_end_local, int n_levels, int64_t row_base, void* workspace,
+                           size_t workspace_bytes, int64_t block_rows, int n_blocks, uint64_t* const* dst_blocks,
+                           void* stream) {
+  HGR_CHECK_ARG(B >= 0 && M_r >= 0 && M_r < (int64_t(1) << 31) - 512, "hgr_hier_level_scatter: bad sizes B=%lld M_r=%lld",
+                (long long)B, (long long)M_r);
+  HGR_CHECK_ARG(D > 0 && D % 8 == 0, "hgr_hier_level_scatter: D = %lld must be a positive multiple of 8", (long long)D);
+  HGR_CHECK_ARG(n_levels >= 1 && n_levels <= 32, "hgr_hier_level_scatter: %d levels outside [1, 32]", n_levels);
+  HGR_CHECK_ARG(row_base >= 0 && row_base + M_r < (int64_t(1) << 31) - 512,
+                "hgr_hier_level_scatter: row_base = %lld puts the shard outside the global sorted bank", (long long)row_base);
+  HGR_CHECK_ARG(n_blocks >= 1 && n_blocks <= kMaxScatterBlocks, "hgr_hier_level_scatter: n_blocks = %d outside [1, %d]",
+                n_blocks, kMaxScatterBlocks);
+  HGR_CHECK_ARG(block_rows >= 1 && block_rows * n_blocks >= B, "hgr_hier_level_scatter: %d blocks of %lld rows do not cover B = %lld",
+                n_blocks, (long long)block_rows, (long long)B);
+  if (B == 0) return HGR_OK;
+  HGR_CHECK_ARG(dst_blocks && workspace && (M_r == 0 || (X && bank_shard && level_end_local)),
+                "hgr_hier_level_scatter: null pointer");
+  for (int g = 0; g < n_blocks; ++g)
+    HGR_CHECK_ARG(dst_blocks[g] && (reinterpret_cast<uintptr_t>(dst_blocks[g]) & 7u) == 0,
+                  "hgr_hier_level_scatter: destination %d null or not 8-byte aligned", g);
+  HGR_CHECK_ARG(aligned16(workspace) && (M_r == 0 || (aligned16(X) && aligned16(bank_shard))),
+                "hgr_hier_level_scatter: X / bank / workspace must be 16-byte aligned");
+  HGR_CHECK_ARG(workspace_bytes >= static_cast<size_t>(B) * n_levels * 8, "hgr_hier_level_scatter: workspace %zu < %zu bytes",
+                workspace_bytes, static_cast<size_t>(B) * n_levels * 8);
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  unsigned long long* best = static_cast<unsigned long long*>(workspace);
+  if (M_r > 0) {          // an empty shard has no GEMM: its workspace is still all zero and the push stores zeros
+    if (!umma_supported(B, M_r, D, 1))
+      return set_error(HGR_ERR_UNSUPPORTED, "hgr_hier_level_scatter: shape not supported by the tcgen05 kernel");
+    const int rc = launch_level_argmax_umma(static_cast<const __nv_bfloat16*>(X), static_cast<const __nv_bfloat16*>(bank_shard),
+                                            B, M_r, D, level_end_local, n_levels, best, s);
+    if (rc != HGR_OK) return rc;
+  }
+  return launch_hier_push(best, B, n_levels, row_base, block_rows, n_blocks,
+                          reinterpret_cast<unsigned long long* const*>(dst_blocks), s);
+}
+
+int hgr_hier_finish_rows_gathered(const uint64_t* parts, int n_parts, int64_t part_stride, int64_t n_rows, int64_t M,
+                                  int n_levels, const int32_t* sorted_to_pos, const int32_t* first_out,
+                                  const int32_t* targets, int64_t n_nodes, const int32_t* chain_ptr,
+                                  const int32_t* chain_pos, const int32_t* chain_level, int32_t* lvl_idx, int32_t* top1,
+                                  int64_t* counts, void* stream) {
+  HGR_CHECK_ARG(n_rows >= 0 && M > 0 && M <= (int64_t(1) << 31) - 512, "hgr_hier_finish_rows_gathered: bad sizes n_rows=%lld M=%lld",
+                (long long)n_rows, (long long)M);
+  HGR_CHECK_ARG(n_nodes > 0 && n_nodes < (int64_t(1) << 31) - 1, "hgr_hier_finish_rows_gathered: n_nodes = %lld",
+                (long long)n_nodes);
+  HGR_CHECK_ARG(n_levels >= 1 && n_levels <= 32, "hgr_hier_finish_rows_gathered: %d levels outside [1, 32]", n_levels);
+  HGR_CHECK_ARG(n_parts >= 1 && n_parts <= kMaxScatterBlocks, "hgr_hier_finish_rows_gathered: n_parts = %d outside [1, %d]",
+                n_parts, kMaxScatterBlocks);
+  HGR_CHECK_ARG(part_stride >= n_rows * n_levels, "hgr_hier_finish_rows_gathered: part_stride < n_rows * n_levels");
+  if (n_rows == 0) return HGR_OK;
+  HGR_CHECK_ARG(parts && sorted_to_pos && first_out && targets && chain_ptr && chain_pos && chain_level && counts,
+                "hgr_hier_finish_rows_gathered: null pointer");
+  HGR_CHECK_ARG((reinterpret_cast<uintptr_t>(parts) & 7u) == 0, "hgr_hier_finish_rows_gathered: parts must be 8-byte aligned");
+  return launch_hier_finish_gathered(reinterpret_cast<const unsigned long long*>(parts), n_parts, part_stride, n_rows, M,
+                                     n_levels, sorted_to_pos, first_out, targets, n_nodes, chain_ptr, chain_pos, chain_level,
+                                     lvl_idx, top1, counts, static_cast<cudaStream_t>(stream));
+}
+
 size_t hgr_masked_ce_workspace_bytes(int64_t B, int64_t U, int64_t T) { return masked_ce_workspace_bytes(B, U, T) + 16; }
 
 int hgr_masked_ce(const float* logits, int64_t ldl, int64_t B, int64_t U, const int32_t* set_ptr, const int32_t* set_col,

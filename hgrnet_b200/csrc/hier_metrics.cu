@@ -153,8 +153,10 @@ hier_metrics_kernel(const float* __restrict__ logits, int64_t ldl, const int32_t
 // as winner words (topk_list.cuh: order key << 32 | ~sorted bank row).  `finish_row` is run by one WARP per image row,
 // lane = level (n_levels <= 32), so every load of a row is issued at once: it decodes the winners, maps the sorted bank
 // row back to its position in `train_index`, and applies the same rules as the kernel above -- the -1 fill (first_out),
-// first position among equal values, chain matching.  It returns the row's counts (warp-uniform) and hands its words of
-// the workspace back zeroed, so the next call needs no memset.  L == 0 decodes the row and counts nothing.
+// first position among equal values, chain matching.  It returns the row's counts (warp-uniform).  L == 0 decodes the
+// row and counts nothing.  `words(row, lane, n_levels)` gives the winner word of level lane (0: no column of that
+// level): `WsWords` reads the fused call's own workspace and hands it back zeroed; `GatheredWords` takes the max over
+// the class shards' words in a peer-exchange slot.
 // kMaxChain: the longest chain the caller passes (<= 64).  At 32 the chain is matched in ONE group of 32 whatever L is,
 // so the warp votes sit under no branch on L (a per-row L from memory would otherwise make the compiler assume
 // divergence there and spill).
@@ -162,9 +164,19 @@ struct RowCounts {
   unsigned long long tor, point, edge;
 };
 
-template <int kMaxChain>
-__device__ __forceinline__ RowCounts finish_row(unsigned long long* __restrict__ lvl_best, int64_t row, int lane,
-                                                int64_t M, int n_levels, const int32_t* __restrict__ sorted_to_pos,
+// The fused calls' own workspace: read the word and hand it back zeroed, so the next call needs no memset.
+struct WsWords {
+  unsigned long long* __restrict__ lvl_best;
+  __device__ __forceinline__ unsigned long long operator()(int64_t row, int lane, int n_levels) const {
+    const unsigned long long w = lvl_best[row * n_levels + lane];
+    lvl_best[row * n_levels + lane] = 0ull;
+    return w;
+  }
+};
+
+template <int kMaxChain, class Words>
+__device__ __forceinline__ RowCounts finish_row(const Words& words, int64_t row, int lane, int64_t M, int n_levels,
+                                                const int32_t* __restrict__ sorted_to_pos,
                                                 const int32_t* __restrict__ first_out, const int32_t* __restrict__ chain,
                                                 const int32_t* __restrict__ chain_level, int L,
                                                 int32_t* __restrict__ lvl_idx, int32_t* __restrict__ top1) {
@@ -172,8 +184,7 @@ __device__ __forceinline__ RowCounts finish_row(unsigned long long* __restrict__
   int32_t j = 0x7FFFFFFF;       // its position in train_index
   int32_t node = 0;             // winner of my level after the -1 rule
   if (lane < n_levels) {
-    const unsigned long long w = lvl_best[row * n_levels + lane];
-    lvl_best[row * n_levels + lane] = 0ull;     // the workspace is handed back zeroed: the next call needs no memset
+    const unsigned long long w = words(row, lane, n_levels);
     const int32_t fo = first_out[lane];
     if (w != 0ull) {
       v = winner_value(w);
@@ -227,8 +238,8 @@ hier_finish_kernel(unsigned long long* __restrict__ lvl_best, int64_t B, int64_t
   const int lane = threadIdx.x & 31;
   const int64_t row = (static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
   if (row >= B) return;
-  const RowCounts c = finish_row<64>(lvl_best, row, lane, M, n_levels, sorted_to_pos, first_out, chain, chain_level, L,
-                                     lvl_idx, top1);
+  const RowCounts c = finish_row<64>(WsWords{lvl_best}, row, lane, M, n_levels, sorted_to_pos,
+                                     first_out, chain, chain_level, L, lvl_idx, top1);
   if (lane == 0) {
     if (c.tor) atomicAdd(counts + 0, c.tor);
     if (c.point) atomicAdd(counts + 1, c.point);
@@ -243,12 +254,15 @@ hier_finish_kernel(unsigned long long* __restrict__ lvl_best, int64_t B, int64_t
 constexpr int kRowsPerBlock = 8;
 constexpr int kHistWords = (HGR_HIER_MAX_CHAIN + 1) * 4;
 
-__global__ void __launch_bounds__(kRowsPerBlock * 32)
-hier_finish_rows_kernel(unsigned long long* __restrict__ lvl_best, int64_t B, int64_t M, int n_levels,
-                        const int32_t* __restrict__ sorted_to_pos, const int32_t* __restrict__ first_out,
-                        const int32_t* __restrict__ targets, int64_t n_nodes, const int32_t* __restrict__ chain_ptr,
-                        const int32_t* __restrict__ chain_pos, const int32_t* __restrict__ chain_level,
-                        int32_t* __restrict__ lvl_idx, int32_t* __restrict__ top1, unsigned long long* counts) {
+template <class Words>
+__device__ __forceinline__ void finish_rows_block(const Words& words, int64_t B, int64_t M, int n_levels,
+                                                  const int32_t* __restrict__ sorted_to_pos,
+                                                  const int32_t* __restrict__ first_out,
+                                                  const int32_t* __restrict__ targets, int64_t n_nodes,
+                                                  const int32_t* __restrict__ chain_ptr,
+                                                  const int32_t* __restrict__ chain_pos,
+                                                  const int32_t* __restrict__ chain_level, int32_t* __restrict__ lvl_idx,
+                                                  int32_t* __restrict__ top1, unsigned long long* counts) {
   __shared__ unsigned int s_cnt[kHistWords];      // <= kRowsPerBlock * HGR_HIER_MAX_CHAIN per word: 32 bits suffice
   for (int i = threadIdx.x; i < kHistWords; i += blockDim.x) s_cnt[i] = 0u;
   __syncthreads();
@@ -269,8 +283,8 @@ hier_finish_rows_kernel(unsigned long long* __restrict__ lvl_best, int64_t B, in
     }
     c0 = __shfl_sync(0xffffffffu, c0, 0);
     L = __shfl_sync(0xffffffffu, L, 0);
-    const RowCounts c = finish_row<HGR_HIER_MAX_CHAIN>(lvl_best, row, lane, M, n_levels, sorted_to_pos, first_out,
-                                                       chain_pos + c0, chain_level + c0, L, lvl_idx, top1);
+    const RowCounts c = finish_row<HGR_HIER_MAX_CHAIN>(words, row, lane, M, n_levels, sorted_to_pos,
+                                                       first_out, chain_pos + c0, chain_level + c0, L, lvl_idx, top1);
     if (lane == 0 && L > 0) {
       unsigned int* bin = s_cnt + 4 * L;
       atomicAdd(bin + 0, 1u);
@@ -284,7 +298,97 @@ hier_finish_rows_kernel(unsigned long long* __restrict__ lvl_best, int64_t B, in
     if (s_cnt[i]) atomicAdd(counts + i, static_cast<unsigned long long>(s_cnt[i]));
 }
 
+__global__ void __launch_bounds__(kRowsPerBlock * 32)
+hier_finish_rows_kernel(unsigned long long* __restrict__ lvl_best, int64_t B, int64_t M, int n_levels,
+                        const int32_t* __restrict__ sorted_to_pos, const int32_t* __restrict__ first_out,
+                        const int32_t* __restrict__ targets, int64_t n_nodes, const int32_t* __restrict__ chain_ptr,
+                        const int32_t* __restrict__ chain_pos, const int32_t* __restrict__ chain_level,
+                        int32_t* __restrict__ lvl_idx, int32_t* __restrict__ top1, unsigned long long* counts) {
+  finish_rows_block(WsWords{lvl_best}, B, M, n_levels, sorted_to_pos, first_out, targets, n_nodes, chain_ptr, chain_pos,
+                    chain_level, lvl_idx, top1, counts);
+}
+
+// ---- class-sharded form (hgr_hier_level_scatter / hgr_hier_finish_rows_gathered) -------------------------------------
+// Every class shard runs the level GEMM on its contiguous slice [row_base, row_base + M_r) of the level-sorted train
+// bank; hier_push_kernel rebases each winner word to the GLOBAL sorted row and stores it into region `rank` of the row
+// owner's exchange slot ([n_parts][block_rows][n_levels] words).  The owner takes the max over its n_parts words per
+// (row, level): that is the word the single-GPU epilogue's atomicMax would have left, because the word's order is
+// (value desc, global sorted row asc), the level-sorted bank keeps train_index order inside a level, and max is
+// associative.  The gathered words then go through the same finish_row.
+
+// Max over the shards' words of a row; the exchange slot is read only (producers overwrite all of it every batch).
+struct GatheredWords {
+  const unsigned long long* __restrict__ parts;
+  int n_parts;
+  int64_t part_stride;
+  __device__ __forceinline__ unsigned long long operator()(int64_t row, int lane, int n_levels) const {
+    unsigned long long w = 0ull;
+    for (int p = 0; p < n_parts; ++p) {
+      const unsigned long long o = parts[p * part_stride + row * n_levels + lane];
+      w = o > w ? o : w;
+    }
+    return w;
+  }
+};
+
+__global__ void __launch_bounds__(kRowsPerBlock * 32)
+hier_finish_gathered_kernel(const unsigned long long* __restrict__ parts, int n_parts, int64_t part_stride, int64_t B,
+                            int64_t M, int n_levels, const int32_t* __restrict__ sorted_to_pos,
+                            const int32_t* __restrict__ first_out, const int32_t* __restrict__ targets, int64_t n_nodes,
+                            const int32_t* __restrict__ chain_ptr, const int32_t* __restrict__ chain_pos,
+                            const int32_t* __restrict__ chain_level, int32_t* __restrict__ lvl_idx,
+                            int32_t* __restrict__ top1, unsigned long long* counts) {
+  finish_rows_block(GatheredWords{parts, n_parts, part_stride}, B, M, n_levels, sorted_to_pos, first_out, targets,
+                    n_nodes, chain_ptr, chain_pos, chain_level, lvl_idx, top1, counts);
+}
+
+struct HierDst {
+  unsigned long long* p[kMaxScatterBlocks];
+};
+
+// One thread per (row, level) word of the shard's workspace: read it, hand it back zeroed, move its item from the
+// shard's sorted row to the global one (0 = no column of that level here: stays 0) and store it -- zeros included, so
+// a slot never holds anything of an earlier batch -- at its row owner.  Plain stores, local or peer memory; the
+// hgr_peer_signal that follows in stream order publishes them.
+constexpr int kPushThreads = 256;
+__global__ void __launch_bounds__(kPushThreads)
+hier_push_kernel(unsigned long long* __restrict__ lvl_best, int64_t n_words, int n_levels, int64_t block_rows,
+                 uint32_t row_base, const __grid_constant__ HierDst dst) {
+  const int64_t i = static_cast<int64_t>(blockIdx.x) * kPushThreads + threadIdx.x;
+  if (i >= n_words) return;
+  unsigned long long w = lvl_best[i];
+  lvl_best[i] = 0ull;
+  if (w != 0ull) w = winner_word(static_cast<uint32_t>(w >> 32), static_cast<uint32_t>(winner_item(w)) + row_base);
+  const int64_t row = i / n_levels;
+  const int g = static_cast<int>(row / block_rows);
+  dst.p[g][i - g * block_rows * n_levels] = w;
+}
+
 }  // namespace
+
+int launch_hier_push(unsigned long long* lvl_best, int64_t B, int n_levels, int64_t row_base, int64_t block_rows,
+                     int n_blocks, unsigned long long* const* dst, cudaStream_t stream) {
+  HierDst d{};
+  for (int g = 0; g < n_blocks; ++g) d.p[g] = dst[g];
+  const int64_t n_words = B * n_levels;
+  hier_push_kernel<<<static_cast<unsigned>((n_words + kPushThreads - 1) / kPushThreads), kPushThreads, 0, stream>>>(
+      lvl_best, n_words, n_levels, block_rows, static_cast<uint32_t>(row_base), d);
+  HGR_CHECK_LAUNCH();
+  return HGR_OK;
+}
+
+int launch_hier_finish_gathered(const unsigned long long* parts, int n_parts, int64_t part_stride, int64_t B, int64_t M,
+                                int n_levels, const int32_t* sorted_to_pos, const int32_t* first_out,
+                                const int32_t* targets, int64_t n_nodes, const int32_t* chain_ptr,
+                                const int32_t* chain_pos, const int32_t* chain_level, int32_t* lvl_idx, int32_t* top1,
+                                int64_t* counts, cudaStream_t stream) {
+  const int blocks = static_cast<int>((B + kRowsPerBlock - 1) / kRowsPerBlock);     // one warp per image row
+  hier_finish_gathered_kernel<<<blocks, kRowsPerBlock * 32, 0, stream>>>(
+      parts, n_parts, part_stride, B, M, n_levels, sorted_to_pos, first_out, targets, n_nodes, chain_ptr, chain_pos,
+      chain_level, lvl_idx, top1, reinterpret_cast<unsigned long long*>(counts));
+  HGR_CHECK_LAUNCH();
+  return HGR_OK;
+}
 
 int launch_hier_finish(unsigned long long* lvl_best, int64_t B, int64_t M, int n_levels, const int32_t* sorted_to_pos,
                        const int32_t* first_out, const int32_t* chain, const int32_t* chain_level, int L, int32_t* lvl_idx,

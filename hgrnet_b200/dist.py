@@ -115,20 +115,27 @@ class _RawCuda:
 X_SLOTS = 4  # feature-ingest slots per exchange (ring length per channel: _ring_len)
 
 
-def exchange_layout(B: int, K: int, world: int, slots: int, D: int = 0):
+def exchange_layout(B: int, K: int, world: int, slots: int, D: int = 0, n_levels: int = 0):
     """Byte layout of one rank's exchange buffer: a 256-byte header (list flags: one word per producer rank at
     byte 0, feature flags at byte 64), then per slot the value lists ``[world, block_rows, K]`` fp32 followed by
     the id lists ``[world, block_rows, K]`` int32 and the bounds ``[world, block_rows]`` fp32 of the global certificate
-    (``hgr_score_topk_scatter_bounded``) and, when ``D`` is given, ``X_SLOTS`` replicas of the normalised
-    image features ``[B, D]`` bf16 (feature ingest, see ``PeerExchange.ingest``)."""
+    (``hgr_score_topk_scatter_bounded``), with ``n_levels`` the per-level winner words ``[world, block_rows, n_levels]``
+    uint64 of class-sharded TOR / POR at ``hier_off`` in the slot (``hgr_hier_level_scatter``) and, when ``D`` is given,
+    ``X_SLOTS`` replicas of the normalised image features ``[B, D]`` bf16 (feature ingest, see
+    ``PeerExchange.ingest``)."""
     block_rows = (B + world - 1) // world
     part = block_rows * K * 4
     bound_bytes = (world * block_rows * 4 + 15) // 16 * 16     # per producer and row: bound of what the shard dropped
     slot_bytes = 2 * world * part + bound_bytes
+    hier = {}
+    if n_levels:
+        # 8-byte aligned: both list areas are multiples of 8 bytes, the bounds of 16, and slots start 16-byte aligned
+        hier = {"hier_off": slot_bytes, "hier_part_bytes": block_rows * n_levels * 8}
+        slot_bytes = (slot_bytes + world * hier["hier_part_bytes"] + 15) // 16 * 16
     x_off = (256 + slots * slot_bytes + 255) // 256 * 256
     x_bytes = (B * D * 2 + 255) // 256 * 256
     return {"block_rows": block_rows, "part_bytes": part, "slot_bytes": slot_bytes, "header": 256,
-            "x_off": x_off, "x_bytes": x_bytes, "total": x_off + (X_SLOTS * x_bytes if D else 0)}
+            "x_off": x_off, "x_bytes": x_bytes, "total": x_off + (X_SLOTS * x_bytes if D else 0), **hier}
 
 
 class PeerMemoryUnavailable(RuntimeError):
@@ -226,6 +233,34 @@ class PeerBank:
             self._own = None
 
 
+class HierShard:
+    """One rank's part of class-sharded TOR / POR (main.py:143,152-191): its contiguous slice ``[row_base, row_base +
+    M_r)`` of the level-sorted train bank (``shard_bounds`` over the sorted rows, so the GEMM columns are balanced) with
+    the global level ends clipped to it, and the global tables the row owner needs to finish its rows.  ``rows_args`` is
+    what ``evaluate.HierMetrics.rows_args()`` returns."""
+
+    def __init__(self, rows_args: dict, rank: int, world: int):
+        bank = rows_args["bank_sorted"]
+        self.M, self.D = bank.shape
+        self.level_end = [int(e) for e in rows_args["level_end"]]
+        self.n_levels = len(self.level_end)
+        if not 1 <= self.n_levels <= 32:
+            raise ValueError("class-sharded TOR / POR supports 1 to 32 levels, got %d" % self.n_levels)
+        lo, hi = shard_bounds(self.M, world)[rank]
+        self.row_base = lo
+        self.bank = bank[lo:hi]                  # a row slice of a contiguous tensor: contiguous, 16-byte aligned
+        self.level_end_local = local_level_ends(self.level_end, lo, hi)
+        self.sorted_to_pos, self.first_out = rows_args["sorted_to_pos"], rows_args["first_out"]
+        self.chain_ptr, self.chain_pos, self.chain_level = (rows_args["chain_ptr"], rows_args["chain_pos"],
+                                                            rows_args["chain_level"])
+
+
+def local_level_ends(level_end, lo: int, hi: int) -> List[int]:
+    """The global level ends of the sorted train bank clipped to the shard ``[lo, hi)``: non-decreasing, ending at
+    ``hi - lo``."""
+    return [min(max(int(e) - lo, 0), hi - lo) for e in level_end]
+
+
 class PeerExchange:
     """Peer-memory exchange of the class-sharded head (no collective call on the data path).
 
@@ -234,11 +269,13 @@ class PeerExchange:
     is mapped into this process (``hgr_peer_open``).  Per batch a rank's scoring kernel then writes its local top-K
     of row block ``g`` directly into list ``rank`` of rank ``g``'s buffer over NVLink (``hgr_score_topk_scatter``)
     and raises its flag there (``hgr_peer_signal``); the owner waits for all ``world`` flags (``hgr_peer_wait``) and
-    merges its ``world`` lists per row (``hgr_topk_merge``).  ``slots`` batches can be in flight.
+    merges its ``world`` lists per row (``hgr_topk_merge``).  ``slots`` batches can be in flight.  With ``n_levels``
+    every slot also carries the per-level winner words of class-sharded TOR / POR (``scatter`` / ``merge`` with
+    ``hier``), published by the same flag.
     """
 
     def __init__(self, B: int, K: int, device, group=None, slots: int = 4, D: int = 0, _bases=None, _rank=None,
-                 _world=None):
+                 _world=None, n_levels: int = 0):
         self.device = torch.device(device)
         self.group = group
         if _bases is None:
@@ -248,8 +285,8 @@ class PeerExchange:
             self.world, self.rank = _world, _rank
         if self.world > 16:
             raise ValueError("PeerExchange supports up to 16 ranks (HGR_MAX_PEERS)")
-        self.B, self.K, self.slots, self.D = B, K, slots, D
-        self.lay = exchange_layout(B, K, self.world, slots, D)
+        self.B, self.K, self.slots, self.D, self.n_levels = B, K, slots, D, n_levels
+        self.lay = exchange_layout(B, K, self.world, slots, D, n_levels)
         self.block_rows = self.lay["block_rows"]
         self.lo = min(B, self.rank * self.block_rows)
         self.hi = min(B, self.lo + self.block_rows)
@@ -293,6 +330,15 @@ class PeerExchange:
         base = self._slot_base(self.bases[self.rank], slot)
         return base, base + self.world * self.lay["part_bytes"], self.block_rows * self.K
 
+    def hier_ptrs(self, slot: int):
+        """Where THIS rank's winner words of row block g go: region ``rank`` of the TOR / POR area of rank g's slot."""
+        off = self.lay["hier_off"] + self.rank * self.lay["hier_part_bytes"]
+        return [self._slot_base(b, slot) + off for b in self.bases]
+
+    def local_hier(self, slot: int):
+        """(pointer, word stride) of the ``world`` winner-word arrays received for my rows."""
+        return self._slot_base(self.bases[self.rank], slot) + self.lay["hier_off"], self.block_rows * self.n_levels
+
     # -- feature ingest ----------------------------------------------------------------------------------------
     def x_ptrs(self, xslot: int):
         return [b + self.lay["x_off"] + xslot * self.lay["x_bytes"] for b in self.bases]
@@ -316,19 +362,26 @@ class PeerExchange:
 
     # -- per batch -------------------------------------------------------------------------------------------
     def scatter(self, x_norm: torch.Tensor, bank: torch.Tensor, id_base: int, slot: int, col_id=None,
-                C_total: int = 0) -> None:
+                C_total: int = 0, hier: Optional[HierShard] = None) -> None:
         """Score the batch against my shard and store the lists at their owners.  ``C_total`` > 0: narrow lists sized
-        for the GLOBAL certificate, with the bound of what was dropped next to every list (``merge(certify=...)``)."""
+        for the GLOBAL certificate, with the bound of what was dropped next to every list (``merge(certify=...)``).
+        ``hier``: also store my train shard's per-level winner words at the owners (``merge(hier=...)``)."""
         val, idx = self.block_ptrs(slot)
         ops.score_topk_scatter(x_norm, bank, val, idx, self.block_rows, col_id=col_id, id_base=id_base, K=self.K,
                                bound_block_ptrs=self.bound_ptrs(slot) if C_total else None, C_total=C_total)
+        if hier is not None:                 # before the signal: the owner's one wait covers lists and words
+            ops.hier_level_scatter(x_norm, hier.bank, hier.level_end_local, hier.row_base, self.hier_ptrs(slot),
+                                   self.block_rows)
         ops.peer_signal(self.flag_ptrs, self.seq[0:1])
 
     def merge(self, slot: int, targets: Optional[torch.Tensor], hits: Optional[torch.Tensor], out=None,
-              targets_local: bool = False, certify=None):
+              targets_local: bool = False, certify=None, hier: Optional[HierShard] = None,
+              counts: Optional[torch.Tensor] = None, hier_out=None):
         """Final top-K (+ hits) of MY rows ``[lo, hi)``; ``targets`` holds the labels of the whole batch (or of my
         rows only with ``targets_local``).  ``certify = (x_norm [B, D], shard table, repair counter)`` after a
-        ``scatter(C_total=...)``: rows whose K-th value does not beat every shard's bound are repaired exactly."""
+        ``scatter(C_total=...)``: rows whose K-th value does not beat every shard's bound are repaired exactly.
+        ``hier`` after a ``scatter(hier=...)``: also count TOR / POR of my rows into ``counts`` (``ops.new_hier_counts``);
+        ``hier_out = (lvl_idx [n, n_levels], top1 [n])`` int32 receives their per-level winners and top-1."""
         ops.peer_wait(self.bases[self.rank], self.world, self.seq[1:2])
         n = self.hi - self.lo
         if n <= 0:
@@ -337,10 +390,18 @@ class PeerExchange:
         t = None if targets is None else (targets if targets_local else targets[self.lo:self.hi])
         if certify is not None:
             x_norm, table, repairs = certify
-            return ops.topk_merge_certified(pv, pi, self.local_bounds(slot), self.world, n, self.K, stride, self.block_rows,
-                                            x_norm[self.lo:self.hi], table, self.device, targets=t, hits=hits,
-                                            repair_count=repairs, out=out)
-        return ops.topk_merge_raw(pv, pi, self.world, n, self.K, stride, self.device, targets=t, hits=hits, out=out)
+            res = ops.topk_merge_certified(pv, pi, self.local_bounds(slot), self.world, n, self.K, stride, self.block_rows,
+                                           x_norm[self.lo:self.hi], table, self.device, targets=t, hits=hits,
+                                           repair_count=repairs, out=out)
+        else:
+            res = ops.topk_merge_raw(pv, pi, self.world, n, self.K, stride, self.device, targets=t, hits=hits, out=out)
+        if hier is not None:
+            parts, part_stride = self.local_hier(slot)
+            lvl_idx, top1 = hier_out if hier_out is not None else (None, None)
+            ops.hier_finish_rows_gathered(parts, self.world, part_stride, n, hier.M, hier.n_levels, hier.sorted_to_pos,
+                                          hier.first_out, t, hier.chain_ptr, hier.chain_pos, hier.chain_level, counts,
+                                          lvl_idx=lvl_idx, top1=top1)
+        return res
 
     def close(self) -> None:
         for p in self._opened:
@@ -375,14 +436,24 @@ class ShardedEvalStream:
       on every rank, the gather of batch i overlapping the GEMM of batch i+1.
 
     A replay is one ``cudaGraphLaunch`` for ``steps`` batches: no interpreter, no per-batch launch latency.
+
+    ``hier`` (a ``HierShard`` of this rank, peer exchange only): every batch also counts TOR / POR (main.py:143,152-191)
+    of the rows this rank owns, against each row's own label.  The rank's slice of the level-sorted train bank runs the
+    per-level arg-max GEMM, its winner words travel to the row owners with the lists, under the same flag, and the owner
+    finishes its rows after the list merge.  The per-chain-length counters share one device buffer with ``hits``
+    (``counters``), so ``host_io`` still makes one D2H copy per batch; ``hier_ratios()`` sums them over ranks.
     """
 
     def __init__(self, bank_shard: torch.Tensor, id_base: int, *, batch: int, K: int = 20, steps: int = 8,
                  feat_dtype=torch.float32, banks=None, group=None, use_graph: bool = True, exchange: str = "p2p",
                  channels: int = 4, host_io: bool = False, col_id: Optional[torch.Tensor] = None,
-                 certify: str = "global"):
+                 certify: str = "global", hier: Optional[HierShard] = None):
         if exchange not in ("p2p", "nccl"):
             raise ValueError("exchange must be 'p2p' or 'nccl'")
+        if hier is not None and exchange != "p2p":
+            raise ValueError("hier (class-sharded TOR / POR) needs the peer-memory exchange")
+        if hier is not None and hier.D != bank_shard.shape[1]:
+            raise ValueError("hier: the train bank has D = %d, the class bank %d" % (hier.D, bank_shard.shape[1]))
         if certify not in ("global", "local"):
             raise ValueError("certify must be 'global' or 'local'")
         if host_io and exchange != "p2p":
@@ -411,7 +482,12 @@ class ShardedEvalStream:
         if not host_io:
             self.dev_feats = [torch.empty((batch, D), dtype=feat_dtype, device=self.device) for _ in range(steps)]
             self.dev_labels = [torch.zeros((batch,), dtype=torch.int32, device=self.device) for _ in range(steps)]
-        self.hits = ops.new_hits(self.device)
+        # hit counters, then (with hier) the per-chain-length TOR / POR counters: one buffer, one D2H copy per batch
+        self.hier = hier
+        n_counters = ops.HGR_NUM_HITS + (0 if hier is None else (ops.HGR_HIER_MAX_CHAIN + 1) * 4)
+        self.counters = torch.zeros(n_counters, dtype=torch.int64, device=self.device)
+        self.hits = self.counters[:ops.HGR_NUM_HITS]
+        self.hier_counts = None if hier is None else self.counters[ops.HGR_NUM_HITS:].view(ops.HGR_HIER_MAX_CHAIN + 1, 4)
         self.val = [None] * steps
         self.idx = [None] * steps
         self.row_lo, self.row_hi = 0, batch
@@ -427,8 +503,8 @@ class ShardedEvalStream:
             if steps < 2:
                 raise ValueError("ShardedEvalStream needs steps >= 2 (two batches per exchange channel and replay)")
             self.channels = max(1, min(channels, steps // 2))
-            self.pxs = [PeerExchange(batch, K, self.device, group=group, slots=self.slots, D=D if host_io else 0)
-                        for _ in range(self.channels)]
+            self.pxs = [PeerExchange(batch, K, self.device, group=group, slots=self.slots, D=D if host_io else 0,
+                                     n_levels=0 if hier is None else hier.n_levels) for _ in range(self.channels)]
             self._ring, self._xring = [], []
             for c in range(self.channels):
                 n_c = (steps - c + self.channels - 1) // self.channels          # batches of channel c per replay
@@ -454,8 +530,9 @@ class ShardedEvalStream:
                 self.dev_pack = [torch.zeros(fbytes + n_my * 4, dtype=torch.uint8, device=self.device) for _ in range(steps)]
                 self.host_feats, self.host_labels = map(list, zip(*[views(p) for p in self.host_pack]))
                 self.dev_feats, self.dev_labels = map(list, zip(*[views(p) for p in self.dev_pack]))
-                self.host_hits = [torch.zeros((ops.HGR_NUM_HITS,), dtype=torch.int64, pin_memory=True)
-                                  for _ in range(steps)]
+                self.host_counters = [torch.zeros((n_counters,), dtype=torch.int64, pin_memory=True)
+                                      for _ in range(steps)]
+                self.host_hits = [c[:ops.HGR_NUM_HITS] for c in self.host_counters]
             if self.world > 1:
                 dist.barrier(group=group)          # every buffer is mapped everywhere before the first store
         else:
@@ -468,7 +545,7 @@ class ShardedEvalStream:
         with torch.cuda.stream(self.stream):
             self._issue()                      # warm-up: NCCL communicator, workspaces
             self.stream.synchronize()
-            self.hits.zero_()
+            self.counters.zero_()
             if use_graph:
                 try:
                     g = torch.cuda.CUDAGraph()
@@ -479,7 +556,7 @@ class ShardedEvalStream:
                     print("ShardedEvalStream: graph capture of the NCCL pipeline failed (%r); running eagerly" % (e,))
                     self.graph = None
         torch.cuda.synchronize(self.device)
-        self.hits.zero_()
+        self.counters.zero_()
 
     def _local(self, s: int):
         bank = self.banks[s % len(self.banks)]
@@ -488,13 +565,14 @@ class ShardedEvalStream:
             self.dev_pack[s].copy_(self.host_pack[s], non_blocking=True)
             x = px.ingest(self.dev_feats[s], j % self._xring[s % self.channels])
             self._x[s] = x
-            px.scatter(x, bank, self.id_base, j % self._ring[s % self.channels], col_id=self.col_id, C_total=self.C_total)
+            px.scatter(x, bank, self.id_base, j % self._ring[s % self.channels], col_id=self.col_id, C_total=self.C_total,
+                       hier=self.hier)
             return None
         x = ops.normalize_rows(self.dev_feats[s])
         if self.exchange == "p2p":
             self._x[s] = x           # the owner's repair reads the row's features (kept alive for the captured graph)
             self.pxs[s % self.channels].scatter(x, bank, self.id_base, (s // self.channels) % self._ring[s % self.channels],
-                                                col_id=self.col_id, C_total=self.C_total)
+                                                col_id=self.col_id, C_total=self.C_total, hier=self.hier)
             return None
         if bank.shape[0] > 0:
             # results go straight into the send record (no pack copies)
@@ -515,9 +593,10 @@ class ShardedEvalStream:
             if self.certify == "global":
                 cert = (self._x[s], self.pbanks[s % len(self.pbanks)].table, self.repairs)
             self.pxs[s % self.channels].merge((s // self.channels) % self._ring[s % self.channels], self.dev_labels[s], self.hits,
-                                              out=(self.val[s], self.idx[s]), targets_local=self.host_io, certify=cert)
+                                              out=(self.val[s], self.idx[s]), targets_local=self.host_io, certify=cert,
+                                              hier=self.hier, counts=self.hier_counts)
             if self.host_io:
-                self.host_hits[s].copy_(self.hits, non_blocking=True)
+                self.host_counters[s].copy_(self.counters, non_blocking=True)
             return
         if work is not None:
             work.wait()
@@ -580,3 +659,19 @@ class ShardedEvalStream:
         if self.exchange == "p2p" and self.world > 1:
             dist.all_reduce(h, group=self.group)
         return h
+
+    def hier_ratios(self):
+        """``(hit_ratio, path_ratio, point_ratio)`` in percent -- the TOR / POR of the reference's ``test()`` line -- over
+        the rows of all ranks scored so far whose label lies in the hierarchy.  A collective (one ``all_reduce`` of the
+        per-chain-length counters): call it on every rank.  Needs ``hier``."""
+        if self.hier is None:
+            raise RuntimeError("ShardedEvalStream was built without hier metrics (pass hier=HierShard(...))")
+        from .evaluate import hier_totals
+        torch.cuda.synchronize(self.device)
+        c = self.hier_counts.clone()
+        if self.world > 1:
+            dist.all_reduce(c, group=self.group)
+        rows, hits, point, path = hier_totals(c).tolist()
+        if rows == 0:
+            return 0.0, 0.0, 0.0
+        return hits / rows * 100.0, path / rows * 100.0, point / rows * 100.0

@@ -481,6 +481,61 @@ def hier_metrics_fused_rows(x_norm: torch.Tensor, bank_sorted: torch.Tensor, lev
                                                 _ptr(lvl_idx), _ptr(top1), _ptr(counts), _stream()))
 
 
+def hier_level_scatter(x_norm: torch.Tensor, bank_shard: torch.Tensor, level_end_local, row_base: int, dst_block_ptrs,
+                       block_rows: int) -> None:
+    """Producer half of class-sharded TOR / POR (``hgr_hier_level_scatter``): the per-level arg-max of ``x_norm``
+    against ``bank_shard`` (sorted rows ``[row_base, row_base + M_r)`` of the level-sorted train bank, ``level_end_local``
+    the global level ends clipped to it), each winner word rebased to the global sorted row and stored at the owner of
+    its row: rows ``[g*block_rows, (g+1)*block_rows)`` go to the ``[block_rows, n_levels]`` uint64 array at
+    ``dst_block_ptrs[g]`` (device pointers, local or peer).  An empty shard stores zeros."""
+    import ctypes
+    lib = _cabi.load()
+    x_norm = _require(x_norm, "x_norm", torch.bfloat16)
+    bank_shard = _require(bank_shard, "bank_shard", torch.bfloat16)
+    B, D = x_norm.shape
+    M_r = bank_shard.shape[0]
+    if M_r and bank_shard.shape[1] != D:
+        raise ValueError("x_norm and bank_shard disagree on D: %d vs %d" % (D, bank_shard.shape[1]))
+    n_levels = len(level_end_local)
+    ends = (ctypes.c_int32 * n_levels)(*[int(e) for e in level_end_local])
+    n = len(dst_block_ptrs)
+    dt = (ctypes.c_void_p * n)(*dst_block_ptrs)
+    ws = _hier_workspace(B * n_levels * 8, x_norm.device)
+    _cabi.check(lib.hgr_hier_level_scatter(_ptr(x_norm), _ptr(bank_shard), B, M_r, D, ends, n_levels, int(row_base),
+                                           _ptr(ws), ws.numel(), block_rows, n, dt, _stream()))
+
+
+def hier_finish_rows_gathered(parts_ptr: int, n_parts: int, part_stride: int, n_rows: int, M: int, n_levels: int,
+                              sorted_to_pos: torch.Tensor, first_out: torch.Tensor, targets: torch.Tensor,
+                              chain_ptr: torch.Tensor, chain_pos: torch.Tensor, chain_level: torch.Tensor,
+                              counts: torch.Tensor, lvl_idx: Optional[torch.Tensor] = None,
+                              top1: Optional[torch.Tensor] = None) -> None:
+    """Owner half of class-sharded TOR / POR (``hgr_hier_finish_rows_gathered``): for ``n_rows`` rows, the max over the
+    ``n_parts`` shards' winner words at ``parts_ptr`` (``part_stride`` words apart, e.g. a peer-exchange slot), then
+    what ``hier_metrics_fused_rows`` does with its own words.  ``targets`` / ``lvl_idx`` / ``top1`` cover these rows;
+    ``M``, ``sorted_to_pos``, ``first_out`` and the chain table are the global ones."""
+    lib = _cabi.load()
+    sorted_to_pos = _require(sorted_to_pos, "sorted_to_pos", torch.int32)
+    first_out = _require(first_out, "first_out", torch.int32)
+    targets = _require(targets, "targets", torch.int32)
+    chain_ptr = _require(chain_ptr, "chain_ptr", torch.int32)
+    chain_pos = _require(chain_pos, "chain_pos", torch.int32)
+    chain_level = _require(chain_level, "chain_level", torch.int32)
+    if not counts.is_cuda or counts.dtype != torch.int64 or counts.numel() != (HGR_HIER_MAX_CHAIN + 1) * 4 \
+            or not counts.is_contiguous():
+        raise ValueError("counts must be a contiguous CUDA int64 [%d, 4] tensor (new_hier_counts)" % (HGR_HIER_MAX_CHAIN + 1))
+    if sorted_to_pos.numel() != M or first_out.numel() != n_levels or targets.numel() != n_rows \
+            or chain_pos.numel() != chain_level.numel():
+        raise ValueError("hier_finish_rows_gathered: inconsistent sizes")
+    for name, t, shape in (("lvl_idx", lvl_idx, (n_rows, n_levels)), ("top1", top1, (n_rows,))):
+        if t is not None and (t.dtype != torch.int32 or tuple(t.shape) != shape or not t.is_contiguous() or not t.is_cuda):
+            raise ValueError("%s must be a contiguous CUDA int32 %s tensor" % (name, list(shape)))
+    _cabi.check(lib.hgr_hier_finish_rows_gathered(parts_ptr, n_parts, part_stride, n_rows, M, n_levels, _ptr(sorted_to_pos),
+                                                  _ptr(first_out), _ptr(targets), chain_ptr.numel() - 1, _ptr(chain_ptr),
+                                                  _ptr(chain_pos), _ptr(chain_level), _ptr(lvl_idx), _ptr(top1),
+                                                  _ptr(counts), _stream()))
+
+
 def masked_ce(logits: torch.Tensor, set_ptr: torch.Tensor, set_col: torch.Tensor, label_pos: torch.Tensor,
               weight: torch.Tensor, need_grad: bool = True):
     """Fused masked CE over T class sets (model/clip_tree.py:241-277).  Returns ``(loss [T], dlogits [B,U] | None)``."""

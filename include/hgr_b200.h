@@ -327,6 +327,39 @@ int hgr_hier_metrics_fused_rows(const void* X, const void* bank_sorted, int64_t 
                                 int64_t* counts, void* stream);
 
 /*
+ * hgr_hier_metrics_fused_rows for the CLASS-SHARDED head (main.py:143,152-191): the level-sorted train bank [M, D] is
+ * cut into contiguous row ranges, one per rank, and image rows are owned block-wise as in hgr_score_topk_scatter.  The
+ * result is bit-identical to hgr_hier_metrics_fused_rows on the whole batch on one GPU: a winner word is
+ * (order key << 32 | ~global sorted row), larger = larger value or else smaller row, the stable level sort keeps
+ * train_index order inside a level across shard boundaries, and max is associative -- so the max over the shards'
+ * words is the word the single-GPU epilogue keeps, whatever the number of shards or the order of arrival.
+ *
+ * hgr_hier_level_scatter          producer: the per-level arg-max GEMM of X [B, D] against this rank's shard
+ *                                 bank_shard [M_r, D] = sorted rows [row_base, row_base + M_r), level_end_local
+ *                                 [n_levels] (HOST) = the global level ends clipped to the shard (non-decreasing, last
+ *                                 = M_r).  Every word of rows [g * block_rows, (g + 1) * block_rows) is rebased to the
+ *                                 global sorted row and stored, zeros included, at dst_blocks[g]
+ *                                 [block_rows][n_levels] uint64 (HOST array of n_blocks device pointers, local or peer,
+ *                                 8-byte aligned).  M_r == 0 runs no GEMM and stores zeros (X / bank_shard unused).
+ *                                 workspace: B * n_levels * 8 bytes, zero on first use, handed back zeroed.  Enqueue it
+ *                                 before hgr_peer_signal: the owner's hgr_peer_wait then covers these words too.
+ * hgr_hier_finish_rows_gathered   owner: for its n_rows rows, the max over the n_parts word arrays parts[p *
+ *                                 part_stride + row * n_levels + level] (part_stride in words), then the decode, -1
+ *                                 rule, tie rule and chain matching of hgr_hier_metrics_fused_rows.  targets, lvl_idx,
+ *                                 top1 cover the owner's rows; M, sorted_to_pos, first_out and the chain table are the
+ *                                 GLOBAL ones; counts as hgr_hier_metrics_fused_rows.  parts is only read.
+ */
+int hgr_hier_level_scatter(const void* X, const void* bank_shard, int64_t B, int64_t M_r, int64_t D,
+                           const int32_t* level_end_local, int n_levels, int64_t row_base, void* workspace,
+                           size_t workspace_bytes, int64_t block_rows, int n_blocks, uint64_t* const* dst_blocks,
+                           void* stream);
+int hgr_hier_finish_rows_gathered(const uint64_t* parts, int n_parts, int64_t part_stride, int64_t n_rows, int64_t M,
+                                  int n_levels, const int32_t* sorted_to_pos, const int32_t* first_out,
+                                  const int32_t* targets, int64_t n_nodes, const int32_t* chain_ptr,
+                                  const int32_t* chain_pos, const int32_t* chain_level, int32_t* lvl_idx, int32_t* top1,
+                                  int64_t* counts, void* stream);
+
+/*
  * Fused masked cross-entropy of the OM training step over T sampled class sets
  * (model/clip_tree.py:241-277 with nn.CrossEntropyLoss, :49,:275).
  *
