@@ -60,11 +60,6 @@ SIGNATURES = {
     "hgr_peer_wait": (c_int, [c_void_p, c_int, c_void_p, c_void_p]),
     "hgr_logits_dense": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int64, c_float, c_void_p, c_int64,
                                  c_int, c_void_p]),
-    "hgr_hier_metrics": (c_int, [c_void_p, c_int64, c_int64, c_int64, c_void_p, c_int64, c_void_p, c_int, c_void_p,
-                                 c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
-    "hgr_hier_metrics_fused": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int64, c_void_p, c_int, c_void_p, c_void_p,
-                                       c_void_p, c_void_p, c_int, c_void_p, c_size_t, c_void_p, c_void_p, c_void_p,
-                                       c_void_p]),
     "hgr_hier_metrics_fused_rows": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int64, c_void_p, c_int, c_void_p,
                                             c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t,
                                             c_void_p, c_void_p, c_void_p, c_void_p]),

@@ -140,9 +140,6 @@ int umma_global_list_len(int64_t B, int64_t C, int64_t D, int K, int64_t C_total
 
 int launch_level_argmax_umma(const __nv_bfloat16* X, const __nv_bfloat16* bank_sorted, int64_t B, int64_t M, int64_t D,
                              const int32_t* level_end, int n_levels, unsigned long long* lvl_best, cudaStream_t stream);
-int launch_hier_finish(unsigned long long* lvl_best, int64_t B, int64_t M, int n_levels, const int32_t* sorted_to_pos,
-                       const int32_t* first_out, const int32_t* chain, const int32_t* chain_level, int L, int32_t* lvl_idx,
-                       int32_t* top1, int64_t* counts, cudaStream_t stream);
 int launch_hier_finish_rows(unsigned long long* lvl_best, int64_t B, int64_t M, int n_levels, const int32_t* sorted_to_pos,
                             const int32_t* first_out, const int32_t* targets, int64_t n_nodes, const int32_t* chain_ptr,
                             const int32_t* chain_pos, const int32_t* chain_level, int32_t* lvl_idx, int32_t* top1,
@@ -155,10 +152,6 @@ int launch_hier_finish_gathered(const unsigned long long* parts, int n_parts, in
                                 const int32_t* targets, int64_t n_nodes, const int32_t* chain_ptr,
                                 const int32_t* chain_pos, const int32_t* chain_level, int32_t* lvl_idx, int32_t* top1,
                                 int64_t* counts, cudaStream_t stream);
-int launch_hier_metrics(const float* logits, int64_t ldl, int64_t B, const int32_t* cols, int64_t M,
-                        const int8_t* level, int n_levels, const int32_t* first_out, const int32_t* chain,
-                        const int32_t* chain_level, int L, int32_t* lvl_idx, int32_t* top1, int64_t* counts,
-                        cudaStream_t stream);
 int launch_normalize_dual(const void* E, int e_dtype, int64_t n_rows, int64_t D, void* out, const int32_t* dst_map,
                           void* out2, cudaStream_t stream);
 int launch_normalize_bcast(const void* E, int e_dtype, int64_t n_rows, int64_t D, int64_t row0, int n_dst,

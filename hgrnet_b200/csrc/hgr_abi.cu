@@ -457,44 +457,6 @@ int hgr_logits_dense(const void* X, const void* bank, int64_t B, int64_t C, int6
   return set_error(HGR_ERR_BAD_ARG, "hgr_logits_dense: unknown impl %d", impl);
 }
 
-int hgr_hier_metrics(const float* logits, int64_t ldl, int64_t B, int64_t N, const int32_t* cols, int64_t M,
-                     const int8_t* level, int n_levels, const int32_t* first_out, const int32_t* chain,
-                     const int32_t* chain_level, int L, int32_t* lvl_idx, int32_t* top1, int64_t* counts, void* stream) {
-  HGR_CHECK_ARG(B >= 0 && N > 0 && M > 0 && M <= (int64_t(1) << 31) - 1, "hgr_hier_metrics: bad sizes B=%lld N=%lld M=%lld",
-                (long long)B, (long long)N, (long long)M);
-  HGR_CHECK_ARG(ldl >= N, "hgr_hier_metrics: ldl < N");
-  HGR_CHECK_ARG(L >= 1 && L <= 64, "hgr_hier_metrics: chain length %d outside [1, 64]", L);
-  if (B == 0) return HGR_OK;
-  HGR_CHECK_ARG(logits && level && first_out && chain && chain_level && counts, "hgr_hier_metrics: null pointer");
-  HGR_CHECK_ARG(cols != nullptr || M == N, "hgr_hier_metrics: cols == NULL needs M == N");
-  return launch_hier_metrics(logits, ldl, B, cols, M, level, n_levels, first_out, chain, chain_level, L, lvl_idx, top1,
-                             counts, static_cast<cudaStream_t>(stream));
-}
-
-int hgr_hier_metrics_fused(const void* X, const void* bank_sorted, int64_t B, int64_t M, int64_t D, const int32_t* level_end,
-                           int n_levels, const int32_t* sorted_to_pos, const int32_t* first_out, const int32_t* chain,
-                           const int32_t* chain_level, int L, void* workspace, size_t workspace_bytes, int32_t* lvl_idx,
-                           int32_t* top1, int64_t* counts, void* stream) {
-  HGR_CHECK_ARG(B >= 0 && M > 0 && M <= (int64_t(1) << 31) - 512, "hgr_hier_metrics_fused: bad sizes B=%lld M=%lld", (long long)B,
-                (long long)M);
-  HGR_CHECK_ARG(D > 0 && D % 8 == 0, "hgr_hier_metrics_fused: D = %lld must be a positive multiple of 8", (long long)D);
-  HGR_CHECK_ARG(L >= 1 && L <= 64, "hgr_hier_metrics_fused: chain length %d outside [1, 64]", L);
-  HGR_CHECK_ARG(n_levels >= 1 && n_levels <= 32, "hgr_hier_metrics_fused: %d levels outside [1, 32]", n_levels);
-  if (B == 0) return HGR_OK;
-  HGR_CHECK_ARG(X && bank_sorted && level_end && sorted_to_pos && first_out && chain && chain_level && counts && workspace,
-                "hgr_hier_metrics_fused: null pointer");
-  HGR_CHECK_ARG(aligned16(X) && aligned16(bank_sorted) && aligned16(workspace), "hgr_hier_metrics_fused: X / bank / workspace must be 16-byte aligned");
-  HGR_CHECK_ARG(workspace_bytes >= static_cast<size_t>(B) * n_levels * 8, "hgr_hier_metrics_fused: workspace %zu < %zu bytes",
-                workspace_bytes, static_cast<size_t>(B) * n_levels * 8);
-  if (!umma_supported(B, M, D, 1)) return set_error(HGR_ERR_UNSUPPORTED, "hgr_hier_metrics_fused: shape not supported by the tcgen05 kernel");
-  cudaStream_t s = static_cast<cudaStream_t>(stream);
-  unsigned long long* best = static_cast<unsigned long long*>(workspace);
-  const int rc = launch_level_argmax_umma(static_cast<const __nv_bfloat16*>(X), static_cast<const __nv_bfloat16*>(bank_sorted), B, M,
-                                          D, level_end, n_levels, best, s);
-  if (rc != HGR_OK) return rc;
-  return launch_hier_finish(best, B, M, n_levels, sorted_to_pos, first_out, chain, chain_level, L, lvl_idx, top1, counts, s);
-}
-
 int hgr_hier_metrics_fused_rows(const void* X, const void* bank_sorted, int64_t B, int64_t M, int64_t D,
                                 const int32_t* level_end, int n_levels, const int32_t* sorted_to_pos,
                                 const int32_t* first_out, const int32_t* targets, int64_t n_nodes,

@@ -286,7 +286,8 @@ int launch_score_topk_umma(const __nv_bfloat16* X, const __nv_bfloat16* bank, co
 int launch_level_argmax_umma(const __nv_bfloat16* X, const __nv_bfloat16* bank_sorted, int64_t B, int64_t M, int64_t D,
                              const int32_t* level_end, int n_levels, unsigned long long* lvl_best, cudaStream_t stream) {
   if (n_levels < 1 || n_levels > kMaxHierLevels)
-    return set_error(HGR_ERR_UNSUPPORTED, "hgr_hier_metrics_fused: %d levels outside [1, %d]", n_levels, kMaxHierLevels);
+    return set_error(HGR_ERR_UNSUPPORTED, "hgr_hier_metrics_fused_rows / hgr_hier_level_scatter: %d levels outside [1, %d]",
+                     n_levels, kMaxHierLevels);
   CUtensorMap mx, mb;
   Params p{};
   int rc = common_setup(X, bank_sorted, B, M, D, &mx, &mb, &p);
@@ -297,11 +298,14 @@ int launch_level_argmax_umma(const __nv_bfloat16* X, const __nv_bfloat16* bank_s
   int32_t prev = 0;
   for (int l = 0; l < n_levels; ++l) {
     if (level_end[l] < prev || level_end[l] > M)
-      return set_error(HGR_ERR_BAD_ARG, "hgr_hier_metrics_fused: level_end must be non-decreasing and <= M");
+      return set_error(HGR_ERR_BAD_ARG,
+                       "hgr_hier_metrics_fused_rows / hgr_hier_level_scatter: level_end must be non-decreasing and <= M");
     p.lvl_end[l] = prev = level_end[l];
   }
-  if (prev != M) return set_error(HGR_ERR_BAD_ARG, "hgr_hier_metrics_fused: level_end[n_levels - 1] must be M");
-  p.lvl_best = lvl_best;   // all zero: on first use by contract, afterwards because hier_finish_kernel zeroes what it reads
+  if (prev != M)
+    return set_error(HGR_ERR_BAD_ARG, "hgr_hier_metrics_fused_rows / hgr_hier_level_scatter: level_end[n_levels - 1] must be M");
+  // all zero: on first use by contract, afterwards because hier_finish_rows_kernel / hier_push_kernel zero what they read
+  p.lvl_best = lvl_best;
   return launch_pair_kernel(kEpiLevel, 8, mx, mb, p, stream);
 }
 

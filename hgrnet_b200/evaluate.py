@@ -5,8 +5,9 @@ Per batch the reference materialises logits [B,N], gathers the test columns, run
 Here that whole chain is ONE fused call, ``model.score_topk`` (kernel (1) + kernel (2)); the
 hit counters stay on the device until the loop ends, as in the reference.  The hierarchical
 metrics TOR / POR (``hit_ratio`` / ``path_ratio`` / ``point_ratio``, main.py:143,152-191) are the
-first "next" row of SURVEY.md section 8f: they are computed from the dense logits of
-``hgr_logits_dense`` with vectorised device ops (no per-sample python loop, no D2H copies).
+first "next" row of SURVEY.md section 8f: a per-level arg-max in the epilogue of the GEMM against
+the level-sorted train bank, then chain matching on the device (``hgr_hier_metrics_fused_rows``);
+no per-sample python loop, no D2H copies.
 Output format: ``count_acc`` (utils.py:135-146) and the log files of main.py:205-222.
 """
 from __future__ import annotations
@@ -71,41 +72,37 @@ def hier_totals(counts: torch.Tensor) -> torch.Tensor:
 
 
 class HierMetrics:
-    """TOR / POR accumulators (main.py:123-127,152-191).  One fused pass per batch (``hgr_hier_metrics``): per-level
-    arg-max over the train columns, chain matching and counting on the device; the per-batch divisions by the chain
+    """TOR / POR accumulators (main.py:123-127,152-191).  One fused call per batch (``hgr_hier_metrics_fused_rows``):
+    per-level arg-max over the train classes in the epilogue of the GEMM against the level-sorted train bank, then
+    chain matching and counting on the device into integer counters per chain length; the divisions by the chain
     length stay device-side float ops, nothing is copied to the host before the ratios are printed.
 
-    ``update`` / ``update_fused`` score a single-label batch against one label (the reference's ``targets[0]``);
     ``update_rows`` scores every row against its own label and needs no host work per batch."""
 
     def __init__(self, model):
         self.model = model
         dev = model.device
-        # (rows counted by update_rows, hits, point, path) -- the order of hier_totals: update_rows folds a batch in with
-        # one add
+        # (rows, hits, point, path) -- the order of hier_totals: update_rows folds a batch in with one add
         self._acc = torch.zeros(4, dtype=torch.float64, device=dev)
         self.hits_all = self._acc[1]
         self.point_all = self._acc[2]
         self.path_all = self._acc[3]
-        self._rows_host = 0                   # rows of update / update_fused (the batch size is known on the host)
         depth = torch.from_numpy(model.hierarchy.depth).to(torch.int64)
         self.n_levels = int(depth.max()) + 1 if depth.numel() else 1
-        # Only the TRAIN columns enter TOR / POR (main.py:143,155,174): the dense logits are taken against the train
-        # rows of the bank alone ([B, M], M = 983 of 18,278 classes on ImageNet-21K-D) instead of all N nodes, and the
-        # kernel works in train POSITIONS: level per position, the label's chain as positions (-1: not a train class).
+        # Only the TRAIN columns enter TOR / POR (main.py:143,155,174): the GEMM runs against the train rows of the bank
+        # alone (M = 983 of 18,278 classes on ImageNet-21K-D) instead of all N nodes, and the kernels work in train
+        # POSITIONS: the label's chain as positions (-1: not a train class).
         train = model.train_index.cpu()
         dt = depth[train]
         M = dt.numel()
-        self._level = dt.to(torch.int8).to(dev)
-        self._pos_of = {int(n): j for j, n in enumerate(train.tolist())}
         # first position of train_index that is NOT at level l: where the reference's -1 fill (main.py:171) sits first
         first_out = []
         for l in range(self.n_levels):
             out = (dt != l).nonzero()
             first_out.append(int(out[0]) if out.numel() else M)
         self._first_out = torch.tensor(first_out, dtype=torch.int32, device=dev)
-        # fused path (hgr_hier_metrics_fused): the train rows of the bank sorted by level -- stable, so that inside a
-        # level the sorted order is the train_index order and "first position among equal values" is preserved
+        # the train rows of the bank sorted by level -- stable, so that inside a level the sorted order is the
+        # train_index order and "first position among equal values" is preserved
         order = torch.sort(dt, stable=True).indices
         self._sorted_to_pos = order.to(torch.int32).to(dev)
         self._level_end = torch.cumsum(torch.bincount(dt, minlength=self.n_levels), 0).tolist()
@@ -117,8 +114,8 @@ class HierMetrics:
 
     @property
     def path_all_count(self) -> int:
-        """Rows scored so far (synchronises when ``update_rows`` has run)."""
-        return self._rows_host + int(self._acc[0])
+        """Rows scored so far (synchronises)."""
+        return int(self._acc[0])
 
     def sorted_bank(self) -> torch.Tensor:
         """The train rows of the bank sorted by level; re-sorted when ``model.bank_train`` was refreshed (new tensor or
@@ -142,47 +139,10 @@ class HierMetrics:
         return dict(bank_sorted=self.sorted_bank(), level_end=self._level_end, sorted_to_pos=self._sorted_to_pos,
                     first_out=self._first_out, chain_ptr=chain_ptr, chain_pos=chain_pos, chain_level=chain_level)
 
-    def update(self, logits_train: torch.Tensor, target: int):
-        """``logits_train`` [B, M]: cosine logits against ``model.bank_train`` (column j = node train_index[j])."""
-        m = self.model
-        B = logits_train.shape[0]
-        parents = list(m.c2p[target]) + [target]
-        L = len(parents)
-        dev = logits_train.device
-        chain = torch.tensor([self._pos_of.get(p, -1) for p in parents], dtype=torch.int32).to(dev, non_blocking=True)
-        chain_level = torch.tensor([len(m.c2p[p]) for p in parents], dtype=torch.int32).to(dev, non_blocking=True)
-        counts = torch.zeros(3, dtype=torch.int64, device=dev)
-        ops.hier_metrics(logits_train, None, self._level, self.n_levels, self._first_out, chain, chain_level, counts)
-        c = counts.double()
-        self.hits_all += c[0]                                               # main.py:158-160
-        self.path_all += c[2] if L == 1 else c[2] / (L - 1)                 # main.py:179-190
-        self.point_all += c[1] / L                                          # main.py:191
-        self._rows_host += B
-
-    def update_fused(self, x_norm: torch.Tensor, target: int):
-        """``update`` without the dense logits: ``x_norm`` [B, D] bf16 normalised image features; the per-level arg-max
-        over the train classes runs in the epilogue of the GEMM against the level-sorted train bank."""
-        m = self.model
-        bank_sorted = self.sorted_bank()
-        B = x_norm.shape[0]
-        parents = list(m.c2p[target]) + [target]
-        L = len(parents)
-        dev = x_norm.device
-        chain = torch.tensor([self._pos_of.get(p, -1) for p in parents], dtype=torch.int32).to(dev, non_blocking=True)
-        chain_level = torch.tensor([len(m.c2p[p]) for p in parents], dtype=torch.int32).to(dev, non_blocking=True)
-        counts = torch.zeros(3, dtype=torch.int64, device=dev)
-        ops.hier_metrics_fused(x_norm, bank_sorted, self._level_end, self._sorted_to_pos, self._first_out, chain,
-                               chain_level, counts)
-        c = counts.double()
-        self.hits_all += c[0]
-        self.path_all += c[2] if L == 1 else c[2] / (L - 1)
-        self.point_all += c[1] / L
-        self._rows_host += B
-
     def update_rows(self, x_norm: torch.Tensor, targets: torch.Tensor):
-        """``update_fused`` with one label per row: row i is scored against the chain of node ``targets[i]``, so a
-        batch may mix classes; for a single-label batch it adds what ``update_fused`` adds.  Rows whose target lies
-        outside ``[0, n_nodes)`` are skipped (padding).  No host work per batch and no synchronisation."""
+        """Score a batch: ``x_norm`` [B, D] bf16 normalised image features, row i scored against the chain of node
+        ``targets[i]``, so a batch may mix classes.  Rows whose target lies outside ``[0, n_nodes)`` are skipped
+        (padding).  No host work per batch and no synchronisation."""
         if self._counts is None:
             self._counts = ops.new_hier_counts(x_norm.device)
         else:
@@ -197,7 +157,10 @@ class HierMetrics:
 
 def test(opts, model, device, splits=None, loader: Optional[Iterable] = None, log: bool = True):
     """Drop-in for main.py:104-222.  ``loader`` yields the reference's batch dicts
-    ``{'img': [1,B,...], 'label': [1,B]}`` (single-label batches, imagenet_group_test.py)."""
+    ``{'img': [1,B,...], 'label': [1,B]}`` (single-label batches, imagenet_group_test.py).
+
+    TOR / POR score every row of a batch against the batch's first label, as the reference does with ``targets[0]``
+    (main.py:152).  A first label outside the hierarchy is counted nowhere (the reference raises ``IndexError``)."""
     print("out", opts.out_ratio)
     print("in", opts.in_ratio)
     model.eval()
@@ -216,12 +179,8 @@ def test(opts, model, device, splits=None, loader: Optional[Iterable] = None, lo
             x = model.encode_image_normalized(imgs)
             model.score_topk(None, targets, hits=hits, feats_normalized=x)   # main.py:135-147, fused
             num_sample += len(targets)
-            if hier is not None:
-                if getattr(opts, "hgr_hier_dense", False):                   # cross-check path: dense [B, M] logits
-                    logits_train = ops.logits_dense(x, model.bank_train)     # clip_tree.py:331, train columns only
-                    hier.update(logits_train, int(data["label"][0][0]))
-                else:                                                        # per-level arg-max in the GEMM epilogue
-                    hier.update_fused(x, int(data["label"][0][0]))
+            if hier is not None:                                             # main.py:152: every row against targets[0]
+                hier.update_rows(x, targets[:1].expand(len(targets)))
             if i % opts.print_freq == 0:
                 out_str = _format(hits, num_sample, hier)
                 print(out_str, flush=True)

@@ -77,8 +77,6 @@ def build_parser() -> argparse.ArgumentParser:
                         "ancestor chain) through the CSR aggregation kernel")
     g.add_argument("--hgr_hier_metrics", type=_bool, default=True, choices=[True, False],
                    help="also compute TOR/POR (hit_ratio/path_ratio/point_ratio, main.py:152-191) during test")
-    g.add_argument("--hgr_hier_dense", type=_bool, default=False, choices=[True, False],
-                   help="TOR/POR from dense [B, M] train logits (cross-check) instead of the per-level arg-max in the GEMM epilogue")
     g.add_argument("--hgr_synthetic", default="", type=str,
                    help="run on a synthetic hierarchy and synthetic features, e.g. '10,100,1000' level sizes")
     return p

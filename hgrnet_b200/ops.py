@@ -371,29 +371,6 @@ def logits_dense(X: torch.Tensor, bank: torch.Tensor, scale: float = 1.0, impl: 
     return out
 
 
-def hier_metrics(logits: torch.Tensor, cols: Optional[torch.Tensor], level: torch.Tensor, n_levels: int,
-                 first_out: torch.Tensor, chain: torch.Tensor, chain_level: torch.Tensor, counts: torch.Tensor,
-                 lvl_idx: Optional[torch.Tensor] = None, top1: Optional[torch.Tensor] = None) -> None:
-    """TOR / POR counters of one single-label batch (main.py:143,152-191) in one pass over the dense logits;
-    ``counts`` (int64 [3]: TOR hits, points, edges) is incremented.  See ``hgr_hier_metrics`` in the header."""
-    lib = _cabi.load()
-    logits = _require(logits, "logits", torch.float32)
-    B, N = logits.shape
-    if cols is not None:
-        cols = _require(cols, "cols", torch.int32)
-    level = _require(level, "level", torch.int8)
-    first_out = _require(first_out, "first_out", torch.int32)
-    chain = _require(chain, "chain", torch.int32)
-    chain_level = _require(chain_level, "chain_level", torch.int32)
-    counts = _require(counts, "counts", torch.int64)
-    if level.numel() != N or first_out.numel() != n_levels or chain.numel() != chain_level.numel():
-        raise ValueError("hier_metrics: inconsistent sizes")
-    M = cols.numel() if cols is not None else N
-    _cabi.check(lib.hgr_hier_metrics(_ptr(logits), logits.stride(0), B, N, _ptr(cols), M, _ptr(level), n_levels,
-                                     _ptr(first_out), _ptr(chain), _ptr(chain_level), chain.numel(), _ptr(lvl_idx),
-                                     _ptr(top1), _ptr(counts), _stream()))
-
-
 def _hier_workspace(nbytes: int, device) -> torch.Tensor:
     """Per-stream scratch of the fused TOR / POR calls: zero when allocated, handed back zeroed by every call (the
     scoring kernel's workspace on the same stream keeps header words, so this is a separate buffer)."""
@@ -407,33 +384,6 @@ def _hier_workspace(nbytes: int, device) -> torch.Tensor:
     return ws
 
 
-def hier_metrics_fused(x_norm: torch.Tensor, bank_sorted: torch.Tensor, level_end, sorted_to_pos: torch.Tensor,
-                       first_out: torch.Tensor, chain: torch.Tensor, chain_level: torch.Tensor, counts: torch.Tensor,
-                       lvl_idx: Optional[torch.Tensor] = None, top1: Optional[torch.Tensor] = None) -> None:
-    """``hier_metrics`` without the dense logits: ``bank_sorted`` holds the train rows of the bank sorted by level
-    (``level_end``: host list of exclusive ends), the per-level arg-max runs in the epilogue of the tcgen05 GEMM
-    (``hgr_hier_metrics_fused``).  Positions (chain, first_out, lvl_idx, top1) are positions in ``train_index``."""
-    import ctypes
-    lib = _cabi.load()
-    x_norm = _require(x_norm, "x_norm", torch.bfloat16)
-    bank_sorted = _require(bank_sorted, "bank_sorted", torch.bfloat16)
-    sorted_to_pos = _require(sorted_to_pos, "sorted_to_pos", torch.int32)
-    first_out = _require(first_out, "first_out", torch.int32)
-    chain = _require(chain, "chain", torch.int32)
-    chain_level = _require(chain_level, "chain_level", torch.int32)
-    counts = _require(counts, "counts", torch.int64)
-    B, D = x_norm.shape
-    M = bank_sorted.shape[0]
-    n_levels = len(level_end)
-    if sorted_to_pos.numel() != M or first_out.numel() != n_levels or chain.numel() != chain_level.numel():
-        raise ValueError("hier_metrics_fused: inconsistent sizes")
-    ends = (ctypes.c_int32 * n_levels)(*[int(e) for e in level_end])
-    ws = _hier_workspace(B * n_levels * 8, x_norm.device)
-    _cabi.check(lib.hgr_hier_metrics_fused(_ptr(x_norm), _ptr(bank_sorted), B, M, D, ends, n_levels, _ptr(sorted_to_pos),
-                                           _ptr(first_out), _ptr(chain), _ptr(chain_level), chain.numel(), _ptr(ws),
-                                           ws.numel(), _ptr(lvl_idx), _ptr(top1), _ptr(counts), _stream()))
-
-
 def new_hier_counts(device) -> torch.Tensor:
     """Zeroed per-chain-length counters of ``hier_metrics_fused_rows``: int64 ``[HGR_HIER_MAX_CHAIN + 1, 4]``, bin L =
     ``{rows, TOR hits, points, edges}`` of the rows whose label chain has L entries."""
@@ -444,11 +394,14 @@ def hier_metrics_fused_rows(x_norm: torch.Tensor, bank_sorted: torch.Tensor, lev
                             first_out: torch.Tensor, targets: torch.Tensor, chain_ptr: torch.Tensor,
                             chain_pos: torch.Tensor, chain_level: torch.Tensor, counts: torch.Tensor,
                             lvl_idx: Optional[torch.Tensor] = None, top1: Optional[torch.Tensor] = None) -> None:
-    """``hier_metrics_fused`` with one label per row: row i is matched against the chain of node ``targets[i]``, read
-    from the chain table ``chain_ptr [n_nodes + 1]`` / ``chain_pos`` / ``chain_level`` (``evaluate.chain_table``).
-    ``counts`` (``new_hier_counts``) is incremented per chain length; rows whose target is outside ``[0, n_nodes)`` are
-    counted nowhere.  No host work depends on the batch's contents, so the call can be captured in a CUDA graph.  See
-    ``hgr_hier_metrics_fused_rows`` in the header."""
+    """TOR / POR counters (main.py:143,152-191) of one batch without the dense logits: ``bank_sorted`` holds the train
+    rows of the bank sorted by level (``level_end``: host list of exclusive ends), the per-level arg-max runs in the
+    epilogue of the tcgen05 GEMM.  Row i is matched against the chain of node ``targets[i]``, read from the chain table
+    ``chain_ptr [n_nodes + 1]`` / ``chain_pos`` / ``chain_level`` (``evaluate.chain_table``).  Positions (chain_pos,
+    first_out, lvl_idx, top1) are positions in ``train_index``.  ``counts`` (``new_hier_counts``) is incremented per
+    chain length; rows whose target is outside ``[0, n_nodes)`` are counted nowhere.  No host work depends on the
+    batch's contents, so the call can be captured in a CUDA graph.  See ``hgr_hier_metrics_fused_rows`` in the
+    header."""
     import ctypes
     lib = _cabi.load()
     x_norm = _require(x_norm, "x_norm", torch.bfloat16)

@@ -260,63 +260,39 @@ int hgr_logits_dense(const void* X, const void* bank, int64_t B, int64_t C, int6
                      float scale, float* out, int64_t ldo, int impl, void* stream);
 
 /*
- * TOR / POR hierarchical metrics of one single-label batch in one pass over dense logits (main.py:143,152-191;
- * SURVEY.md 8-f1).  Replaces the L clone + index_fill + gather + topk passes over [B, N] and the Python B x L
- * loop with device->host copies of the reference's test().
+ * TOR / POR hierarchical metrics (main.py:143,152-191; SURVEY.md 8-f1) of a batch in which every row is matched
+ * against the chain of ITS OWN label, without the dense matrix.  For a single-label batch this is exactly the
+ * reference's metric, whose per-batch edge / (L-1) and point / L are sums of per-row terms.  Replaces the L clone +
+ * index_fill + gather + topk passes over [B, N] and the Python B x L loop with device->host copies of the reference's
+ * test().  Needs no host work per batch and no memset, so it can be captured in a CUDA graph.
  *
- *  logits      [B, N] fp32 (hgr_logits_dense), row pitch ldl
- *  cols        [M] int32 train_index (columns that take part), or NULL = all N columns
- *  level       [N] int8 depth of every node (len(c2p[n])); n_levels <= 32
- *  first_out   [n_levels] int32: first position j whose column is NOT at level l (a masked column holds -1.0,
- *              so that position wins when no in-level logit exceeds -1; >= M when there is none)
- *  chain       [L] int32 the label's ancestor chain + the label itself; chain_level [L] their depths
- *  lvl_idx     [B, n_levels] int32 per-level arg-max node (optional), top1 [B] int32 arg-max over cols (optional)
- *  counts      [3] int64, INCREMENTED: {TOR hits (sum over rows of #{k: top1 == chain[k]}),
- *              points (#{k: lvl[chain_level[k]] == chain[k]}), edges (#{k: matches at k and k+1}; L == 1: match[0])}
- * Ties: first position in `cols` (the CPU arg-max rule; torch's CUDA top-k leaves it unspecified).
- */
-int hgr_hier_metrics(const float* logits, int64_t ldl, int64_t B, int64_t N, const int32_t* cols, int64_t M,
-                     const int8_t* level, int n_levels, const int32_t* first_out, const int32_t* chain,
-                     const int32_t* chain_level, int L, int32_t* lvl_idx, int32_t* top1, int64_t* counts,
-                     void* stream);
-
-/*
- * The same metrics WITHOUT the dense matrix (SURVEY.md 8-f1 as written: "per-depth-level masked arg-max ... in the
- * epilogue").  The train rows of the bank are handed over SORTED BY LEVEL (stable: inside a level in train_index
- * order); X . bank_sorted^T runs on the tcgen05 main loop and the epilogue keeps, per image row, a running arg-max of
- * the current level -- the level of a column is warp-uniform and changes n_levels - 1 times over the whole bank -- and
+ * The train rows of the bank are handed over SORTED BY LEVEL (stable: inside a level in train_index order);
+ * X . bank_sorted^T runs on the tcgen05 main loop and the epilogue keeps, per image row, a running arg-max of the
+ * current level -- the level of a column is warp-uniform and changes n_levels - 1 times over the whole bank -- and
  * publishes it with one 64-bit atomicMax per (row, level, worker).  A second, tiny kernel decodes the winners, maps
- * sorted rows back to train POSITIONS (positions in train_index; chain / first_out / lvl_idx / top1 are positions too,
- * i.e. hgr_hier_metrics with cols == NULL on the [B, M] train logits), applies the -1 rule and counts.
+ * sorted rows back to train POSITIONS (positions in train_index; chain_pos / first_out / lvl_idx / top1 are positions
+ * too), applies the -1 rule and counts.
  *
  *  X            [B, D] bf16, row-normalised          bank_sorted [M, D] bf16, train rows sorted by level
- *  level_end    [n_levels] int32 HOST array: level l = sorted rows [level_end[l-1], level_end[l]); last entry = M
+ *  level_end    [n_levels] int32 HOST array: level l = sorted rows [level_end[l-1], level_end[l]); last entry = M;
+ *               n_levels <= 32
  *  sorted_to_pos [M] int32 (device): position in train_index of sorted row s
+ *  first_out    [n_levels] int32: first position j whose column is NOT at level l (a masked column holds -1.0, so that
+ *               position wins when no in-level logit exceeds -1; >= M when there is none)
  *  workspace    B * n_levels * 8 bytes (device): ZERO on first use; the call hands it back zeroed (no memset per batch)
- * Same results as hgr_hier_metrics on hgr_logits_dense(X, bank_train) -- ties included.
- */
-int hgr_hier_metrics_fused(const void* X, const void* bank_sorted, int64_t B, int64_t M, int64_t D,
-                           const int32_t* level_end, int n_levels, const int32_t* sorted_to_pos,
-                           const int32_t* first_out, const int32_t* chain, const int32_t* chain_level, int L,
-                           void* workspace, size_t workspace_bytes, int32_t* lvl_idx, int32_t* top1, int64_t* counts,
-                           void* stream);
-
-/*
- * hgr_hier_metrics_fused for batches that mix labels: every row is matched against the chain of ITS OWN label.  For a
- * single-label batch this is exactly the reference's metric, whose per-batch edge / (L-1) and point / L are sums of
- * per-row terms.  Needs no host work per batch and no memset, so it can be captured in a CUDA graph.
- *
- *  X, bank_sorted, B, M, D, level_end, n_levels, sorted_to_pos, first_out, workspace, lvl_idx, top1:
- *               as hgr_hier_metrics_fused (lvl_idx / top1 do not depend on the labels; both optional)
+ *  lvl_idx      [B, n_levels] int32 per-level arg-max position after the -1 rule (optional), top1 [B] int32 arg-max
+ *               position over the train columns (optional); neither depends on the labels
  *  targets      [B] int32 node id of each row's label
  *  chain table  CSR over all n_nodes nodes, built once per model: the chain of node n is c2p[n] + [n], entries
  *               [chain_ptr[n], chain_ptr[n+1]); per entry chain_pos = its position in train_index (-1: not a train
  *               class) and chain_level = its depth.  chain_ptr [n_nodes + 1] int32, chain_pos / chain_level int32.
- *  counts       [HGR_HIER_MAX_CHAIN + 1][4] int64, INCREMENTED: bin L (chain length) holds {rows, TOR hits, points,
- *               edges} of the rows whose chain has L entries (bin 0 stays zero).  The reference's totals follow on the
- *               host: hits = sum_L tor_L, path = sum_L edges_L / max(L-1, 1), point = sum_L points_L / L.
+ *  counts       [HGR_HIER_MAX_CHAIN + 1][4] int64, INCREMENTED: bin L (chain length) holds {rows, TOR hits (#{k: top1 ==
+ *               chain[k]}), points (#{k: lvl[chain_level[k]] == chain[k]}), edges (#{k: matches at k and k+1}; L == 1:
+ *               match[0])} of the rows whose chain has L entries (bin 0 stays zero).  The reference's totals follow on
+ *               the host: hits = sum_L tor_L, path = sum_L edges_L / max(L-1, 1), point = sum_L points_L / L.
  * A row whose target lies outside [0, n_nodes), or whose chain length lies outside [1, HGR_HIER_MAX_CHAIN], is counted
  * nowhere (its lvl_idx / top1 are still written): callers pad a fixed-shape batch with target -1.
+ * Ties: first position in train_index (the CPU arg-max rule; torch's CUDA top-k leaves it unspecified).
  */
 #define HGR_HIER_MAX_CHAIN 32 /* = the 32-level limit of the per-level arg-max epilogue */
 int hgr_hier_metrics_fused_rows(const void* X, const void* bank_sorted, int64_t B, int64_t M, int64_t D,

@@ -223,6 +223,26 @@ def count_acc(hits_dict, num_tot):
     return ", ".join(parts) + ".", acc
 
 
+def tor_por_winners(logits: torch.Tensor, train_index: torch.Tensor, c2p, d2n, n_nodes: int, target: int):
+    """The arg-maxes behind ``tor_por`` (main.py:155-156,162-176): ``(top1 [B], dict_path [B, L])`` int64 node ids,
+    the top-1 over ``train_index`` and, per node of the label's chain ``c2p[target] + [target]``, the top-1 over
+    ``train_index`` after every column not at that node's depth is filled with -1."""
+    B = logits.shape[0]
+    parents = list(c2p[target]) + [target]
+    L = len(parents)
+    top1 = train_index[logits[:, train_index].topk(1, 1, True, True)[1]].squeeze(1)
+    dict_path = torch.zeros(B, L, dtype=torch.long)
+    for kk, p in enumerate(parents):
+        level = len(c2p[p])
+        same_l = list(d2n[level])
+        if p not in same_l:
+            same_l.append(p)
+        rest = torch.tensor(sorted(set(range(n_nodes)) - set(same_l)), dtype=torch.long)
+        lk = logits.clone().index_fill(1, rest, -1)[:, train_index]
+        dict_path[:, kk] = train_index[lk.topk(1, 1, True, True)[1]].squeeze(1)
+    return top1, dict_path
+
+
 def tor_por(logits: torch.Tensor, train_index: torch.Tensor, c2p, d2n, n_nodes: int,
             target: int):
     """Hierarchical metrics of one single-label batch, main.py:143,152-191.
@@ -234,18 +254,9 @@ def tor_por(logits: torch.Tensor, train_index: torch.Tensor, c2p, d2n, n_nodes: 
     parents = list(c2p[target]) + [target]
     L = len(parents)
     # TOR (main.py:143,155-160): top-1 over train_index matched against the whole chain
-    top1 = train_index[logits[:, train_index].topk(1, 1, True, True)[1]]  # [B,1]
-    tor_hits = float(top1.expand(B, L).eq(torch.tensor(parents).expand(B, L)).float().sum())
     # POR (main.py:162-176): per chain level, arg-max restricted to that level's nodes
-    dict_path = torch.zeros(B, L)
-    for kk, p in enumerate(parents):
-        level = len(c2p[p])
-        same_l = list(d2n[level])
-        if p not in same_l:
-            same_l.append(p)
-        rest = torch.tensor(sorted(set(range(n_nodes)) - set(same_l)), dtype=torch.long)
-        lk = logits.clone().index_fill(1, rest, -1)[:, train_index]
-        dict_path[:, kk] = train_index[lk.topk(1, 1, True, True)[1]].squeeze(1).float()
+    top1, dict_path = tor_por_winners(logits, train_index, c2p, d2n, n_nodes, target)
+    tor_hits = float(top1[:, None].expand(B, L).eq(torch.tensor(parents).expand(B, L)).float().sum())
     # main.py:177-191
     path_add = 0.0
     edge = 0

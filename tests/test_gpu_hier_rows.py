@@ -1,14 +1,15 @@
-"""TOR / POR with one label per row (``hgr_hier_metrics_fused_rows``, main.py:143,152-191): against the single-label
-fused call on each label's sub-batch, against ``HierMetrics.update_fused`` on single-label batches, and inside the
-graph-replayed ``EvalStream``."""
+"""TOR / POR with one label per row (``hgr_hier_metrics_fused_rows``, main.py:143,152-191) against the oracle's
+restatement of the reference, directly and through ``HierMetrics.update_rows``, and inside the graph-replayed
+``EvalStream``."""
 from __future__ import annotations
 
 import ctypes
+import types
 
 import pytest
 import torch
 
-from oracle import cases
+from oracle import cases, hgr_oracle as orc
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
@@ -22,8 +23,8 @@ def _emb(n, d, seed, normalize=True):
 
 
 def _setup(levels, B, D, train_every):
-    """The inputs of test_hier_metrics_fused_matches_dense_pass (tests/test_gpu_kernels.py), duplicated bank rows
-    included, plus the chain table."""
+    """Seeded inputs with exact ties from duplicated bank rows (inside a level and across two levels), the arguments of
+    ``hier_metrics_fused_rows``, the chain table and the train rows of the bank in ``train_index`` order."""
     from hgrnet_b200 import ops
     from hgrnet_b200.evaluate import chain_table
     from hgrnet_b200.hierarchy import synthetic_hierarchy
@@ -32,7 +33,8 @@ def _setup(levels, B, D, train_every):
     bank = _emb(N, D, 21).to(torch.bfloat16)
     bank[5] = bank[3]
     bank[N - 2] = bank[N // 2]
-    bank[7] = bank[N - 1]                                       # a tie across two levels
+    if N > 7:
+        bank[7] = bank[N - 1]                                   # a tie across two levels
     x = ops.normalize_rows(_emb(B, D, 22, normalize=False).to(DEV))
     train_index = torch.arange(0, N, train_every)
     depth = torch.from_numpy(h.depth).long()
@@ -42,11 +44,68 @@ def _setup(levels, B, D, train_every):
     first_out = torch.tensor([int((dt != l).nonzero()[0]) if (dt != l).any() else M for l in range(n_levels)],
                              dtype=torch.int32, device=DEV)
     order = torch.sort(dt, stable=True).indices
-    args = dict(bank_sorted=bank[train_index].to(DEV)[order.to(DEV)].contiguous(),
+    bank_train = bank[train_index].to(DEV).contiguous()
+    args = dict(bank_sorted=bank_train[order.to(DEV)].contiguous(),
                 level_end=torch.cumsum(torch.bincount(dt, minlength=n_levels), 0).tolist(),
                 sorted_to_pos=order.to(torch.int32).to(DEV), first_out=first_out)
     table = [torch.from_numpy(a).to(DEV) for a in chain_table(h.c2p, h.depth, train_index.tolist())]
-    return h, x, train_index, n_levels, args, dict(zip(("chain_ptr", "chain_pos", "chain_level"), table))
+    return h, x, train_index, n_levels, args, dict(zip(("chain_ptr", "chain_pos", "chain_level"), table)), bank_train
+
+
+def _oracle_logits(x, bank_train, train_index, n_nodes):
+    """The fp32 logits of the fused GEMM (bit-identical to ``hgr_logits_dense`` on the same inputs) at the train columns
+    of a ``[B, n_nodes]`` matrix; ``oracle.tor_por`` reads no other column."""
+    from hgrnet_b200 import ops
+    logits = torch.zeros(x.shape[0], n_nodes)
+    logits[:, train_index] = ops.logits_dense(x, bank_train).cpu()
+    return logits
+
+
+def _oracle_bin(logits, train_index, h, target):
+    """``oracle.tor_por`` of a single-label batch as the integers of bin L: ``[rows, TOR hits, points, edges]``."""
+    tor, path_add, point_add = orc.tor_por(logits, train_index, h.c2p, h.d2n, len(h), target)
+    L = len(h.c2p[target]) + 1
+    return torch.tensor([logits.shape[0], int(tor), round(point_add * L), round(path_add * max(L - 1, 1))])
+
+
+def _check_winners(logits, train_index, h, lvl, top1):
+    """Per-level winners and top-1 (train positions) against the oracle's arg-maxes; the chain of the last node (the
+    deepest level) covers every level."""
+    _, dict_path = orc.tor_por_winners(logits, train_index, h.c2p, h.d2n, len(h), len(h) - 1)
+    assert dict_path.shape[1] == lvl.shape[1]
+    assert torch.equal(train_index[lvl.cpu().long()], dict_path), "per-level winners differ"
+    assert torch.equal(train_index[top1.cpu().long()], train_index[logits[:, train_index].argmax(1)]), \
+        "top-1 over the train classes differs"
+
+
+_LEVELS6 = (6, 60, 600, 2400, 1500, 400)
+_LEVELS12 = (20, 150, 900, 3000, 5500, 5500, 3500, 1800, 900, 400, 120, 51)      # cfg 2: 21,841 nodes, 12 levels
+_LEVELS20 = tuple(1 + i // 2 for i in range(20))
+
+
+@pytest.mark.parametrize("levels,B,D,train_every", [((4, 20, 200), 64, 64, 1), ((4, 20, 200), 64, 128, 1),
+                                                    ((3, 9, 40, 160), 33, 64, 2), ((3, 9, 40, 160), 33, 128, 2),
+                                                    ((1, 5), 7, 64, 1), (_LEVELS20, 9, 64, 1), (_LEVELS20, 9, 128, 1),
+                                                    (_LEVELS6, 12, 128, 1), (_LEVELS6, 5, 64, 3),
+                                                    (_LEVELS6, 300, 256, 1), (_LEVELS12, 512, 1024, 1)])
+def test_hier_rows_match_oracle(levels, B, D, train_every):
+    """Single-label batches: bin L of the counters, the per-level winners and the top-1 equal the oracle's on the same
+    logits -- exact ties (duplicated bank rows, inside a level and across levels) included."""
+    from hgrnet_b200 import ops
+    h, x, train_index, n_levels, args, table, bank_train = _setup(levels, B, D, train_every)
+    N = len(h)
+    logits = _oracle_logits(x, bank_train, train_index, N)
+    for target in sorted({N - 1, 0, N // 2, min(7, N - 1)}):
+        L = len(h.c2p[target]) + 1
+        counts = ops.new_hier_counts(DEV)
+        lvl = torch.empty((B, n_levels), dtype=torch.int32, device=DEV)
+        top1 = torch.empty((B,), dtype=torch.int32, device=DEV)
+        ops.hier_metrics_fused_rows(x, targets=torch.full((B,), target, dtype=torch.int32, device=DEV), counts=counts,
+                                    lvl_idx=lvl, top1=top1, **args, **table)
+        want = torch.zeros_like(counts, device="cpu")
+        want[L] = _oracle_bin(logits, train_index, h, target)
+        assert torch.equal(counts.cpu(), want), (target, counts.cpu()[L], want[L])
+        _check_winners(logits, train_index, h, lvl, top1)
 
 
 def _mixed_targets(h, B, seed):
@@ -63,28 +122,23 @@ def _mixed_targets(h, B, seed):
 
 
 @pytest.mark.parametrize("levels,B,D,train_every", [((4, 20, 200), 64, 128, 1), ((3, 9, 40, 160), 33, 64, 2),
-                                                    (tuple(1 + i // 2 for i in range(20)), 40, 64, 1),
-                                                    ((20, 150, 900, 3000, 5500, 5500, 3500, 1800, 900, 400, 120, 51), 512, 1024, 1)])
-def test_rows_equal_per_label_calls(levels, B, D, train_every):
+                                                    (_LEVELS20, 40, 64, 1), (_LEVELS12, 512, 1024, 1)])
+def test_mixed_rows_match_oracle_per_label(levels, B, D, train_every):
+    """A batch that mixes labels (padding rows included): bin L holds the oracle's counts of each label's sub-batch."""
     from hgrnet_b200 import ops
-    h, x, train_index, n_levels, args, table = _setup(levels, B, D, train_every)
+    h, x, train_index, n_levels, args, table, bank_train = _setup(levels, B, D, train_every)
     N = len(h)
     targets = _mixed_targets(h, B, seed=B)
-    pos_of = {int(n): j for j, n in enumerate(train_index.tolist())}
     labels = sorted({int(t) for t in targets.tolist() if 0 <= t < N})
     assert len(labels) >= 5 and len({len(h.c2p[l]) for l in labels}) >= min(5, h.max_depth + 1)
     assert any(len(h.c2p[l]) == 0 for l in labels)
 
-    # expected: ops.hier_metrics_fused on each label's sub-batch, in bin L; the padded rows nowhere
+    # expected: the oracle on each label's sub-batch, in bin L; the padded rows nowhere
+    logits = _oracle_logits(x, bank_train, train_index, N)
     want = torch.zeros((ops.HGR_HIER_MAX_CHAIN + 1, 4), dtype=torch.int64)
     for lab in labels:
         rows = (targets == lab).nonzero().flatten()
-        parents = list(h.c2p[lab]) + [lab]
-        c = torch.zeros(3, dtype=torch.int64, device=DEV)
-        ops.hier_metrics_fused(x[rows.to(DEV)].contiguous(), args["bank_sorted"], args["level_end"], args["sorted_to_pos"],
-                               args["first_out"], torch.tensor([pos_of.get(p, -1) for p in parents], dtype=torch.int32, device=DEV),
-                               torch.tensor([len(h.c2p[p]) for p in parents], dtype=torch.int32, device=DEV), c)
-        want[len(parents)] += torch.cat([torch.tensor([rows.numel()]), c.cpu()])
+        want[len(h.c2p[lab]) + 1] += _oracle_bin(logits[rows], train_index, h, lab)
 
     t_dev = targets.to(DEV)
     got = ops.new_hier_counts(DEV)
@@ -94,13 +148,8 @@ def test_rows_equal_per_label_calls(levels, B, D, train_every):
     assert torch.equal(got.cpu(), want), (got.cpu()[got.cpu().any(1)], want[want.any(1)])
     assert int(want[:, 0].sum()) == B - 2
 
-    # per-level winners and top-1 do not depend on the labels: a single-label call on the full batch
-    lvl1 = torch.empty_like(lvl)
-    top11 = torch.empty_like(top1)
-    ops.hier_metrics_fused(x, args["bank_sorted"], args["level_end"], args["sorted_to_pos"], args["first_out"],
-                           torch.tensor([0], dtype=torch.int32, device=DEV), torch.tensor([0], dtype=torch.int32, device=DEV),
-                           torch.zeros(3, dtype=torch.int64, device=DEV), lvl_idx=lvl1, top1=top11)
-    assert torch.equal(lvl, lvl1) and torch.equal(top1, top11)
+    # per-level winners and top-1 do not depend on the labels: those of every row, padding included, are the oracle's
+    _check_winners(logits, train_index, h, lvl, top1)
 
     # the workspace came back zeroed: the same call again gives the same counters
     again = ops.new_hier_counts(DEV)
@@ -133,24 +182,30 @@ def _model(spec, tmp_path):
 
 
 @pytest.mark.parametrize("spec", cases.EVAL_CASES, ids=[s["name"] for s in cases.EVAL_CASES])
-def test_update_rows_reproduces_update_fused(spec, tmp_path):
+def test_update_rows_matches_oracle(spec, tmp_path):
+    """``HierMetrics.update_rows`` over single-label batches against the sum of the oracle's per-batch increments."""
     from hgrnet_b200 import ops
     from hgrnet_b200.evaluate import HierMetrics, _format
     model, h, test_ids = _model(spec, tmp_path)
-    hm_f, hm_r = HierMetrics(model), HierMetrics(model)
+    N = len(h)
+    train_index = model.train_index.cpu()
+    hm = HierMetrics(model)
     hits = ops.new_hits(DEV)
     n = 0
+    tor = path = point = 0.0
     for feats, label in cases.eval_batches(spec, test_ids):
         x = model.encode_image_normalized(feats.to(DEV))
         tg = torch.full((feats.shape[0],), label, dtype=torch.long, device=DEV)
         model.score_topk(None, tg, hits=hits, feats_normalized=x)
-        hm_f.update_fused(x, label)
-        hm_r.update_rows(x, tg)
+        hm.update_rows(x, tg)
+        a, b, c = orc.tor_por(_oracle_logits(x, model.bank_train, train_index, N), train_index, h.c2p, h.d2n, N, label)
+        tor, path, point = tor + a, path + b, point + c
         n += feats.shape[0]
-    assert hm_r.path_all_count == hm_f.path_all_count == n
-    for a, b in zip(hm_r.ratios(n), hm_f.ratios(n)):
-        assert abs(a - b) < 1e-9, (hm_r.ratios(n), hm_f.ratios(n))
-    assert _format(hits, n, hm_r) == _format(hits, n, hm_f)
+    want = (tor / n * 100.0, path / n * 100.0, point / n * 100.0)
+    assert hm.path_all_count == n
+    for a, b in zip(hm.ratios(n), want):
+        assert abs(a - b) < 1e-9, (hm.ratios(n), want)
+    assert _format(hits, n, hm) == _format(hits, n, types.SimpleNamespace(ratios=lambda _: want))
 
 
 def test_eval_stream_hier_matches_eager(tmp_path):
@@ -193,7 +248,7 @@ def test_eval_stream_hier_matches_eager(tmp_path):
 def test_hier_rows_rejects_bad_arguments():
     from hgrnet_b200 import _cabi, ops
     from hgrnet_b200._cabi import HgrError
-    h, x, train_index, n_levels, args, table = _setup((4, 20, 200), 64, 128, 1)
+    h, x, train_index, n_levels, args, table, _ = _setup((4, 20, 200), 64, 128, 1)
     t = _mixed_targets(h, 64, seed=1).to(DEV)
     counts = ops.new_hier_counts(DEV)
     lib = _cabi.load()

@@ -308,95 +308,3 @@ def test_masked_ce_matches_crossentropy(B, U, T):
     loss2, none = ops.masked_ce(logits.to(DEV), t(set_ptr), t(set_col), t(np.asarray(lps, np.int32)), t(weight),
                                 need_grad=False)
     assert none is None and torch.equal(loss2, loss)
-
-
-# ---------------------------------------------------------------------------------------------------------------
-# TOR / POR fused pass (hgr_hier_metrics) against the oracle's restatement of main.py:143,152-191
-@pytest.mark.parametrize("levels,B,train_every", [((4, 20, 200), 64, 1), ((3, 9, 40, 160), 33, 2), ((1, 5), 7, 1),
-                                                  (tuple(1 + i // 2 for i in range(20)), 9, 1),    # 20 levels: the 32-level variant
-                                                  ((6, 60, 600, 2400, 1500, 400), 12, 1),          # several passes of the column loop
-                                                  ((6, 60, 600, 2400, 1500, 400), 5, 3)])
-def test_hier_metrics_match_oracle(levels, B, train_every):
-    from hgrnet_b200 import ops
-    from hgrnet_b200.hierarchy import synthetic_hierarchy
-    from oracle import hgr_oracle as orc
-    h = synthetic_hierarchy(list(levels), seed=3)
-    N = len(h)
-    g = torch.Generator().manual_seed(11)
-    logits = torch.randn(B, N, generator=g).clamp_(-0.99, 0.99)
-    logits[:, 5] = logits[:, 3]                                       # exact ties between two columns
-    train_index = torch.arange(0, N, train_every)
-    depth = torch.from_numpy(h.depth).long()
-    n_levels = int(depth.max()) + 1
-    dt = depth[train_index]
-    first_out = torch.tensor([int((dt != l).nonzero()[0]) if (dt != l).any() else len(dt) for l in range(n_levels)],
-                             dtype=torch.int32, device=DEV)
-    for target in (N - 1, 0, N // 2):
-        parents = list(h.c2p[target]) + [target]
-        L = len(parents)
-        tor, path_add, point_add = orc.tor_por(logits, train_index, h.c2p, h.d2n, N, target)
-        counts = torch.zeros(3, dtype=torch.int64, device=DEV)
-        lvl = torch.empty((B, n_levels), dtype=torch.int32, device=DEV)
-        top1 = torch.empty((B,), dtype=torch.int32, device=DEV)
-        ops.hier_metrics(logits.to(DEV), train_index.int().to(DEV), depth.to(torch.int8).to(DEV), n_levels, first_out,
-                         torch.tensor(parents, dtype=torch.int32, device=DEV),
-                         torch.tensor([len(h.c2p[p]) for p in parents], dtype=torch.int32, device=DEV), counts,
-                         lvl_idx=lvl, top1=top1)
-        # position mode (evaluate.HierMetrics): logits of the train columns only, chain as train positions
-        pos_of = {int(n): j for j, n in enumerate(train_index.tolist())}
-        counts2 = torch.zeros(3, dtype=torch.int64, device=DEV)
-        ops.hier_metrics(logits[:, train_index].contiguous().to(DEV), None, dt.to(torch.int8).to(DEV), n_levels, first_out,
-                         torch.tensor([pos_of.get(p, -1) for p in parents], dtype=torch.int32, device=DEV),
-                         torch.tensor([len(h.c2p[p]) for p in parents], dtype=torch.int32, device=DEV), counts2)
-        assert counts2.tolist() == counts.tolist()
-        c = counts.tolist()
-        assert c[0] == int(tor)
-        assert abs((c[2] if L == 1 else c[2] / (L - 1)) - path_add) < 1e-9
-        assert abs(c[1] / L - point_add) < 1e-9
-        ref_top1 = train_index[logits[:, train_index].argmax(1)]
-        assert torch.equal(top1.cpu().long(), ref_top1)
-
-
-@pytest.mark.parametrize("levels,B,D,train_every", [((4, 20, 200), 64, 128, 1), ((3, 9, 40, 160), 33, 64, 2),
-                                                    ((6, 60, 600, 2400, 1500, 400), 300, 256, 1),
-                                                    (tuple(1 + i // 2 for i in range(20)), 9, 64, 1),
-                                                    ((20, 150, 900, 3000, 5500, 5500, 3500, 1800, 900, 400, 120, 51), 512, 1024, 1)])
-def test_hier_metrics_fused_matches_dense_pass(levels, B, D, train_every):
-    """TOR / POR without the dense matrix (hgr_hier_metrics_fused: per-level arg-max in the GEMM epilogue over the
-    level-sorted train bank, main.py:143,152-191) against the dense pass (hgr_logits_dense + hgr_hier_metrics), which is
-    itself pinned on the oracle above: same counters, same per-level winners, same top-1 -- exact ties (duplicated bank
-    rows, inside a level and across levels) included."""
-    from hgrnet_b200.hierarchy import synthetic_hierarchy
-    h = synthetic_hierarchy(list(levels), seed=3)
-    N = len(h)
-    bank = _emb(N, D, 21).to(torch.bfloat16)
-    bank[5] = bank[3]
-    bank[N - 2] = bank[N // 2]
-    bank[7] = bank[N - 1]                                       # a tie across two levels
-    x = ops.normalize_rows(_emb(B, D, 22, normalize=False).to(DEV))
-    train_index = torch.arange(0, N, train_every)
-    depth = torch.from_numpy(h.depth).long()
-    n_levels = int(depth.max()) + 1
-    dt = depth[train_index]
-    M = len(train_index)
-    first_out = torch.tensor([int((dt != l).nonzero()[0]) if (dt != l).any() else M for l in range(n_levels)],
-                             dtype=torch.int32, device=DEV)
-    bank_train = bank[train_index].to(DEV).contiguous()
-    order = torch.sort(dt, stable=True).indices
-    bank_sorted = bank_train[order.to(DEV)].contiguous()
-    level_end = torch.cumsum(torch.bincount(dt, minlength=n_levels), 0).tolist()
-    dense = ops.logits_dense(x, bank_train)
-    pos_of = {int(n): j for j, n in enumerate(train_index.tolist())}
-    for target in (N - 1, 0, N // 2, 7):
-        parents = list(h.c2p[target]) + [target]
-        chain = torch.tensor([pos_of.get(p, -1) for p in parents], dtype=torch.int32, device=DEV)
-        chain_level = torch.tensor([len(h.c2p[p]) for p in parents], dtype=torch.int32, device=DEV)
-        c1, c2 = torch.zeros(3, dtype=torch.int64, device=DEV), torch.zeros(3, dtype=torch.int64, device=DEV)
-        l1, l2 = (torch.empty((B, n_levels), dtype=torch.int32, device=DEV) for _ in range(2))
-        t1, t2 = (torch.empty((B,), dtype=torch.int32, device=DEV) for _ in range(2))
-        ops.hier_metrics(dense, None, dt.to(torch.int8).to(DEV), n_levels, first_out, chain, chain_level, c1, lvl_idx=l1, top1=t1)
-        ops.hier_metrics_fused(x, bank_sorted, level_end, order.to(torch.int32).to(DEV), first_out, chain, chain_level, c2,
-                               lvl_idx=l2, top1=t2)
-        assert torch.equal(l1, l2), "per-level winners differ"
-        assert torch.equal(t1, t2), "top-1 over the train classes differs"
-        assert c1.tolist() == c2.tolist()

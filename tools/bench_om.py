@@ -167,15 +167,16 @@ def main():
         "identity_bf16_in": {"us": us_id16, "bytes": b_id16, "GBs": b_id16 / us_id16 / 1e3, "frac": b_id16 / us_id16 / 1e3 / HBM},
         "chain_csr_bf16_in": {"us": us_ch, "nnz": nnz, "compulsory_bytes": b_ch, "GBs": b_ch / us_ch / 1e3,
                               "frac": b_ch / us_ch / 1e3 / HBM, "gathered_GBs": (nnz * D * 2 + N * D * 2) / us_ch / 1e3}}
-    # ---- row f1: TOR / POR pass at cfg-2 shape (B=512 rows of dense logits over 21,841 nodes, chain of 12)
+    # ---- row f1: TOR / POR at cfg-2 shape (B=512 rows against 21,841 nodes, chain of 12)
     from hgrnet_b200.evaluate import HierMetrics
     Bt = 512
     xt = ops.normalize_rows(synthetic_embeddings(Bt, D, 7, normalize=False).to(DEV))
     model.update_classifier()
     dense = ops.logits_dense(xt, model.bank_train)           # train columns only (here: every node is a train class)
     hm = HierMetrics(model)
+    tt = torch.full((Bt,), target, dtype=torch.int32, device=DEV)
     us_dense = graph_us(lambda i: ops.logits_dense(xt, model.bank_train, out=dense))
-    us_fused = events(lambda: hm.update(dense, target), 50)
+    us_fused = events(lambda: hm.update_rows(xt, tt), 50)
     parents = list(model.c2p[target]) + [target]
     depth_t = torch.from_numpy(hier.depth).to(DEV)
 
@@ -187,24 +188,19 @@ def main():
             lk = dense.detach().clone().index_fill(1, rest, -1)[:, model.train_index]
             _ = model.train_index[lk.topk(1, 1, True, True)[1]].squeeze()
     us_ref = events(reference_passes, 5)
-    kb = Bt * N * 4 + N * 5
-    ch_, cl_ = torch.zeros(12, dtype=torch.int32, device=DEV), torch.arange(12, dtype=torch.int32, device=DEV)
-    cnt_ = torch.zeros(3, dtype=torch.int64, device=DEV)
-    us_kernel = graph_us(lambda i: ops.hier_metrics(dense, None, hm._level, hm.n_levels, hm._first_out, ch_, cl_, cnt_))
-    # the same metrics WITHOUT the dense matrix: per-level arg-max in the GEMM epilogue over the level-sorted bank
-    hm.update_fused(xt, target)
-    us_nodense = graph_us(lambda i: ops.hier_metrics_fused(xt, hm._bank_sorted, hm._level_end, hm._sorted_to_pos, hm._first_out,
-                                                            ch_, cl_, cnt_))
+    # the metrics WITHOUT the dense matrix: per-level arg-max in the GEMM epilogue over the level-sorted bank
+    args, cnt_ = hm.rows_args(), ops.new_hier_counts(DEV)
+    us_nodense = graph_us(lambda i: ops.hier_metrics_fused_rows(xt, targets=tt, counts=cnt_, **args))
     out["hier_metrics_f1"] = {"B": Bt, "N": N, "L": len(parents), "us_kernel_plus_host_glue": us_fused,
-                              "us_fused_in_gemm_epilogue": us_nodense,
-                              "us_kernel_call": us_kernel, "kernel_bytes": kb, "kernel_GBs": kb / us_kernel / 1e3,
-                              "frac_hbm": kb / us_kernel / 1e3 / HBM, "us_dense_logits": us_dense,
+                              "us_fused_in_gemm_epilogue": us_nodense, "us_dense_logits": us_dense,
                               "us_reference_torch_passes_gpu": us_ref,
-                              "speedup_vs_torch_passes": us_ref / (us_fused + us_dense),
-                              "note": "reference = L+1 clone/index_fill/gather/topk passes over [B,N] (without its Python BxL loop)"}
+                              "speedup_vs_torch_passes": us_ref / us_fused,
+                              "note": "reference = L+1 clone/index_fill/gather/topk passes over [B,N] (without its Python "
+                                      "BxL loop and without the dense logits they read); ours = HierMetrics.update_rows "
+                                      "(GEMM + finish + totals)"}
     # ---- the same row with a REAL-SHAPED train split: 1,000 train classes + their ancestors (ImageNet-1K inside the
     # 21K hierarchy: ~1,900 of 21,841 nodes), test bank = all 21,841 nodes.  What `evaluate.test` runs per batch with
-    # the metrics on: fused top-20 head + dense logits over the TRAIN columns + hier_metrics, against the head alone.
+    # the metrics on: fused top-20 head + the per-level arg-max GEMM over the TRAIN rows, against the head alone.
     rs = np.random.RandomState(3)
     deep = [n for n in range(N) if hier.depth[n] >= 5]
     picked = set()
@@ -219,30 +215,18 @@ def main():
     tgt2 = sorted(picked)[-1]
     lab2 = torch.full((Bt,), tgt2, dtype=torch.int32, device=DEV)
     hits2 = ops.new_hits(DEV)
-    dense2 = ops.logits_dense(xt, m2.bank_train)
-    ch2 = torch.tensor([hm2._pos_of.get(p_, -1) for p_ in list(m2.c2p[tgt2]) + [tgt2]], dtype=torch.int32, device=DEV)
-    cl2 = torch.tensor([len(m2.c2p[p_]) for p_ in list(m2.c2p[tgt2]) + [tgt2]], dtype=torch.int32, device=DEV)
-    cnt2 = torch.zeros(3, dtype=torch.int64, device=DEV)
+    args2, cnt2 = hm2.rows_args(), ops.new_hier_counts(DEV)
     us_head = graph_us(lambda i: ops.score_topk(xt, m2.bank_test, col_id=m2._test_index_i32, targets=lab2, K=20, hits=hits2))
-
-    def with_metrics_dense(i):
-        ops.score_topk(xt, m2.bank_test, col_id=m2._test_index_i32, targets=lab2, K=20, hits=hits2)
-        ops.logits_dense(xt, m2.bank_train, out=dense2)
-        ops.hier_metrics(dense2, None, hm2._level, hm2.n_levels, hm2._first_out, ch2, cl2, cnt2)
-    us_with_dense = graph_us(with_metrics_dense)
-    hm2.update_fused(xt, tgt2)
 
     def with_metrics(i):
         ops.score_topk(xt, m2.bank_test, col_id=m2._test_index_i32, targets=lab2, K=20, hits=hits2)
-        ops.hier_metrics_fused(xt, hm2._bank_sorted, hm2._level_end, hm2._sorted_to_pos, hm2._first_out, ch2, cl2, cnt2)
+        ops.hier_metrics_fused_rows(xt, targets=lab2, counts=cnt2, **args2)
     us_with = graph_us(with_metrics)
     out["hier_metrics_f1_real_split"] = {
         "B": Bt, "test_classes": int(m2.bank_test.shape[0]), "train_columns": int(m2.bank_train.shape[0]),
         "us_head_alone": us_head, "us_head_plus_metrics": us_with, "ratio": us_with / us_head,
-        "us_head_plus_metrics_dense_pass": us_with_dense, "ratio_dense_pass": us_with_dense / us_head,
         "note": "kernels of one eval batch (one CUDA graph replay each, same bank every replay: L2-warm); metrics = "
-                "hgr_hier_metrics_fused (per-level arg-max in the GEMM epilogue over the train rows); dense pass = dense "
-                "logits over the train columns + hgr_hier_metrics"}
+                "hgr_hier_metrics_fused_rows (per-level arg-max in the GEMM epilogue over the train rows)"}
     print(json.dumps(out, indent=1))
 
 
