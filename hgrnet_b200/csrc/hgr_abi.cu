@@ -554,7 +554,14 @@ int hgr_masked_ce(const float* logits, int64_t ldl, int64_t B, int64_t U, const 
                   size_t workspace_bytes, void* stream) {
   HGR_CHECK_ARG(B > 0 && U > 0 && T >= 0, "hgr_masked_ce: bad sizes B=%lld U=%lld T=%lld", (long long)B, (long long)U, (long long)T);
   HGR_CHECK_ARG(ldl >= U, "hgr_masked_ce: ldl < U");
-  if (T == 0) return HGR_OK;
+  if (T == 0) {
+    // no set: the loss is empty and the gradient is zero everywhere, still overwritten as documented
+    if (dlogits)
+      HGR_CHECK_CUDA(cudaMemset2DAsync(dlogits, static_cast<size_t>(ldl) * sizeof(float), 0,
+                                       static_cast<size_t>(U) * sizeof(float), static_cast<size_t>(B),
+                                       static_cast<cudaStream_t>(stream)));
+    return HGR_OK;
+  }
   HGR_CHECK_ARG(logits && set_ptr && set_col && label_pos && weight && loss, "hgr_masked_ce: null pointer");
   return launch_masked_ce(logits, ldl, B, U, set_ptr, set_col, label_pos, weight, T, loss, dlogits, workspace,
                           workspace_bytes, static_cast<cudaStream_t>(stream));

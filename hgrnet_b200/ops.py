@@ -358,7 +358,9 @@ def peer_wait(flags_ptr: int, n: int, seq: torch.Tensor) -> None:
 
 def logits_dense(X: torch.Tensor, bank: torch.Tensor, scale: float = 1.0, impl: int = HGR_IMPL_AUTO,
                  out: Optional[torch.Tensor] = None) -> torch.Tensor:
-    """``scale * X @ bank.T`` in fp32 (model/clip_tree.py:331 / :263) on the tcgen05 main loop."""
+    """``scale * X @ bank.T`` in fp32 (model/clip_tree.py:331 / :263) on the tcgen05 main loop.
+    ``out`` (optional): fp32 ``[B, C]`` on X's device with unit column stride and, when B > 1, stride(0) >= C; its rows
+    may be further apart than C (a column slice of a wider buffer), the cells between them are left untouched."""
     lib = _cabi.load()
     X = _require(X, "X", torch.bfloat16)
     bank = _require(bank, "bank", torch.bfloat16)
@@ -366,8 +368,13 @@ def logits_dense(X: torch.Tensor, bank: torch.Tensor, scale: float = 1.0, impl: 
     C = bank.shape[0]
     if out is None:
         out = torch.empty((B, C), dtype=torch.float32, device=X.device)
-    _cabi.check(lib.hgr_logits_dense(_ptr(X), _ptr(bank), B, C, D, float(scale), _ptr(out), out.stride(0), impl,
-                                     _stream()))
+    elif out.dtype != torch.float32 or out.device != X.device or tuple(out.shape) != (B, C) or out.stride(1) != 1 \
+            or (B > 1 and out.stride(0) < C):
+        raise ValueError("out must be a float32 [%d, %d] tensor on %s with stride(1) == 1 and stride(0) >= %d, got %s %s "
+                         "on %s with strides %s" % (B, C, X.device, C, out.dtype, list(out.shape), out.device,
+                                                     list(out.stride())))
+    ldo = out.stride(0) if B > 1 else C        # one row: its stride is never used
+    _cabi.check(lib.hgr_logits_dense(_ptr(X), _ptr(bank), B, C, D, float(scale), _ptr(out), ldo, impl, _stream()))
     return out
 
 

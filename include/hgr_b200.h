@@ -345,7 +345,7 @@ int hgr_hier_finish_rows_gathered(const uint64_t* parts, int n_parts, int64_t pa
  *           of the positive inside its set (:139); weight [T] fp32 = w_in[m] * w_out[k] (:275)
  *  loss     [T] fp32: weight[t] * mean_b( logsumexp_j - logit_label )   (overwritten)
  *  dlogits  [B, U] fp32 (ld = ldl): sum_t weight[t]/B * (softmax_t - onehot_t), zero outside
- *           every set (overwritten); NULL to skip the backward.
+ *           every set (overwritten, all zero when T == 0); NULL to skip the backward.
  *  workspace at least hgr_masked_ce_workspace_bytes(B, U, T) bytes.
  */
 size_t hgr_masked_ce_workspace_bytes(int64_t B, int64_t U, int64_t T);

@@ -11,7 +11,7 @@ import pytest
 import torch
 
 from oracle import cases, hgr_oracle as orc
-from tests.util import bf16_input_atol, compare_topk, hits_from_idx
+from tests.util import bf16_input_atol, compare_topk, hits_from_idx, row_rel_err
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
@@ -129,6 +129,9 @@ def test_om_step_matches_reference_run(spec, tmp_path, golden, golden_dir):
     assert d_text[mask].abs().max() == 0                               # only sampled classes receive gradient
     assert rel(d_text[rows], torch.from_numpy(z["d_text"])) < 1e-2
     assert rel(img.grad.cpu(), torch.from_numpy(z["d_x"])) < 1e-2
+    # per row too: the global measure would pass with one sampled row lost
+    assert row_rel_err(d_text[rows], torch.from_numpy(z["d_text"])) < 1e-2
+    assert row_rel_err(img.grad.cpu(), torch.from_numpy(z["d_x"])) < 1e-2
     assert abs(float(enc.logit_scale.grad) - float(z["d_log_scale"])) <= 5e-3 * abs(float(z["d_log_scale"])) + 1e-6
     if o["weights"] == "adaptive":
         assert model.layer_weight.grad is not None and model.layer_weight.grad.abs().sum() > 0

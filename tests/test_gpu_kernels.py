@@ -55,7 +55,7 @@ def test_normalize_identity_matches_update_classifier(n, d, in_dtype):
     assert int((got16.cpu() != ref16).sum()) <= max(2, int(1e-3 * ref16.numel()))
 
 
-@pytest.mark.parametrize("d", [64, 1024])
+@pytest.mark.parametrize("d", [8, 64, 520, 1024, 2048, 2056, 4096])
 def test_aggregate_general_csr_and_row_map(d):
     n_src, n_rows = 500, 211
     rng = np.random.RandomState(3)
@@ -95,14 +95,23 @@ def test_aggregate_empty_and_errors():
 # --------------------------------------------------------------------------- dense logits
 @pytest.mark.parametrize("impl", ["simt", "tcgen05"])
 @pytest.mark.parametrize("B,C,D", [(64, 1000, 1024), (37, 313, 256), (1, 16, 64), (129, 4097, 520), (300, 777, 8),
-                                   (256, 257, 1024)])
+                                   (256, 257, 1024),
+                                   # the OM backward's GEMMs: M = U over 12-18 row tiles, N = D, K = B or U
+                                   (3000, 1024, 256), (4369, 1024, 264), (256, 1024, 3000), (1024, 2731, 1024)])
 def test_logits_dense_matches_forward(impl, B, C, D):
-    """`feats @ zsl_weights.T` (clip_tree.py:331) / scaled training logits (:263)."""
+    """`feats @ zsl_weights.T` (clip_tree.py:331) / scaled training logits (:263).  Also per element against float64:
+    the products of bf16 inputs are exact in fp32 and D of them are summed in fp32 (<= D 2^-24 of the absolute sum),
+    then scaled (2^-24); doubled, |got - ref| <= (D + 2) 2^-23 scale |x| @ |w|."""
     x, w = _emb(B, D, 1), _emb(C, D, 2)
     want = x @ w.T
+    ref = x.double() @ w.double().T
+    mag = x.double().abs() @ w.double().abs().T
     for scale in (1.0, 14.285714):
         got = ops.logits_dense(x.to(DEV).bfloat16(), w.to(DEV).bfloat16(), scale=scale, impl=IMPLS[impl])
         torch.testing.assert_close(got.cpu(), want * scale, rtol=1e-4, atol=2e-5)
+        err = (got.cpu().double() - scale * ref).abs()
+        bnd = (D + 2) * 2.0 ** -23 * scale * mag
+        assert (err <= bnd).all(), "%d elements outside the bound" % int((err > bnd).sum())
 
 
 # --------------------------------------------------------------------------- kernel (2)

@@ -62,6 +62,19 @@ def compare_topk(val, idx, oracle_logits, col_ids, K, rtol=LOGIT_RTOL, atol=LOGI
     return tie_rows
 
 
+def row_rel_err(got, ref):
+    """Largest per-row relative error ``|got_r - ref_r| / |ref_r|`` over the rows of ``ref`` that are not zero; a zero
+    row of ``ref`` must be zero in ``got`` too (inf otherwise).  A global Frobenius measure hides a lost row."""
+    got, ref = got.detach().cpu().double(), ref.detach().cpu().double()
+    rn = ref.norm(dim=1)
+    zero = rn == 0
+    if (got[zero] != 0).any():
+        return float("inf")
+    if not (~zero).any():
+        return 0.0
+    return float(((got - ref).norm(dim=1)[~zero] / rn[~zero]).max())
+
+
 def hits_from_idx(idx, targets, cuts=(1, 2, 5, 10, 20)):
     idx = idx.detach().cpu().long()
     targets = torch.as_tensor(targets).long().reshape(-1, 1)
