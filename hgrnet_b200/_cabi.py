@@ -21,6 +21,8 @@ HGR_IMPL_FLAG_NO_MERGE = 0x100
 HGR_NUM_HITS = 5
 HGR_TOPK_MAX = 32
 HGR_HIER_MAX_CHAIN = 32
+HGR_MAX_SPLITS = 8   # hgr_score_topk_splits: splits per call
+HGR_MAX_GROUPS = 16  # ... and groups of equal split membership
 HIT_CUTS = (1, 2, 5, 10, 20)  # main.py:120
 
 # every symbol include/hgr_b200.h declares: name -> (restype, argtypes)
@@ -63,6 +65,13 @@ SIGNATURES = {
     "hgr_hier_metrics_fused_rows": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int64, c_void_p, c_int, c_void_p,
                                             c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t,
                                             c_void_p, c_void_p, c_void_p, c_void_p]),
+    "hgr_score_topk_splits_workspace_bytes": (c_size_t, [c_int64, c_int64, c_int64, c_int, c_int, c_void_p]),
+    "hgr_score_topk_splits": (c_int, [c_void_p, c_void_p, c_void_p, c_int32, c_void_p, c_void_p, c_int64, c_int64, c_int64,
+                                      c_int64, c_float, c_int, c_int, c_void_p, c_void_p, c_int, c_void_p, c_size_t,
+                                      c_void_p, c_void_p, c_void_p, c_int, c_void_p]),
+    "hgr_hier_metrics_fused_rows_splits": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int64, c_void_p, c_int, c_void_p,
+                                                   c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_int,
+                                                   c_void_p, c_size_t, c_void_p, c_void_p]),
     "hgr_hier_level_scatter": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int64, c_void_p, c_int, c_int64, c_void_p,
                                        c_size_t, c_int64, c_int, c_void_p, c_void_p]),
     "hgr_hier_finish_rows_gathered": (c_int, [c_void_p, c_int, c_int64, c_int64, c_int64, c_int, c_void_p, c_void_p,

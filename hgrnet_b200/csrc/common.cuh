@@ -117,6 +117,34 @@ struct MergeArgs {
 };
 int launch_topk_merge(const MergeArgs& args, cudaStream_t stream);
 
+// Arguments of the per-split merge (hgr_score_topk_splits, topk_merge.cu): the scoring kernel's lists on the grouped
+// schedule, group_parts(mt) lists of length KL per row, list slot p of row tile mt covering the bank rows
+// group_slot_range(p) of one group.  Split s is the union of the groups g with bit s of group_splits[g].
+constexpr int kMaxSplits = 8;
+struct SplitMergeArgs {
+  const float* part_val;       // [slots][B][KL]
+  const int32_t* part_idx;     // [slots][B][KL] bank rows
+  int64_t B, C;
+  int KL, K, S;
+  Sched sched;
+  Groups groups;
+  uint8_t group_splits[kMaxGroups];
+  const int32_t* col_id;
+  int32_t id_base;
+  float scale;
+  const int32_t* targets;      // [B] node ids, or null
+  const uint8_t* node_splits;  // [n_nodes] split bits of every node
+  int64_t n_nodes;
+  float* topk_val;             // [S][B][K]
+  int32_t* topk_idx;           // [S][B][K] node ids
+  int64_t* counts;             // [S][HGR_NUM_HITS + 1]: Hit@{1,2,5,10,20}, rows; or null
+  const void* X;               // [B, D] bf16 -- exact re-scan only
+  const void* bank;            // [C, D] bf16
+  int D8;
+  unsigned int* rescan_count;  // (row, split) pairs re-scanned
+};
+int launch_topk_split_merge(const SplitMergeArgs& args, cudaStream_t stream);
+
 size_t simt_score_workspace_bytes(int64_t B, int64_t C, int K);
 int launch_score_topk_simt(const __nv_bfloat16* X, const __nv_bfloat16* bank, const int32_t* col_id,
                            int32_t id_base, const int32_t* targets, int64_t B, int64_t C, int64_t D,
@@ -137,6 +165,12 @@ int launch_score_topk_umma(const __nv_bfloat16* X, const __nv_bfloat16* bank, co
                            int32_t* topk_idx, int64_t* hits, int variant, bool skip_merge,
                            cudaStream_t stream, const OutScatter* scatter = nullptr, int64_t C_total = 0);
 int umma_global_list_len(int64_t B, int64_t C, int64_t D, int K, int64_t C_total);
+size_t umma_split_workspace_bytes(int64_t B, const Groups& gr, int K);
+int launch_score_topk_splits_umma(const __nv_bfloat16* X, const __nv_bfloat16* bank, const int32_t* col_id,
+                                  int32_t id_base, const int32_t* targets, const uint8_t* node_splits, int64_t n_nodes,
+                                  int64_t B, int64_t C, int64_t D, float scale, int K, const Groups& gr,
+                                  const uint8_t* group_splits, int S, void* ws, size_t ws_bytes, float* topk_val,
+                                  int32_t* topk_idx, int64_t* counts, bool exact, cudaStream_t stream);
 
 int launch_level_argmax_umma(const __nv_bfloat16* X, const __nv_bfloat16* bank_sorted, int64_t B, int64_t M, int64_t D,
                              const int32_t* level_end, int n_levels, unsigned long long* lvl_best, cudaStream_t stream);
@@ -152,6 +186,12 @@ int launch_hier_finish_gathered(const unsigned long long* parts, int n_parts, in
                                 const int32_t* targets, int64_t n_nodes, const int32_t* chain_ptr,
                                 const int32_t* chain_pos, const int32_t* chain_level, int32_t* lvl_idx, int32_t* top1,
                                 int64_t* counts, cudaStream_t stream);
+// hgr_hier_metrics_fused_rows_splits: counts [n_splits][HGR_HIER_MAX_CHAIN + 1][4], a row in every split of its label
+int launch_hier_finish_rows_splits(unsigned long long* lvl_best, int64_t B, int64_t M, int n_levels,
+                                   const int32_t* sorted_to_pos, const int32_t* first_out, const int32_t* targets,
+                                   int64_t n_nodes, const int32_t* chain_ptr, const int32_t* chain_pos,
+                                   const int32_t* chain_level, const uint8_t* node_splits, int n_splits,
+                                   int64_t* counts, cudaStream_t stream);
 int launch_normalize_dual(const void* E, int e_dtype, int64_t n_rows, int64_t D, void* out, const int32_t* dst_map,
                           void* out2, cudaStream_t stream);
 int launch_normalize_bcast(const void* E, int e_dtype, int64_t n_rows, int64_t D, int64_t row0, int n_dst,

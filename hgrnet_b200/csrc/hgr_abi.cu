@@ -134,6 +134,55 @@ static int score_topk_impl(const void* X, const void* bank, const int32_t* col_i
   return set_error(HGR_ERR_BAD_ARG, "hgr_score_topk: unknown impl %d", impl);
 }
 
+// main.py:104-222 run once per split (`--model_test` / `--data_test` = 2-hops, 3-hops, all): one GEMM over the union
+// bank, per split the top-K of main.py:136-138 and the hit / row counts of main.py:139-147.
+static int split_table(int64_t C, int n_groups, const int32_t* group_end, const uint8_t* group_splits, int n_splits,
+                       Groups* gr) {
+  HGR_CHECK_ARG(n_splits >= 1 && n_splits <= kMaxSplits, "hgr_score_topk_splits: %d splits outside [1, %d]", n_splits,
+                kMaxSplits);
+  HGR_CHECK_ARG(group_end != nullptr && group_splits != nullptr, "hgr_score_topk_splits: null group table");
+  HGR_CHECK_ARG(make_groups(C, n_groups, group_end, gr),
+                "hgr_score_topk_splits: %d groups: need 1..%d strictly ascending ends, the last = C = %lld", n_groups,
+                kMaxGroups, (long long)C);
+  for (int g = 0; g < n_groups; ++g)
+    HGR_CHECK_ARG(group_splits[g] < (1u << n_splits), "hgr_score_topk_splits: group %d names a split >= %d", g, n_splits);
+  return HGR_OK;
+}
+
+size_t hgr_score_topk_splits_workspace_bytes(int64_t B, int64_t C, int64_t D, int K, int n_groups, const int32_t* group_end) {
+  Groups gr;
+  if (B <= 0 || C <= 0 || K <= 0 || K > HGR_TOPK_MAX || group_end == nullptr || !make_groups(C, n_groups, group_end, &gr))
+    return 16;
+  return umma_split_workspace_bytes(B, gr, K) + 16;
+}
+
+int hgr_score_topk_splits(const void* X, const void* bank, const int32_t* col_id, int32_t id_base, const int32_t* targets,
+                          const uint8_t* node_splits, int64_t n_nodes, int64_t B, int64_t C, int64_t D, float scale, int K,
+                          int n_groups, const int32_t* group_end, const uint8_t* group_splits, int n_splits,
+                          void* workspace, size_t workspace_bytes, float* topk_val, int32_t* topk_idx, int64_t* counts,
+                          int impl, void* stream) {
+  HGR_CHECK_ARG(B >= 0 && C >= 1, "hgr_score_topk_splits: bad sizes B=%lld C=%lld", (long long)B, (long long)C);
+  HGR_CHECK_ARG(D > 0 && D % 8 == 0, "hgr_score_topk_splits: D = %lld must be a positive multiple of 8", (long long)D);
+  HGR_CHECK_ARG(K >= 1 && K <= HGR_TOPK_MAX, "hgr_score_topk_splits: K = %d outside [1, %d]", K, HGR_TOPK_MAX);
+  HGR_CHECK_ARG(scale > 0.f, "hgr_score_topk_splits: scale must be > 0 (top-k order is taken on unscaled cosines)");
+  Groups gr;
+  const int rc = split_table(C, n_groups, group_end, group_splits, n_splits, &gr);
+  if (rc != HGR_OK) return rc;
+  if (impl != HGR_IMPL_AUTO && impl != HGR_IMPL_TCGEN05 && impl != HGR_IMPL_TCGEN05_EXACT)
+    return set_error(HGR_ERR_UNSUPPORTED, "hgr_score_topk_splits: impl %d (only the tcgen05 kernel has the grouped schedule)",
+                     impl);
+  if (B == 0) return HGR_OK;
+  HGR_CHECK_ARG(X && bank && topk_val && topk_idx, "hgr_score_topk_splits: null X / bank / output");
+  HGR_CHECK_ARG(counts == nullptr || (targets && node_splits && n_nodes > 0),
+                "hgr_score_topk_splits: counting needs targets and node_splits");
+  HGR_CHECK_ARG(aligned16(X) && aligned16(bank) && aligned16(workspace), "hgr_score_topk_splits: X/bank/workspace must be 16-byte aligned");
+  if (!umma_supported(B, C, D, K)) return set_error(HGR_ERR_UNSUPPORTED, "hgr_score_topk_splits: shape not supported by the tcgen05 kernel");
+  return launch_score_topk_splits_umma(static_cast<const __nv_bfloat16*>(X), static_cast<const __nv_bfloat16*>(bank), col_id,
+                                       id_base, counts ? targets : nullptr, node_splits, n_nodes, B, C, D, scale, K, gr,
+                                       group_splits, n_splits, workspace, workspace_bytes, topk_val, topk_idx, counts,
+                                       impl == HGR_IMPL_TCGEN05_EXACT, static_cast<cudaStream_t>(stream));
+}
+
 int hgr_score_topk_plan(int64_t B, int64_t C, int64_t D, int K, int32_t* plan) {
   HGR_CHECK_ARG(plan != nullptr, "hgr_score_topk_plan: null plan");
   HGR_CHECK_ARG(K >= 1 && K <= HGR_TOPK_MAX, "hgr_score_topk_plan: K = %d outside [1, %d]", K, HGR_TOPK_MAX);
@@ -486,6 +535,41 @@ int hgr_hier_metrics_fused_rows(const void* X, const void* bank_sorted, int64_t 
   if (rc != HGR_OK) return rc;
   return launch_hier_finish_rows(best, B, M, n_levels, sorted_to_pos, first_out, targets, n_nodes, chain_ptr, chain_pos,
                                  chain_level, lvl_idx, top1, counts, s);
+}
+
+// main.py:143,152-191 run once per split: hgr_hier_metrics_fused_rows with the counters binned per split of the label.
+int hgr_hier_metrics_fused_rows_splits(const void* X, const void* bank_sorted, int64_t B, int64_t M, int64_t D,
+                                       const int32_t* level_end, int n_levels, const int32_t* sorted_to_pos,
+                                       const int32_t* first_out, const int32_t* targets, int64_t n_nodes,
+                                       const int32_t* chain_ptr, const int32_t* chain_pos, const int32_t* chain_level,
+                                       const uint8_t* node_splits, int n_splits, void* workspace, size_t workspace_bytes,
+                                       int64_t* counts, void* stream) {
+  HGR_CHECK_ARG(B >= 0 && M > 0 && M <= (int64_t(1) << 31) - 512, "hgr_hier_metrics_fused_rows_splits: bad sizes B=%lld M=%lld",
+                (long long)B, (long long)M);
+  HGR_CHECK_ARG(D > 0 && D % 8 == 0, "hgr_hier_metrics_fused_rows_splits: D = %lld must be a positive multiple of 8", (long long)D);
+  HGR_CHECK_ARG(n_nodes > 0 && n_nodes < (int64_t(1) << 31) - 1, "hgr_hier_metrics_fused_rows_splits: n_nodes = %lld",
+                (long long)n_nodes);
+  HGR_CHECK_ARG(n_levels >= 1 && n_levels <= 32, "hgr_hier_metrics_fused_rows_splits: %d levels outside [1, 32]", n_levels);
+  HGR_CHECK_ARG(n_splits >= 1 && n_splits <= kMaxSplits, "hgr_hier_metrics_fused_rows_splits: %d splits outside [1, %d]",
+                n_splits, kMaxSplits);
+  if (B == 0) return HGR_OK;
+  HGR_CHECK_ARG(X && bank_sorted && level_end && sorted_to_pos && first_out && targets && chain_ptr && chain_pos &&
+                    chain_level && node_splits && counts && workspace,
+                "hgr_hier_metrics_fused_rows_splits: null pointer");
+  HGR_CHECK_ARG(aligned16(X) && aligned16(bank_sorted) && aligned16(workspace),
+                "hgr_hier_metrics_fused_rows_splits: X / bank / workspace must be 16-byte aligned");
+  HGR_CHECK_ARG(workspace_bytes >= static_cast<size_t>(B) * n_levels * 8,
+                "hgr_hier_metrics_fused_rows_splits: workspace %zu < %zu bytes", workspace_bytes,
+                static_cast<size_t>(B) * n_levels * 8);
+  if (!umma_supported(B, M, D, 1))
+    return set_error(HGR_ERR_UNSUPPORTED, "hgr_hier_metrics_fused_rows_splits: shape not supported by the tcgen05 kernel");
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  unsigned long long* best = static_cast<unsigned long long*>(workspace);
+  const int rc = launch_level_argmax_umma(static_cast<const __nv_bfloat16*>(X), static_cast<const __nv_bfloat16*>(bank_sorted), B, M,
+                                          D, level_end, n_levels, best, s);
+  if (rc != HGR_OK) return rc;
+  return launch_hier_finish_rows_splits(best, B, M, n_levels, sorted_to_pos, first_out, targets, n_nodes, chain_ptr,
+                                        chain_pos, chain_level, node_splits, n_splits, counts, s);
 }
 
 int hgr_hier_level_scatter(const void* X, const void* bank_shard, int64_t B, int64_t M_r, int64_t D,

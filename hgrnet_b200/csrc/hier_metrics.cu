@@ -109,7 +109,9 @@ __device__ __forceinline__ RowCounts finish_row(const Words& words, int64_t row,
 constexpr int kRowsPerBlock = 8;
 constexpr int kHistWords = (HGR_HIER_MAX_CHAIN + 1) * 4;
 
-template <class Words>
+// kSplits (hgr_hier_metrics_fused_rows_splits): counter set s ([s][kHistWords]) takes the rows whose label has bit s in
+// node_splits -- a row in several splits is added to each of them.
+template <class Words, bool kSplits = false>
 __device__ __forceinline__ void finish_rows_block(const Words& words, int64_t B, int64_t M, int n_levels,
                                                   const int32_t* __restrict__ sorted_to_pos,
                                                   const int32_t* __restrict__ first_out,
@@ -117,9 +119,11 @@ __device__ __forceinline__ void finish_rows_block(const Words& words, int64_t B,
                                                   const int32_t* __restrict__ chain_ptr,
                                                   const int32_t* __restrict__ chain_pos,
                                                   const int32_t* __restrict__ chain_level, int32_t* __restrict__ lvl_idx,
-                                                  int32_t* __restrict__ top1, unsigned long long* counts) {
-  __shared__ unsigned int s_cnt[kHistWords];      // <= kRowsPerBlock * HGR_HIER_MAX_CHAIN per word: 32 bits suffice
-  for (int i = threadIdx.x; i < kHistWords; i += blockDim.x) s_cnt[i] = 0u;
+                                                  int32_t* __restrict__ top1, unsigned long long* counts,
+                                                  const uint8_t* __restrict__ node_splits = nullptr, int n_splits = 1) {
+  constexpr int kSets = kSplits ? kMaxSplits : 1;
+  __shared__ unsigned int s_cnt[kSets * kHistWords];   // <= kRowsPerBlock * HGR_HIER_MAX_CHAIN per word: 32 bits suffice
+  for (int i = threadIdx.x; i < kSets * kHistWords; i += blockDim.x) s_cnt[i] = 0u;
   __syncthreads();
   const int lane = threadIdx.x & 31;
   const int64_t row = static_cast<int64_t>(blockIdx.x) * kRowsPerBlock + (threadIdx.x >> 5);
@@ -141,15 +145,19 @@ __device__ __forceinline__ void finish_rows_block(const Words& words, int64_t B,
     const RowCounts c = finish_row(words, row, lane, M, n_levels, sorted_to_pos, first_out, chain_pos + c0,
                                    chain_level + c0, L, lvl_idx, top1);
     if (lane == 0 && L > 0) {
-      unsigned int* bin = s_cnt + 4 * L;
-      atomicAdd(bin + 0, 1u);
-      if (c.tor) atomicAdd(bin + 1, static_cast<unsigned int>(c.tor));
-      if (c.point) atomicAdd(bin + 2, static_cast<unsigned int>(c.point));
-      if (c.edge) atomicAdd(bin + 3, static_cast<unsigned int>(c.edge));
+      const unsigned bits = kSplits ? node_splits[targets[row]] : 1u;   // L > 0: the target is a node
+      for (int sp = 0; sp < kSets; ++sp) {
+        if (!((bits >> sp) & 1u)) continue;
+        unsigned int* bin = s_cnt + sp * kHistWords + 4 * L;
+        atomicAdd(bin + 0, 1u);
+        if (c.tor) atomicAdd(bin + 1, static_cast<unsigned int>(c.tor));
+        if (c.point) atomicAdd(bin + 2, static_cast<unsigned int>(c.point));
+        if (c.edge) atomicAdd(bin + 3, static_cast<unsigned int>(c.edge));
+      }
     }
   }
   __syncthreads();
-  for (int i = threadIdx.x; i < kHistWords; i += blockDim.x)
+  for (int i = threadIdx.x; i < (kSplits ? n_splits : 1) * kHistWords; i += blockDim.x)
     if (s_cnt[i]) atomicAdd(counts + i, static_cast<unsigned long long>(s_cnt[i]));
 }
 
@@ -161,6 +169,17 @@ hier_finish_rows_kernel(unsigned long long* __restrict__ lvl_best, int64_t B, in
                         int32_t* __restrict__ lvl_idx, int32_t* __restrict__ top1, unsigned long long* counts) {
   finish_rows_block(WsWords{lvl_best}, B, M, n_levels, sorted_to_pos, first_out, targets, n_nodes, chain_ptr, chain_pos,
                     chain_level, lvl_idx, top1, counts);
+}
+
+__global__ void __launch_bounds__(kRowsPerBlock * 32)
+hier_finish_rows_splits_kernel(unsigned long long* __restrict__ lvl_best, int64_t B, int64_t M, int n_levels,
+                               const int32_t* __restrict__ sorted_to_pos, const int32_t* __restrict__ first_out,
+                               const int32_t* __restrict__ targets, int64_t n_nodes,
+                               const int32_t* __restrict__ chain_ptr, const int32_t* __restrict__ chain_pos,
+                               const int32_t* __restrict__ chain_level, const uint8_t* __restrict__ node_splits,
+                               int n_splits, unsigned long long* counts) {
+  finish_rows_block<WsWords, true>(WsWords{lvl_best}, B, M, n_levels, sorted_to_pos, first_out, targets, n_nodes,
+                                   chain_ptr, chain_pos, chain_level, nullptr, nullptr, counts, node_splits, n_splits);
 }
 
 // ---- class-sharded form (hgr_hier_level_scatter / hgr_hier_finish_rows_gathered) -------------------------------------
@@ -255,6 +274,22 @@ int launch_hier_finish_rows(unsigned long long* lvl_best, int64_t B, int64_t M, 
   hier_finish_rows_kernel<<<blocks, kRowsPerBlock * 32, 0, stream>>>(
       lvl_best, B, M, n_levels, sorted_to_pos, first_out, targets, n_nodes, chain_ptr, chain_pos, chain_level, lvl_idx,
       top1, reinterpret_cast<unsigned long long*>(counts));
+  HGR_CHECK_LAUNCH();
+  return HGR_OK;
+}
+
+int launch_hier_finish_rows_splits(unsigned long long* lvl_best, int64_t B, int64_t M, int n_levels,
+                                   const int32_t* sorted_to_pos, const int32_t* first_out, const int32_t* targets,
+                                   int64_t n_nodes, const int32_t* chain_ptr, const int32_t* chain_pos,
+                                   const int32_t* chain_level, const uint8_t* node_splits, int n_splits,
+                                   int64_t* counts, cudaStream_t stream) {
+  if (n_levels < 1 || n_levels > kMaxLevels)
+    return set_error(HGR_ERR_UNSUPPORTED, "hgr_hier_metrics_fused_rows_splits: %d levels outside [1, %d]", n_levels,
+                     kMaxLevels);
+  const int blocks = static_cast<int>((B + kRowsPerBlock - 1) / kRowsPerBlock);     // one warp per image row
+  hier_finish_rows_splits_kernel<<<blocks, kRowsPerBlock * 32, 0, stream>>>(
+      lvl_best, B, M, n_levels, sorted_to_pos, first_out, targets, n_nodes, chain_ptr, chain_pos, chain_level,
+      node_splits, n_splits, reinterpret_cast<unsigned long long*>(counts));
   HGR_CHECK_LAUNCH();
   return HGR_OK;
 }

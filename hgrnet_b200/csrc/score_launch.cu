@@ -8,6 +8,8 @@
 
 #include <cmath>
 #include <cstdlib>
+#include <cstring>
+#include <mutex>
 
 #include "sketch_epi.cuh"
 #include "umma_common.cuh"
@@ -280,6 +282,150 @@ int launch_score_topk_umma(const __nv_bfloat16* X, const __nv_bfloat16* bank, co
   m.C = C;
   if (scatter) m.scatter = *scatter;
   return launch_topk_merge(m, stream);
+}
+
+// ---- several test splits in one pass (hgr_score_topk_splits) --------------------------------------------------------
+// Grouped schedule over all workers (sched.cuh): no list crosses a group, so split s is served by the lists of its
+// groups alone.  The list length comes from the split that is worst off: for split s a list holds at most `cols_s` of
+// its C_s columns (share_s = cols_s / C_s), and each row has `lists_s` lists of s; the narrowest length whose expected
+// repair time stays below 1.5 % of the call (the rule of pick_list_len, the call being the GEMM over all C columns)
+// for EVERY split is taken -- so a small split covered by a few long lists per row does not get repaired on every row.
+
+static int pick_list_len_splits(int K, int64_t B, int64_t C, int64_t D, const Sched& s, const Groups& gr,
+                                const uint8_t* group_splits, int S) {
+  const int exact = K <= 8 ? 8 : (K <= 12 ? 12 : (K <= 20 ? 20 : 32));
+  int64_t cs[kMaxSplits] = {}, cols[kMaxSplits] = {};
+  int lists[kMaxSplits] = {};
+  for (int g = 0; g < gr.n; ++g)
+    for (int sp = 0; sp < S; ++sp)
+      if ((group_splits[g] >> sp) & 1u) cs[sp] += gr.end[g] - gr.begin(g);
+  for (int32_t mt = 0; mt < s.MT; ++mt) {
+    int n[kMaxSplits] = {};
+    const int parts = group_parts(s, gr, mt);
+    for (int p = 0; p < parts; ++p) {
+      int64_t c0, c1;
+      const int g = group_slot_range(s, gr, mt, p, c0, c1);
+      for (int sp = 0; sp < S; ++sp) {
+        if (!((group_splits[g] >> sp) & 1u)) continue;
+        ++n[sp];
+        cols[sp] = c1 - c0 > cols[sp] ? c1 - c0 : cols[sp];
+      }
+    }
+    for (int sp = 0; sp < S; ++sp) lists[sp] = n[sp] > lists[sp] ? n[sp] : lists[sp];
+  }
+  const double t_call = 2.0 * static_cast<double>(B) * static_cast<double>(C) * static_cast<double>(D) / (0.6 * 1.6e15);
+  const int cand[4] = {8, 10, 12, 16};
+  for (int i = 0; i < 4; ++i) {
+    const int kl = cand[i];
+    if (kl >= K) break;
+    bool ok = true;
+    for (int sp = 0; sp < S && ok; ++sp) {
+      if (cs[sp] == 0) continue;
+      const double share = static_cast<double>(cols[sp]) / static_cast<double>(cs[sp]);
+      const double repairs = static_cast<double>(B) * lists[sp] * overflow_bound(K, kl, share);
+      const double t_repair = static_cast<double>(cols[sp]) * (static_cast<double>(D) / 1024.0) * 0.6e-6;
+      ok = repairs * t_repair < 0.015 * t_call;
+    }
+    if (ok) return kl;
+  }
+  return exact;
+}
+
+// The schedule and the list length of a call depend only on (B, C, D, K, group table, split bits) and visit every
+// (row tile, slot): eager callers (evaluate.test, SplitEval.update) make the same call every batch, so the last few
+// plans are kept.
+struct SplitPlan {
+  int64_t B = -1, C = -1, D = -1;
+  int K = 0, S = 0;
+  bool exact = false;
+  Groups gr{};
+  uint8_t splits[kMaxGroups] = {};
+  Sched sched{};
+  int KL = 0;
+};
+
+static SplitPlan split_plan(int64_t B, int64_t C, int64_t D, int K, const Groups& gr, const uint8_t* group_splits, int S,
+                            bool exact) {
+  constexpr int kSlots = 8;
+  static SplitPlan cache[kSlots];
+  static int next = 0;
+  static std::mutex mu;
+  SplitPlan key;
+  key.B = B, key.C = C, key.D = D, key.K = K, key.S = S, key.exact = exact;
+  key.gr = gr;
+  for (int g = 0; g < gr.n && group_splits; ++g) key.splits[g] = group_splits[g];
+  auto same = [&](const SplitPlan& e) {
+    return e.B == key.B && e.C == key.C && e.D == key.D && e.K == key.K && e.S == key.S && e.exact == key.exact &&
+           std::memcmp(&e.gr, &key.gr, sizeof(Groups)) == 0 && std::memcmp(e.splits, key.splits, kMaxGroups) == 0;
+  };
+  {
+    std::lock_guard<std::mutex> lk(mu);
+    for (const SplitPlan& e : cache)
+      if (same(e)) return e;
+  }
+  key.sched = make_sched_groups(B, gr, usable_sms() / 2, 2 * kTileM);
+  const int exact_kl = K <= 8 ? 8 : (K <= 12 ? 12 : (K <= 20 ? 20 : 32));
+  key.KL = exact || group_splits == nullptr ? exact_kl : pick_list_len_splits(K, B, C, D, key.sched, gr, group_splits, S);
+  std::lock_guard<std::mutex> lk(mu);
+  cache[next] = key;
+  next = (next + 1) % kSlots;
+  return key;
+}
+
+size_t umma_split_workspace_bytes(int64_t B, const Groups& gr, int K) {
+  // sized for exact lists: the plan without split bits (the list length does not change the schedule)
+  const SplitPlan plan = split_plan(B, gr.end[gr.n - 1], 0, K, gr, nullptr, 0, true);
+  return static_cast<size_t>(plan.sched.P) * B * plan.KL * (sizeof(float) + sizeof(int32_t)) + kWsHeaderBytes;
+}
+
+int launch_score_topk_splits_umma(const __nv_bfloat16* X, const __nv_bfloat16* bank, const int32_t* col_id,
+                                  int32_t id_base, const int32_t* targets, const uint8_t* node_splits, int64_t n_nodes,
+                                  int64_t B, int64_t C, int64_t D, float scale, int K, const Groups& gr,
+                                  const uint8_t* group_splits, int S, void* ws, size_t ws_bytes, float* topk_val,
+                                  int32_t* topk_idx, int64_t* counts, bool exact, cudaStream_t stream) {
+  if (ws == nullptr || ws_bytes < umma_split_workspace_bytes(B, gr, K))
+    return set_error(HGR_ERR_WORKSPACE, "hgr_score_topk_splits: workspace %zu < %zu bytes", ws_bytes,
+                     umma_split_workspace_bytes(B, gr, K));
+  CUtensorMap mx, mb;
+  Params p{};
+  int rc = common_setup(X, bank, B, C, D, &mx, &mb, &p);
+  if (rc != HGR_OK) return rc;
+  const SplitPlan plan = split_plan(B, C, D, K, gr, group_splits, S, exact);
+  p.sched = plan.sched;
+  p.groups = gr;
+  p.scale = scale;
+  p.stats = static_cast<unsigned int*>(ws);
+  const int KL = plan.KL;
+  p.KL = KL;
+  p.part_val = reinterpret_cast<float*>(static_cast<uint8_t*>(ws) + kWsHeaderBytes);
+  p.part_idx = reinterpret_cast<int32_t*>(p.part_val + static_cast<size_t>(p.sched.P) * B * KL);
+  rc = launch_pair_kernel(kEpiTopkGroups, KL, mx, mb, p, stream);
+  if (rc != HGR_OK) return rc;
+  SplitMergeArgs m{};
+  m.part_val = p.part_val;
+  m.part_idx = p.part_idx;
+  m.B = B;
+  m.C = C;
+  m.KL = KL;
+  m.K = K;
+  m.S = S;
+  m.sched = p.sched;
+  m.groups = gr;
+  for (int g = 0; g < gr.n; ++g) m.group_splits[g] = group_splits[g];
+  m.col_id = col_id;
+  m.id_base = id_base;
+  m.scale = scale;
+  m.targets = targets;
+  m.node_splits = node_splits;
+  m.n_nodes = n_nodes;
+  m.topk_val = topk_val;
+  m.topk_idx = topk_idx;
+  m.counts = counts;
+  m.X = X;
+  m.bank = bank;
+  m.D8 = static_cast<int>(D / 8);
+  m.rescan_count = p.stats;
+  return launch_topk_split_merge(m, stream);
 }
 
 // Row f1 without the dense matrix: X . bank_sorted^T on the tcgen05 loop, per-level arg-max in the epilogue.

@@ -42,12 +42,13 @@ struct PairCtl {
 // its launcher (threads, dynamic shared memory, opt-in limit).
 template <int EPI>
 struct EpiRes {
-  static constexpr bool kQueue = EPI == kEpiTopkDefer || EPI == kEpiSketch;   // a candidate queue per thread
+  static constexpr bool kTopk = EPI == kEpiTopkDefer || EPI == kEpiTopkGroups;
+  static constexpr bool kQueue = kTopk || EPI == kEpiSketch;   // a candidate queue per thread
   // one warp per TMEM lane quarter; the dense epilogue has two, which take alternate chunks of every sub-tile
   static constexpr int kWarps = EPI == kEpiDense ? 8 : 4;
   static constexpr int kThreads = 64 + 32 * kWarps;           // + the TMA and the MMA warp
   static constexpr int kStagingBytes = EPI == kEpiSketch ? kSkQueueBytes
-                                     : EPI == kEpiTopkDefer ? (kDeferQueue + 1) * kDeferStride
+                                     : kTopk ? (kDeferQueue + 1) * kDeferStride
                                      : EPI == kEpiDense ? kWarps * kDenseTileFloats * 4 : 0;
   // Operand stages: as many 32 KB stages as fit beside the staging memory (measured: 4 stages cost ~2 us of main loop
   // at cfg 2, and leaving room for co-resident small kernels bought nothing).
@@ -65,12 +66,27 @@ struct EpiRes {
 static_assert(EpiRes<kEpiSketch>::kWarps * 32 * 8 == kSkStride &&
               EpiRes<kEpiTopkDefer>::kWarps * 32 * 8 == kDeferStride, "queue stride = one entry per epilogue thread");
 
+// The walk of a worker over its chunk: the plain schedule, or the grouped one (kEpiTopkGroups).
+template <bool kGroups>
+struct WalkerOf {
+  using type = TileWalker;
+  __device__ __forceinline__ static TileWalker make(const Params& p, int pair) { return TileWalker(p.sched, pair, p.C); }
+};
+template <>
+struct WalkerOf<true> {
+  using type = GroupWalker;
+  __device__ __forceinline__ static GroupWalker make(const Params& p, int pair) {
+    return GroupWalker(p.sched, pair, p.groups);
+  }
+};
+
 // TMA producer (warp 0 of both CTAs; convergent warp, elected issue -- see ptx.cuh): per K block this CTA's 128 image
 // rows and its half of the bank sub-tile, both signalled on the LEADER's `full` barrier.
+template <bool kGroups>
 __device__ __forceinline__ void produce(const CUtensorMap* map_x, const CUtensorMap* map_bank, const Params& p,
                                         PairCtl* ctl, uint8_t* stage_base, uint32_t rank, int pair) {
   const uint64_t pol = ptx::policy_evict_last();
-  TileWalker walk(p.sched, pair, p.C);
+  auto walk = WalkerOf<kGroups>::make(p, pair);
   SubTile t;
   int stage = 0;
   uint32_t phase = 0;
@@ -101,9 +117,10 @@ __device__ __forceinline__ void produce(const CUtensorMap* map_x, const CUtensor
 
 // MMA issuer (warp 1 of the leader CTA; convergent warp, elected issue): M = 256 over both CTAs, accumulators
 // alternate between the two TMEM buffers.
+template <bool kGroups>
 __device__ __forceinline__ void issue_mma(const Params& p, PairCtl* ctl, uint8_t* stage_base, uint32_t tmem_base,
                                           int pair, int lane) {
-  TileWalker walk(p.sched, pair, p.C);
+  auto walk = WalkerOf<kGroups>::make(p, pair);
   SubTile t;
   int stage = 0;
   uint32_t phase = 0;
@@ -266,10 +283,11 @@ __device__ __forceinline__ void epi_null(const Params& p, const EpiWarp& w) {
 // ===================== epilogue: deferred-insert top-K lists (production; umma_common.cuh) =====================
 // A sorted register list per row.  Every sub-tile is filtered against a threshold fixed for the sub-tile into the
 // thread's candidate queue; the queue is drained into the list once the accumulator buffer is back with the tensor core.
-template <int KL>
+// kGroups: on the grouped schedule -- only the walk and the list slot differ.
+template <int KL, bool kGroups>
 __device__ __forceinline__ void epi_topk_defer(const Params& p, const EpiWarp& w, float* staging) {
   const int epi_tid = w.epi_tid();
-  TileWalker walk(p.sched, w.pair, p.C);
+  auto walk = WalkerOf<kGroups>::make(p, w.pair);
   SubTile t;
   SortedList<KL> list;
   list.init();
@@ -337,8 +355,13 @@ __device__ __forceinline__ void epi_topk_defer(const Params& p, const EpiWarp& w
     ck.lap(ck.drain);
     if (epi_tid == 0 && it < 4) stamp(p, 8 + it);   // this warp is done with sub-tile `it`
     if (t.last && row < p.B) {
-      float* pv = p.part_val + list_offset(p, w.pair, t.mt, row);
-      int32_t* pi = p.part_idx + list_offset(p, w.pair, t.mt, row);
+      int64_t li;
+      if constexpr (kGroups)
+        li = (static_cast<int64_t>(group_slot(p.sched, p.groups, t.mt, walk.unit_of(t), t.group)) * p.B + row) * p.KL;
+      else
+        li = list_offset(p, w.pair, t.mt, row);
+      float* pv = p.part_val + li;
+      int32_t* pi = p.part_idx + li;
 #pragma unroll
       for (int k = 0; k < KL; ++k) {
         if (k < p.KL) {
@@ -607,15 +630,17 @@ score_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_c
   const uint32_t tmem_base = ctl->tmem_base;
   if (threadIdx.x == 0) stamp(p, 1);  // set-up done (barriers, TMEM, cluster sync)
 
+  constexpr bool kGroups = EPI == kEpiTopkGroups;
   if (warp == 0) {
-    produce(&map_x, &map_bank, p, ctl, smem, rank, pair);
+    produce<kGroups>(&map_x, &map_bank, p, ctl, smem, rank, pair);
   } else if (warp == 1) {
-    if (rank == 0) issue_mma(p, ctl, smem, tmem_base, pair, lane);   // the leader's MMAs cover both CTAs
+    if (rank == 0) issue_mma<kGroups>(p, ctl, smem, tmem_base, pair, lane);   // the leader's MMAs cover both CTAs
   } else {
     const EpiWarp w{ctl, tmem_base, rank, pair, warp, lane};
     if constexpr (EPI == kEpiDense) epi_dense(p, w, staging);
     else if constexpr (EPI == kEpiNull) epi_null(p, w);
-    else if constexpr (EPI == kEpiTopkDefer) epi_topk_defer<KL>(p, w, staging);
+    else if constexpr (EPI == kEpiTopkDefer) epi_topk_defer<KL, false>(p, w, staging);
+    else if constexpr (EPI == kEpiTopkGroups) epi_topk_defer<KL, true>(p, w, staging);
     else if constexpr (EPI == kEpiSketch) epi_sketch(p, w, staging);
     else epi_level(p, w);
   }
@@ -658,6 +683,19 @@ int launch_one(const CUtensorMap& mx, const CUtensorMap& mb, const Params& p, cu
 
 int pair_ring_depth(int64_t B) { return EpiRes<kEpiTopkDefer>::stages(B); }
 
+template <int EPI>
+int launch_topk(int KL, const CUtensorMap& mx, const CUtensorMap& mb, const Params& p, cudaStream_t stream) {
+  switch (KL) {
+    case 8: return launch_one<EPI, 8>(mx, mb, p, stream);
+    case 10: return launch_one<EPI, 10>(mx, mb, p, stream);
+    case 12: return launch_one<EPI, 12>(mx, mb, p, stream);
+    case 16: return launch_one<EPI, 16>(mx, mb, p, stream);
+    case 20: return launch_one<EPI, 20>(mx, mb, p, stream);
+    case 32: return launch_one<EPI, 32>(mx, mb, p, stream);
+  }
+  return set_error(HGR_ERR_UNSUPPORTED, "hgr_score_topk(tcgen05): list length %d", KL);
+}
+
 // Epilogue arrangement of the top-K kernels: ONE warp per TMEM lane quarter, one list per row, inserts deferred off the
 // tensor core's critical path (measured against two warps per quarter with in-place inserts: exact 20-entry lists at
 // B = 4096 40 / 57 / 87 / 154 us against 46 / 66 / 98 / 164 us).  The dense epilogue uses two warps per quarter.
@@ -667,15 +705,8 @@ int launch_pair_kernel(int epi, int KL, const CUtensorMap& mx, const CUtensorMap
   if (epi == kEpiNull) return launch_one<kEpiNull, 8>(mx, mb, p, stream);
   if (epi == kEpiSketch) return launch_one<kEpiSketch, 8>(mx, mb, p, stream);
   if (epi == kEpiLevel) return launch_one<kEpiLevel, 8>(mx, mb, p, stream);
-  switch (KL) {
-    case 8: return launch_one<kEpiTopkDefer, 8>(mx, mb, p, stream);
-    case 10: return launch_one<kEpiTopkDefer, 10>(mx, mb, p, stream);
-    case 12: return launch_one<kEpiTopkDefer, 12>(mx, mb, p, stream);
-    case 16: return launch_one<kEpiTopkDefer, 16>(mx, mb, p, stream);
-    case 20: return launch_one<kEpiTopkDefer, 20>(mx, mb, p, stream);
-    case 32: return launch_one<kEpiTopkDefer, 32>(mx, mb, p, stream);
-  }
-  return set_error(HGR_ERR_UNSUPPORTED, "hgr_score_topk(tcgen05): list length %d", KL);
+  if (epi == kEpiTopkGroups) return launch_topk<kEpiTopkGroups>(KL, mx, mb, p, stream);
+  return launch_topk<kEpiTopkDefer>(KL, mx, mb, p, stream);
 }
 
 }  // namespace umma

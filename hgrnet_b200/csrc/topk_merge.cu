@@ -684,6 +684,203 @@ topk_merge_counts_kernel(const __grid_constant__ MergeArgs a) {
   flush_hits(a, s_hits, threadIdx.x);
 }
 
+// ---- per-split merge (hgr_score_topk_splits) --------------------------------------------------------------------
+// The lists of a row on the grouped schedule never cross a group, so the lists of the row's groups in split s cover
+// exactly the columns of s.  One warp per row stages all the row's lists in shared memory, then for every split runs
+// the K rounds of the P-way merge of topk_merge_kernel over that split's lists only, certifies the result against the
+// split's own K-th value and, for an uncertified (row, split), re-scans that split's doubtful lists exactly.
+constexpr int kSplitDoubtWords = 4;   // bit per list, up to 128 lists per row
+
+// Exact repair of split s of a row (cold): the doubtful lists of s are re-scanned over their bank rows, the others of s
+// inserted as they are -- in column order, as repair_row does.  Returns rank `lane` of the repaired row.
+__device__ __noinline__ Cand split_repair_cold(const SplitMergeArgs* a, int64_t row, int lane, int cnt, int s,
+                                               const uint32_t* dmask) {
+  if (lane == 0 && a->rescan_count) atomicAdd(a->rescan_count, 1u);
+  SortedList<HGR_TOPK_MAX> full;
+  full.init();
+  const int32_t mt = static_cast<int32_t>(row / a->sched.rows);
+  const int KL = a->KL;
+  for (int p = 0; p < cnt; ++p) {
+    int64_t c0, c1;
+    const int g = group_slot_range(a->sched, a->groups, mt, p, c0, c1);
+    if (!((a->group_splits[g] >> s) & 1u)) continue;
+    if ((dmask[p >> 5] >> (p & 31)) & 1u) {
+      scan_row_range_lanes<HGR_TOPK_MAX>(reinterpret_cast<const uint4*>(a->X) + row * a->D8,
+                                         reinterpret_cast<const uint4*>(a->bank), c0, c1, a->D8, lane, full);
+    } else {
+      for (int k = 0; k < KL; ++k) {
+        const int64_t e = (p * a->B + row) * KL + k;
+        const int32_t it = a->part_idx[e];
+        const float v = a->part_val[e];
+        if (it >= 0 && v > full.thr()) full.insert(v, it);
+      }
+    }
+  }
+  Cand c;
+  c.v = -INFINITY;
+  c.i = -1;
+#pragma unroll
+  for (int k = 0; k < HGR_TOPK_MAX; ++k) {
+    if (lane == k) {
+      c.v = full.v[k];
+      c.i = full.i[k];
+    }
+  }
+  return c;
+}
+
+template <int kMaxListsPerLane>
+__global__ void __launch_bounds__(kMergeWarps * 32, 4)  // (the cold repair function must not set the register count)
+topk_split_merge_kernel(const __grid_constant__ SplitMergeArgs a) {
+  extern __shared__ uint8_t smem_raw[];
+  __shared__ unsigned int s_cnt[kMaxSplits][HGR_NUM_HITS + 1];
+  __shared__ uint32_t s_dmask[kMergeWarps][kSplitDoubtWords];
+  for (int i = threadIdx.x; i < kMaxSplits * (HGR_NUM_HITS + 1); i += blockDim.x) (&s_cnt[0][0])[i] = 0u;
+  if (threadIdx.x < kMergeWarps * kSplitDoubtWords) (&s_dmask[0][0])[threadIdx.x] = 0u;
+  __syncthreads();
+
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int KL = a.KL, K = a.K;
+  const int slots = a.sched.P;
+  float* lv = reinterpret_cast<float*>(smem_raw) + warp * slots * KL;                   // [slots][KL] of this row
+  int32_t* li = reinterpret_cast<int32_t*>(reinterpret_cast<float*>(smem_raw) + kMergeWarps * slots * KL) + warp * slots * KL;
+  const int64_t row = static_cast<int64_t>(blockIdx.x) * kMergeWarps + warp;
+  if (row < a.B) {
+    const int32_t mt = static_cast<int32_t>(row / a.sched.rows);
+    const int cnt = group_parts(a.sched, a.groups, mt);
+    for (int e = lane; e < cnt * KL; e += 32) {
+      const int p = e / KL, k = e - p * KL;
+      const int64_t g = (p * a.B + row) * KL + k;
+      lv[e] = a.part_val[g];
+      li[e] = a.part_idx[g];
+    }
+    // split bits of my lists: lane h holds the first slot of group h
+    const int ng = a.groups.n;
+    const int fs = lane < ng ? group_first_slot(a.sched, a.groups, mt, lane) : 0x7FFFFFFF;
+    int grp[kMaxListsPerLane];
+#pragma unroll
+    for (int q = 0; q < kMaxListsPerLane; ++q) grp[q] = 0;
+    for (int h = 1; h < ng; ++h) {
+      const int f = __shfl_sync(0xffffffffu, fs, h);
+#pragma unroll
+      for (int q = 0; q < kMaxListsPerLane; ++q)
+        if (lane + 32 * q >= f) grp[q] = h;
+    }
+    uint32_t lmask[kMaxListsPerLane];
+#pragma unroll
+    for (int q = 0; q < kMaxListsPerLane; ++q) lmask[q] = lane + 32 * q < cnt ? a.group_splits[grp[q]] : 0u;
+    __syncwarp();
+    const int32_t target = a.targets ? a.targets[row] : -1;
+    const uint32_t tbits = (target >= 0 && target < a.n_nodes) ? a.node_splits[target] : 0u;
+
+    for (int s = 0; s < a.S; ++s) {
+      int head[kMaxListsPerLane];
+      float hv[kMaxListsPerLane];
+      int32_t hi[kMaxListsPerLane];
+#pragma unroll
+      for (int q = 0; q < kMaxListsPerLane; ++q) {
+        const int p = lane + 32 * q;
+        head[q] = 0;
+        hi[q] = ((lmask[q] >> s) & 1u) ? li[p * KL] : -1;
+        hv[q] = hi[q] >= 0 ? lv[p * KL] : -INFINITY;
+      }
+      float my_v = -INFINITY;
+      int32_t my_i = -1;
+      float kth = -INFINITY;
+      for (int r = 0; r < K; ++r) {
+        float bv = hv[0];
+        int32_t bi = hi[0];
+#pragma unroll
+        for (int q = 1; q < kMaxListsPerLane; ++q) {
+          if (hv[q] > bv || (hv[q] == bv && hi[q] < bi && hi[q] >= 0)) {
+            bv = hv[q];
+            bi = hi[q];
+          }
+        }
+        const float lbv = bv;
+        const int32_t lbi = bi;
+        const uint32_t lkey = order_key(lbv);
+        const uint32_t mkey = __reduce_max_sync(0xffffffffu, lkey);
+        const uint32_t mitem =
+            __reduce_min_sync(0xffffffffu, (lkey == mkey && lbi >= 0) ? static_cast<uint32_t>(lbi) : 0xFFFFFFFFu);
+        if (mitem == 0xFFFFFFFFu) {   // the split's lists are exhausted: the rest stays (-inf, -1)
+          kth = -INFINITY;
+          break;
+        }
+        bv = order_key_value(mkey);
+        bi = static_cast<int32_t>(mitem);
+        kth = bv;
+        const unsigned holders = __ballot_sync(0xffffffffu, lbv == bv && lbi == bi);
+        if (lane == __ffs(holders) - 1) {
+          bool done = false;
+#pragma unroll
+          for (int q = 0; q < kMaxListsPerLane; ++q) {
+            if (!done && hv[q] == bv && hi[q] == bi) {
+              const int p = lane + 32 * q;
+              const int h = ++head[q];
+              hi[q] = h < KL ? li[p * KL + h] : -1;
+              hv[q] = hi[q] >= 0 ? lv[p * KL + h] : -INFINITY;
+              done = true;
+            }
+          }
+        }
+        if (lane == r) {
+          my_v = bv;
+          my_i = bi;
+        }
+      }
+      // certificate against the split's own K-th value: a full narrow list of s that ends at or above it may hide
+      // members of the split's top-K
+      bool doubt = false;
+      if (KL < K) {
+#pragma unroll
+        for (int q = 0; q < kMaxListsPerLane; ++q) {
+          const int p = lane + 32 * q;
+          if (((lmask[q] >> s) & 1u) && li[p * KL + KL - 1] >= 0 && lv[p * KL + KL - 1] >= kth) {
+            doubt = true;
+            atomicOr(&s_dmask[warp][p >> 5], 1u << (p & 31));
+          }
+        }
+      }
+      if (__any_sync(0xffffffffu, doubt)) {
+        __syncwarp();
+        const Cand c = split_repair_cold(&a, row, lane, cnt, s, s_dmask[warp]);
+        my_v = c.v;
+        my_i = c.i;
+        __syncwarp();
+        if (lane < kSplitDoubtWords) s_dmask[warp][lane] = 0u;
+        __syncwarp();
+      }
+      int32_t gid = -1;
+      if (lane < K && my_i >= 0) gid = a.col_id ? a.col_id[my_i] : a.id_base + my_i;
+      if (lane < K) {
+        const int64_t o = (s * a.B + row) * K + lane;
+        a.topk_val[o] = my_i >= 0 ? my_v * a.scale : -INFINITY;
+        a.topk_idx[o] = gid;
+      }
+      if (a.counts && ((tbits >> s) & 1u)) {   // the row's label is a class of split s
+        const unsigned m = __ballot_sync(0xffffffffu, lane < K && gid >= 0 && gid == target);
+        if (lane == 0) {
+          atomicAdd(&s_cnt[s][HGR_NUM_HITS], 1u);
+          if (m != 0) {
+            const int pos = __ffs(m) - 1;
+#pragma unroll
+            for (int c = 0; c < HGR_NUM_HITS; ++c)
+              if (pos < hit_cut(c)) atomicAdd(&s_cnt[s][c], 1u);
+          }
+        }
+      }
+    }
+  }
+  __syncthreads();
+  if (a.counts) {
+    for (int i = threadIdx.x; i < a.S * (HGR_NUM_HITS + 1); i += blockDim.x) {
+      const unsigned int v = (&s_cnt[0][0])[i];
+      if (v) atomicAdd(reinterpret_cast<unsigned long long*>(a.counts) + i, static_cast<unsigned long long>(v));
+    }
+  }
+}
+
 // ---- cross-GPU sequencing of the peer-memory exchange ---------------------------------------------------------
 // Every rank keeps `n` flag words (one per producer rank) in its exchange buffer.  After the kernel that wrote its
 // candidates into the peers' buffers, a rank launches peer_signal: thread g stores the rank's running sequence
@@ -803,6 +1000,28 @@ int launch_topk_merge(const MergeArgs& args, cudaStream_t stream) {
       HGR_CHECK_CUDA(cudaFuncSetAttribute(topk_merge_kernel<10>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                           static_cast<int>(smem)));
     topk_merge_kernel<10><<<blocks, kMergeWarps * 32, smem, stream>>>(args);
+  }
+  HGR_CHECK_LAUNCH();
+  return HGR_OK;
+}
+
+int launch_topk_split_merge(const SplitMergeArgs& args, cudaStream_t stream) {
+  if (args.B == 0) return HGR_OK;
+  if (args.sched.P > 32 * kSplitDoubtWords)
+    return set_error(HGR_ERR_UNSUPPORTED, "topk split merge: %d lists per row exceed %d", args.sched.P, 32 * kSplitDoubtWords);
+  const int blocks = static_cast<int>((args.B + kMergeWarps - 1) / kMergeWarps);
+  const size_t smem = static_cast<size_t>(kMergeWarps) * args.sched.P * args.KL * 8;
+  if (smem > 200 * 1024) return set_error(HGR_ERR_UNSUPPORTED, "topk split merge: %zu bytes of lists per CTA", smem);
+  if (args.sched.P <= 64) {
+    if (smem > 48 * 1024)
+      HGR_CHECK_CUDA(cudaFuncSetAttribute(topk_split_merge_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                          static_cast<int>(smem)));
+    topk_split_merge_kernel<2><<<blocks, kMergeWarps * 32, smem, stream>>>(args);
+  } else {
+    if (smem > 48 * 1024)
+      HGR_CHECK_CUDA(cudaFuncSetAttribute(topk_split_merge_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                          static_cast<int>(smem)));
+    topk_split_merge_kernel<4><<<blocks, kMergeWarps * 32, smem, stream>>>(args);
   }
   HGR_CHECK_LAUNCH();
   return HGR_OK;

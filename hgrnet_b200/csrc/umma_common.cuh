@@ -20,7 +20,8 @@ constexpr int kTmemCols = 512;
 constexpr int kChunk = 32;                          // accumulator columns per tcgen05.ld
 constexpr int kMaxHierLevels = 32;                  // hierarchy levels of the per-level arg-max epilogue
 
-enum EpiMode { kEpiDense = 0, kEpiNull = 3, kEpiTopkDefer = 4, kEpiSketch = 5, kEpiLevel = 6 };
+// kEpiTopkGroups: the kEpiTopkDefer epilogue on the grouped schedule (Params::groups, hgr_score_topk_splits)
+enum EpiMode { kEpiDense = 0, kEpiNull = 3, kEpiTopkDefer = 4, kEpiSketch = 5, kEpiLevel = 6, kEpiTopkGroups = 7 };
 enum Variant { kVarProd = 0, kVarExact = 2, kVarNull = 3, kVarSketch = 10 };   // impl code - HGR_IMPL_TCGEN05
 
 // SubTile / TileWalker (the walk of one worker over its chunk of the schedule) live in sched.cuh: plain integer
@@ -51,6 +52,8 @@ struct Params {
   uint2* sk_part;                  // [slots][B][kSkCap] (value bits, bank row)
   int32_t* sk_cnt;                 // [slots][B] entries of each list
   unsigned long long* sk_floors;   // [B][kSkSlots] (epoch << 32 | order key)
+  // grouped schedule (kEpiTopkGroups): no list holds rows of two groups, list slots per group_slot (sched.cuh)
+  Groups groups;
 };
 
 constexpr int kTimelineSlots = 32;

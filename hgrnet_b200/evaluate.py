@@ -20,7 +20,7 @@ import numpy as np
 import torch
 
 from . import ops
-from ._cabi import HIT_CUTS
+from ._cabi import HGR_HIER_MAX_CHAIN, HIT_CUTS
 
 
 def count_acc(hits_dict, num_tot):
@@ -155,6 +155,122 @@ class HierMetrics:
                 float(self.point_all) / num_sample * 100.0)
 
 
+_BANK_SEED = 0x48475221   # the seed of tree_model's test-bank permutation (head.py)
+
+
+def split_groups(splits, n_nodes: int):
+    """Host layout of the multi-split bank.  ``splits``: ``{name: node ids}`` (at most 8).  Every class of the union
+    gets the bit mask of the splits that hold it; classes of equal mask form one GROUP, groups in ascending mask order,
+    and inside a group the rows follow a fixed pseudo-random permutation (as ``tree_model``'s test bank does, so that an
+    image's top-20 are not packed into a few adjacent rows).  Returns ``(names, bank_nodes int64 [C], group_end,
+    group_splits, node_splits uint8 [n_nodes])``."""
+    names = list(splits)
+    if not 1 <= len(names) <= 8:
+        raise ValueError("between 1 and 8 splits, got %d" % len(names))
+    node_splits = np.zeros(n_nodes, dtype=np.uint8)
+    for s, name in enumerate(names):
+        ids = np.asarray(list(splits[name]), dtype=np.int64)
+        if ids.size == 0:
+            raise ValueError("split %r is empty" % name)
+        node_splits[ids] |= np.uint8(1 << s)
+    masks = sorted(set(node_splits[node_splits != 0].tolist()))
+    if len(masks) > 16:
+        raise ValueError("%d groups of equal split membership; at most 16" % len(masks))
+    gen = torch.Generator().manual_seed(_BANK_SEED)
+    rows, group_end = [], []
+    for m in masks:
+        ids = np.nonzero(node_splits == m)[0]
+        perm = torch.randperm(ids.size, generator=gen).numpy() if ids.size > 1 else np.zeros(1, dtype=np.int64)
+        rows.append(ids[perm])
+        group_end.append((group_end[-1] if group_end else 0) + ids.size)
+    return names, np.concatenate(rows), group_end, masks, node_splits
+
+
+def split_line(name, hits, rows, hier=None):
+    """The reference's ``test()`` line of one split (``count_acc`` + TOR / POR), prefixed with the split's name.
+    ``hier``: ``(hits, point, path, path_rows)`` sums or None."""
+    out_str, _ = count_acc(dict(zip(HIT_CUTS, hits)), rows)
+    if hier is not None:
+        tor, point, path, path_rows = hier
+        out_str += " hit_ratio(%):{:.2f}".format(tor / rows * 100.0)
+        out_str += " path_ratio(%):{:.2f}".format(path / path_rows * 100.0 if path_rows else 0.0)
+        out_str += " point_ratio(%):{:.2f}".format(point / rows * 100.0)
+    return "{}: {}".format(name, out_str)
+
+
+class SplitEval:
+    """Several test splits of one hierarchy scored in ONE pass per batch (``hgr_score_topk_splits``): the union bank is
+    built from ``model.zsl_weights`` in the group layout of ``split_groups`` and rebuilt after a bank refresh; the hit
+    counters of every split stay on the device.  With ``hier=True`` the TOR / POR counters of every split follow from
+    one level GEMM per batch (``hgr_hier_metrics_fused_rows_splits``).  ``lines()`` gives one line per split."""
+
+    def __init__(self, model, splits, hier: bool = True, K: int = 20):
+        self.model = model
+        self.K = K
+        dev = model.device
+        names, bank_nodes, self.group_end, self.group_splits, node_splits = split_groups(splits, len(model.nodes))
+        self.names = names
+        self.S = len(names)
+        self._bank_nodes = torch.from_numpy(bank_nodes).to(dev)
+        self.col_id = self._bank_nodes.to(torch.int32)
+        self.node_splits = torch.from_numpy(node_splits).to(dev)
+        self.counts = torch.zeros((self.S, ops.HGR_NUM_HITS + 1), dtype=torch.int64, device=dev)
+        self.hier = HierMetrics(model) if hier else None
+        self._hier_counts = None
+        self._hier_acc = torch.zeros((self.S, 4), dtype=torch.float64, device=dev)   # (rows, hits, point, path)
+        self._bank = None
+        self._bank_version = None
+
+    def bank(self) -> torch.Tensor:
+        """The union bank in group layout; rebuilt when ``model.zsl_weights`` was refreshed (new tensor or in place)."""
+        w = self.model.zsl_weights
+        stamp = (w.data_ptr(), w._version)
+        if self._bank is None or self._bank_version != stamp:
+            self._bank = w.index_select(0, self._bank_nodes).contiguous()
+            self._bank_version = stamp
+        return self._bank
+
+    def score_args(self) -> dict:
+        return dict(bank=self.bank(), group_end=self.group_end, group_splits=self.group_splits, n_splits=self.S,
+                    col_id=self.col_id, node_splits=self.node_splits, K=self.K)
+
+    def update(self, x_norm: torch.Tensor, targets: torch.Tensor, hier_targets: Optional[torch.Tensor] = None):
+        """Score a batch against every split: ``x_norm`` [B, D] bf16, ``targets`` [B] node ids (a row counts toward
+        the splits its label belongs to).  TOR / POR match row i against ``hier_targets[i]`` (default: ``targets``).
+        Returns ``(val [S,B,K], idx [S,B,K])``.  No host synchronisation."""
+        t = targets.to(torch.int32)
+        out = ops.score_topk_splits(x_norm, targets=t, counts=self.counts, **self.score_args())
+        if self.hier is not None:
+            if self._hier_counts is None:
+                self._hier_counts = torch.zeros((self.S, HGR_HIER_MAX_CHAIN + 1, 4), dtype=torch.int64,
+                                                device=x_norm.device)
+            else:
+                self._hier_counts.zero_()
+            ht = t if hier_targets is None else hier_targets.to(torch.int32)
+            ops.hier_metrics_fused_rows_splits(x_norm, targets=ht, node_splits=self.node_splits,
+                                               counts=self._hier_counts, **self.hier.rows_args())
+            self._hier_acc += torch.stack([hier_totals(c) for c in self._hier_counts])
+        return out
+
+    def hit_counts(self):
+        """Per split ``[Hit@1, @2, @5, @10, @20, rows]`` so far (synchronises)."""
+        return self.counts.tolist()
+
+    def lines(self):
+        """One line per split: ``name: Top@1(%):..., ... .`` plus TOR / POR with ``hier`` (synchronises)."""
+        counts = self.counts.tolist()
+        acc = self._hier_acc.tolist()
+        out = []
+        for s, name in enumerate(self.names):
+            rows = counts[s][ops.HGR_NUM_HITS]
+            h = None
+            if self.hier is not None:
+                r, tor, point, path = acc[s]
+                h = (tor, point, path, r)
+            out.append(split_line(name, counts[s][:ops.HGR_NUM_HITS], max(rows, 1), h))
+        return out
+
+
 def test(opts, model, device, splits=None, loader: Optional[Iterable] = None, log: bool = True):
     """Drop-in for main.py:104-222.  ``loader`` yields the reference's batch dicts
     ``{'img': [1,B,...], 'label': [1,B]}`` (single-label batches, imagenet_group_test.py).
@@ -169,6 +285,9 @@ def test(opts, model, device, splits=None, loader: Optional[Iterable] = None, lo
         raise ValueError("hgrnet_b200.evaluate.test needs a loader: image I/O (dataset/imagenet_group_test.py) is "
                          "an upstream component; pass loader=DataManager_test(...).get_data_loader()")
     print("Running.", flush=True)
+    split_keys = [k for k in (getattr(opts, "hgr_eval_splits", "") or "").split(",") if k]
+    if split_keys:
+        return _test_splits(opts, model, device, splits, split_keys, loader, log)
     hier = HierMetrics(model) if getattr(opts, "hgr_hier_metrics", True) else None
     hits = ops.new_hits(model.device)
     num_sample = 0
@@ -186,6 +305,32 @@ def test(opts, model, device, splits=None, loader: Optional[Iterable] = None, lo
                 print(out_str, flush=True)
     print("End of testing.")
     out_str = _format(hits, num_sample, hier)
+    print(out_str, flush=True)
+    if log:
+        with open(model.save_path + "arugements.log", "a") as f:       # [sic] main.py:217
+            f.writelines(out_str + "\n")
+        with open("{}.txt".format(opts.weights), "a") as f:            # main.py:219-222
+            method = "{},{},{}:".format(opts.weights, opts.out_ratio, opts.in_ratio)
+            f.writelines(method + "\n" + out_str + "\n")
+    return out_str
+
+
+def _test_splits(opts, model, device, splits, split_keys, loader, log):
+    """``test`` for several split-file keys at once: one scoring pass per batch, one line per split."""
+    if splits is None:
+        raise ValueError("--hgr_eval_splits needs the split file's class lists (splits)")
+    index = model.hierarchy.index
+    se = SplitEval(model, {k: [index[c] for c in splits[k]] for k in split_keys},
+                   hier=getattr(opts, "hgr_hier_metrics", True))
+    with torch.no_grad():
+        for i, data in enumerate(loader):
+            imgs, targets = data["img"].to(device, non_blocking=True)[0], data["label"].to(device, non_blocking=True)[0]
+            x = model.encode_image_normalized(imgs)
+            se.update(x, targets, targets[:1].expand(len(targets)))        # TOR / POR: main.py:152, targets[0]
+            if i % opts.print_freq == 0:
+                print("\n" + "\n".join(se.lines()), flush=True)
+    print("End of testing.")
+    out_str = "\n" + "\n".join(se.lines())
     print(out_str, flush=True)
     if log:
         with open(model.save_path + "arugements.log", "a") as f:       # [sic] main.py:217

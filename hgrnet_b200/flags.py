@@ -79,6 +79,9 @@ def build_parser() -> argparse.ArgumentParser:
                    help="also compute TOR/POR (hit_ratio/path_ratio/point_ratio, main.py:152-191) during test")
     g.add_argument("--hgr_synthetic", default="", type=str,
                    help="run on a synthetic hierarchy and synthetic features, e.g. '10,100,1000' level sizes")
+    g.add_argument("--hgr_eval_splits", default="", type=str,
+                   help="comma-separated split-file keys (e.g. 2-hops,3-hops,all): test scores every batch against all of "
+                        "them in one pass and prints one line per split")
     return p
 
 

@@ -242,19 +242,26 @@ class tree_model(nn.Module):
         return ops.score_topk(x, self.bank_test, col_id=self._test_index_i32, targets=t, K=K, hits=hits)
 
     def make_eval_stream(self, batch: int, slots: int = 4, streams: int = 2, feat_dtype=torch.float32, K: int = 20,
-                         banks=None, host_io: bool = True, hier_metrics: bool = False):
+                         banks=None, host_io: bool = True, hier_metrics: bool = False, eval_splits=None):
         """CUDA-graph replayed eval step over pre-computed image features (hgrnet_b200.stream.EvalStream).
 
         ``hier_metrics=True`` adds TOR / POR (``EvalStream.hier_ratios``), every row scored against its own label.  The
         stream keeps the device pointers of ``bank_test`` and of the level-sorted ``bank_train`` taken now: after
-        ``update_classifier`` refreshes the banks, build a new stream."""
+        ``update_classifier`` refreshes the banks, build a new stream.
+
+        ``eval_splits`` (``{name: node ids}``, at most 8 splits): every step scores against all of these test splits
+        in one pass instead of against ``bank_test`` (``EvalStream.split_hit_counts``; with ``hier_metrics`` also the
+        per-split TOR / POR, ``EvalStream.split_ratios``)."""
         from .stream import EvalStream
-        hier = None
-        if hier_metrics:
+        hier = splits = None
+        if eval_splits is not None:
+            from .evaluate import SplitEval
+            splits = SplitEval(self, eval_splits, hier=hier_metrics, K=K)
+        elif hier_metrics:
             from .evaluate import HierMetrics
             hier = HierMetrics(self)
         return EvalStream(self.bank_test, col_id=self._test_index_i32, batch=batch, feat_dtype=feat_dtype, K=K,
-                          slots=slots, streams=streams, banks=banks, host_io=host_io, hier=hier)
+                          slots=slots, streams=streams, banks=banks, host_io=host_io, hier=hier, splits=splits)
 
     # ------------------------------------------------------------------ training step
     def _schedule(self, training_method, target):

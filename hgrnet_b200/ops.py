@@ -172,6 +172,63 @@ def score_topk(X: torch.Tensor, bank: torch.Tensor, *, col_id: Optional[torch.Te
     return val, idx
 
 
+def score_topk_splits(X: torch.Tensor, bank: torch.Tensor, group_end, group_splits, n_splits: int, *,
+                      col_id: Optional[torch.Tensor] = None, id_base: int = 0, targets: Optional[torch.Tensor] = None,
+                      node_splits: Optional[torch.Tensor] = None, counts: Optional[torch.Tensor] = None, K: int = 20,
+                      scale: float = 1.0, impl: int = HGR_IMPL_AUTO,
+                      out: Optional[Tuple[torch.Tensor, torch.Tensor]] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """``score_topk`` for ``n_splits`` test splits in one pass (``hgr_score_topk_splits``, main.py:104-222 once per
+    split).  ``bank`` is the union of the splits' classes with the classes of equal membership in contiguous groups:
+    ``group_end`` (host ints, exclusive ends, the last = C) and ``group_splits`` (host ints, bit s = the group belongs to
+    split s).  ``counts`` (int64 ``[n_splits, HGR_NUM_HITS + 1]``, optional) is incremented by Hit@{1,2,5,10,20} and the
+    row count of every split, a row counting toward split s when bit s of ``node_splits[targets[row]]`` (uint8 per node)
+    is set.  Returns ``(val [S,B,K] fp32, idx [S,B,K] int32 node ids)``."""
+    import ctypes
+    lib = _cabi.load()
+    X = _require(X, "X", torch.bfloat16)
+    bank = _require(bank, "bank", torch.bfloat16)
+    B, D = X.shape
+    C = bank.shape[0]
+    if bank.shape[1] != D:
+        raise ValueError("X and bank disagree on D: %d vs %d" % (D, bank.shape[1]))
+    n_groups = len(group_end)
+    if len(group_splits) != n_groups:
+        raise ValueError("group_end and group_splits disagree")
+    if col_id is not None:
+        col_id = _require(col_id, "col_id", torch.int32)
+        if col_id.numel() != C:
+            raise ValueError("col_id must have one entry per bank row")
+    if counts is not None:
+        if targets is None or node_splits is None:
+            raise ValueError("counts need targets and node_splits")
+        if not counts.is_cuda or counts.dtype != torch.int64 or counts.numel() != n_splits * (HGR_NUM_HITS + 1) \
+                or not counts.is_contiguous():
+            raise ValueError("counts must be a contiguous CUDA int64 [%d, %d] tensor" % (n_splits, HGR_NUM_HITS + 1))
+    if targets is not None:
+        targets = _require(targets, "targets", torch.int32)
+        if targets.numel() != B:
+            raise ValueError("targets must have one entry per image row")
+    if node_splits is not None:
+        node_splits = _require(node_splits, "node_splits", torch.uint8)
+    if out is not None:
+        val, idx = out
+        if val.shape != (n_splits, B, K) or idx.shape != (n_splits, B, K) or val.dtype != torch.float32 \
+                or idx.dtype != torch.int32 or not val.is_contiguous() or not idx.is_contiguous():
+            raise ValueError("out must be contiguous (float32 [S,B,K], int32 [S,B,K])")
+    else:
+        val = torch.empty((n_splits, B, K), dtype=torch.float32, device=X.device)
+        idx = torch.empty((n_splits, B, K), dtype=torch.int32, device=X.device)
+    ends = (ctypes.c_int32 * n_groups)(*[int(e) for e in group_end])
+    gsp = (ctypes.c_uint8 * n_groups)(*[int(m) for m in group_splits])
+    nbytes = lib.hgr_score_topk_splits_workspace_bytes(B, C, D, K, n_groups, ends)
+    ws = _workspace(nbytes, X.device)      # the stream's scoring workspace: last_rescan_count() reads it
+    n_nodes = node_splits.numel() if node_splits is not None else 0
+    _cabi.check(lib.hgr_score_topk_splits(_ptr(X), _ptr(bank), _ptr(col_id), id_base, _ptr(targets), _ptr(node_splits),
+                                          n_nodes, B, C, D, float(scale), K, n_groups, ends, gsp, n_splits, _ptr(ws),
+                                          ws.numel(), _ptr(val), _ptr(idx), _ptr(counts), impl, _stream()))
+    return val, idx
+
+
 def score_topk_plan(B: int, C: int, D: int, K: int = 20) -> dict:
     """What ``score_topk`` would do for this shape on the tcgen05 path (no launch, works without a GPU)."""
     import ctypes
@@ -439,6 +496,44 @@ def hier_metrics_fused_rows(x_norm: torch.Tensor, bank_sorted: torch.Tensor, lev
                                                 _ptr(sorted_to_pos), _ptr(first_out), _ptr(targets), n_nodes,
                                                 _ptr(chain_ptr), _ptr(chain_pos), _ptr(chain_level), _ptr(ws), ws.numel(),
                                                 _ptr(lvl_idx), _ptr(top1), _ptr(counts), _stream()))
+
+
+def hier_metrics_fused_rows_splits(x_norm: torch.Tensor, bank_sorted: torch.Tensor, level_end, sorted_to_pos: torch.Tensor,
+                                   first_out: torch.Tensor, targets: torch.Tensor, chain_ptr: torch.Tensor,
+                                   chain_pos: torch.Tensor, chain_level: torch.Tensor, node_splits: torch.Tensor,
+                                   counts: torch.Tensor) -> None:
+    """``hier_metrics_fused_rows`` with one counter set per split (``hgr_hier_metrics_fused_rows_splits``): ``counts``
+    int64 ``[S, HGR_HIER_MAX_CHAIN + 1, 4]``; a row is added to set s for every bit s of ``node_splits[targets[row]]``
+    (uint8 per node).  One GEMM per batch whatever S is."""
+    import ctypes
+    lib = _cabi.load()
+    x_norm = _require(x_norm, "x_norm", torch.bfloat16)
+    bank_sorted = _require(bank_sorted, "bank_sorted", torch.bfloat16)
+    sorted_to_pos = _require(sorted_to_pos, "sorted_to_pos", torch.int32)
+    first_out = _require(first_out, "first_out", torch.int32)
+    targets = _require(targets, "targets", torch.int32)
+    chain_ptr = _require(chain_ptr, "chain_ptr", torch.int32)
+    chain_pos = _require(chain_pos, "chain_pos", torch.int32)
+    chain_level = _require(chain_level, "chain_level", torch.int32)
+    node_splits = _require(node_splits, "node_splits", torch.uint8)
+    S = counts.shape[0] if counts.dim() == 3 else -1
+    if not counts.is_cuda or counts.dtype != torch.int64 or tuple(counts.shape[1:]) != (HGR_HIER_MAX_CHAIN + 1, 4) \
+            or not counts.is_contiguous():
+        raise ValueError("counts must be a contiguous CUDA int64 [S, %d, 4] tensor" % (HGR_HIER_MAX_CHAIN + 1))
+    B, D = x_norm.shape
+    M = bank_sorted.shape[0]
+    n_levels = len(level_end)
+    n_nodes = chain_ptr.numel() - 1
+    if sorted_to_pos.numel() != M or first_out.numel() != n_levels or targets.numel() != B \
+            or chain_pos.numel() != chain_level.numel() or node_splits.numel() != n_nodes:
+        raise ValueError("hier_metrics_fused_rows_splits: inconsistent sizes")
+    ends = (ctypes.c_int32 * n_levels)(*[int(e) for e in level_end])
+    ws = _hier_workspace(B * n_levels * 8, x_norm.device)
+    _cabi.check(lib.hgr_hier_metrics_fused_rows_splits(_ptr(x_norm), _ptr(bank_sorted), B, M, D, ends, n_levels,
+                                                       _ptr(sorted_to_pos), _ptr(first_out), _ptr(targets), n_nodes,
+                                                       _ptr(chain_ptr), _ptr(chain_pos), _ptr(chain_level),
+                                                       _ptr(node_splits), S, _ptr(ws), ws.numel(), _ptr(counts),
+                                                       _stream()))
 
 
 def hier_level_scatter(x_norm: torch.Tensor, bank_shard: torch.Tensor, level_end_local, row_base: int, dst_block_ptrs,

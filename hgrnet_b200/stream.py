@@ -23,6 +23,12 @@ With ``hier`` (an ``evaluate.HierMetrics``) each graph also runs the hierarchica
 per-row chain matching).  Its per-chain-length counters share one device buffer with the hit counters, so a step still
 makes one D2H copy.  The level-sorted train bank, like ``bank``, is taken when the stream is built: after a bank
 refresh, build a new stream.
+
+With ``splits`` (an ``evaluate.SplitEval``) each graph scores the batch against all of the SplitEval's test splits in
+one pass instead of against ``bank`` (``ops.score_topk_splits`` over the union bank, plus the per-split TOR / POR when
+the SplitEval has them): one line per split, same graph shape, and the per-split counters sit in the same device buffer
+as the others, so a step still makes one D2H copy (``split_hit_counts`` / ``split_ratios``).  The union bank too is taken
+when the stream is built.
 """
 from __future__ import annotations
 
@@ -37,12 +43,14 @@ from ._cabi import HGR_HIER_MAX_CHAIN
 class EvalStream:
     def __init__(self, bank: torch.Tensor, col_id: Optional[torch.Tensor] = None, id_base: int = 0, *, batch: int,
                  feat_dtype=torch.float32, K: int = 20, slots: int = 4, streams: int = 2, banks=None,
-                 host_io: bool = True, hier=None):
+                 host_io: bool = True, hier=None, splits=None):
         """``bank`` [C, D] bf16 on the device.  ``banks``: optional list of bank tensors to rotate over per slot
         (benchmarks use it to keep the working set larger than L2).  ``host_io=False`` skips the H2D / D2H nodes
         (features are then written straight into ``dev_feats`` / ``dev_labels``).  ``hier``: optional
         ``evaluate.HierMetrics`` of the model; when given, every step also counts TOR / POR (``hier_ratios``).  Labels
-        are node ids; a label outside the hierarchy (e.g. -1 padding) is counted by neither metric."""
+        are node ids; a label outside the hierarchy (e.g. -1 padding) is counted by neither metric.  ``splits``: optional
+        ``evaluate.SplitEval``; every step then scores against its splits instead of ``bank`` (``val`` / ``idx`` are
+        ``[S, B, K]``, ``hit_counts`` stays zero, ``split_hit_counts`` / ``split_ratios`` give the per-split results)."""
         self.device = bank.device
         self.K = K
         self.B = batch
@@ -64,7 +72,13 @@ class EvalStream:
         # hit counters, then (with hier) the per-chain-length TOR / POR counters: one buffer, one D2H copy per step
         self.hier = hier
         self._hier_args = hier.rows_args() if hier is not None else None
-        n_counters = ops.HGR_NUM_HITS + (0 if hier is None else (HGR_HIER_MAX_CHAIN + 1) * 4)
+        self.splits = splits
+        self._split_args = splits.score_args() if splits is not None else None
+        self._split_hier_args = splits.hier.rows_args() if splits is not None and splits.hier is not None else None
+        n_hier = 0 if hier is None else (HGR_HIER_MAX_CHAIN + 1) * 4
+        n_split = 0 if splits is None else splits.S * (ops.HGR_NUM_HITS + 1)
+        n_split_hier = 0 if self._split_hier_args is None else splits.S * (HGR_HIER_MAX_CHAIN + 1) * 4
+        n_counters = ops.HGR_NUM_HITS + n_hier + n_split + n_split_hier
         if host_io:
             self.host_pack = [torch.zeros(nbytes, dtype=torch.uint8).pin_memory() for _ in range(slots)]
             self.host_feats, self.host_labels = map(list, zip(*[views(p) for p in self.host_pack]))
@@ -72,7 +86,13 @@ class EvalStream:
             self.host_hits = self.host_counters[:ops.HGR_NUM_HITS]
         self.counters = torch.zeros(n_counters, dtype=torch.int64, device=self.device)
         self.hits = self.counters[:ops.HGR_NUM_HITS]
-        self.hier_counts = self.counters[ops.HGR_NUM_HITS:].view(HGR_HIER_MAX_CHAIN + 1, 4) if hier is not None else None
+        o = ops.HGR_NUM_HITS
+        self.hier_counts = self.counters[o:o + n_hier].view(HGR_HIER_MAX_CHAIN + 1, 4) if hier is not None else None
+        o += n_hier
+        self.split_counts = self.counters[o:o + n_split].view(-1, ops.HGR_NUM_HITS + 1) if n_split else None
+        o += n_split
+        self.split_hier_counts = (self.counters[o:o + n_split_hier].view(-1, HGR_HIER_MAX_CHAIN + 1, 4)
+                                  if n_split_hier else None)
         self.val = [None] * slots
         self.idx = [None] * slots
         self.streams = [torch.cuda.Stream(device=self.device) for _ in range(max(1, min(streams, slots)))]
@@ -87,9 +107,16 @@ class EvalStream:
         if self.host_io:
             self.dev_pack[s].copy_(self.host_pack[s], non_blocking=True)
         x = ops.normalize_rows(self.dev_feats[s])                                    # clip_tree.py:330
-        self.val[s], self.idx[s] = ops.score_topk(x, self.banks[s % len(self.banks)], col_id=self.col_id,
-                                                  id_base=self.id_base, targets=self.dev_labels[s], K=self.K,
-                                                  hits=self.hits)                    # clip_tree.py:331 + main.py:136-147
+        if self._split_args is None:
+            self.val[s], self.idx[s] = ops.score_topk(x, self.banks[s % len(self.banks)], col_id=self.col_id,
+                                                      id_base=self.id_base, targets=self.dev_labels[s], K=self.K,
+                                                      hits=self.hits)                # clip_tree.py:331 + main.py:136-147
+        else:                                                                        # the same, once per test split
+            self.val[s], self.idx[s] = ops.score_topk_splits(x, targets=self.dev_labels[s], counts=self.split_counts,
+                                                             **self._split_args)
+            if self._split_hier_args is not None:
+                ops.hier_metrics_fused_rows_splits(x, targets=self.dev_labels[s], node_splits=self.splits.node_splits,
+                                                   counts=self.split_hier_counts, **self._split_hier_args)
         if self._hier_args is not None:                                              # main.py:143,152-191
             ops.hier_metrics_fused_rows(x, targets=self.dev_labels[s], counts=self.hier_counts, **self._hier_args)
         if self.host_io:
@@ -157,3 +184,24 @@ class EvalStream:
         if rows == 0:
             return 0.0, 0.0, 0.0
         return hits / rows * 100.0, path / rows * 100.0, point / rows * 100.0
+
+    def split_hit_counts(self):
+        """Per split ``[Hit@1, @2, @5, @10, @20, rows]`` so far, in the order of ``splits.names`` (synchronises).
+        Needs ``splits``."""
+        if self.splits is None:
+            raise RuntimeError("EvalStream was built without splits (pass splits=SplitEval(model, {...}))")
+        self.synchronize()
+        return self.split_counts.tolist()
+
+    def split_ratios(self):
+        """Per split ``(hit_ratio, path_ratio, point_ratio)`` in percent over the rows whose label is in the split
+        (synchronises).  Needs ``splits`` with TOR / POR."""
+        if self.split_hier_counts is None:
+            raise RuntimeError("EvalStream was built without per-split TOR / POR (SplitEval(..., hier=True))")
+        from .evaluate import hier_totals
+        self.synchronize()
+        out = []
+        for c in self.split_hier_counts:
+            rows, hits, point, path = hier_totals(c).tolist()
+            out.append((0.0, 0.0, 0.0) if rows == 0 else (hits / rows * 100.0, path / rows * 100.0, point / rows * 100.0))
+        return out

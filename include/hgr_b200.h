@@ -303,6 +303,47 @@ int hgr_hier_metrics_fused_rows(const void* X, const void* bank_sorted, int64_t 
                                 int64_t* counts, void* stream);
 
 /*
+ * Several test splits of one hierarchy in ONE scoring pass (the reference prints one line per run of main.py:104-222
+ * with --model_test / --data_test = 2-hops, 3-hops, all).  The bank [C, D] is the union of the splits' classes, ordered
+ * so that the classes of equal split membership form contiguous GROUPS; the scoring kernel's partial lists never cross
+ * a group, so for every split the merge takes exactly the lists of its groups -- certified against that split's own
+ * K-th value and repaired exactly like hgr_score_topk.  Per split the result is hgr_score_topk on the split's rows of
+ * the bank (same values, same (value desc, bank row asc) order).
+ *
+ *  n_groups, group_end   HOST [n_groups] int32 (n_groups <= 16): group g = bank rows [group_end[g-1], group_end[g]),
+ *                        strictly ascending, group_end[n_groups-1] == C.  Copied into the kernel parameters: the call
+ *                        can be captured in a CUDA graph.
+ *  group_splits          HOST [n_groups] uint8: bit s set = the group's classes belong to split s (n_splits <= 8)
+ *  node_splits           [n_nodes] uint8 split bits of every node id: a row counts toward split s only if bit s of
+ *                        node_splits[targets[row]] is set (its label is a class of s); NULL with counts == NULL
+ *  topk_val / topk_idx   [n_splits, B, K] fp32 / int32 node ids (col_id applied), as hgr_score_topk per split
+ *  counts                [n_splits][HGR_NUM_HITS + 1] int64, INCREMENTED: Hit@{1,2,5,10,20} and the number of rows
+ *                        counted -- the numerator and denominator of the split's line; NULL to skip
+ *  impl                  HGR_IMPL_AUTO / HGR_IMPL_TCGEN05 / HGR_IMPL_TCGEN05_EXACT; others: HGR_ERR_UNSUPPORTED
+ *  workspace             hgr_score_topk_splits_workspace_bytes(...) bytes, 16-byte aligned, ZERO on first use, left
+ *                        reusable (no memset per batch); the rows re-scanned exactly are counted in its first word
+ */
+size_t hgr_score_topk_splits_workspace_bytes(int64_t B, int64_t C, int64_t D, int K, int n_groups, const int32_t* group_end);
+int hgr_score_topk_splits(const void* X, const void* bank, const int32_t* col_id, int32_t id_base, const int32_t* targets,
+                          const uint8_t* node_splits, int64_t n_nodes, int64_t B, int64_t C, int64_t D, float scale, int K,
+                          int n_groups, const int32_t* group_end, const uint8_t* group_splits, int n_splits,
+                          void* workspace, size_t workspace_bytes, float* topk_val, int32_t* topk_idx, int64_t* counts,
+                          int impl, void* stream);
+
+/*
+ * hgr_hier_metrics_fused_rows with the counters of every split (main.py:143,152-191 run once per split): the same GEMM
+ * and row decoding, once per batch, and each row is added to counter set s for every bit s of node_splits[targets[row]]
+ * (a row outside the hierarchy nowhere).  counts [n_splits][HGR_HIER_MAX_CHAIN + 1][4] int64, incremented; n_splits
+ * <= 8.  workspace as hgr_hier_metrics_fused_rows.
+ */
+int hgr_hier_metrics_fused_rows_splits(const void* X, const void* bank_sorted, int64_t B, int64_t M, int64_t D,
+                                       const int32_t* level_end, int n_levels, const int32_t* sorted_to_pos,
+                                       const int32_t* first_out, const int32_t* targets, int64_t n_nodes,
+                                       const int32_t* chain_ptr, const int32_t* chain_pos, const int32_t* chain_level,
+                                       const uint8_t* node_splits, int n_splits, void* workspace, size_t workspace_bytes,
+                                       int64_t* counts, void* stream);
+
+/*
  * hgr_hier_metrics_fused_rows for the CLASS-SHARDED head (main.py:143,152-191): the level-sorted train bank [M, D] is
  * cut into contiguous row ranges, one per rank, and image rows are owned block-wise as in hgr_score_topk_scatter.  The
  * result is bit-identical to hgr_hier_metrics_fused_rows on the whole batch on one GPU: a winner word is

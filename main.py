@@ -65,7 +65,11 @@ def _synthetic_setup(opts, device):
     dim = 1024 if opts.arch == "RN50" else 512
     enc = TableEncoder(synthetic_embeddings(n, dim, 1, normalize=False)).to(device)
     leaves = hier.nodes[n - levels[-1]:]
-    splits = {"train": hier.nodes, "rest": leaves, "all": hier.nodes}
+    # two seeded nested splits of the leaves (the shape of the 2-hops / 3-hops sets inside "rest"), for --hgr_eval_splits
+    order = torch.randperm(len(leaves), generator=torch.Generator().manual_seed(5)).tolist()
+    hops3 = [leaves[i] for i in sorted(order[:max(1, len(leaves) // 2)])]
+    hops2 = [leaves[i] for i in sorted(order[:max(1, len(leaves) // 8)])]
+    splits = {"train": hier.nodes, "rest": leaves, "all": hier.nodes, "hops2": hops2, "hops3": hops3}
     model = tree_model(opts, splits[opts.model_train], splits[opts.model_test], clip_model=enc, hierarchy=hier,
                        node_tokens=node_id_tokens(n))
     g = torch.Generator().manual_seed(3)
