@@ -77,6 +77,19 @@ SIGNATURES = {
     "hgr_hier_finish_rows_gathered": (c_int, [c_void_p, c_int, c_int64, c_int64, c_int64, c_int, c_void_p, c_void_p,
                                               c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                               c_void_p]),
+    "hgr_score_topk_splits_scatter_bounded_workspace_bytes": (c_size_t, [c_int64, c_int64, c_int64, c_int, c_int, c_void_p]),
+    "hgr_score_topk_splits_global_list_len": (c_int, [c_int64, c_int64, c_int64, c_int, c_int, c_void_p, c_void_p, c_int,
+                                                      c_void_p]),
+    "hgr_score_topk_splits_scatter_bounded": (c_int, [c_void_p, c_void_p, c_void_p, c_int32, c_int64, c_int64, c_int64,
+                                                      c_float, c_int, c_int, c_void_p, c_void_p, c_int, c_void_p, c_void_p,
+                                                      c_size_t, c_int64, c_int, c_void_p, c_void_p, c_void_p, c_int64,
+                                                      c_int, c_void_p]),
+    "hgr_topk_merge_splits_certified": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int, c_int, c_int64,
+                                                c_int64, c_int64, c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p,
+                                                c_void_p, c_int64, c_void_p, c_float, c_void_p, c_void_p]),
+    "hgr_hier_finish_rows_gathered_splits": (c_int, [c_void_p, c_int, c_int64, c_int64, c_int64, c_int, c_void_p, c_void_p,
+                                                     c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_int,
+                                                     c_void_p, c_void_p]),
     "hgr_masked_ce_workspace_bytes":(c_size_t, [c_int64, c_int64, c_int64]),
     "hgr_om_backward_workspace_bytes": (c_size_t, [c_int64, c_int64, c_int64]),
     "hgr_om_backward": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int64, c_int64, c_void_p, c_void_p, c_void_p,

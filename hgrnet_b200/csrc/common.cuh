@@ -142,8 +142,36 @@ struct SplitMergeArgs {
   const void* bank;            // [C, D] bf16
   int D8;
   unsigned int* rescan_count;  // (row, split) pairs re-scanned
+  // bounded scatter (hgr_score_topk_splits_scatter_bounded): instead of topk_val / topk_idx / counts, split s of row
+  // block g goes to scatter.val[g] / idx[g] / bound[g] + s * split_stride elements; no local certificate, no repair
+  OutScatter scatter;
+  int64_t split_stride;
 };
 int launch_topk_split_merge(const SplitMergeArgs& args, cudaStream_t stream);
+
+// Owner side of the class-sharded per-split certificate (hgr_topk_merge_splits_certified): split s of list p (class
+// shard p) sits at part_val / part_idx + s * split_stride + p * part_stride + row * K (node ids, scaled values), its
+// bound at part_bound + s * split_stride + p * bound_stride + row.
+struct SplitCertArgs {
+  const float* part_val;
+  const int32_t* part_idx;
+  const float* part_bound;
+  int64_t P, B;
+  int K, S;
+  int64_t part_stride, bound_stride, split_stride;
+  const int32_t* targets;      // [B] node ids, or null
+  const uint8_t* node_splits;  // [n_nodes] split bits of every node
+  int64_t n_nodes;
+  float* topk_val;             // [S][B][K]
+  int32_t* topk_idx;           // [S][B][K] node ids
+  int64_t* counts;             // [S][HGR_NUM_HITS + 1], or null
+  const hgr_shard_t* shards;   // [P] the shards' banks (peer memory) for the exact repair
+  const void* xrows;           // [B, D] bf16
+  int xD8;
+  float scale;
+  unsigned int* repair_count;  // (row, split) pairs repaired
+};
+int launch_topk_split_merge_certified(const SplitCertArgs& args, cudaStream_t stream);
 
 size_t simt_score_workspace_bytes(int64_t B, int64_t C, int K);
 int launch_score_topk_simt(const __nv_bfloat16* X, const __nv_bfloat16* bank, const int32_t* col_id,
@@ -171,6 +199,15 @@ int launch_score_topk_splits_umma(const __nv_bfloat16* X, const __nv_bfloat16* b
                                   int64_t B, int64_t C, int64_t D, float scale, int K, const Groups& gr,
                                   const uint8_t* group_splits, int S, void* ws, size_t ws_bytes, float* topk_val,
                                   int32_t* topk_idx, int64_t* counts, bool exact, cudaStream_t stream);
+// class shard of the union bank (hgr_score_topk_splits_scatter_bounded): lists sized for each split's GLOBAL stream of
+// split_C_total[s] classes, per split the local top-K and the bound of what was dropped scattered to the row owners
+int launch_score_topk_splits_scatter_umma(const __nv_bfloat16* X, const __nv_bfloat16* bank, const int32_t* col_id,
+                                          int32_t id_base, int64_t B, int64_t C, int64_t D, float scale, int K,
+                                          const Groups& gr, const uint8_t* group_splits, int S,
+                                          const int64_t* split_C_total, void* ws, size_t ws_bytes,
+                                          const OutScatter& scatter, int64_t split_stride, cudaStream_t stream);
+int umma_split_global_list_len(int64_t B, int64_t C, int64_t D, int K, const Groups& gr, const uint8_t* group_splits,
+                               int S, const int64_t* split_C_total);
 
 int launch_level_argmax_umma(const __nv_bfloat16* X, const __nv_bfloat16* bank_sorted, int64_t B, int64_t M, int64_t D,
                              const int32_t* level_end, int n_levels, unsigned long long* lvl_best, cudaStream_t stream);
@@ -192,6 +229,12 @@ int launch_hier_finish_rows_splits(unsigned long long* lvl_best, int64_t B, int6
                                    int64_t n_nodes, const int32_t* chain_ptr, const int32_t* chain_pos,
                                    const int32_t* chain_level, const uint8_t* node_splits, int n_splits,
                                    int64_t* counts, cudaStream_t stream);
+// hgr_hier_finish_rows_gathered_splits: the gathered words, counted per split as above
+int launch_hier_finish_gathered_splits(const unsigned long long* parts, int n_parts, int64_t part_stride, int64_t B,
+                                       int64_t M, int n_levels, const int32_t* sorted_to_pos, const int32_t* first_out,
+                                       const int32_t* targets, int64_t n_nodes, const int32_t* chain_ptr,
+                                       const int32_t* chain_pos, const int32_t* chain_level, const uint8_t* node_splits,
+                                       int n_splits, int64_t* counts, cudaStream_t stream);
 int launch_normalize_dual(const void* E, int e_dtype, int64_t n_rows, int64_t D, void* out, const int32_t* dst_map,
                           void* out2, cudaStream_t stream);
 int launch_normalize_bcast(const void* E, int e_dtype, int64_t n_rows, int64_t D, int64_t row0, int n_dst,

@@ -183,6 +183,111 @@ int hgr_score_topk_splits(const void* X, const void* bank, const int32_t* col_id
                                        impl == HGR_IMPL_TCGEN05_EXACT, static_cast<cudaStream_t>(stream));
 }
 
+// Class shard of the union bank, one rank's part of main.py:104-222 run once per split: per split the rank's top-K and
+// the bound of what it dropped, scattered to the row owners (hgr_topk_merge_splits_certified).
+static int split_totals(int n_splits, const int64_t* split_C_total) {
+  HGR_CHECK_ARG(split_C_total != nullptr, "hgr_score_topk_splits_scatter_bounded: null split_C_total");
+  for (int sp = 0; sp < n_splits; ++sp)
+    HGR_CHECK_ARG(split_C_total[sp] >= 0, "hgr_score_topk_splits_scatter_bounded: split_C_total[%d] = %lld < 0", sp,
+                  (long long)split_C_total[sp]);
+  return HGR_OK;
+}
+
+size_t hgr_score_topk_splits_scatter_bounded_workspace_bytes(int64_t B, int64_t C, int64_t D, int K, int n_groups,
+                                                             const int32_t* group_end) {
+  return hgr_score_topk_splits_workspace_bytes(B, C, D, K, n_groups, group_end);
+}
+
+int hgr_score_topk_splits_scatter_bounded(const void* X, const void* bank, const int32_t* col_id, int32_t id_base,
+                                          int64_t B, int64_t C, int64_t D, float scale, int K, int n_groups,
+                                          const int32_t* group_end, const uint8_t* group_splits, int n_splits,
+                                          const int64_t* split_C_total, void* workspace, size_t workspace_bytes,
+                                          int64_t block_rows, int n_blocks, float* const* val_blocks,
+                                          int32_t* const* idx_blocks, float* const* bound_blocks, int64_t split_stride,
+                                          int impl, void* stream) {
+  HGR_CHECK_ARG(B >= 0 && C >= 0, "hgr_score_topk_splits_scatter_bounded: bad sizes B=%lld C=%lld", (long long)B,
+                (long long)C);
+  HGR_CHECK_ARG(D > 0 && D % 8 == 0, "hgr_score_topk_splits_scatter_bounded: D = %lld must be a positive multiple of 8",
+                (long long)D);
+  HGR_CHECK_ARG(K >= 1 && K <= HGR_TOPK_MAX, "hgr_score_topk_splits_scatter_bounded: K = %d outside [1, %d]", K, HGR_TOPK_MAX);
+  HGR_CHECK_ARG(scale > 0.f, "hgr_score_topk_splits_scatter_bounded: scale must be > 0");
+  HGR_CHECK_ARG(n_splits >= 1 && n_splits <= kMaxSplits, "hgr_score_topk_splits_scatter_bounded: %d splits outside [1, %d]",
+                n_splits, kMaxSplits);
+  Groups gr;
+  if (C > 0) {
+    const int rc = split_table(C, n_groups, group_end, group_splits, n_splits, &gr);
+    if (rc != HGR_OK) return rc;
+  }
+  int rc = split_totals(n_splits, split_C_total);
+  if (rc != HGR_OK) return rc;
+  if (impl != HGR_IMPL_AUTO && impl != HGR_IMPL_TCGEN05)
+    return set_error(HGR_ERR_UNSUPPORTED, "hgr_score_topk_splits_scatter_bounded: impl %d (only the tcgen05 kernel has the "
+                     "grouped schedule)", impl);
+  HGR_CHECK_ARG(n_blocks >= 1 && n_blocks <= kMaxScatterBlocks,
+                "hgr_score_topk_splits_scatter_bounded: n_blocks = %d outside [1, %d]", n_blocks, kMaxScatterBlocks);
+  HGR_CHECK_ARG(block_rows >= 1 && block_rows * n_blocks >= B,
+                "hgr_score_topk_splits_scatter_bounded: %d blocks of %lld rows do not cover B = %lld", n_blocks,
+                (long long)block_rows, (long long)B);
+  HGR_CHECK_ARG(val_blocks && idx_blocks && bound_blocks, "hgr_score_topk_splits_scatter_bounded: null block tables");
+  // a split's area in an owner's slot: the value and id lists [n_blocks, block_rows, K] and the bounds [n_blocks,
+  // block_rows] of all producers
+  HGR_CHECK_ARG(n_splits == 1 || split_stride >= n_blocks * block_rows * (2 * K + 1),
+                "hgr_score_topk_splits_scatter_bounded: split_stride %lld < %lld: the areas of two splits overlap",
+                (long long)split_stride, (long long)(n_blocks * block_rows * (2 * K + 1)));
+  if (B == 0) return HGR_OK;
+  OutScatter sc;
+  sc.n_blocks = n_blocks;
+  sc.block_rows = block_rows;
+  sc.emit_bound = 1;
+  for (int g = 0; g < n_blocks; ++g) {
+    HGR_CHECK_ARG(val_blocks[g] && idx_blocks[g] && bound_blocks[g], "hgr_score_topk_splits_scatter_bounded: null block %d", g);
+    sc.val[g] = val_blocks[g];
+    sc.idx[g] = idx_blocks[g];
+    sc.bound[g] = bound_blocks[g];
+  }
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  if (C == 0) {
+    // no rows on this rank: every split stores (-inf, -1) lists and a -inf bound (the merge of zero lists)
+    for (int sp = 0; sp < n_splits; ++sp) {
+      MergeArgs m{};
+      m.B = B;
+      m.KL = K;
+      m.K = K;
+      m.scale = 1.f;
+      m.scatter = sc;
+      for (int g = 0; g < n_blocks; ++g) {
+        m.scatter.val[g] += sp * split_stride;
+        m.scatter.idx[g] += sp * split_stride;
+        m.scatter.bound[g] += sp * split_stride;
+      }
+      rc = launch_topk_merge(m, s);
+      if (rc != HGR_OK) return rc;
+    }
+    return HGR_OK;
+  }
+  HGR_CHECK_ARG(X && bank, "hgr_score_topk_splits_scatter_bounded: null X / bank");
+  HGR_CHECK_ARG(aligned16(X) && aligned16(bank) && aligned16(workspace),
+                "hgr_score_topk_splits_scatter_bounded: X/bank/workspace must be 16-byte aligned");
+  if (!umma_supported(B, C, D, K))
+    return set_error(HGR_ERR_UNSUPPORTED, "hgr_score_topk_splits_scatter_bounded: shape not supported by the tcgen05 kernel");
+  return launch_score_topk_splits_scatter_umma(static_cast<const __nv_bfloat16*>(X), static_cast<const __nv_bfloat16*>(bank),
+                                               col_id, id_base, B, C, D, scale, K, gr, group_splits, n_splits,
+                                               split_C_total, workspace, workspace_bytes, sc, split_stride, s);
+}
+
+int hgr_score_topk_splits_global_list_len(int64_t B, int64_t C, int64_t D, int K, int n_groups, const int32_t* group_end,
+                                          const uint8_t* group_splits, int n_splits, const int64_t* split_C_total) {
+  HGR_CHECK_ARG(K >= 1 && K <= HGR_TOPK_MAX, "hgr_score_topk_splits_global_list_len: K = %d outside [1, %d]", K, HGR_TOPK_MAX);
+  Groups gr;
+  int rc = split_table(C, n_groups, group_end, group_splits, n_splits, &gr);
+  if (rc != HGR_OK) return rc;
+  rc = split_totals(n_splits, split_C_total);
+  if (rc != HGR_OK) return rc;
+  if (!umma_supported(B, C, D, K))
+    return set_error(HGR_ERR_UNSUPPORTED, "hgr_score_topk_splits_global_list_len: shape not supported by the tcgen05 kernel");
+  return umma_split_global_list_len(B, C, D, K, gr, group_splits, n_splits, split_C_total);
+}
+
 int hgr_score_topk_plan(int64_t B, int64_t C, int64_t D, int K, int32_t* plan) {
   HGR_CHECK_ARG(plan != nullptr, "hgr_score_topk_plan: null plan");
   HGR_CHECK_ARG(K >= 1 && K <= HGR_TOPK_MAX, "hgr_score_topk_plan: K = %d outside [1, %d]", K, HGR_TOPK_MAX);
@@ -366,6 +471,56 @@ int hgr_topk_merge_certified(const float* part_val, const int32_t* part_idx, con
   m.shard_scale = scale;
   m.repair_count = repair_count;
   return launch_topk_merge(m, static_cast<cudaStream_t>(stream));
+}
+
+int hgr_topk_merge_splits_certified(const float* part_val, const int32_t* part_idx, const float* part_bound, int64_t P,
+                                    int64_t B, int K, int n_splits, int64_t part_stride, int64_t bound_stride,
+                                    int64_t split_stride, const int32_t* targets, const uint8_t* node_splits,
+                                    int64_t n_nodes, float* topk_val, int32_t* topk_idx, int64_t* counts, const void* X,
+                                    int64_t D, const hgr_shard_t* shards, float scale, unsigned int* repair_count,
+                                    void* stream) {
+  HGR_CHECK_ARG(P >= 1 && P <= kMaxScatterBlocks && B >= 0, "hgr_topk_merge_splits_certified: P = %lld outside [1, %d]",
+                (long long)P, kMaxScatterBlocks);
+  HGR_CHECK_ARG(K >= 1 && K <= HGR_TOPK_MAX, "hgr_topk_merge_splits_certified: K = %d outside [1, %d]", K, HGR_TOPK_MAX);
+  HGR_CHECK_ARG(n_splits >= 1 && n_splits <= kMaxSplits, "hgr_topk_merge_splits_certified: %d splits outside [1, %d]",
+                n_splits, kMaxSplits);
+  if (B == 0) return HGR_OK;
+  HGR_CHECK_ARG(topk_val && topk_idx && part_val && part_idx && part_bound,
+                "hgr_topk_merge_splits_certified: null lists / bounds / output");
+  HGR_CHECK_ARG(node_splits && n_nodes > 0, "hgr_topk_merge_splits_certified: the repair needs node_splits");
+  HGR_CHECK_ARG(counts == nullptr || targets, "hgr_topk_merge_splits_certified: counting needs targets");
+  HGR_CHECK_ARG(X && shards && D > 0 && D % 8 == 0 && aligned16(X),
+                "hgr_topk_merge_splits_certified: the repair needs X (16-byte aligned, D %% 8 == 0) and the shard table");
+  HGR_CHECK_ARG(part_stride >= B * K, "hgr_topk_merge_splits_certified: part_stride < B*K");
+  HGR_CHECK_ARG(bound_stride >= B, "hgr_topk_merge_splits_certified: bound_stride < B");
+  // value lists, id lists and bounds of a split all sit at + s * split_stride: its area spans all three
+  HGR_CHECK_ARG(n_splits == 1 || split_stride >= 2 * P * part_stride + P * bound_stride,
+                "hgr_topk_merge_splits_certified: split_stride %lld < %lld: the areas of two splits overlap",
+                (long long)split_stride, (long long)(2 * P * part_stride + P * bound_stride));
+  HGR_CHECK_ARG(scale > 0.f, "hgr_topk_merge_splits_certified: scale must be > 0");
+  SplitCertArgs m{};
+  m.part_val = part_val;
+  m.part_idx = part_idx;
+  m.part_bound = part_bound;
+  m.P = P;
+  m.B = B;
+  m.K = K;
+  m.S = n_splits;
+  m.part_stride = part_stride;
+  m.bound_stride = bound_stride;
+  m.split_stride = split_stride;
+  m.targets = targets;
+  m.node_splits = node_splits;
+  m.n_nodes = n_nodes;
+  m.topk_val = topk_val;
+  m.topk_idx = topk_idx;
+  m.counts = counts;
+  m.shards = shards;
+  m.xrows = X;
+  m.xD8 = static_cast<int>(D / 8);
+  m.scale = scale;
+  m.repair_count = repair_count;
+  return launch_topk_split_merge_certified(m, static_cast<cudaStream_t>(stream));
 }
 
 int64_t hgr_sample_replay(const uint32_t* words, int64_t n_words, int64_t n, int64_t k, int64_t setsize, int32_t* out_pos,
@@ -629,6 +784,33 @@ int hgr_hier_finish_rows_gathered(const uint64_t* parts, int n_parts, int64_t pa
   return launch_hier_finish_gathered(reinterpret_cast<const unsigned long long*>(parts), n_parts, part_stride, n_rows, M,
                                      n_levels, sorted_to_pos, first_out, targets, n_nodes, chain_ptr, chain_pos, chain_level,
                                      lvl_idx, top1, counts, static_cast<cudaStream_t>(stream));
+}
+
+int hgr_hier_finish_rows_gathered_splits(const uint64_t* parts, int n_parts, int64_t part_stride, int64_t n_rows,
+                                         int64_t M, int n_levels, const int32_t* sorted_to_pos, const int32_t* first_out,
+                                         const int32_t* targets, int64_t n_nodes, const int32_t* chain_ptr,
+                                         const int32_t* chain_pos, const int32_t* chain_level, const uint8_t* node_splits,
+                                         int n_splits, int64_t* counts, void* stream) {
+  HGR_CHECK_ARG(n_rows >= 0 && M > 0 && M <= (int64_t(1) << 31) - 512,
+                "hgr_hier_finish_rows_gathered_splits: bad sizes n_rows=%lld M=%lld", (long long)n_rows, (long long)M);
+  HGR_CHECK_ARG(n_nodes > 0 && n_nodes < (int64_t(1) << 31) - 1, "hgr_hier_finish_rows_gathered_splits: n_nodes = %lld",
+                (long long)n_nodes);
+  HGR_CHECK_ARG(n_levels >= 1 && n_levels <= 32, "hgr_hier_finish_rows_gathered_splits: %d levels outside [1, 32]", n_levels);
+  HGR_CHECK_ARG(n_parts >= 1 && n_parts <= kMaxScatterBlocks,
+                "hgr_hier_finish_rows_gathered_splits: n_parts = %d outside [1, %d]", n_parts, kMaxScatterBlocks);
+  HGR_CHECK_ARG(n_splits >= 1 && n_splits <= kMaxSplits, "hgr_hier_finish_rows_gathered_splits: %d splits outside [1, %d]",
+                n_splits, kMaxSplits);
+  HGR_CHECK_ARG(part_stride >= n_rows * n_levels, "hgr_hier_finish_rows_gathered_splits: part_stride < n_rows * n_levels");
+  if (n_rows == 0) return HGR_OK;
+  HGR_CHECK_ARG(parts && sorted_to_pos && first_out && targets && chain_ptr && chain_pos && chain_level && node_splits &&
+                    counts,
+                "hgr_hier_finish_rows_gathered_splits: null pointer");
+  HGR_CHECK_ARG((reinterpret_cast<uintptr_t>(parts) & 7u) == 0,
+                "hgr_hier_finish_rows_gathered_splits: parts must be 8-byte aligned");
+  return launch_hier_finish_gathered_splits(reinterpret_cast<const unsigned long long*>(parts), n_parts, part_stride,
+                                            n_rows, M, n_levels, sorted_to_pos, first_out, targets, n_nodes, chain_ptr,
+                                            chain_pos, chain_level, node_splits, n_splits, counts,
+                                            static_cast<cudaStream_t>(stream));
 }
 
 size_t hgr_masked_ce_workspace_bytes(int64_t B, int64_t U, int64_t T) { return masked_ce_workspace_bytes(B, U, T) + 16; }

@@ -216,6 +216,19 @@ hier_finish_gathered_kernel(const unsigned long long* __restrict__ parts, int n_
                     n_nodes, chain_ptr, chain_pos, chain_level, lvl_idx, top1, counts);
 }
 
+// hgr_hier_finish_rows_gathered_splits: the gathered words, counted per split of the row's label
+__global__ void __launch_bounds__(kRowsPerBlock * 32)
+hier_finish_gathered_splits_kernel(const unsigned long long* __restrict__ parts, int n_parts, int64_t part_stride,
+                                   int64_t B, int64_t M, int n_levels, const int32_t* __restrict__ sorted_to_pos,
+                                   const int32_t* __restrict__ first_out, const int32_t* __restrict__ targets,
+                                   int64_t n_nodes, const int32_t* __restrict__ chain_ptr,
+                                   const int32_t* __restrict__ chain_pos, const int32_t* __restrict__ chain_level,
+                                   const uint8_t* __restrict__ node_splits, int n_splits, unsigned long long* counts) {
+  finish_rows_block<GatheredWords, true>(GatheredWords{parts, n_parts, part_stride}, B, M, n_levels, sorted_to_pos,
+                                         first_out, targets, n_nodes, chain_ptr, chain_pos, chain_level, nullptr, nullptr,
+                                         counts, node_splits, n_splits);
+}
+
 struct HierDst {
   unsigned long long* p[kMaxScatterBlocks];
 };
@@ -290,6 +303,19 @@ int launch_hier_finish_rows_splits(unsigned long long* lvl_best, int64_t B, int6
   hier_finish_rows_splits_kernel<<<blocks, kRowsPerBlock * 32, 0, stream>>>(
       lvl_best, B, M, n_levels, sorted_to_pos, first_out, targets, n_nodes, chain_ptr, chain_pos, chain_level,
       node_splits, n_splits, reinterpret_cast<unsigned long long*>(counts));
+  HGR_CHECK_LAUNCH();
+  return HGR_OK;
+}
+
+int launch_hier_finish_gathered_splits(const unsigned long long* parts, int n_parts, int64_t part_stride, int64_t B,
+                                       int64_t M, int n_levels, const int32_t* sorted_to_pos, const int32_t* first_out,
+                                       const int32_t* targets, int64_t n_nodes, const int32_t* chain_ptr,
+                                       const int32_t* chain_pos, const int32_t* chain_level, const uint8_t* node_splits,
+                                       int n_splits, int64_t* counts, cudaStream_t stream) {
+  const int blocks = static_cast<int>((B + kRowsPerBlock - 1) / kRowsPerBlock);     // one warp per image row
+  hier_finish_gathered_splits_kernel<<<blocks, kRowsPerBlock * 32, 0, stream>>>(
+      parts, n_parts, part_stride, B, M, n_levels, sorted_to_pos, first_out, targets, n_nodes, chain_ptr, chain_pos,
+      chain_level, node_splits, n_splits, reinterpret_cast<unsigned long long*>(counts));
   HGR_CHECK_LAUNCH();
   return HGR_OK;
 }

@@ -291,14 +291,17 @@ int launch_score_topk_umma(const __nv_bfloat16* X, const __nv_bfloat16* bank, co
 // repair time stays below 1.5 % of the call (the rule of pick_list_len, the call being the GEMM over all C columns)
 // for EVERY split is taken -- so a small split covered by a few long lists per row does not get repaired on every row.
 
-static int pick_list_len_splits(int K, int64_t B, int64_t C, int64_t D, const Sched& s, const Groups& gr,
-                                const uint8_t* group_splits, int S) {
-  const int exact = K <= 8 ? 8 : (K <= 12 ? 12 : (K <= 20 ? 20 : 32));
+// Per split: its columns in this bank (cs), the columns of its largest list (cols) and the most lists of it a row has.
+struct SplitStats {
   int64_t cs[kMaxSplits] = {}, cols[kMaxSplits] = {};
   int lists[kMaxSplits] = {};
+};
+
+static SplitStats split_stats(const Sched& s, const Groups& gr, const uint8_t* group_splits, int S) {
+  SplitStats st;
   for (int g = 0; g < gr.n; ++g)
     for (int sp = 0; sp < S; ++sp)
-      if ((group_splits[g] >> sp) & 1u) cs[sp] += gr.end[g] - gr.begin(g);
+      if ((group_splits[g] >> sp) & 1u) st.cs[sp] += gr.end[g] - gr.begin(g);
   for (int32_t mt = 0; mt < s.MT; ++mt) {
     int n[kMaxSplits] = {};
     const int parts = group_parts(s, gr, mt);
@@ -308,11 +311,21 @@ static int pick_list_len_splits(int K, int64_t B, int64_t C, int64_t D, const Sc
       for (int sp = 0; sp < S; ++sp) {
         if (!((group_splits[g] >> sp) & 1u)) continue;
         ++n[sp];
-        cols[sp] = c1 - c0 > cols[sp] ? c1 - c0 : cols[sp];
+        st.cols[sp] = c1 - c0 > st.cols[sp] ? c1 - c0 : st.cols[sp];
       }
     }
-    for (int sp = 0; sp < S; ++sp) lists[sp] = n[sp] > lists[sp] ? n[sp] : lists[sp];
+    for (int sp = 0; sp < S; ++sp) st.lists[sp] = n[sp] > st.lists[sp] ? n[sp] : st.lists[sp];
   }
+  return st;
+}
+
+static int pick_list_len_splits(int K, int64_t B, int64_t C, int64_t D, const Sched& s, const Groups& gr,
+                                const uint8_t* group_splits, int S) {
+  const int exact = K <= 8 ? 8 : (K <= 12 ? 12 : (K <= 20 ? 20 : 32));
+  const SplitStats st = split_stats(s, gr, group_splits, S);
+  const int64_t* cs = st.cs;
+  const int64_t* cols = st.cols;
+  const int* lists = st.lists;
   const double t_call = 2.0 * static_cast<double>(B) * static_cast<double>(C) * static_cast<double>(D) / (0.6 * 1.6e15);
   const int cand[4] = {8, 10, 12, 16};
   for (int i = 0; i < 4; ++i) {
@@ -331,6 +344,35 @@ static int pick_list_len_splits(int K, int64_t B, int64_t C, int64_t D, const Sc
   return exact;
 }
 
+// Class shard of the union bank (hgr_score_topk_splits_scatter_bounded): the certificate of split s is taken by the row
+// owner against s's GLOBAL K-th value, so -- as pick_list_len_global does for one bank -- a list's share is its columns
+// over the split's global class count split_C_total[s], a row has lists_s * split_C_total[s] / cs_s lists of s over all
+// ranks, and a repair re-scans s's rows of one shard (budgeted at 1.5 us per bank row of 1024 elements, NVLink).  The
+// narrowest length whose expected repair time stays below 1.5 % of this rank's GEMM for every split is taken.
+static int pick_list_len_splits_global(int K, int64_t B, int64_t C, int64_t D, const Sched& s, const Groups& gr,
+                                       const uint8_t* group_splits, int S, const int64_t* split_C_total) {
+  const int exact = K <= 8 ? 8 : (K <= 12 ? 12 : (K <= 20 ? 20 : 32));
+  const SplitStats st = split_stats(s, gr, group_splits, S);
+  const double t_call = 2.0 * static_cast<double>(B) * static_cast<double>(C) * static_cast<double>(D) / (0.6 * 1.6e15);
+  const int cand[4] = {8, 10, 12, 16};
+  for (int i = 0; i < 4; ++i) {
+    const int kl = cand[i];
+    if (kl >= K) break;
+    bool ok = true;
+    for (int sp = 0; sp < S && ok; ++sp) {
+      if (st.cs[sp] == 0) continue;
+      const double total = static_cast<double>(split_C_total[sp] > st.cs[sp] ? split_C_total[sp] : st.cs[sp]);
+      const double share = static_cast<double>(st.cols[sp]) / total > 1.0 ? 1.0 : static_cast<double>(st.cols[sp]) / total;
+      const double lists = static_cast<double>(st.lists[sp]) * total / static_cast<double>(st.cs[sp]);
+      const double repairs = static_cast<double>(B) * lists * overflow_bound(K, kl, share);
+      const double t_repair = static_cast<double>(st.cs[sp]) * (static_cast<double>(D) / 1024.0) * 1.5e-6;
+      ok = repairs * t_repair < 0.015 * t_call;
+    }
+    if (ok) return kl;
+  }
+  return exact;
+}
+
 // The schedule and the list length of a call depend only on (B, C, D, K, group table, split bits) and visit every
 // (row tile, slot): eager callers (evaluate.test, SplitEval.update) make the same call every batch, so the last few
 // plans are kept.
@@ -340,12 +382,13 @@ struct SplitPlan {
   bool exact = false;
   Groups gr{};
   uint8_t splits[kMaxGroups] = {};
+  int64_t ctot[kMaxSplits] = {};   // global class count of every split (class shard), all 0 otherwise
   Sched sched{};
   int KL = 0;
 };
 
 static SplitPlan split_plan(int64_t B, int64_t C, int64_t D, int K, const Groups& gr, const uint8_t* group_splits, int S,
-                            bool exact) {
+                            bool exact, const int64_t* split_C_total = nullptr) {
   constexpr int kSlots = 8;
   static SplitPlan cache[kSlots];
   static int next = 0;
@@ -354,9 +397,11 @@ static SplitPlan split_plan(int64_t B, int64_t C, int64_t D, int K, const Groups
   key.B = B, key.C = C, key.D = D, key.K = K, key.S = S, key.exact = exact;
   key.gr = gr;
   for (int g = 0; g < gr.n && group_splits; ++g) key.splits[g] = group_splits[g];
+  for (int sp = 0; sp < S && split_C_total; ++sp) key.ctot[sp] = split_C_total[sp];
   auto same = [&](const SplitPlan& e) {
     return e.B == key.B && e.C == key.C && e.D == key.D && e.K == key.K && e.S == key.S && e.exact == key.exact &&
-           std::memcmp(&e.gr, &key.gr, sizeof(Groups)) == 0 && std::memcmp(e.splits, key.splits, kMaxGroups) == 0;
+           std::memcmp(&e.gr, &key.gr, sizeof(Groups)) == 0 && std::memcmp(e.splits, key.splits, kMaxGroups) == 0 &&
+           std::memcmp(e.ctot, key.ctot, sizeof(key.ctot)) == 0;
   };
   {
     std::lock_guard<std::mutex> lk(mu);
@@ -365,7 +410,9 @@ static SplitPlan split_plan(int64_t B, int64_t C, int64_t D, int K, const Groups
   }
   key.sched = make_sched_groups(B, gr, usable_sms() / 2, 2 * kTileM);
   const int exact_kl = K <= 8 ? 8 : (K <= 12 ? 12 : (K <= 20 ? 20 : 32));
-  key.KL = exact || group_splits == nullptr ? exact_kl : pick_list_len_splits(K, B, C, D, key.sched, gr, group_splits, S);
+  key.KL = exact || group_splits == nullptr ? exact_kl
+           : split_C_total ? pick_list_len_splits_global(K, B, C, D, key.sched, gr, group_splits, S, split_C_total)
+                           : pick_list_len_splits(K, B, C, D, key.sched, gr, group_splits, S);
   std::lock_guard<std::mutex> lk(mu);
   cache[next] = key;
   next = (next + 1) % kSlots;
@@ -425,6 +472,53 @@ int launch_score_topk_splits_umma(const __nv_bfloat16* X, const __nv_bfloat16* b
   m.bank = bank;
   m.D8 = static_cast<int>(D / 8);
   m.rescan_count = p.stats;
+  return launch_topk_split_merge(m, stream);
+}
+
+int umma_split_global_list_len(int64_t B, int64_t C, int64_t D, int K, const Groups& gr, const uint8_t* group_splits,
+                               int S, const int64_t* split_C_total) {
+  return split_plan(B, C, D, K, gr, group_splits, S, false, split_C_total).KL;
+}
+
+int launch_score_topk_splits_scatter_umma(const __nv_bfloat16* X, const __nv_bfloat16* bank, const int32_t* col_id,
+                                          int32_t id_base, int64_t B, int64_t C, int64_t D, float scale, int K,
+                                          const Groups& gr, const uint8_t* group_splits, int S,
+                                          const int64_t* split_C_total, void* ws, size_t ws_bytes,
+                                          const OutScatter& scatter, int64_t split_stride, cudaStream_t stream) {
+  if (ws == nullptr || ws_bytes < umma_split_workspace_bytes(B, gr, K))
+    return set_error(HGR_ERR_WORKSPACE, "hgr_score_topk_splits_scatter_bounded: workspace %zu < %zu bytes", ws_bytes,
+                     umma_split_workspace_bytes(B, gr, K));
+  CUtensorMap mx, mb;
+  Params p{};
+  int rc = common_setup(X, bank, B, C, D, &mx, &mb, &p);
+  if (rc != HGR_OK) return rc;
+  const SplitPlan plan = split_plan(B, C, D, K, gr, group_splits, S, false, split_C_total);
+  p.sched = plan.sched;
+  p.groups = gr;
+  p.scale = scale;
+  p.stats = static_cast<unsigned int*>(ws);
+  const int KL = plan.KL;
+  p.KL = KL;
+  p.part_val = reinterpret_cast<float*>(static_cast<uint8_t*>(ws) + kWsHeaderBytes);
+  p.part_idx = reinterpret_cast<int32_t*>(p.part_val + static_cast<size_t>(p.sched.P) * B * KL);
+  rc = launch_pair_kernel(kEpiTopkGroups, KL, mx, mb, p, stream);
+  if (rc != HGR_OK) return rc;
+  SplitMergeArgs m{};
+  m.part_val = p.part_val;
+  m.part_idx = p.part_idx;
+  m.B = B;
+  m.C = C;
+  m.KL = KL;
+  m.K = K;
+  m.S = S;
+  m.sched = p.sched;
+  m.groups = gr;
+  for (int g = 0; g < gr.n; ++g) m.group_splits[g] = group_splits[g];
+  m.col_id = col_id;
+  m.id_base = id_base;
+  m.scale = scale;
+  m.scatter = scatter;
+  m.split_stride = split_stride;
   return launch_topk_split_merge(m, stream);
 }
 

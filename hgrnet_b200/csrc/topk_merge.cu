@@ -729,7 +729,9 @@ __device__ __noinline__ Cand split_repair_cold(const SplitMergeArgs* a, int64_t 
   return c;
 }
 
-template <int kMaxListsPerLane>
+// kScatter (hgr_score_topk_splits_scatter_bounded, producer of the class-sharded head): no local certificate or repair;
+// split s of the row goes to its owner's slot next to the bound of what the split's full narrow lists dropped.
+template <int kMaxListsPerLane, bool kScatter>
 __global__ void __launch_bounds__(kMergeWarps * 32, 4)  // (the cold repair function must not set the register count)
 topk_split_merge_kernel(const __grid_constant__ SplitMergeArgs a) {
   extern __shared__ uint8_t smem_raw[];
@@ -829,6 +831,28 @@ topk_split_merge_kernel(const __grid_constant__ SplitMergeArgs a) {
           my_i = bi;
         }
       }
+      if constexpr (kScatter) {
+        // bound of split s: the largest last entry of a full narrow list of s (K-entry lists drop nothing that matters)
+        float b = -INFINITY;
+        if (KL < K) {
+#pragma unroll
+          for (int q = 0; q < kMaxListsPerLane; ++q) {
+            const int p = lane + 32 * q;
+            if (((lmask[q] >> s) & 1u) && li[p * KL + KL - 1] >= 0) b = fmaxf(b, lv[p * KL + KL - 1]);
+          }
+        }
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) b = fmaxf(b, __shfl_xor_sync(0xffffffffu, b, o));
+        const int64_t g = row / a.scatter.block_rows;
+        const int64_t orow = row - g * a.scatter.block_rows;
+        const int64_t so = s * a.split_stride;
+        if (lane < K) {
+          a.scatter.val[g][so + orow * K + lane] = my_i >= 0 ? my_v * a.scale : -INFINITY;
+          a.scatter.idx[g][so + orow * K + lane] = my_i >= 0 ? (a.col_id ? a.col_id[my_i] : a.id_base + my_i) : -1;
+        }
+        if (lane == 0) a.scatter.bound[g][so + orow] = b * a.scale;
+        continue;
+      }
       // certificate against the split's own K-th value: a full narrow list of s that ends at or above it may hide
       // members of the split's top-K
       bool doubt = false;
@@ -860,6 +884,175 @@ topk_split_merge_kernel(const __grid_constant__ SplitMergeArgs a) {
       }
       if (a.counts && ((tbits >> s) & 1u)) {   // the row's label is a class of split s
         const unsigned m = __ballot_sync(0xffffffffu, lane < K && gid >= 0 && gid == target);
+        if (lane == 0) {
+          atomicAdd(&s_cnt[s][HGR_NUM_HITS], 1u);
+          if (m != 0) {
+            const int pos = __ffs(m) - 1;
+#pragma unroll
+            for (int c = 0; c < HGR_NUM_HITS; ++c)
+              if (pos < hit_cut(c)) atomicAdd(&s_cnt[s][c], 1u);
+          }
+        }
+      }
+    }
+  }
+  __syncthreads();
+  if (a.counts) {
+    for (int i = threadIdx.x; i < a.S * (HGR_NUM_HITS + 1); i += blockDim.x) {
+      const unsigned int v = (&s_cnt[0][0])[i];
+      if (v) atomicAdd(reinterpret_cast<unsigned long long*>(a.counts) + i, static_cast<unsigned long long>(v));
+    }
+  }
+}
+
+// ---- per-split certified merge of the class-sharded head (hgr_topk_merge_splits_certified) -------------------------
+// Owner side of hgr_score_topk_splits_scatter_bounded.  For every owned row and split s the P shard lists of s are merged
+// in the order (value desc, shard asc, position in the list asc): each list is the shard's top-K of s in (value desc,
+// local bank row asc) order, so the result is the top-K of s's rows concatenated in rank-major order -- what score_topk
+// returns on that bank.  The merged K-th value must strictly beat every shard's bound of s; a doubtful (row, split,
+// shard) is re-scanned exactly from the shard table.
+
+// Exact local top-K of split s on one shard: its rows whose node has bit s in node_splits, in ascending row order (as
+// scan_row_range_lanes; membership is tested before the dot product).  Every lane holds the same list.
+__device__ __forceinline__ void scan_shard_split(const uint4* __restrict__ xr, const hgr_shard_t& sh, const uint8_t* node_splits,
+                                                 int64_t n_nodes, int s, int D8, int lane, SortedList<HGR_TOPK_MAX>& list) {
+  const uint4* bank4 = reinterpret_cast<const uint4*>(sh.bank);
+  for (int64_t cb = 0; cb < sh.C; cb += 32) {
+    const int64_t c = cb + lane;
+    bool ok = c < sh.C;
+    if (ok) {
+      const int64_t node = sh.col_id ? sh.col_id[c] : sh.id_base + c;
+      ok = node >= 0 && node < n_nodes && ((node_splits[node] >> s) & 1u);
+    }
+    float v = -INFINITY;
+    if (ok) {
+      const uint4* b = bank4 + c * D8;
+      float a0 = 0.f, a1 = 0.f;
+      int idx = 0;
+      for (; idx + 1 < D8; idx += 2) {
+        a0 = dot8_bf16(__ldg(b + idx), __ldg(xr + idx), a0);
+        a1 = dot8_bf16(__ldg(b + idx + 1), __ldg(xr + idx + 1), a1);
+      }
+      if (idx < D8) a0 = dot8_bf16(__ldg(b + idx), __ldg(xr + idx), a0);
+      v = a0 + a1;
+    }
+    const unsigned members = __ballot_sync(0xffffffffu, ok);
+    float vmax = v;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) vmax = fmaxf(vmax, __shfl_xor_sync(0xffffffffu, vmax, o));
+    if (members != 0u && vmax > list.thr()) {
+      for (int l = 0; l < 32; ++l) {
+        const float vl = __shfl_sync(0xffffffffu, v, l);
+        if (((members >> l) & 1u) && vl > list.thr()) list.insert(vl, static_cast<int32_t>(cb + l));
+      }
+    }
+  }
+}
+
+// Exact repair of split s of a row (cold): the doubtful shards (bits of `dm`) are re-scanned, their exact top-K of s
+// mapped to node ids and scaled like the producer did; the lists of the other shards are final as they are (what such
+// a shard dropped is below the old K-th value, which can only rise).  Shards are visited in ascending order and
+// SortedList keeps the first of equal values, so the tie order stays (value desc, shard asc, local row asc).
+// Returns rank `lane` of the repaired row.
+__device__ __noinline__ Cand split_cert_repair_cold(const SplitCertArgs* a, int64_t row, int lane, int s, unsigned dm) {
+  if (lane == 0 && a->repair_count) atomicAdd(a->repair_count, 1u);
+  SortedList<HGR_TOPK_MAX> full;
+  full.init();
+  const int K = a->K;
+  const uint4* xr = reinterpret_cast<const uint4*>(a->xrows) + row * a->xD8;
+  for (int p = 0; p < static_cast<int>(a->P); ++p) {
+    if ((dm >> p) & 1u) {
+      const hgr_shard_t sh = a->shards[p];
+      SortedList<HGR_TOPK_MAX> sub;
+      sub.init();
+      scan_shard_split(xr, sh, a->node_splits, a->n_nodes, s, a->xD8, lane, sub);
+      for (int k = 0; k < K; ++k) {
+        const int32_t it = sub.i[k];
+        const float v = sub.v[k] * a->scale;
+        if (it >= 0 && v > full.thr()) full.insert(v, sh.col_id ? sh.col_id[it] : sh.id_base + it);
+      }
+    } else {
+      const int64_t base = s * a->split_stride + p * a->part_stride + row * K;
+      for (int k = 0; k < K; ++k) {
+        const int32_t it = a->part_idx[base + k];
+        const float v = a->part_val[base + k];
+        if (it >= 0 && v > full.thr()) full.insert(v, it);
+      }
+    }
+  }
+  Cand c;
+  c.v = -INFINITY;
+  c.i = -1;
+#pragma unroll
+  for (int k = 0; k < HGR_TOPK_MAX; ++k) {
+    if (lane == k) {
+      c.v = full.v[k];
+      c.i = full.i[k];
+    }
+  }
+  return c;
+}
+
+// One warp per row; lane p holds the head of shard p's list.  Per output rank: the largest head value, the lowest lane
+// among equals, and that lane advances.
+__global__ void __launch_bounds__(kMergeWarps * 32)   // (a cap on the registers makes the merge spill around the call)
+topk_split_cert_kernel(const __grid_constant__ SplitCertArgs a) {
+  __shared__ unsigned int s_cnt[kMaxSplits][HGR_NUM_HITS + 1];
+  for (int i = threadIdx.x; i < kMaxSplits * (HGR_NUM_HITS + 1); i += blockDim.x) (&s_cnt[0][0])[i] = 0u;
+  __syncthreads();
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int K = a.K;
+  const int P = static_cast<int>(a.P);
+  const int64_t row = static_cast<int64_t>(blockIdx.x) * kMergeWarps + warp;
+  if (row < a.B) {
+    const int32_t target = a.targets ? a.targets[row] : -1;
+    const uint32_t tbits = (target >= 0 && target < a.n_nodes) ? a.node_splits[target] : 0u;
+    for (int s = 0; s < a.S; ++s) {
+      const int64_t lbase = s * a.split_stride + lane * a.part_stride + row * K;
+      int head = 0;
+      float hv = -INFINITY;
+      int32_t hi = -1;
+      if (lane < P) {
+        hi = a.part_idx[lbase];
+        hv = a.part_val[lbase];
+      }
+      float my_v = -INFINITY;
+      int32_t my_i = -1;
+      for (int r = 0; r < K; ++r) {
+        const bool live = hi >= 0;
+        const uint32_t mkey = __reduce_max_sync(0xffffffffu, live ? order_key(hv) : 0u);
+        const unsigned cand = __ballot_sync(0xffffffffu, live && order_key(hv) == mkey);
+        if (cand == 0u) break;                      // every list exhausted: the rest stays (-inf, -1)
+        const int win = __ffs(cand) - 1;
+        const float bv = __shfl_sync(0xffffffffu, hv, win);
+        const int32_t bi = __shfl_sync(0xffffffffu, hi, win);
+        if (lane == r) {
+          my_v = bv;
+          my_i = bi;
+        }
+        if (lane == win) {
+          ++head;
+          hi = head < K ? a.part_idx[lbase + head] : -1;
+          hv = hi >= 0 ? a.part_val[lbase + head] : -INFINITY;
+        }
+      }
+      // certificate: the merged K-th value strictly above every shard's bound of s (fewer than K merged: -inf, so any
+      // shard that dropped something is doubtful)
+      const float kth = __shfl_sync(0xffffffffu, my_i >= 0 ? my_v : -INFINITY, K - 1);
+      const float bnd = lane < P ? a.part_bound[s * a.split_stride + lane * a.bound_stride + row] : -INFINITY;
+      const unsigned dm = __ballot_sync(0xffffffffu, bnd > -INFINITY && bnd >= kth);
+      if (dm != 0u) {
+        const Cand c = split_cert_repair_cold(&a, row, lane, s, dm);
+        my_v = c.v;
+        my_i = c.i;
+      }
+      if (lane < K) {
+        const int64_t o = (s * a.B + row) * K + lane;
+        a.topk_val[o] = my_i >= 0 ? my_v : -INFINITY;
+        a.topk_idx[o] = my_i;
+      }
+      if (a.counts && ((tbits >> s) & 1u)) {   // the row's label is a class of split s
+        const unsigned m = __ballot_sync(0xffffffffu, lane < K && my_i >= 0 && my_i == target);
         if (lane == 0) {
           atomicAdd(&s_cnt[s][HGR_NUM_HITS], 1u);
           if (m != 0) {
@@ -1005,6 +1198,16 @@ int launch_topk_merge(const MergeArgs& args, cudaStream_t stream) {
   return HGR_OK;
 }
 
+template <int kMaxListsPerLane, bool kScatter>
+static int launch_split_merge_kernel(const SplitMergeArgs& args, int blocks, size_t smem, cudaStream_t stream) {
+  if (smem > 48 * 1024)
+    HGR_CHECK_CUDA(cudaFuncSetAttribute(topk_split_merge_kernel<kMaxListsPerLane, kScatter>,
+                                        cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
+  topk_split_merge_kernel<kMaxListsPerLane, kScatter><<<blocks, kMergeWarps * 32, smem, stream>>>(args);
+  HGR_CHECK_LAUNCH();
+  return HGR_OK;
+}
+
 int launch_topk_split_merge(const SplitMergeArgs& args, cudaStream_t stream) {
   if (args.B == 0) return HGR_OK;
   if (args.sched.P > 32 * kSplitDoubtWords)
@@ -1012,17 +1215,18 @@ int launch_topk_split_merge(const SplitMergeArgs& args, cudaStream_t stream) {
   const int blocks = static_cast<int>((args.B + kMergeWarps - 1) / kMergeWarps);
   const size_t smem = static_cast<size_t>(kMergeWarps) * args.sched.P * args.KL * 8;
   if (smem > 200 * 1024) return set_error(HGR_ERR_UNSUPPORTED, "topk split merge: %zu bytes of lists per CTA", smem);
-  if (args.sched.P <= 64) {
-    if (smem > 48 * 1024)
-      HGR_CHECK_CUDA(cudaFuncSetAttribute(topk_split_merge_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                          static_cast<int>(smem)));
-    topk_split_merge_kernel<2><<<blocks, kMergeWarps * 32, smem, stream>>>(args);
-  } else {
-    if (smem > 48 * 1024)
-      HGR_CHECK_CUDA(cudaFuncSetAttribute(topk_split_merge_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                          static_cast<int>(smem)));
-    topk_split_merge_kernel<4><<<blocks, kMergeWarps * 32, smem, stream>>>(args);
-  }
+  const bool scatter = args.scatter.n_blocks > 0;
+  if (args.sched.P <= 64)
+    return scatter ? launch_split_merge_kernel<2, true>(args, blocks, smem, stream)
+                   : launch_split_merge_kernel<2, false>(args, blocks, smem, stream);
+  return scatter ? launch_split_merge_kernel<4, true>(args, blocks, smem, stream)
+                 : launch_split_merge_kernel<4, false>(args, blocks, smem, stream);
+}
+
+int launch_topk_split_merge_certified(const SplitCertArgs& args, cudaStream_t stream) {
+  if (args.B == 0) return HGR_OK;
+  const int blocks = static_cast<int>((args.B + kMergeWarps - 1) / kMergeWarps);
+  topk_split_cert_kernel<<<blocks, kMergeWarps * 32, 0, stream>>>(args);
   HGR_CHECK_LAUNCH();
   return HGR_OK;
 }

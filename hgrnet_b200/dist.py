@@ -115,18 +115,23 @@ class _RawCuda:
 X_SLOTS = 4  # feature-ingest slots per exchange (ring length per channel: _ring_len)
 
 
-def exchange_layout(B: int, K: int, world: int, slots: int, D: int = 0, n_levels: int = 0):
+def exchange_layout(B: int, K: int, world: int, slots: int, D: int = 0, n_levels: int = 0, n_splits: int = 0):
     """Byte layout of one rank's exchange buffer: a 256-byte header (list flags: one word per producer rank at
     byte 0, feature flags at byte 64), then per slot the value lists ``[world, block_rows, K]`` fp32 followed by
     the id lists ``[world, block_rows, K]`` int32 and the bounds ``[world, block_rows]`` fp32 of the global certificate
-    (``hgr_score_topk_scatter_bounded``), with ``n_levels`` the per-level winner words ``[world, block_rows, n_levels]``
-    uint64 of class-sharded TOR / POR at ``hier_off`` in the slot (``hgr_hier_level_scatter``) and, when ``D`` is given,
-    ``X_SLOTS`` replicas of the normalised image features ``[B, D]`` bf16 (feature ingest, see
+    (``hgr_score_topk_scatter_bounded``) -- with ``n_splits`` one such area per split, ``split_bytes`` apart
+    (``hgr_score_topk_splits_scatter_bounded``) --, with ``n_levels`` the per-level winner words ``[world, block_rows,
+    n_levels]`` uint64 of class-sharded TOR / POR at ``hier_off`` in the slot (``hgr_hier_level_scatter``) and, when
+    ``D`` is given, ``X_SLOTS`` replicas of the normalised image features ``[B, D]`` bf16 (feature ingest, see
     ``PeerExchange.ingest``)."""
     block_rows = (B + world - 1) // world
     part = block_rows * K * 4
     bound_bytes = (world * block_rows * 4 + 15) // 16 * 16     # per producer and row: bound of what the shard dropped
     slot_bytes = 2 * world * part + bound_bytes
+    split = {}
+    if n_splits:
+        split = {"split_bytes": (slot_bytes + 15) // 16 * 16}  # every split's area 16-byte aligned
+        slot_bytes = n_splits * split["split_bytes"]
     hier = {}
     if n_levels:
         # 8-byte aligned: both list areas are multiples of 8 bytes, the bounds of 16, and slots start 16-byte aligned
@@ -135,7 +140,7 @@ def exchange_layout(B: int, K: int, world: int, slots: int, D: int = 0, n_levels
     x_off = (256 + slots * slot_bytes + 255) // 256 * 256
     x_bytes = (B * D * 2 + 255) // 256 * 256
     return {"block_rows": block_rows, "part_bytes": part, "slot_bytes": slot_bytes, "header": 256,
-            "x_off": x_off, "x_bytes": x_bytes, "total": x_off + (X_SLOTS * x_bytes if D else 0), **hier}
+            "x_off": x_off, "x_bytes": x_bytes, "total": x_off + (X_SLOTS * x_bytes if D else 0), **split, **hier}
 
 
 class PeerMemoryUnavailable(RuntimeError):
@@ -261,6 +266,56 @@ def local_level_ends(level_end, lo: int, hi: int) -> List[int]:
     return [min(max(int(e) - lo, 0), hi - lo) for e in level_end]
 
 
+def split_shard_bounds(group_end, world: int):
+    """How the union bank of ``evaluate.split_groups`` is cut over ``world`` ranks: every rank takes its balanced slice
+    ``[floor(r * C_g / world), floor((r + 1) * C_g / world))`` of EVERY group g, so it holds about 1/world of every
+    split (a contiguous cut would leave a small split on one or two ranks).  Returns, per rank, ``(ranges, local_end,
+    kept)``: the union-bank row ranges ``[lo, hi)`` of the groups it holds rows of (``kept``, ascending), concatenated in
+    that order its local bank, and their clipped ends ``local_end`` (strictly ascending: groups without rows here are
+    dropped).  A rank may hold no rows at all."""
+    out = []
+    begins = [0] + [int(e) for e in group_end[:-1]]
+    for r in range(world):
+        ranges, local_end, kept, n = [], [], [], 0
+        for g, (b, e) in enumerate(zip(begins, [int(e) for e in group_end])):
+            lo, hi = b + (e - b) * r // world, b + (e - b) * (r + 1) // world
+            if hi > lo:
+                ranges.append((lo, hi))
+                n += hi - lo
+                local_end.append(n)
+                kept.append(g)
+        out.append((ranges, local_end, kept))
+    return out
+
+
+class SplitShard:
+    """One rank's part of several test splits scored in one pass on the class-sharded head (main.py:104-222 once per
+    split): its slice of every group of ``split_eval``'s union bank (``split_shard_bounds``) with its node ids
+    (``col_id``), its own group table (``group_end`` / ``group_splits``, the masks of the groups it holds), the global
+    class count of every split (``split_C``) and ``node_splits`` / ``names`` / ``S``.  With ``split_eval.hier`` it also
+    holds the rank's ``HierShard`` of the level-sorted train bank (per-split TOR / POR).  ``split_eval`` is an
+    ``evaluate.SplitEval`` (or anything with its ``group_end``, ``group_splits``, ``names``, ``S``, ``node_splits``,
+    ``col_id``, ``bank()`` and ``hier``)."""
+
+    def __init__(self, split_eval, rank: int, world: int):
+        ranges, self.group_end, kept = split_shard_bounds(split_eval.group_end, world)[rank]
+        union = split_eval.bank()
+        self.device = union.device
+        rows = (torch.cat([torch.arange(lo, hi) for lo, hi in ranges]) if ranges
+                else torch.zeros(0, dtype=torch.int64)).to(self.device)
+        self.bank = union.index_select(0, rows).contiguous()
+        self.col_id = split_eval.col_id.index_select(0, rows).to(torch.int32).contiguous()
+        self.C, self.D = self.bank.shape
+        self.group_splits = [int(split_eval.group_splits[g]) for g in kept]
+        self.names, self.S = list(split_eval.names), int(split_eval.S)
+        self.node_splits = split_eval.node_splits
+        ends = [int(e) for e in split_eval.group_end]
+        sizes = [e - b for b, e in zip([0] + ends[:-1], ends)]
+        self.split_C = [sum(n for n, m in zip(sizes, split_eval.group_splits) if (int(m) >> s) & 1) for s in range(self.S)]
+        h = getattr(split_eval, "hier", None)
+        self.hier = HierShard(h.rows_args(), rank, world) if h is not None else None
+
+
 class PeerExchange:
     """Peer-memory exchange of the class-sharded head (no collective call on the data path).
 
@@ -271,11 +326,12 @@ class PeerExchange:
     and raises its flag there (``hgr_peer_signal``); the owner waits for all ``world`` flags (``hgr_peer_wait``) and
     merges its ``world`` lists per row (``hgr_topk_merge``).  ``slots`` batches can be in flight.  With ``n_levels``
     every slot also carries the per-level winner words of class-sharded TOR / POR (``scatter`` / ``merge`` with
-    ``hier``), published by the same flag.
+    ``hier``), published by the same flag.  With ``n_splits`` every slot holds the lists and bounds of that many test
+    splits (``scatter`` / ``merge`` with ``splits``).
     """
 
     def __init__(self, B: int, K: int, device, group=None, slots: int = 4, D: int = 0, _bases=None, _rank=None,
-                 _world=None, n_levels: int = 0):
+                 _world=None, n_levels: int = 0, n_splits: int = 0):
         self.device = torch.device(device)
         self.group = group
         if _bases is None:
@@ -286,7 +342,8 @@ class PeerExchange:
         if self.world > 16:
             raise ValueError("PeerExchange supports up to 16 ranks (HGR_MAX_PEERS)")
         self.B, self.K, self.slots, self.D, self.n_levels = B, K, slots, D, n_levels
-        self.lay = exchange_layout(B, K, self.world, slots, D, n_levels)
+        self.lay = exchange_layout(B, K, self.world, slots, D, n_levels, n_splits)
+        self.split_stride = self.lay.get("split_bytes", 0) // 4     # elements between two splits' areas
         self.block_rows = self.lay["block_rows"]
         self.lo = min(B, self.rank * self.block_rows)
         self.hi = min(B, self.lo + self.block_rows)
@@ -362,13 +419,20 @@ class PeerExchange:
 
     # -- per batch -------------------------------------------------------------------------------------------
     def scatter(self, x_norm: torch.Tensor, bank: torch.Tensor, id_base: int, slot: int, col_id=None,
-                C_total: int = 0, hier: Optional[HierShard] = None) -> None:
+                C_total: int = 0, hier: Optional[HierShard] = None, splits: Optional[SplitShard] = None) -> None:
         """Score the batch against my shard and store the lists at their owners.  ``C_total`` > 0: narrow lists sized
         for the GLOBAL certificate, with the bound of what was dropped next to every list (``merge(certify=...)``).
-        ``hier``: also store my train shard's per-level winner words at the owners (``merge(hier=...)``)."""
+        ``hier``: also store my train shard's per-level winner words at the owners (``merge(hier=...)``).  ``splits``:
+        ``bank`` / ``col_id`` are my part of the split union bank; every split's lists and bounds are stored
+        (``merge(splits=...)``)."""
         val, idx = self.block_ptrs(slot)
-        ops.score_topk_scatter(x_norm, bank, val, idx, self.block_rows, col_id=col_id, id_base=id_base, K=self.K,
-                               bound_block_ptrs=self.bound_ptrs(slot) if C_total else None, C_total=C_total)
+        if splits is not None:
+            ops.score_topk_splits_scatter(x_norm, bank, splits.group_end, splits.group_splits, splits.split_C, val, idx,
+                                          self.bound_ptrs(slot), self.block_rows, self.split_stride, col_id=col_id,
+                                          K=self.K)
+        else:
+            ops.score_topk_scatter(x_norm, bank, val, idx, self.block_rows, col_id=col_id, id_base=id_base, K=self.K,
+                                   bound_block_ptrs=self.bound_ptrs(slot) if C_total else None, C_total=C_total)
         if hier is not None:                 # before the signal: the owner's one wait covers lists and words
             ops.hier_level_scatter(x_norm, hier.bank, hier.level_end_local, hier.row_base, self.hier_ptrs(slot),
                                    self.block_rows)
@@ -376,18 +440,34 @@ class PeerExchange:
 
     def merge(self, slot: int, targets: Optional[torch.Tensor], hits: Optional[torch.Tensor], out=None,
               targets_local: bool = False, certify=None, hier: Optional[HierShard] = None,
-              counts: Optional[torch.Tensor] = None, hier_out=None):
+              counts: Optional[torch.Tensor] = None, hier_out=None, splits: Optional[SplitShard] = None,
+              split_counts: Optional[torch.Tensor] = None):
         """Final top-K (+ hits) of MY rows ``[lo, hi)``; ``targets`` holds the labels of the whole batch (or of my
         rows only with ``targets_local``).  ``certify = (x_norm [B, D], shard table, repair counter)`` after a
         ``scatter(C_total=...)``: rows whose K-th value does not beat every shard's bound are repaired exactly.
         ``hier`` after a ``scatter(hier=...)``: also count TOR / POR of my rows into ``counts`` (``ops.new_hier_counts``);
-        ``hier_out = (lvl_idx [n, n_levels], top1 [n])`` int32 receives their per-level winners and top-1."""
+        ``hier_out = (lvl_idx [n, n_levels], top1 [n])`` int32 receives their per-level winners and top-1.
+        ``splits`` after a ``scatter(splits=...)`` (needs ``certify``): per split the certified top-K of my rows
+        (``[S, n, K]``), Hit@k and rows counted into ``split_counts`` ``[S, HGR_NUM_HITS + 1]``; with ``hier``, ``counts``
+        holds the per-split TOR / POR counters ``[S, HGR_HIER_MAX_CHAIN + 1, 4]``."""
         ops.peer_wait(self.bases[self.rank], self.world, self.seq[1:2])
         n = self.hi - self.lo
         if n <= 0:
             return None
         pv, pi, stride = self.local_parts(slot)
         t = None if targets is None else (targets if targets_local else targets[self.lo:self.hi])
+        if splits is not None:
+            x_norm, table, repairs = certify
+            res = ops.topk_merge_splits_certified(pv, pi, self.local_bounds(slot), self.world, n, self.K, splits.S, stride,
+                                                  self.block_rows, self.split_stride, x_norm[self.lo:self.hi], table,
+                                                  splits.node_splits, self.device, targets=t, counts=split_counts,
+                                                  repair_count=repairs, out=out)
+            if hier is not None:
+                parts, part_stride = self.local_hier(slot)
+                ops.hier_finish_rows_gathered_splits(parts, self.world, part_stride, n, hier.M, hier.n_levels,
+                                                     hier.sorted_to_pos, hier.first_out, t, hier.chain_ptr, hier.chain_pos,
+                                                     hier.chain_level, splits.node_splits, counts)
+            return res
         if certify is not None:
             x_norm, table, repairs = certify
             res = ops.topk_merge_certified(pv, pi, self.local_bounds(slot), self.world, n, self.K, stride, self.block_rows,
@@ -442,14 +522,34 @@ class ShardedEvalStream:
     per-level arg-max GEMM, its winner words travel to the row owners with the lists, under the same flag, and the owner
     finishes its rows after the list merge.  The per-chain-length counters share one device buffer with ``hits``
     (``counters``), so ``host_io`` still makes one D2H copy per batch; ``hier_ratios()`` sums them over ranks.
+
+    ``splits`` (a ``SplitShard`` of this rank, peer exchange with the global certificate only): every batch is scored
+    against the rank's part of several test splits instead of ``bank_shard``, in one pass, as ``EvalStream(splits=...)``
+    does on one GPU.  ``val`` / ``idx`` are ``[S, rows, K]``; the per-split Hit@k / row counters ``split_counts``
+    ``[S, HGR_NUM_HITS + 1]`` and, when the ``SplitShard`` has ``hier``, the per-split TOR / POR counters
+    ``split_hier_counts`` live in ``counters`` too.  ``split_hit_counts()`` / ``split_ratios()`` / ``split_lines()`` sum
+    them over ranks.  With ``splits`` the stream scores nothing against ``bank_shard`` / ``id_base``: ``bank_shard`` only
+    has to agree with the ``SplitShard`` on D and device (pass e.g. ``split_eval.bank()``), and ``id_base`` is unused.
     """
 
     def __init__(self, bank_shard: torch.Tensor, id_base: int, *, batch: int, K: int = 20, steps: int = 8,
                  feat_dtype=torch.float32, banks=None, group=None, use_graph: bool = True, exchange: str = "p2p",
                  channels: int = 4, host_io: bool = False, col_id: Optional[torch.Tensor] = None,
-                 certify: str = "global", hier: Optional[HierShard] = None):
+                 certify: str = "global", hier: Optional[HierShard] = None, splits: Optional[SplitShard] = None):
         if exchange not in ("p2p", "nccl"):
             raise ValueError("exchange must be 'p2p' or 'nccl'")
+        if splits is not None:
+            if exchange != "p2p":
+                raise ValueError("splits need the peer-memory exchange")
+            if certify != "global":
+                raise ValueError("splits need certify='global'")
+            if hier is not None:
+                raise ValueError("splits and hier together: the splits' TOR / POR come with the SplitShard's hier")
+            if banks is not None:
+                raise ValueError("splits do not take a banks= rotation")
+            if splits.D != bank_shard.shape[1] or splits.device != bank_shard.device:
+                raise ValueError("splits: the SplitShard has D = %d on %s, the stream D = %d on %s" % (
+                    splits.D, splits.device, bank_shard.shape[1], bank_shard.device))
         if hier is not None and exchange != "p2p":
             raise ValueError("hier (class-sharded TOR / POR) needs the peer-memory exchange")
         if hier is not None and hier.D != bank_shard.shape[1]:
@@ -474,8 +574,11 @@ class ShardedEvalStream:
         self.C_total = 0
         self.repairs = torch.zeros(1, dtype=torch.int32, device=self.device)
         self._x = [None] * steps
+        self.splits = splits
+        if splits is not None:
+            self.banks, col_id, self.id_base = [splits.bank], splits.col_id, 0
         if self.certify == "global":
-            self.pbanks = [PeerBank(b, col_id, id_base, group) for b in self.banks]
+            self.pbanks = [PeerBank(b, col_id, self.id_base, group) for b in self.banks]
             self.banks = [pb.bank for pb in self.pbanks]
             self.col_id = self.pbanks[0].col_id
             self.C_total = self.pbanks[0].C_total
@@ -484,10 +587,20 @@ class ShardedEvalStream:
             self.dev_labels = [torch.zeros((batch,), dtype=torch.int32, device=self.device) for _ in range(steps)]
         # hit counters, then (with hier) the per-chain-length TOR / POR counters: one buffer, one D2H copy per batch
         self.hier = hier
-        n_counters = ops.HGR_NUM_HITS + (0 if hier is None else (ops.HGR_HIER_MAX_CHAIN + 1) * 4)
+        n_hier = 0 if hier is None else (ops.HGR_HIER_MAX_CHAIN + 1) * 4
+        S = 0 if splits is None else splits.S
+        n_split = S * (ops.HGR_NUM_HITS + 1)
+        n_split_hier = 0 if splits is None or splits.hier is None else S * (ops.HGR_HIER_MAX_CHAIN + 1) * 4
+        n_counters = ops.HGR_NUM_HITS + n_hier + n_split + n_split_hier
         self.counters = torch.zeros(n_counters, dtype=torch.int64, device=self.device)
         self.hits = self.counters[:ops.HGR_NUM_HITS]
-        self.hier_counts = None if hier is None else self.counters[ops.HGR_NUM_HITS:].view(ops.HGR_HIER_MAX_CHAIN + 1, 4)
+        o = ops.HGR_NUM_HITS
+        self.hier_counts = None if hier is None else self.counters[o:o + n_hier].view(ops.HGR_HIER_MAX_CHAIN + 1, 4)
+        o += n_hier
+        self.split_counts = None if splits is None else self.counters[o:o + n_split].view(S, ops.HGR_NUM_HITS + 1)
+        o += n_split
+        self.split_hier_counts = (self.counters[o:o + n_split_hier].view(S, ops.HGR_HIER_MAX_CHAIN + 1, 4)
+                                  if n_split_hier else None)
         self.val = [None] * steps
         self.idx = [None] * steps
         self.row_lo, self.row_hi = 0, batch
@@ -503,8 +616,10 @@ class ShardedEvalStream:
             if steps < 2:
                 raise ValueError("ShardedEvalStream needs steps >= 2 (two batches per exchange channel and replay)")
             self.channels = max(1, min(channels, steps // 2))
+            hs = hier if splits is None else splits.hier
             self.pxs = [PeerExchange(batch, K, self.device, group=group, slots=self.slots, D=D if host_io else 0,
-                                     n_levels=0 if hier is None else hier.n_levels) for _ in range(self.channels)]
+                                     n_levels=0 if hs is None else hs.n_levels, n_splits=S)
+                        for _ in range(self.channels)]
             self._ring, self._xring = [], []
             for c in range(self.channels):
                 n_c = (steps - c + self.channels - 1) // self.channels          # batches of channel c per replay
@@ -514,8 +629,9 @@ class ShardedEvalStream:
             self.side = [torch.cuda.Stream(device=self.device) for _ in range(self.channels)]
             self.row_lo, self.row_hi = self.px.lo, self.px.hi
             n_my = max(0, self.row_hi - self.row_lo)
-            self.val = [torch.empty((n_my, K), dtype=torch.float32, device=self.device) for _ in range(steps)]
-            self.idx = [torch.empty((n_my, K), dtype=torch.int32, device=self.device) for _ in range(steps)]
+            shape = (n_my, K) if splits is None else (S, n_my, K)
+            self.val = [torch.empty(shape, dtype=torch.float32, device=self.device) for _ in range(steps)]
+            self.idx = [torch.empty(shape, dtype=torch.int32, device=self.device) for _ in range(steps)]
             if host_io:
                 # feature ingest: this rank copies only ITS rows (and their labels) from pinned host memory; the
                 # normalised rows reach the other ranks over NVLink (PeerExchange.ingest); Hit@k counters go back
@@ -566,13 +682,14 @@ class ShardedEvalStream:
             x = px.ingest(self.dev_feats[s], j % self._xring[s % self.channels])
             self._x[s] = x
             px.scatter(x, bank, self.id_base, j % self._ring[s % self.channels], col_id=self.col_id, C_total=self.C_total,
-                       hier=self.hier)
+                       hier=self._hier_shard(), splits=self.splits)
             return None
         x = ops.normalize_rows(self.dev_feats[s])
         if self.exchange == "p2p":
             self._x[s] = x           # the owner's repair reads the row's features (kept alive for the captured graph)
             self.pxs[s % self.channels].scatter(x, bank, self.id_base, (s // self.channels) % self._ring[s % self.channels],
-                                                col_id=self.col_id, C_total=self.C_total, hier=self.hier)
+                                                col_id=self.col_id, C_total=self.C_total, hier=self._hier_shard(),
+                                                splits=self.splits)
             return None
         if bank.shape[0] > 0:
             # results go straight into the send record (no pack copies)
@@ -594,7 +711,9 @@ class ShardedEvalStream:
                 cert = (self._x[s], self.pbanks[s % len(self.pbanks)].table, self.repairs)
             self.pxs[s % self.channels].merge((s // self.channels) % self._ring[s % self.channels], self.dev_labels[s], self.hits,
                                               out=(self.val[s], self.idx[s]), targets_local=self.host_io, certify=cert,
-                                              hier=self.hier, counts=self.hier_counts)
+                                              hier=self._hier_shard(),
+                                              counts=self.hier_counts if self.splits is None else self.split_hier_counts,
+                                              splits=self.splits, split_counts=self.split_counts)
             if self.host_io:
                 self.host_counters[s].copy_(self.counters, non_blocking=True)
             return
@@ -602,6 +721,9 @@ class ShardedEvalStream:
             work.wait()
         pv, pi = unpack_gathered(self.recv[s])
         self.val[s], self.idx[s] = ops.topk_merge(pv, pi, targets=self.dev_labels[s], hits=self.hits)
+
+    def _hier_shard(self) -> Optional[HierShard]:
+        return self.hier if self.splits is None else self.splits.hier
 
     def _issue(self):
         if self.exchange == "p2p":
@@ -675,3 +797,47 @@ class ShardedEvalStream:
         if rows == 0:
             return 0.0, 0.0, 0.0
         return hits / rows * 100.0, path / rows * 100.0, point / rows * 100.0
+
+    def split_hit_counts(self):
+        """Per split ``[Hit@1, @2, @5, @10, @20, rows]`` over the rows of all ranks scored so far, in the order of
+        ``splits.names``.  A collective (one ``all_reduce`` of the integer counters): call it on every rank.  Needs
+        ``splits``."""
+        if self.splits is None:
+            raise RuntimeError("ShardedEvalStream was built without splits (pass splits=SplitShard(...))")
+        torch.cuda.synchronize(self.device)
+        c = self.split_counts.clone()
+        if self.world > 1:
+            dist.all_reduce(c, group=self.group)
+        return c.tolist()
+
+    def _split_hier_totals(self):
+        from .evaluate import hier_totals
+        torch.cuda.synchronize(self.device)
+        c = self.split_hier_counts.clone()
+        if self.world > 1:
+            dist.all_reduce(c, group=self.group)
+        return [hier_totals(x).tolist() for x in c]
+
+    def split_ratios(self):
+        """Per split ``(hit_ratio, path_ratio, point_ratio)`` in percent over the rows of all ranks whose label is in the
+        split.  A collective (one ``all_reduce``): call it on every rank.  Needs a ``SplitShard`` with ``hier``."""
+        if self.split_hier_counts is None:
+            raise RuntimeError("ShardedEvalStream was built without per-split TOR / POR (a SplitShard with hier)")
+        return [(0.0, 0.0, 0.0) if rows == 0 else (hits / rows * 100.0, path / rows * 100.0, point / rows * 100.0)
+                for rows, hits, point, path in self._split_hier_totals()]
+
+    def split_lines(self):
+        """One ``evaluate.split_line`` per split (Hit@k, plus TOR / POR when the ``SplitShard`` has ``hier``).  A
+        collective: call it on every rank."""
+        from .evaluate import split_line
+        counts = self.split_hit_counts()
+        hier = self._split_hier_totals() if self.split_hier_counts is not None else None
+        out = []
+        for s, name in enumerate(self.splits.names):
+            rows = counts[s][ops.HGR_NUM_HITS]
+            h = None
+            if hier is not None:
+                r, tor, point, path = hier[s]
+                h = (tor, point, path, r)
+            out.append(split_line(name, counts[s][:ops.HGR_NUM_HITS], max(rows, 1), h))
+        return out

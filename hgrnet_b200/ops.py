@@ -325,6 +325,99 @@ def global_list_len(B: int, C: int, D: int, K: int, C_total: int) -> int:
     return int(r)
 
 
+def _split_tables(group_end, group_splits, split_C_total):
+    import ctypes
+    n_groups, S = len(group_end), len(split_C_total)
+    if len(group_splits) != n_groups:
+        raise ValueError("group_end and group_splits disagree")
+    return ((ctypes.c_int32 * max(n_groups, 1))(*[int(e) for e in group_end]),
+            (ctypes.c_uint8 * max(n_groups, 1))(*[int(m) for m in group_splits]),
+            (ctypes.c_int64 * S)(*[int(c) for c in split_C_total]))
+
+
+def score_topk_splits_scatter(X: torch.Tensor, bank: torch.Tensor, group_end, group_splits, split_C_total,
+                              val_block_ptrs, idx_block_ptrs, bound_block_ptrs, block_rows: int, split_stride: int, *,
+                              col_id: Optional[torch.Tensor] = None, id_base: int = 0, K: int = 20,
+                              scale: float = 1.0) -> None:
+    """Producer of the class-sharded multi-split head (``hgr_score_topk_splits_scatter_bounded``, main.py:104-222 once
+    per split): ``bank`` is this rank's part of the union bank with its own group table (``group_end`` / ``group_splits``,
+    host ints, as ``score_topk_splits``; empty for a rank without rows), ``split_C_total`` the GLOBAL class count of every
+    split.  Per split s the rank's top-K of rows ``[g*block_rows, (g+1)*block_rows)`` and the bound of what it dropped go
+    to ``val_block_ptrs[g]`` / ``idx_block_ptrs[g]`` / ``bound_block_ptrs[g]`` + ``s * split_stride`` elements (device
+    pointers, local or peer); the owner runs ``topk_merge_splits_certified``."""
+    lib = _cabi.load()
+    X = _require(X, "X", torch.bfloat16)
+    B, D = X.shape
+    C = bank.shape[0]
+    if C:
+        bank = _require(bank, "bank", torch.bfloat16)
+        if bank.shape[1] != D:
+            raise ValueError("X and bank disagree on D: %d vs %d" % (D, bank.shape[1]))
+    if col_id is not None:
+        col_id = _require(col_id, "col_id", torch.int32)
+        if col_id.numel() != C:
+            raise ValueError("col_id must have one entry per bank row")
+    n = len(val_block_ptrs)
+    if len(idx_block_ptrs) != n or len(bound_block_ptrs) != n:
+        raise ValueError("val/idx/bound block tables disagree")
+    import ctypes
+    vt = (ctypes.c_void_p * n)(*val_block_ptrs)
+    it = (ctypes.c_void_p * n)(*idx_block_ptrs)
+    bt = (ctypes.c_void_p * n)(*bound_block_ptrs)
+    ends, gsp, ctot = _split_tables(group_end, group_splits, split_C_total)
+    n_groups = len(group_end)
+    nbytes = lib.hgr_score_topk_splits_scatter_bounded_workspace_bytes(B, C, D, K, n_groups, ends)
+    ws = _workspace(nbytes, X.device)
+    _cabi.check(lib.hgr_score_topk_splits_scatter_bounded(_ptr(X), _ptr(bank) if C else None, _ptr(col_id), id_base, B, C,
+                                                          D, float(scale), K, n_groups, ends, gsp, len(split_C_total),
+                                                          ctot, _ptr(ws), ws.numel(), block_rows, n, vt, it, bt,
+                                                          int(split_stride), HGR_IMPL_AUTO, _stream()))
+
+
+def splits_global_list_len(B: int, C: int, D: int, K: int, group_end, group_splits, split_C_total) -> int:
+    """Entries per list ``score_topk_splits_scatter`` keeps on a rank's part of the union bank (host only)."""
+    ends, gsp, ctot = _split_tables(group_end, group_splits, split_C_total)
+    r = _cabi.load().hgr_score_topk_splits_global_list_len(B, C, D, K, len(group_end), ends, gsp, len(split_C_total), ctot)
+    if r < 0:
+        _cabi.check(r)
+    return int(r)
+
+
+def topk_merge_splits_certified(part_val_ptr: int, part_idx_ptr: int, part_bound_ptr: int, P: int, B: int, K: int,
+                                n_splits: int, part_stride: int, bound_stride: int, split_stride: int,
+                                x_rows: torch.Tensor, shards: torch.Tensor, node_splits: torch.Tensor, device, *,
+                                scale: float = 1.0, targets: Optional[torch.Tensor] = None,
+                                counts: Optional[torch.Tensor] = None, repair_count: Optional[torch.Tensor] = None,
+                                out: Optional[Tuple[torch.Tensor, torch.Tensor]] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Owner side of the class-sharded multi-split head (``hgr_topk_merge_splits_certified``): per split, merge the
+    ``P`` shard lists of ``B`` rows, certify against the shards' bounds and repair the rest exactly from ``shards``
+    (``shard_table``) with the rows' features ``x_rows [B, D]`` bf16.  ``counts`` int64 ``[n_splits, HGR_NUM_HITS + 1]``
+    as in ``score_topk_splits``.  Returns ``(val [S,B,K], idx [S,B,K])``."""
+    lib = _cabi.load()
+    x_rows = _require(x_rows, "x_rows", torch.bfloat16)
+    if x_rows.shape[0] != B:
+        raise ValueError("x_rows must hold the %d rows being merged" % B)
+    if shards.dtype != torch.int64 or tuple(shards.shape) != (P, 4) or not shards.is_cuda:
+        raise ValueError("shards must be the [P, 4] int64 device tensor shard_table() builds")
+    node_splits = _require(node_splits, "node_splits", torch.uint8)
+    if targets is not None:
+        targets = _require(targets, "targets", torch.int32)
+    if counts is not None and (not counts.is_cuda or counts.dtype != torch.int64 or not counts.is_contiguous()
+                               or counts.numel() != n_splits * (HGR_NUM_HITS + 1)):
+        raise ValueError("counts must be a contiguous CUDA int64 [%d, %d] tensor" % (n_splits, HGR_NUM_HITS + 1))
+    if repair_count is not None:
+        repair_count = _require(repair_count, "repair_count", torch.int32)
+    if out is None:
+        out = (torch.empty((n_splits, B, K), dtype=torch.float32, device=device),
+               torch.empty((n_splits, B, K), dtype=torch.int32, device=device))
+    _cabi.check(lib.hgr_topk_merge_splits_certified(part_val_ptr, part_idx_ptr, part_bound_ptr, P, B, K, n_splits,
+                                                    part_stride, bound_stride, split_stride, _ptr(targets),
+                                                    _ptr(node_splits), node_splits.numel(), _ptr(out[0]), _ptr(out[1]),
+                                                    _ptr(counts), _ptr(x_rows), x_rows.shape[1], _ptr(shards),
+                                                    float(scale), _ptr(repair_count), _stream()))
+    return out
+
+
 def shard_table(shards, device) -> torch.Tensor:
     """Device copy of an ``hgr_shard_t`` array: ``shards`` = [(bank pointer, col_id pointer or 0, C, id_base), ...]
     (32 bytes per entry: two pointers, int64 C, int32 id_base + padding)."""
@@ -589,6 +682,33 @@ def hier_finish_rows_gathered(parts_ptr: int, n_parts: int, part_stride: int, n_
                                                   _ptr(first_out), _ptr(targets), chain_ptr.numel() - 1, _ptr(chain_ptr),
                                                   _ptr(chain_pos), _ptr(chain_level), _ptr(lvl_idx), _ptr(top1),
                                                   _ptr(counts), _stream()))
+
+
+def hier_finish_rows_gathered_splits(parts_ptr: int, n_parts: int, part_stride: int, n_rows: int, M: int, n_levels: int,
+                                     sorted_to_pos: torch.Tensor, first_out: torch.Tensor, targets: torch.Tensor,
+                                     chain_ptr: torch.Tensor, chain_pos: torch.Tensor, chain_level: torch.Tensor,
+                                     node_splits: torch.Tensor, counts: torch.Tensor) -> None:
+    """``hier_finish_rows_gathered`` with one counter set per split (``hgr_hier_finish_rows_gathered_splits``):
+    ``counts`` int64 ``[S, HGR_HIER_MAX_CHAIN + 1, 4]`` as in ``hier_metrics_fused_rows_splits``."""
+    lib = _cabi.load()
+    sorted_to_pos = _require(sorted_to_pos, "sorted_to_pos", torch.int32)
+    first_out = _require(first_out, "first_out", torch.int32)
+    targets = _require(targets, "targets", torch.int32)
+    chain_ptr = _require(chain_ptr, "chain_ptr", torch.int32)
+    chain_pos = _require(chain_pos, "chain_pos", torch.int32)
+    chain_level = _require(chain_level, "chain_level", torch.int32)
+    node_splits = _require(node_splits, "node_splits", torch.uint8)
+    if not counts.is_cuda or counts.dtype != torch.int64 or counts.dim() != 3 \
+            or tuple(counts.shape[1:]) != (HGR_HIER_MAX_CHAIN + 1, 4) or not counts.is_contiguous():
+        raise ValueError("counts must be a contiguous CUDA int64 [S, %d, 4] tensor" % (HGR_HIER_MAX_CHAIN + 1))
+    n_nodes = chain_ptr.numel() - 1
+    if sorted_to_pos.numel() != M or first_out.numel() != n_levels or targets.numel() != n_rows \
+            or chain_pos.numel() != chain_level.numel() or node_splits.numel() != n_nodes:
+        raise ValueError("hier_finish_rows_gathered_splits: inconsistent sizes")
+    _cabi.check(lib.hgr_hier_finish_rows_gathered_splits(parts_ptr, n_parts, part_stride, n_rows, M, n_levels,
+                                                         _ptr(sorted_to_pos), _ptr(first_out), _ptr(targets), n_nodes,
+                                                         _ptr(chain_ptr), _ptr(chain_pos), _ptr(chain_level),
+                                                         _ptr(node_splits), counts.shape[0], _ptr(counts), _stream()))
 
 
 def masked_ce(logits: torch.Tensor, set_ptr: torch.Tensor, set_col: torch.Tensor, label_pos: torch.Tensor,

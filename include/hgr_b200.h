@@ -377,6 +377,67 @@ int hgr_hier_finish_rows_gathered(const uint64_t* parts, int n_parts, int64_t pa
                                   int64_t* counts, void* stream);
 
 /*
+ * Several test splits in one scoring pass on the CLASS-SHARDED head (main.py:104-222 run once per split, as
+ * hgr_score_topk_splits, over G ranks).  Every rank holds about 1/G of EVERY group of the union bank (its slice of each
+ * group, concatenated in group order, with the clipped group ends as its own group table), so every rank holds about
+ * 1/G of every split.  Image rows are owned block-wise as in hgr_score_topk_scatter.
+ *
+ * Result and tie order: for split s the top-K of s's classes in the order (value desc, rank asc, local bank row asc) --
+ * hgr_score_topk on s's rows of the ranks' banks concatenated rank after rank.  At G = 1 that is the union bank's own
+ * order: the result is hgr_score_topk_splits's, bit for bit when neither call repairs a row (a repaired list carries
+ * the CUDA cores' values of its re-scanned rows, which may differ from the GEMM's in the last bits).
+ *
+ * hgr_score_topk_splits_scatter_bounded   producer: the grouped scoring kernel of hgr_score_topk_splits on this rank's
+ *                                 bank [C, D] (group table n_groups / group_end / group_splits as there), lists sized
+ *                                 for each split's GLOBAL stream of split_C_total[s] classes (HOST [n_splits] int64;
+ *                                 hgr_score_topk_splits_global_list_len), then per split s and row: the rank's top-K of
+ *                                 s (node ids, values times scale) at val_blocks[g] / idx_blocks[g] + s * split_stride +
+ *                                 (row - g * block_rows) * K and the bound -- scale * the largest last entry of its FULL
+ *                                 narrow lists of s, -inf when none dropped anything -- at bound_blocks[g] + s *
+ *                                 split_stride + row - g * block_rows (HOST arrays of n_blocks device pointers, local or
+ *                                 peer; split_stride in 4-byte elements, >= n_blocks * block_rows * (2K + 1):
+ *                                 a split's lists and bounds of all producers).  No local certificate, no repair, no counting.
+ *                                 C == 0 (a rank without rows) and splits without rows here store (-inf, -1) lists and
+ *                                 -inf bounds.  impl: HGR_IMPL_AUTO / HGR_IMPL_TCGEN05.  workspace:
+ *                                 hgr_score_topk_splits_scatter_bounded_workspace_bytes(...), as hgr_score_topk_splits.
+ * hgr_topk_merge_splits_certified owner: for its B rows and every split s, the merge of the P = G shard lists of s at
+ *                                 part_val / part_idx + s * split_stride + p * part_stride + row * K in the order above,
+ *                                 certified when the merged K-th value beats every shard's bound of s (part_bound + s *
+ *                                 split_stride + p * bound_stride + row) STRICTLY.  A doubtful (row, split, shard) is
+ *                                 re-scanned exactly on the CUDA cores: the rows of shards[p] whose node (col_id or
+ *                                 id_base + row) has bit s in node_splits, over NVLink for a peer's bank.  topk_val /
+ *                                 topk_idx [n_splits, B, K]; counts [n_splits][HGR_NUM_HITS + 1] int64, INCREMENTED as
+ *                                 in hgr_score_topk_splits (optional); *repair_count (optional) counts (row, split) pairs
+ *                                 repaired.  split_stride >= 2 * P * part_stride + P * bound_stride: a split's
+ *                                 value lists, id lists and bounds all sit at + s * split_stride.
+ * hgr_hier_finish_rows_gathered_splits   hgr_hier_finish_rows_gathered with the counters of every split: counts
+ *                                 [n_splits][HGR_HIER_MAX_CHAIN + 1][4], a row added to set s for every bit s of
+ *                                 node_splits[targets[row]] (hgr_hier_metrics_fused_rows_splits); no lvl_idx / top1.
+ */
+size_t hgr_score_topk_splits_scatter_bounded_workspace_bytes(int64_t B, int64_t C, int64_t D, int K, int n_groups,
+                                                             const int32_t* group_end);
+int hgr_score_topk_splits_global_list_len(int64_t B, int64_t C, int64_t D, int K, int n_groups, const int32_t* group_end,
+                                          const uint8_t* group_splits, int n_splits, const int64_t* split_C_total);
+int hgr_score_topk_splits_scatter_bounded(const void* X, const void* bank, const int32_t* col_id, int32_t id_base,
+                                          int64_t B, int64_t C, int64_t D, float scale, int K, int n_groups,
+                                          const int32_t* group_end, const uint8_t* group_splits, int n_splits,
+                                          const int64_t* split_C_total, void* workspace, size_t workspace_bytes,
+                                          int64_t block_rows, int n_blocks, float* const* val_blocks,
+                                          int32_t* const* idx_blocks, float* const* bound_blocks, int64_t split_stride,
+                                          int impl, void* stream);
+int hgr_topk_merge_splits_certified(const float* part_val, const int32_t* part_idx, const float* part_bound, int64_t P,
+                                    int64_t B, int K, int n_splits, int64_t part_stride, int64_t bound_stride,
+                                    int64_t split_stride, const int32_t* targets, const uint8_t* node_splits,
+                                    int64_t n_nodes, float* topk_val, int32_t* topk_idx, int64_t* counts, const void* X,
+                                    int64_t D, const hgr_shard_t* shards, float scale, unsigned int* repair_count,
+                                    void* stream);
+int hgr_hier_finish_rows_gathered_splits(const uint64_t* parts, int n_parts, int64_t part_stride, int64_t n_rows,
+                                         int64_t M, int n_levels, const int32_t* sorted_to_pos, const int32_t* first_out,
+                                         const int32_t* targets, int64_t n_nodes, const int32_t* chain_ptr,
+                                         const int32_t* chain_pos, const int32_t* chain_level, const uint8_t* node_splits,
+                                         int n_splits, int64_t* counts, void* stream);
+
+/*
  * Fused masked cross-entropy of the OM training step over T sampled class sets
  * (model/clip_tree.py:241-277 with nn.CrossEntropyLoss, :49,:275).
  *
