@@ -24,6 +24,7 @@ HGR_HIER_MAX_CHAIN = 32
 HGR_MAX_SPLITS = 8   # hgr_score_topk_splits: splits per call
 HGR_MAX_GROUPS = 16  # ... and groups of equal split membership
 HIT_CUTS = (1, 2, 5, 10, 20)  # main.py:120
+HGR_MISTAKE_COUNTERS = 2 + 2 * HGR_NUM_HITS + 2 * HGR_HIER_MAX_CHAIN + 2   # hgr_hier_mistakes: counters per set
 
 # every symbol include/hgr_b200.h declares: name -> (restype, argtypes)
 SIGNATURES = {
@@ -90,6 +91,8 @@ SIGNATURES = {
     "hgr_hier_finish_rows_gathered_splits": (c_int, [c_void_p, c_int, c_int64, c_int64, c_int64, c_int, c_void_p, c_void_p,
                                                      c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_int,
                                                      c_void_p, c_void_p]),
+    "hgr_hier_mistakes": (c_int, [c_void_p, c_int64, c_int, c_int64, c_int, c_void_p, c_void_p, c_void_p, c_void_p,
+                                  c_int64, c_void_p, c_void_p]),
     "hgr_masked_ce_workspace_bytes":(c_size_t, [c_int64, c_int64, c_int64]),
     "hgr_om_backward_workspace_bytes": (c_size_t, [c_int64, c_int64, c_int64]),
     "hgr_om_backward": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int64, c_int64, c_void_p, c_void_p, c_void_p,

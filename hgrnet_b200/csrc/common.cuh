@@ -235,6 +235,9 @@ int launch_hier_finish_gathered_splits(const unsigned long long* parts, int n_pa
                                        const int32_t* targets, int64_t n_nodes, const int32_t* chain_ptr,
                                        const int32_t* chain_pos, const int32_t* chain_level, const uint8_t* node_splits,
                                        int n_splits, int64_t* counts, cudaStream_t stream);
+int launch_hier_mistakes(const int32_t* topk_idx, int64_t B, int K, int64_t set_stride, int n_sets,
+                         const int32_t* targets, const uint8_t* node_splits, const int32_t* chain_ptr,
+                         const int32_t* chain_node, int64_t n_nodes, int64_t* counts, cudaStream_t stream);
 int launch_normalize_dual(const void* E, int e_dtype, int64_t n_rows, int64_t D, void* out, const int32_t* dst_map,
                           void* out2, cudaStream_t stream);
 int launch_normalize_bcast(const void* E, int e_dtype, int64_t n_rows, int64_t D, int64_t row0, int n_dst,

@@ -316,6 +316,32 @@ class SplitShard:
         self.hier = HierShard(h.rows_args(), rank, world) if h is not None else None
 
 
+class MistakeShard:
+    """One rank's part of the class-sharded mistake severity and LCA distance@k (``evaluate.MistakeMetrics``): the
+    chain table, which every rank holds whole, and the image rows this rank owns and counts.  The owner runs
+    ``ops.hier_mistakes`` on its merged lists, so nothing of it crosses the exchange.  ``rank`` / ``world`` default to
+    the process group's."""
+
+    def __init__(self, mistakes, rank: Optional[int] = None, world: Optional[int] = None, group=None):
+        if world is None:
+            world = dist.get_world_size(group) if dist.is_initialized() else 1
+        if rank is None:
+            rank = dist.get_rank(group) if dist.is_initialized() else 0
+        if not 0 <= rank < world:
+            raise ValueError("rank %d outside [0, %d)" % (rank, world))
+        self.rank, self.world = rank, world
+        self.chain_ptr, self.chain_node = mistakes.chain_ptr, mistakes.chain_node
+
+    def args(self) -> dict:
+        return dict(chain_ptr=self.chain_ptr, chain_node=self.chain_node)
+
+    def row_bounds(self, B: int) -> Tuple[int, int]:
+        """The rows ``[lo, hi)`` of a batch of ``B`` this rank owns, merges and counts (``PeerExchange``'s blocks)."""
+        block_rows = (B + self.world - 1) // self.world
+        lo = min(B, self.rank * block_rows)
+        return lo, min(B, lo + block_rows)
+
+
 class PeerExchange:
     """Peer-memory exchange of the class-sharded head (no collective call on the data path).
 
@@ -530,12 +556,18 @@ class ShardedEvalStream:
     ``split_hier_counts`` live in ``counters`` too.  ``split_hit_counts()`` / ``split_ratios()`` / ``split_lines()`` sum
     them over ranks.  With ``splits`` the stream scores nothing against ``bank_shard`` / ``id_base``: ``bank_shard`` only
     has to agree with the ``SplitShard`` on D and device (pass e.g. ``split_eval.bank()``), and ``id_base`` is unused.
+
+    ``mistakes`` (a ``MistakeShard`` of this rank, peer exchange only, with or without ``splits``): after the merge the
+    row owner counts the mistake severity and LCA distance@k of its merged lists against each row's own label
+    (``ops.hier_mistakes``; one counter set per split with ``splits``).  No exchange data and no flag is added; the
+    counters sit in ``counters``, and ``mistake_summary()`` / ``split_mistake_summary()`` sum them over ranks.
     """
 
     def __init__(self, bank_shard: torch.Tensor, id_base: int, *, batch: int, K: int = 20, steps: int = 8,
                  feat_dtype=torch.float32, banks=None, group=None, use_graph: bool = True, exchange: str = "p2p",
                  channels: int = 4, host_io: bool = False, col_id: Optional[torch.Tensor] = None,
-                 certify: str = "global", hier: Optional[HierShard] = None, splits: Optional[SplitShard] = None):
+                 certify: str = "global", hier: Optional[HierShard] = None, splits: Optional[SplitShard] = None,
+                 mistakes: Optional[MistakeShard] = None):
         if exchange not in ("p2p", "nccl"):
             raise ValueError("exchange must be 'p2p' or 'nccl'")
         if splits is not None:
@@ -550,6 +582,12 @@ class ShardedEvalStream:
             if splits.D != bank_shard.shape[1] or splits.device != bank_shard.device:
                 raise ValueError("splits: the SplitShard has D = %d on %s, the stream D = %d on %s" % (
                     splits.D, splits.device, bank_shard.shape[1], bank_shard.device))
+        if mistakes is not None:
+            if exchange != "p2p":
+                raise ValueError("mistakes (class-sharded mistake metrics) need the peer-memory exchange")
+            if mistakes.chain_ptr.device != bank_shard.device:
+                raise ValueError("mistakes: the chain table is on %s, the bank on %s" % (mistakes.chain_ptr.device,
+                                                                                       bank_shard.device))
         if hier is not None and exchange != "p2p":
             raise ValueError("hier (class-sharded TOR / POR) needs the peer-memory exchange")
         if hier is not None and hier.D != bank_shard.shape[1]:
@@ -591,7 +629,9 @@ class ShardedEvalStream:
         S = 0 if splits is None else splits.S
         n_split = S * (ops.HGR_NUM_HITS + 1)
         n_split_hier = 0 if splits is None or splits.hier is None else S * (ops.HGR_HIER_MAX_CHAIN + 1) * 4
-        n_counters = ops.HGR_NUM_HITS + n_hier + n_split + n_split_hier
+        self.mistakes = mistakes
+        n_mist = 0 if mistakes is None else max(S, 1) * ops.HGR_MISTAKE_COUNTERS
+        n_counters = ops.HGR_NUM_HITS + n_hier + n_split + n_split_hier + n_mist
         self.counters = torch.zeros(n_counters, dtype=torch.int64, device=self.device)
         self.hits = self.counters[:ops.HGR_NUM_HITS]
         o = ops.HGR_NUM_HITS
@@ -601,6 +641,8 @@ class ShardedEvalStream:
         o += n_split
         self.split_hier_counts = (self.counters[o:o + n_split_hier].view(S, ops.HGR_HIER_MAX_CHAIN + 1, 4)
                                   if n_split_hier else None)
+        o += n_split_hier
+        self.mistake_counts = self.counters[o:o + n_mist].view(-1, ops.HGR_MISTAKE_COUNTERS) if n_mist else None
         self.val = [None] * steps
         self.idx = [None] * steps
         self.row_lo, self.row_hi = 0, batch
@@ -714,6 +756,11 @@ class ShardedEvalStream:
                                               hier=self._hier_shard(),
                                               counts=self.hier_counts if self.splits is None else self.split_hier_counts,
                                               splits=self.splits, split_counts=self.split_counts)
+            if self.mistakes is not None and self.row_hi > self.row_lo:     # the owner's merged lists, after the merge
+                t = self.dev_labels[s] if self.host_io else self.dev_labels[s][self.row_lo:self.row_hi]
+                ops.hier_mistakes(self.idx[s], t, counts=self.mistake_counts,
+                                  node_splits=None if self.splits is None else self.splits.node_splits,
+                                  **self.mistakes.args())
             if self.host_io:
                 self.host_counters[s].copy_(self.counters, non_blocking=True)
             return
@@ -827,11 +874,12 @@ class ShardedEvalStream:
                 for rows, hits, point, path in self._split_hier_totals()]
 
     def split_lines(self):
-        """One ``evaluate.split_line`` per split (Hit@k, plus TOR / POR when the ``SplitShard`` has ``hier``).  A
-        collective: call it on every rank."""
+        """One ``evaluate.split_line`` per split (Hit@k, plus TOR / POR when the ``SplitShard`` has ``hier`` and the
+        mistake metrics with ``mistakes``).  A collective: call it on every rank."""
         from .evaluate import split_line
         counts = self.split_hit_counts()
         hier = self._split_hier_totals() if self.split_hier_counts is not None else None
+        mist = self.split_mistake_summary() if self.mistake_counts is not None else [None] * self.splits.S
         out = []
         for s, name in enumerate(self.splits.names):
             rows = counts[s][ops.HGR_NUM_HITS]
@@ -839,5 +887,30 @@ class ShardedEvalStream:
             if hier is not None:
                 r, tor, point, path = hier[s]
                 h = (tor, point, path, r)
-            out.append(split_line(name, counts[s][:ops.HGR_NUM_HITS], max(rows, 1), h))
+            out.append(split_line(name, counts[s][:ops.HGR_NUM_HITS], max(rows, 1), h, mist[s]))
         return out
+
+    def _mistake_totals(self):
+        if self.mistake_counts is None:
+            raise RuntimeError("ShardedEvalStream was built without mistake metrics (pass mistakes=MistakeShard(...))")
+        torch.cuda.synchronize(self.device)
+        c = self.mistake_counts.clone()
+        if self.world > 1:
+            dist.all_reduce(c, group=self.group)
+        return c
+
+    def mistake_summary(self):
+        """``evaluate.mistake_summary`` over the rows of all ranks scored so far.  A collective (one ``all_reduce``):
+        call it on every rank.  Needs ``mistakes`` without ``splits``."""
+        from .evaluate import mistake_summary
+        if self.splits is not None:
+            raise RuntimeError("ShardedEvalStream has splits: use split_mistake_summary()")
+        return mistake_summary(self._mistake_totals()[0], self.K)
+
+    def split_mistake_summary(self):
+        """Per split ``evaluate.mistake_summary`` over the rows of all ranks whose label is in the split.  A collective
+        (one ``all_reduce``): call it on every rank.  Needs ``mistakes`` and ``splits``."""
+        from .evaluate import mistake_summary
+        if self.splits is None:
+            raise RuntimeError("ShardedEvalStream was built without splits: use mistake_summary()")
+        return [mistake_summary(c, self.K) for c in self._mistake_totals()]

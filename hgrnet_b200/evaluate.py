@@ -20,7 +20,7 @@ import numpy as np
 import torch
 
 from . import ops
-from ._cabi import HGR_HIER_MAX_CHAIN, HIT_CUTS
+from ._cabi import HGR_HIER_MAX_CHAIN, HGR_MISTAKE_COUNTERS, HIT_CUTS
 
 
 def count_acc(hits_dict, num_tot):
@@ -36,17 +36,25 @@ def count_acc(hits_dict, num_tot):
     return out_str, acc_dict
 
 
-def chain_table(c2p: Sequence[Sequence[int]], depth: np.ndarray, train_ids: Sequence[int]
-                ) -> Tuple[np.ndarray, np.ndarray, np.ndarray]:
-    """The chain table of ``hgr_hier_metrics_fused_rows``: a CSR over all nodes whose row n is the reference's label
-    chain ``c2p[n] + [n]`` (main.py:152).  Returns int32 ``(chain_ptr [N + 1], chain_pos, chain_level)``: per entry the
-    node's position in ``train_ids`` (the last one if it repeats, -1 if it is not a train class) and its depth."""
+def chain_csr(c2p: Sequence[Sequence[int]]) -> Tuple[np.ndarray, np.ndarray]:
+    """A CSR over all nodes whose row n is the reference's label chain ``c2p[n] + [n]`` (main.py:152): int64
+    ``(chain_ptr [N + 1], nodes)``, the node ids of every chain.  ``hgr_hier_mistakes`` takes it as it is (as int32)."""
     n = len(c2p)
     lens = np.fromiter((len(c) + 1 for c in c2p), dtype=np.int64, count=n)
     chain_ptr = np.zeros(n + 1, dtype=np.int64)
     np.cumsum(lens, out=chain_ptr[1:])
     nodes = np.fromiter(itertools.chain.from_iterable((*c, i) for i, c in enumerate(c2p)), dtype=np.int64,
                         count=int(chain_ptr[-1]))
+    return chain_ptr, nodes
+
+
+def chain_table(c2p: Sequence[Sequence[int]], depth: np.ndarray, train_ids: Sequence[int]
+                ) -> Tuple[np.ndarray, np.ndarray, np.ndarray]:
+    """The chain table of ``hgr_hier_metrics_fused_rows``: the CSR of ``chain_csr``.  Returns int32 ``(chain_ptr
+    [N + 1], chain_pos, chain_level)``: per entry the node's position in ``train_ids`` (the last one if it repeats, -1 if
+    it is not a train class) and its depth."""
+    n = len(c2p)
+    chain_ptr, nodes = chain_csr(c2p)
     pos_of = np.full(n, -1, dtype=np.int64)
     train = np.asarray(train_ids, dtype=np.int64)
     pos_of[train] = np.arange(train.size)                # repeated ids: the last assignment stays, as in a dict
@@ -155,6 +163,67 @@ class HierMetrics:
                 float(self.point_all) / num_sample * 100.0)
 
 
+def mistake_summary(counts, K: int = 20) -> dict:
+    """The derived values of one set of ``hier_mistakes`` counters (``[HGR_MISTAKE_COUNTERS]``, tensor or list), as
+    float64: ``rows``, ``mistakes``, ``mistake_rate`` = mistakes / rows, ``severity_h`` / ``severity_d`` = the sum of
+    h / d at top-1 over the mistakes (0 without mistakes; a correct top-1 adds 0), ``hdist@k`` / ``dist@k`` = the sum of
+    h / d over the first min(k, K) entries / (rows * min(k, K)), and ``hist_d`` the histogram of d at top-1 (last bin:
+    larger than 2 * HGR_HIER_MAX_CHAIN).  ``K`` is the list length.  All zero without rows."""
+    c = [int(v) for v in (counts.tolist() if hasattr(counts, "tolist") else counts)]
+    if len(c) != HGR_MISTAKE_COUNTERS:
+        raise ValueError("one set of %d mistake counters expected, got %d" % (HGR_MISTAKE_COUNTERS, len(c)))
+    rows, mistakes = float(c[0]), float(c[1])
+    nh = len(HIT_CUTS)
+    out = {"rows": rows, "mistakes": mistakes, "mistake_rate": mistakes / rows if rows else 0.0,
+           "severity_h": c[2] / mistakes if mistakes else 0.0, "severity_d": c[2 + nh] / mistakes if mistakes else 0.0}
+    for i, k in enumerate(HIT_CUTS):
+        n = rows * min(k, K)
+        out["hdist@%d" % k] = c[2 + i] / n if n else 0.0
+        out["dist@%d" % k] = c[2 + nh + i] / n if n else 0.0
+    out["hist_d"] = [float(v) for v in c[2 + 2 * nh:]]
+    return out
+
+
+def mistake_line(summary: dict) -> str:
+    """The suffix ``test()`` appends to its line with ``--hgr_mistake_metrics``."""
+    return " mistake_rate(%):{:.2f} severity:{:.2f} hdist@1:{:.2f} hdist@5:{:.2f} hdist@20:{:.2f}".format(
+        summary["mistake_rate"] * 100.0, summary["severity_h"], summary["hdist@1"], summary["hdist@5"],
+        summary["hdist@20"])
+
+
+class MistakeMetrics:
+    """Hierarchical mistake severity and LCA distance@k (Bertinetto et al., "Making Better Mistakes", CVPR 2020) of
+    the top-K lists of every batch: how far from the label in the hierarchy the predictions are, not only whether the
+    label is among them (main.py:135-148).  Holds the chain table (``chain_csr`` of ``model.c2p``, on the device) and
+    the counters, one set per list set; ``update`` counts a batch on the device (``ops.hier_mistakes``) with no host
+    synchronisation.  ``n_sets`` > 1 counts ``[n_sets, B, K]`` lists of several test splits (``SplitEval``)."""
+
+    def __init__(self, model, n_sets: int = 1, K: int = 20):
+        dev = model.device
+        ptr, nodes = chain_csr(model.c2p)
+        self.chain_ptr = torch.from_numpy(ptr.astype(np.int32)).to(dev)
+        self.chain_node = torch.from_numpy(nodes.astype(np.int32)).to(dev)
+        self.n_sets, self.K = n_sets, K
+        self.counts = ops.new_mistake_counts(dev, n_sets)
+
+    def args(self) -> dict:
+        """The chain table arguments of ``ops.hier_mistakes``."""
+        return dict(chain_ptr=self.chain_ptr, chain_node=self.chain_node)
+
+    def update(self, idx: torch.Tensor, targets: torch.Tensor, node_splits: Optional[torch.Tensor] = None,
+               counts: Optional[torch.Tensor] = None):
+        """Count a batch: ``idx`` int32 node ids ``[B, K]`` (or ``[n_sets, B, K]`` with ``node_splits``), ``targets``
+        [B] node ids, one per row (-1 padding counts nowhere).  Into ``counts`` (default: the object's own)."""
+        ops.hier_mistakes(idx, targets.to(torch.int32), counts=self.counts if counts is None else counts,
+                          node_splits=node_splits, **self.args())
+
+    def summary(self, counts: Optional[torch.Tensor] = None):
+        """``mistake_summary`` of every set (synchronises): a dict, or a list of dicts for several sets."""
+        c = (self.counts if counts is None else counts).view(-1, HGR_MISTAKE_COUNTERS).tolist()
+        out = [mistake_summary(x, self.K) for x in c]
+        return out[0] if self.n_sets == 1 else out
+
+
 _BANK_SEED = 0x48475221   # the seed of tree_model's test-bank permutation (head.py)
 
 
@@ -186,15 +255,17 @@ def split_groups(splits, n_nodes: int):
     return names, np.concatenate(rows), group_end, masks, node_splits
 
 
-def split_line(name, hits, rows, hier=None):
+def split_line(name, hits, rows, hier=None, mistakes=None):
     """The reference's ``test()`` line of one split (``count_acc`` + TOR / POR), prefixed with the split's name.
-    ``hier``: ``(hits, point, path, path_rows)`` sums or None."""
+    ``hier``: ``(hits, point, path, path_rows)`` sums or None; ``mistakes``: the split's ``mistake_summary`` or None."""
     out_str, _ = count_acc(dict(zip(HIT_CUTS, hits)), rows)
     if hier is not None:
         tor, point, path, path_rows = hier
         out_str += " hit_ratio(%):{:.2f}".format(tor / rows * 100.0)
         out_str += " path_ratio(%):{:.2f}".format(path / path_rows * 100.0 if path_rows else 0.0)
         out_str += " point_ratio(%):{:.2f}".format(point / rows * 100.0)
+    if mistakes is not None:
+        out_str += mistake_line(mistakes)
     return "{}: {}".format(name, out_str)
 
 
@@ -202,9 +273,11 @@ class SplitEval:
     """Several test splits of one hierarchy scored in ONE pass per batch (``hgr_score_topk_splits``): the union bank is
     built from ``model.zsl_weights`` in the group layout of ``split_groups`` and rebuilt after a bank refresh; the hit
     counters of every split stay on the device.  With ``hier=True`` the TOR / POR counters of every split follow from
-    one level GEMM per batch (``hgr_hier_metrics_fused_rows_splits``).  ``lines()`` gives one line per split."""
+    one level GEMM per batch (``hgr_hier_metrics_fused_rows_splits``).  With ``mistakes=True`` the mistake severity and
+    LCA distance@k of every split are counted from the ``[S, B, K]`` lists (``MistakeMetrics``, one set per split).
+    ``lines()`` gives one line per split."""
 
-    def __init__(self, model, splits, hier: bool = True, K: int = 20):
+    def __init__(self, model, splits, hier: bool = True, K: int = 20, mistakes: bool = False):
         self.model = model
         self.K = K
         dev = model.device
@@ -218,6 +291,7 @@ class SplitEval:
         self.hier = HierMetrics(model) if hier else None
         self._hier_counts = None
         self._hier_acc = torch.zeros((self.S, 4), dtype=torch.float64, device=dev)   # (rows, hits, point, path)
+        self.mistakes = MistakeMetrics(model, n_sets=self.S, K=K) if mistakes else None
         self._bank = None
         self._bank_version = None
 
@@ -250,6 +324,8 @@ class SplitEval:
             ops.hier_metrics_fused_rows_splits(x_norm, targets=ht, node_splits=self.node_splits,
                                                counts=self._hier_counts, **self.hier.rows_args())
             self._hier_acc += torch.stack([hier_totals(c) for c in self._hier_counts])
+        if self.mistakes is not None:
+            self.mistakes.update(out[1], t, node_splits=self.node_splits)
         return out
 
     def hit_counts(self):
@@ -257,9 +333,11 @@ class SplitEval:
         return self.counts.tolist()
 
     def lines(self):
-        """One line per split: ``name: Top@1(%):..., ... .`` plus TOR / POR with ``hier`` (synchronises)."""
+        """One line per split: ``name: Top@1(%):..., ... .`` plus TOR / POR with ``hier`` and the mistake metrics with
+        ``mistakes`` (synchronises)."""
         counts = self.counts.tolist()
         acc = self._hier_acc.tolist()
+        mist = self.mistakes.summary() if self.mistakes is not None else [None] * self.S
         out = []
         for s, name in enumerate(self.names):
             rows = counts[s][ops.HGR_NUM_HITS]
@@ -267,7 +345,7 @@ class SplitEval:
             if self.hier is not None:
                 r, tor, point, path = acc[s]
                 h = (tor, point, path, r)
-            out.append(split_line(name, counts[s][:ops.HGR_NUM_HITS], max(rows, 1), h))
+            out.append(split_line(name, counts[s][:ops.HGR_NUM_HITS], max(rows, 1), h, mist[s]))
         return out
 
 
@@ -276,7 +354,9 @@ def test(opts, model, device, splits=None, loader: Optional[Iterable] = None, lo
     ``{'img': [1,B,...], 'label': [1,B]}`` (single-label batches, imagenet_group_test.py).
 
     TOR / POR score every row of a batch against the batch's first label, as the reference does with ``targets[0]``
-    (main.py:152).  A first label outside the hierarchy is counted nowhere (the reference raises ``IndexError``)."""
+    (main.py:152).  A first label outside the hierarchy is counted nowhere (the reference raises ``IndexError``).
+    With ``--hgr_mistake_metrics`` the line also gets the mistake rate, the mistake severity and the LCA distance@k
+    (``MistakeMetrics``), every row against its own label."""
     print("out", opts.out_ratio)
     print("in", opts.in_ratio)
     model.eval()
@@ -289,6 +369,7 @@ def test(opts, model, device, splits=None, loader: Optional[Iterable] = None, lo
     if split_keys:
         return _test_splits(opts, model, device, splits, split_keys, loader, log)
     hier = HierMetrics(model) if getattr(opts, "hgr_hier_metrics", True) else None
+    mist = MistakeMetrics(model) if getattr(opts, "hgr_mistake_metrics", False) else None
     hits = ops.new_hits(model.device)
     num_sample = 0
     out_str = ""
@@ -296,15 +377,17 @@ def test(opts, model, device, splits=None, loader: Optional[Iterable] = None, lo
         for i, data in enumerate(loader):
             imgs, targets = data["img"].to(device, non_blocking=True)[0], data["label"].to(device, non_blocking=True)[0]
             x = model.encode_image_normalized(imgs)
-            model.score_topk(None, targets, hits=hits, feats_normalized=x)   # main.py:135-147, fused
+            _, idx = model.score_topk(None, targets, hits=hits, feats_normalized=x)   # main.py:135-147, fused
             num_sample += len(targets)
             if hier is not None:                                             # main.py:152: every row against targets[0]
                 hier.update_rows(x, targets[:1].expand(len(targets)))
+            if mist is not None:
+                mist.update(idx, targets)
             if i % opts.print_freq == 0:
-                out_str = _format(hits, num_sample, hier)
+                out_str = _format(hits, num_sample, hier, mist)
                 print(out_str, flush=True)
     print("End of testing.")
-    out_str = _format(hits, num_sample, hier)
+    out_str = _format(hits, num_sample, hier, mist)
     print(out_str, flush=True)
     if log:
         with open(model.save_path + "arugements.log", "a") as f:       # [sic] main.py:217
@@ -321,7 +404,7 @@ def _test_splits(opts, model, device, splits, split_keys, loader, log):
         raise ValueError("--hgr_eval_splits needs the split file's class lists (splits)")
     index = model.hierarchy.index
     se = SplitEval(model, {k: [index[c] for c in splits[k]] for k in split_keys},
-                   hier=getattr(opts, "hgr_hier_metrics", True))
+                   hier=getattr(opts, "hgr_hier_metrics", True), mistakes=getattr(opts, "hgr_mistake_metrics", False))
     with torch.no_grad():
         for i, data in enumerate(loader):
             imgs, targets = data["img"].to(device, non_blocking=True)[0], data["label"].to(device, non_blocking=True)[0]
@@ -341,7 +424,7 @@ def _test_splits(opts, model, device, splits, split_keys, loader, log):
     return out_str
 
 
-def _format(hits, num_sample, hier):
+def _format(hits, num_sample, hier, mist=None):
     h = hits.tolist()
     hits_dict = dict(zip(HIT_CUTS, h))
     out_str = "\n"
@@ -352,4 +435,6 @@ def _format(hits, num_sample, hier):
         out_str += " hit_ratio(%):{:.2f}".format(hit_ratio)
         out_str += " path_ratio(%):{:.2f}".format(path_ratio)
         out_str += " point_ratio(%):{:.2f}".format(point_ratio)
+    if mist is not None:
+        out_str += mistake_line(mist.summary())
     return out_str

@@ -82,6 +82,9 @@ def build_parser() -> argparse.ArgumentParser:
     g.add_argument("--hgr_eval_splits", default="", type=str,
                    help="comma-separated split-file keys (e.g. 2-hops,3-hops,all): test scores every batch against all of "
                         "them in one pass and prints one line per split")
+    g.add_argument("--hgr_mistake_metrics", type=_bool, default=False, choices=[True, False],
+                   help="also report the mistake rate, the mistake severity (mean LCA height of the wrong top-1) and "
+                        "the LCA distance@k of the top-k during test, per split with --hgr_eval_splits")
     return p
 
 

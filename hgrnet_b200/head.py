@@ -242,7 +242,8 @@ class tree_model(nn.Module):
         return ops.score_topk(x, self.bank_test, col_id=self._test_index_i32, targets=t, K=K, hits=hits)
 
     def make_eval_stream(self, batch: int, slots: int = 4, streams: int = 2, feat_dtype=torch.float32, K: int = 20,
-                         banks=None, host_io: bool = True, hier_metrics: bool = False, eval_splits=None):
+                         banks=None, host_io: bool = True, hier_metrics: bool = False, eval_splits=None,
+                         mistake_metrics: bool = False):
         """CUDA-graph replayed eval step over pre-computed image features (hgrnet_b200.stream.EvalStream).
 
         ``hier_metrics=True`` adds TOR / POR (``EvalStream.hier_ratios``), every row scored against its own label.  The
@@ -251,9 +252,15 @@ class tree_model(nn.Module):
 
         ``eval_splits`` (``{name: node ids}``, at most 8 splits): every step scores against all of these test splits
         in one pass instead of against ``bank_test`` (``EvalStream.split_hit_counts``; with ``hier_metrics`` also the
-        per-split TOR / POR, ``EvalStream.split_ratios``)."""
+        per-split TOR / POR, ``EvalStream.split_ratios``).
+
+        ``mistake_metrics=True`` adds the mistake severity and LCA distance@k of every row's top-K against its own label
+        (``EvalStream.mistake_summary``, per split ``EvalStream.split_mistake_summary``)."""
         from .stream import EvalStream
-        hier = splits = None
+        hier = splits = mistakes = None
+        if mistake_metrics:
+            from .evaluate import MistakeMetrics
+            mistakes = MistakeMetrics(self, K=K)
         if eval_splits is not None:
             from .evaluate import SplitEval
             splits = SplitEval(self, eval_splits, hier=hier_metrics, K=K)
@@ -261,7 +268,8 @@ class tree_model(nn.Module):
             from .evaluate import HierMetrics
             hier = HierMetrics(self)
         return EvalStream(self.bank_test, col_id=self._test_index_i32, batch=batch, feat_dtype=feat_dtype, K=K,
-                          slots=slots, streams=streams, banks=banks, host_io=host_io, hier=hier, splits=splits)
+                          slots=slots, streams=streams, banks=banks, host_io=host_io, hier=hier, splits=splits,
+                          mistakes=mistakes)
 
     # ------------------------------------------------------------------ training step
     def _schedule(self, training_method, target):

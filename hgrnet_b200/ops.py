@@ -13,7 +13,7 @@ import torch
 from . import _cabi
 from ._cabi import (HGR_IMPL_AUTO, HGR_IMPL_SIMT, HGR_IMPL_TCGEN05,  # noqa: F401
                     HGR_IMPL_TCGEN05_EXACT, HGR_IMPL_TCGEN05_NULL, HGR_IMPL_TCGEN05_SKETCH,
-                    HGR_HIER_MAX_CHAIN, HGR_NUM_HITS)
+                    HGR_HIER_MAX_CHAIN, HGR_MISTAKE_COUNTERS, HGR_NUM_HITS)
 
 _DTYPE_CODE = {torch.float32: _cabi.HGR_F32, torch.bfloat16: _cabi.HGR_BF16, torch.float16: _cabi.HGR_F16}
 _workspaces = {}
@@ -709,6 +709,47 @@ def hier_finish_rows_gathered_splits(parts_ptr: int, n_parts: int, part_stride: 
                                                          _ptr(sorted_to_pos), _ptr(first_out), _ptr(targets), n_nodes,
                                                          _ptr(chain_ptr), _ptr(chain_pos), _ptr(chain_level),
                                                          _ptr(node_splits), counts.shape[0], _ptr(counts), _stream()))
+
+
+def new_mistake_counts(device, n_sets: int = 1) -> torch.Tensor:
+    """Zeroed counters of ``hier_mistakes``: int64 ``[n_sets, HGR_MISTAKE_COUNTERS]`` (rows, mistakes, sums of h and of d
+    over the first 1/2/5/10/20 entries, histogram of d at top-1; see ``hgr_hier_mistakes`` in the header)."""
+    return torch.zeros((n_sets, HGR_MISTAKE_COUNTERS), dtype=torch.int64, device=device)
+
+
+def hier_mistakes(idx: torch.Tensor, targets: torch.Tensor, chain_ptr: torch.Tensor, chain_node: torch.Tensor,
+                  counts: torch.Tensor, node_splits: Optional[torch.Tensor] = None) -> None:
+    """Mistake severity and LCA distance@k counters (``hgr_hier_mistakes``) of top-K lists on the device: ``idx`` int32
+    node ids ``[B, K]`` (one set) or ``[S, B, K]`` (one set per test split, with ``node_splits``: list set s counts a row
+    only when bit s of ``node_splits[targets[row]]`` is set).  ``targets`` [B] node ids, row by row; ``chain_ptr`` /
+    ``chain_node`` the chain table of ``evaluate.chain_csr``.  ``counts`` (``new_mistake_counts(device, S)``) is
+    incremented.  No host work depends on the batch: the call can be captured in a CUDA graph."""
+    lib = _cabi.load()
+    if idx.dim() == 2:
+        idx = idx.unsqueeze(0)
+    if idx.dim() != 3 or idx.dtype != torch.int32 or not idx.is_cuda:
+        raise ValueError("idx must be a CUDA int32 [B, K] or [S, B, K] tensor")
+    if not (idx.stride(2) == 1 and idx.stride(1) == idx.shape[2]):
+        idx = idx.contiguous()
+    S, B, K = idx.shape
+    targets = _require(targets, "targets", torch.int32)
+    chain_ptr = _require(chain_ptr, "chain_ptr", torch.int32)
+    chain_node = _require(chain_node, "chain_node", torch.int32)
+    if node_splits is not None:
+        node_splits = _require(node_splits, "node_splits", torch.uint8)
+        if node_splits.numel() != chain_ptr.numel() - 1:
+            raise ValueError("node_splits must have one entry per node")
+    elif S != 1:
+        raise ValueError("%d list sets need node_splits" % S)
+    if targets.numel() != B:
+        raise ValueError("targets must have one entry per list row")
+    if not counts.is_cuda or counts.dtype != torch.int64 or counts.numel() != S * HGR_MISTAKE_COUNTERS \
+            or not counts.is_contiguous():
+        raise ValueError("counts must be a contiguous CUDA int64 [%d, %d] tensor (new_mistake_counts)"
+                         % (S, HGR_MISTAKE_COUNTERS))
+    _cabi.check(lib.hgr_hier_mistakes(_ptr(idx), B, K, idx.stride(0) if S > 1 else B * K, S, _ptr(targets),
+                                      _ptr(node_splits), _ptr(chain_ptr), _ptr(chain_node), chain_ptr.numel() - 1,
+                                      _ptr(counts), _stream()))
 
 
 def masked_ce(logits: torch.Tensor, set_ptr: torch.Tensor, set_col: torch.Tensor, label_pos: torch.Tensor,

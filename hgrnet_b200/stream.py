@@ -29,6 +29,10 @@ one pass instead of against ``bank`` (``ops.score_topk_splits`` over the union b
 the SplitEval has them): one line per split, same graph shape, and the per-split counters sit in the same device buffer
 as the others, so a step still makes one D2H copy (``split_hit_counts`` / ``split_ratios``).  The union bank too is taken
 when the stream is built.
+
+With ``mistakes`` (an ``evaluate.MistakeMetrics``) each graph also counts the mistake severity and LCA distance@k of
+the slot's top-K lists against its per-row labels (``ops.hier_mistakes``, one warp per row), one counter set per split
+with ``splits``.  These counters too sit in the one device buffer (``mistake_summary`` / ``split_mistake_summary``).
 """
 from __future__ import annotations
 
@@ -43,14 +47,16 @@ from ._cabi import HGR_HIER_MAX_CHAIN
 class EvalStream:
     def __init__(self, bank: torch.Tensor, col_id: Optional[torch.Tensor] = None, id_base: int = 0, *, batch: int,
                  feat_dtype=torch.float32, K: int = 20, slots: int = 4, streams: int = 2, banks=None,
-                 host_io: bool = True, hier=None, splits=None):
+                 host_io: bool = True, hier=None, splits=None, mistakes=None):
         """``bank`` [C, D] bf16 on the device.  ``banks``: optional list of bank tensors to rotate over per slot
         (benchmarks use it to keep the working set larger than L2).  ``host_io=False`` skips the H2D / D2H nodes
         (features are then written straight into ``dev_feats`` / ``dev_labels``).  ``hier``: optional
         ``evaluate.HierMetrics`` of the model; when given, every step also counts TOR / POR (``hier_ratios``).  Labels
         are node ids; a label outside the hierarchy (e.g. -1 padding) is counted by neither metric.  ``splits``: optional
         ``evaluate.SplitEval``; every step then scores against its splits instead of ``bank`` (``val`` / ``idx`` are
-        ``[S, B, K]``, ``hit_counts`` stays zero, ``split_hit_counts`` / ``split_ratios`` give the per-split results)."""
+        ``[S, B, K]``, ``hit_counts`` stays zero, ``split_hit_counts`` / ``split_ratios`` give the per-split results).
+        ``mistakes``: optional ``evaluate.MistakeMetrics`` of the model (its chain table); every step then also counts the
+        mistake severity and LCA distance@k of the slot's lists (``mistake_summary`` / ``split_mistake_summary``)."""
         self.device = bank.device
         self.K = K
         self.B = batch
@@ -78,7 +84,10 @@ class EvalStream:
         n_hier = 0 if hier is None else (HGR_HIER_MAX_CHAIN + 1) * 4
         n_split = 0 if splits is None else splits.S * (ops.HGR_NUM_HITS + 1)
         n_split_hier = 0 if self._split_hier_args is None else splits.S * (HGR_HIER_MAX_CHAIN + 1) * 4
-        n_counters = ops.HGR_NUM_HITS + n_hier + n_split + n_split_hier
+        self.mistakes = mistakes
+        self._mistake_args = mistakes.args() if mistakes is not None else None
+        n_mist = 0 if mistakes is None else (1 if splits is None else splits.S) * ops.HGR_MISTAKE_COUNTERS
+        n_counters = ops.HGR_NUM_HITS + n_hier + n_split + n_split_hier + n_mist
         if host_io:
             self.host_pack = [torch.zeros(nbytes, dtype=torch.uint8).pin_memory() for _ in range(slots)]
             self.host_feats, self.host_labels = map(list, zip(*[views(p) for p in self.host_pack]))
@@ -93,6 +102,8 @@ class EvalStream:
         o += n_split
         self.split_hier_counts = (self.counters[o:o + n_split_hier].view(-1, HGR_HIER_MAX_CHAIN + 1, 4)
                                   if n_split_hier else None)
+        o += n_split_hier
+        self.mistake_counts = self.counters[o:o + n_mist].view(-1, ops.HGR_MISTAKE_COUNTERS) if n_mist else None
         self.val = [None] * slots
         self.idx = [None] * slots
         self.streams = [torch.cuda.Stream(device=self.device) for _ in range(max(1, min(streams, slots)))]
@@ -119,6 +130,9 @@ class EvalStream:
                                                    counts=self.split_hier_counts, **self._split_hier_args)
         if self._hier_args is not None:                                              # main.py:143,152-191
             ops.hier_metrics_fused_rows(x, targets=self.dev_labels[s], counts=self.hier_counts, **self._hier_args)
+        if self._mistake_args is not None:                                           # main.py:135-148, hierarchy distance
+            ops.hier_mistakes(self.idx[s], self.dev_labels[s], counts=self.mistake_counts,
+                              node_splits=None if self.splits is None else self.splits.node_splits, **self._mistake_args)
         if self.host_io:
             self.host_counters.copy_(self.counters, non_blocking=True)
 
@@ -205,3 +219,22 @@ class EvalStream:
             rows, hits, point, path = hier_totals(c).tolist()
             out.append((0.0, 0.0, 0.0) if rows == 0 else (hits / rows * 100.0, path / rows * 100.0, point / rows * 100.0))
         return out
+
+    def mistake_summary(self):
+        """``evaluate.mistake_summary`` of the rows scored so far (synchronises).  Needs ``mistakes`` without
+        ``splits``."""
+        if self.mistake_counts is None or self.splits is not None:
+            raise RuntimeError("EvalStream was built without mistakes=MistakeMetrics(model), or with splits "
+                               "(use split_mistake_summary)")
+        from .evaluate import mistake_summary
+        self.synchronize()
+        return mistake_summary(self.mistake_counts[0], self.K)
+
+    def split_mistake_summary(self):
+        """Per split ``evaluate.mistake_summary`` over the rows whose label is in the split, in the order of
+        ``splits.names`` (synchronises).  Needs ``mistakes`` and ``splits``."""
+        if self.mistake_counts is None or self.splits is None:
+            raise RuntimeError("EvalStream was built without per-split mistake metrics (pass splits= and mistakes=)")
+        from .evaluate import mistake_summary
+        self.synchronize()
+        return [mistake_summary(c, self.K) for c in self.mistake_counts]

@@ -438,6 +438,35 @@ int hgr_hier_finish_rows_gathered_splits(const uint64_t* parts, int n_parts, int
                                          int n_splits, int64_t* counts, void* stream);
 
 /*
+ * Hierarchical mistake severity and LCA distance@k (Bertinetto et al., "Making Better Mistakes", CVPR 2020) of top-K
+ * lists already on the device -- the lists of hgr_score_topk / hgr_score_topk_splits / the certified merges.  It
+ * extends the Hit@k count of the reference's test() (main.py:135-148) from "is the label in the first k" to "how far
+ * from the label are the first k".  Chain table as in hgr_hier_metrics_fused_rows, with the NODE ids per entry:
+ * chain(n) = c2p[n] + [n] = chain_node[chain_ptr[n] .. chain_ptr[n+1]), depth(n) = len(c2p[n]).  Every c2p[n] is a
+ * shortest root path, so the entry at index i of a chain has depth i.  For a label t and a prediction p:
+ *   lca(t, p) = the largest index i with chain(t)[i] == chain(p)[i] (on a DAG the deepest match, not the end of the
+ *               common prefix); -1 (a virtual super-root) without one
+ *   h(t, p)   = depth(t) - depth(lca)          d(t, p) = depth(t) + depth(p) - 2 depth(lca)
+ * A list entry outside [0, n_nodes) (-1: an empty entry when C < K) counts as the super-root: h = d = depth(t) + 1.
+ * A row counts when 0 <= targets[row] < n_nodes and its chain has 1 .. HGR_HIER_MAX_CHAIN entries (the TOR / POR rule).
+ *
+ *  topk_idx    n_sets lists [B, K] int32 node ids, list set s at topk_idx + s * set_stride; K <= HGR_TOPK_MAX
+ *  node_splits NULL: n_sets must be 1.  Otherwise [n_nodes] uint8 and n_sets <= 8: list set s counts a row only when
+ *              bit s of node_splits[targets[row]] is set (the rule of hgr_score_topk_splits)
+ *  counts      [n_sets][HGR_MISTAKE_COUNTERS] int64, INCREMENTED, per set:
+ *                0      rows
+ *                1      mistakes: rows whose first entry is not the label
+ *                2..6   sum over rows of sum_{j < min(k, K)} h(t, p_j), k in {1, 2, 5, 10, 20}
+ *                7..11  the same sums of d
+ *                12..   histogram of d(t, p_0): bins 0 .. 2 * HGR_HIER_MAX_CHAIN, then one overflow bin
+ * One warp per row, one ballot per list entry.  No allocation, no host work per batch: capturable in a CUDA graph.
+ */
+#define HGR_MISTAKE_COUNTERS (2 + 2 * HGR_NUM_HITS + 2 * HGR_HIER_MAX_CHAIN + 2)
+int hgr_hier_mistakes(const int32_t* topk_idx, int64_t B, int K, int64_t set_stride, int n_sets, const int32_t* targets,
+                      const uint8_t* node_splits, const int32_t* chain_ptr, const int32_t* chain_node, int64_t n_nodes,
+                      int64_t* counts, void* stream);
+
+/*
  * Fused masked cross-entropy of the OM training step over T sampled class sets
  * (model/clip_tree.py:241-277 with nn.CrossEntropyLoss, :49,:275).
  *
