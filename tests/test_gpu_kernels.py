@@ -259,11 +259,13 @@ def test_score_topk_empty_and_bad_args():
         ops.score_topk(x, x, K=20, scale=-1.0)
     with pytest.raises(TypeError):
         ops.score_topk(x.float(), x, K=20)
+    with pytest.raises(HgrError, match="320"):         # more lists per row than the merge kernels hold
+        ops.topk_merge(torch.zeros(321, 4, 7, device=DEV), torch.zeros(321, 4, 7, dtype=torch.int32, device=DEV))
 
 
 # --------------------------------------------------------------------------- merge
 @pytest.mark.parametrize("P,B,K", [(1, 5, 20), (2, 64, 20), (4, 70, 20), (3, 40, 32), (5, 1000, 20), (8, 130, 20), (37, 33, 20),
-                                   (128, 9, 7)])
+                                   (128, 9, 7), (129, 9, 20), (320, 5, 7)])
 def test_topk_merge_matches_sort(P, B, K):
     g = torch.Generator().manual_seed(P * 100 + B)
     vals = torch.randn(P, B, K, generator=g)

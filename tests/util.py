@@ -62,6 +62,84 @@ def compare_topk(val, idx, oracle_logits, col_ids, K, rtol=LOGIT_RTOL, atol=LOGI
     return tie_rows
 
 
+def order_key(v):
+    """int64 restatement of ``topk_list.cuh::order_key``: a larger key is a larger value, and -0 sorts below +0."""
+    b = v.float().contiguous().view(torch.int32).long() & 0xFFFFFFFF
+    return torch.where(b >= 0x80000000, b ^ 0xFFFFFFFF, b | 0x80000000)
+
+
+def _ids_of_rows(rows, col_id, id_base):
+    rows = rows.long()
+    ids = col_id.long()[rows.clamp_min(0)] if col_id is not None else rows + id_base
+    return torch.where(rows >= 0, ids, torch.full_like(ids, -1)).int()
+
+
+def reference_topk(X, bank, K, scale=1.0, col_id=None, id_base=0):
+    """Bit-exact reference of every tcgen05 top-K epilogue: a sort of the dense logits of the same GEMM.
+
+    ``ops.logits_dense`` (tcgen05) holds the fp32 accumulators each epilogue sees -- their rounding does not depend on
+    the element's place in the tile.  Rows are ordered by (value desc, bank row asc), the value compared through the
+    kernels' order key (a stable descending sort of that key).  The ORDER comes from the unscaled accumulators and the
+    VALUES from ``logits_dense(scale=s)``: the lists are sorted before the merge multiplies by ``scale``, so where two
+    distinct accumulators round to the same scaled value the kernels keep the unscaled order, and so does this.
+    Returns device ``(val [B, K] fp32, idx [B, K] int32 ids)``, padded with (-inf, -1) when C < K."""
+    from hgrnet_b200 import ops
+    B, C = X.shape[0], bank.shape[0]
+    acc = ops.logits_dense(X, bank, scale=1.0, impl=ops.HGR_IMPL_TCGEN05)
+    scaled = acc if scale == 1.0 else ops.logits_dense(X, bank, scale=scale, impl=ops.HGR_IMPL_TCGEN05)
+    Kv = min(K, C)
+    rows = torch.sort(order_key(acc), dim=1, descending=True, stable=True).indices[:, :Kv]
+    val = torch.full((B, K), float("-inf"), device=X.device)
+    idx = torch.full((B, K), -1, dtype=torch.int32, device=X.device)
+    val[:, :Kv] = scaled.gather(1, rows)
+    idx[:, :Kv] = _ids_of_rows(rows, None if col_id is None else col_id.to(X.device), id_base)
+    return val, idx
+
+
+def reference_hits(idx, targets):
+    """Hit@{1,2,5,10,20} the kernels count for lists ``idx``: a target below 0 (padding) is never a hit, also not
+    against the -1 that pads a list when C < K."""
+    t = torch.as_tensor(targets).long().cpu()
+    return hits_from_idx(idx, torch.where(t < 0, torch.full_like(t, -2), t))
+
+
+def check_topk_f64(val, idx, X, bank, K, scale=1.0, col_id=None, id_base=0, rows=None):
+    """Float64-certified check of top-K lists whose sums are not the tensor core's (``simt``, rows the production
+    kernel repaired on the CUDA cores).  R = float64 logits (exact products of the bf16 inputs), E = (D + 2) 2^-23
+    scale |x| @ |w| the bound of an fp32 sum of D products and the scaling.  Per row: every value is within E of
+    scale * R of its bank row; values do not increase, ids are distinct, the padding (-inf, -1) appears exactly when
+    C < K; and no bank row left out has scale * R - E above the K-th value.  ``rows``: the rows to check (all)."""
+    B, D = X.shape
+    C = bank.shape[0]
+    dev = X.device
+    sel = torch.arange(B, device=dev) if rows is None else torch.as_tensor(rows, device=dev).long()
+    if sel.numel() == 0:
+        return
+    x, w = X[sel].double(), bank.double()
+    R = scale * (x @ w.T)
+    E = (D + 2) * 2.0 ** -23 * scale * (x.abs() @ w.abs().T)
+    v, ids = val.to(dev)[sel].double(), idx.to(dev)[sel].long()
+    Kv = min(K, C)
+    if Kv < K:
+        assert torch.isinf(v[:, Kv:]).all() and (v[:, Kv:] < 0).all() and (ids[:, Kv:] == -1).all(), "padding"
+    v, ids = v[:, :Kv], ids[:, :Kv]
+    assert (ids >= 0).all(), "a list of C >= K columns holds an empty entry"
+    if col_id is not None:
+        row_of = torch.full((int(col_id.max()) + 1,), -1, dtype=torch.long, device=dev)
+        row_of[col_id.to(dev).long()] = torch.arange(C, device=dev)
+        r = row_of[ids]
+    else:
+        r = ids - id_base
+    assert ((r >= 0) & (r < C)).all(), "an id names no bank row"
+    assert (r.sort(1).values[:, 1:] != r.sort(1).values[:, :-1]).all(), "an id appears twice in a row"
+    assert (v[:, :-1] >= v[:, 1:]).all(), "values not sorted descending"
+    err = (v - R.gather(1, r)).abs() - E.gather(1, r)
+    assert (err <= 0).all(), "value off its float64 logit by more than the bound: %g" % float(err.max())
+    left = torch.ones_like(R, dtype=torch.bool).scatter_(1, r, False)
+    beat = left & ((R - E) > v[:, -1:])
+    assert not beat.any(), "row %d: bank rows left out beat the K-th value" % int(sel[beat.any(1)][0])
+
+
 def row_rel_err(got, ref):
     """Largest per-row relative error ``|got_r - ref_r| / |ref_r|`` over the rows of ``ref`` that are not zero; a zero
     row of ``ref`` must be zero in ``got`` too (inf otherwise).  A global Frobenius measure hides a lost row."""
