@@ -194,18 +194,16 @@ int launch_score_topk_umma(const __nv_bfloat16* X, const __nv_bfloat16* bank, co
                            cudaStream_t stream, const OutScatter* scatter = nullptr, int64_t C_total = 0);
 int umma_global_list_len(int64_t B, int64_t C, int64_t D, int K, int64_t C_total);
 size_t umma_split_workspace_bytes(int64_t B, const Groups& gr, int K);
+// scatter (class shard of the union bank, hgr_score_topk_splits_scatter_bounded): lists sized for each split's GLOBAL
+// stream of split_C_total[s] classes; per split the local top-K and the bound of what was dropped go to the row owners,
+// split s at + s * split_stride, instead of topk_val / topk_idx / counts
 int launch_score_topk_splits_umma(const __nv_bfloat16* X, const __nv_bfloat16* bank, const int32_t* col_id,
                                   int32_t id_base, const int32_t* targets, const uint8_t* node_splits, int64_t n_nodes,
                                   int64_t B, int64_t C, int64_t D, float scale, int K, const Groups& gr,
                                   const uint8_t* group_splits, int S, void* ws, size_t ws_bytes, float* topk_val,
-                                  int32_t* topk_idx, int64_t* counts, bool exact, cudaStream_t stream);
-// class shard of the union bank (hgr_score_topk_splits_scatter_bounded): lists sized for each split's GLOBAL stream of
-// split_C_total[s] classes, per split the local top-K and the bound of what was dropped scattered to the row owners
-int launch_score_topk_splits_scatter_umma(const __nv_bfloat16* X, const __nv_bfloat16* bank, const int32_t* col_id,
-                                          int32_t id_base, int64_t B, int64_t C, int64_t D, float scale, int K,
-                                          const Groups& gr, const uint8_t* group_splits, int S,
-                                          const int64_t* split_C_total, void* ws, size_t ws_bytes,
-                                          const OutScatter& scatter, int64_t split_stride, cudaStream_t stream);
+                                  int32_t* topk_idx, int64_t* counts, bool exact, cudaStream_t stream,
+                                  const OutScatter* scatter = nullptr, const int64_t* split_C_total = nullptr,
+                                  int64_t split_stride = 0);
 int umma_split_global_list_len(int64_t B, int64_t C, int64_t D, int K, const Groups& gr, const uint8_t* group_splits,
                                int S, const int64_t* split_C_total);
 

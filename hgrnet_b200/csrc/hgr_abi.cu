@@ -91,6 +91,20 @@ size_t hgr_score_topk_workspace_bytes(int64_t B, int64_t C, int64_t D, int K) {
   return (a > b ? a : b) + 16;
 }
 
+// The merge of zero lists: every row gets (-inf, -1) -- and, scattered with bounds, a -inf bound.
+static int merge_zero_lists(int64_t B, int K, float* topk_val, int32_t* topk_idx, const OutScatter* scatter,
+                            cudaStream_t stream) {
+  MergeArgs m{};
+  m.B = B;
+  m.KL = K;
+  m.K = K;
+  m.scale = 1.f;
+  m.topk_val = topk_val;
+  m.topk_idx = topk_idx;
+  if (scatter) m.scatter = *scatter;
+  return launch_topk_merge(m, stream);
+}
+
 static int score_topk_impl(const void* X, const void* bank, const int32_t* col_id, int32_t id_base, const int32_t* targets,
                            int64_t B, int64_t C, int64_t D, float scale, int K, void* workspace, size_t workspace_bytes,
                            float* topk_val, int32_t* topk_idx, int64_t* hits, int impl, void* stream,
@@ -104,18 +118,7 @@ static int score_topk_impl(const void* X, const void* bank, const int32_t* col_i
   HGR_CHECK_ARG(C == 0 || (X && bank), "hgr_score_topk: null X/bank");
   HGR_CHECK_ARG(aligned16(X) && aligned16(bank) && aligned16(workspace), "hgr_score_topk: X/bank/workspace must be 16-byte aligned");
   cudaStream_t s = static_cast<cudaStream_t>(stream);
-  if (C == 0) {
-    // empty class set: every list is (-inf, -1); the merge of zero lists writes exactly that
-    MergeArgs m{};
-    m.B = B;
-    m.KL = K;
-    m.K = K;
-    m.scale = 1.f;
-    m.topk_val = topk_val;
-    m.topk_idx = topk_idx;
-    if (scatter) m.scatter = *scatter;
-    return launch_topk_merge(m, s);
-  }
+  if (C == 0) return merge_zero_lists(B, K, topk_val, topk_idx, scatter, s);   // empty class set
   const bool skip_merge = (impl & HGR_IMPL_FLAG_NO_MERGE) != 0;
   impl &= ~HGR_IMPL_FLAG_NO_MERGE;
   const int which = pick_impl(impl, B, C, D, K);
@@ -249,18 +252,13 @@ int hgr_score_topk_splits_scatter_bounded(const void* X, const void* bank, const
   if (C == 0) {
     // no rows on this rank: every split stores (-inf, -1) lists and a -inf bound (the merge of zero lists)
     for (int sp = 0; sp < n_splits; ++sp) {
-      MergeArgs m{};
-      m.B = B;
-      m.KL = K;
-      m.K = K;
-      m.scale = 1.f;
-      m.scatter = sc;
+      OutScatter split_sc = sc;
       for (int g = 0; g < n_blocks; ++g) {
-        m.scatter.val[g] += sp * split_stride;
-        m.scatter.idx[g] += sp * split_stride;
-        m.scatter.bound[g] += sp * split_stride;
+        split_sc.val[g] += sp * split_stride;
+        split_sc.idx[g] += sp * split_stride;
+        split_sc.bound[g] += sp * split_stride;
       }
-      rc = launch_topk_merge(m, s);
+      rc = merge_zero_lists(B, K, nullptr, nullptr, &split_sc, s);
       if (rc != HGR_OK) return rc;
     }
     return HGR_OK;
@@ -270,9 +268,10 @@ int hgr_score_topk_splits_scatter_bounded(const void* X, const void* bank, const
                 "hgr_score_topk_splits_scatter_bounded: X/bank/workspace must be 16-byte aligned");
   if (!umma_supported(B, C, D, K))
     return set_error(HGR_ERR_UNSUPPORTED, "hgr_score_topk_splits_scatter_bounded: shape not supported by the tcgen05 kernel");
-  return launch_score_topk_splits_scatter_umma(static_cast<const __nv_bfloat16*>(X), static_cast<const __nv_bfloat16*>(bank),
-                                               col_id, id_base, B, C, D, scale, K, gr, group_splits, n_splits,
-                                               split_C_total, workspace, workspace_bytes, sc, split_stride, s);
+  return launch_score_topk_splits_umma(static_cast<const __nv_bfloat16*>(X), static_cast<const __nv_bfloat16*>(bank), col_id,
+                                       id_base, nullptr, nullptr, 0, B, C, D, scale, K, gr, group_splits, n_splits,
+                                       workspace, workspace_bytes, nullptr, nullptr, nullptr, false, s, &sc,
+                                       split_C_total, split_stride);
 }
 
 int hgr_score_topk_splits_global_list_len(int64_t B, int64_t C, int64_t D, int K, int n_groups, const int32_t* group_end,
@@ -413,14 +412,11 @@ int hgr_peer_wait(const uint32_t* flags, int n, uint32_t* seq, void* stream) {
   return launch_peer_wait(flags, n, seq, static_cast<cudaStream_t>(stream));
 }
 
-int hgr_topk_merge(const float* part_val, const int32_t* part_idx, int64_t P, int64_t B, int K, int64_t part_stride,
-                   const int32_t* targets, float* topk_val, int32_t* topk_idx, int64_t* hits, void* stream) {
-  HGR_CHECK_ARG(P >= 0 && B >= 0, "hgr_topk_merge: negative size");
-  HGR_CHECK_ARG(K >= 1 && K <= HGR_TOPK_MAX, "hgr_topk_merge: K = %d outside [1, %d]", K, HGR_TOPK_MAX);
-  if (B == 0) return HGR_OK;
-  HGR_CHECK_ARG(topk_val && topk_idx, "hgr_topk_merge: null output");
-  HGR_CHECK_ARG(P == 0 || (part_val && part_idx), "hgr_topk_merge: null parts");
-  HGR_CHECK_ARG(part_stride == 0 || part_stride >= B * K, "hgr_topk_merge: part_stride < B*K");
+// P lists of K entries per row (node ids), merged and counted: hgr_topk_merge, and hgr_topk_merge_certified before it
+// adds its certificate.
+static MergeArgs list_merge_args(const float* part_val, const int32_t* part_idx, int64_t P, int64_t B, int K,
+                                 int64_t part_stride, const int32_t* targets, float* topk_val, int32_t* topk_idx,
+                                 int64_t* hits) {
   MergeArgs m{};
   m.part_val = part_val;
   m.part_idx = part_idx;
@@ -434,7 +430,19 @@ int hgr_topk_merge(const float* part_val, const int32_t* part_idx, int64_t P, in
   m.topk_val = topk_val;
   m.topk_idx = topk_idx;
   m.hits = hits;
-  return launch_topk_merge(m, static_cast<cudaStream_t>(stream));
+  return m;
+}
+
+int hgr_topk_merge(const float* part_val, const int32_t* part_idx, int64_t P, int64_t B, int K, int64_t part_stride,
+                   const int32_t* targets, float* topk_val, int32_t* topk_idx, int64_t* hits, void* stream) {
+  HGR_CHECK_ARG(P >= 0 && B >= 0, "hgr_topk_merge: negative size");
+  HGR_CHECK_ARG(K >= 1 && K <= HGR_TOPK_MAX, "hgr_topk_merge: K = %d outside [1, %d]", K, HGR_TOPK_MAX);
+  if (B == 0) return HGR_OK;
+  HGR_CHECK_ARG(topk_val && topk_idx, "hgr_topk_merge: null output");
+  HGR_CHECK_ARG(P == 0 || (part_val && part_idx), "hgr_topk_merge: null parts");
+  HGR_CHECK_ARG(part_stride == 0 || part_stride >= B * K, "hgr_topk_merge: part_stride < B*K");
+  return launch_topk_merge(list_merge_args(part_val, part_idx, P, B, K, part_stride, targets, topk_val, topk_idx, hits),
+                           static_cast<cudaStream_t>(stream));
 }
 
 int hgr_topk_merge_certified(const float* part_val, const int32_t* part_idx, const float* part_bound, int64_t P, int64_t B,
@@ -450,19 +458,7 @@ int hgr_topk_merge_certified(const float* part_val, const int32_t* part_idx, con
   HGR_CHECK_ARG(part_stride == 0 || part_stride >= B * K, "hgr_topk_merge_certified: part_stride < B*K");
   HGR_CHECK_ARG(bound_stride >= B, "hgr_topk_merge_certified: bound_stride < B");
   HGR_CHECK_ARG(scale > 0.f, "hgr_topk_merge_certified: scale must be > 0");
-  MergeArgs m{};
-  m.part_val = part_val;
-  m.part_idx = part_idx;
-  m.P = P;
-  m.B = B;
-  m.KL = K;
-  m.K = K;
-  m.part_stride = part_stride;
-  m.scale = 1.f;
-  m.targets = targets;
-  m.topk_val = topk_val;
-  m.topk_idx = topk_idx;
-  m.hits = hits;
+  MergeArgs m = list_merge_args(part_val, part_idx, P, B, K, part_stride, targets, topk_val, topk_idx, hits);
   m.part_bound = part_bound;
   m.bound_stride = bound_stride;
   m.shards = shards;

@@ -429,15 +429,17 @@ int launch_score_topk_splits_umma(const __nv_bfloat16* X, const __nv_bfloat16* b
                                   int32_t id_base, const int32_t* targets, const uint8_t* node_splits, int64_t n_nodes,
                                   int64_t B, int64_t C, int64_t D, float scale, int K, const Groups& gr,
                                   const uint8_t* group_splits, int S, void* ws, size_t ws_bytes, float* topk_val,
-                                  int32_t* topk_idx, int64_t* counts, bool exact, cudaStream_t stream) {
+                                  int32_t* topk_idx, int64_t* counts, bool exact, cudaStream_t stream,
+                                  const OutScatter* scatter, const int64_t* split_C_total, int64_t split_stride) {
   if (ws == nullptr || ws_bytes < umma_split_workspace_bytes(B, gr, K))
-    return set_error(HGR_ERR_WORKSPACE, "hgr_score_topk_splits: workspace %zu < %zu bytes", ws_bytes,
+    return set_error(HGR_ERR_WORKSPACE, "%s: workspace %zu < %zu bytes",
+                     scatter ? "hgr_score_topk_splits_scatter_bounded" : "hgr_score_topk_splits", ws_bytes,
                      umma_split_workspace_bytes(B, gr, K));
   CUtensorMap mx, mb;
   Params p{};
   int rc = common_setup(X, bank, B, C, D, &mx, &mb, &p);
   if (rc != HGR_OK) return rc;
-  const SplitPlan plan = split_plan(B, C, D, K, gr, group_splits, S, exact);
+  const SplitPlan plan = split_plan(B, C, D, K, gr, group_splits, S, exact, split_C_total);
   p.sched = plan.sched;
   p.groups = gr;
   p.scale = scale;
@@ -472,54 +474,14 @@ int launch_score_topk_splits_umma(const __nv_bfloat16* X, const __nv_bfloat16* b
   m.bank = bank;
   m.D8 = static_cast<int>(D / 8);
   m.rescan_count = p.stats;
+  if (scatter) m.scatter = *scatter;
+  m.split_stride = split_stride;
   return launch_topk_split_merge(m, stream);
 }
 
 int umma_split_global_list_len(int64_t B, int64_t C, int64_t D, int K, const Groups& gr, const uint8_t* group_splits,
                                int S, const int64_t* split_C_total) {
   return split_plan(B, C, D, K, gr, group_splits, S, false, split_C_total).KL;
-}
-
-int launch_score_topk_splits_scatter_umma(const __nv_bfloat16* X, const __nv_bfloat16* bank, const int32_t* col_id,
-                                          int32_t id_base, int64_t B, int64_t C, int64_t D, float scale, int K,
-                                          const Groups& gr, const uint8_t* group_splits, int S,
-                                          const int64_t* split_C_total, void* ws, size_t ws_bytes,
-                                          const OutScatter& scatter, int64_t split_stride, cudaStream_t stream) {
-  if (ws == nullptr || ws_bytes < umma_split_workspace_bytes(B, gr, K))
-    return set_error(HGR_ERR_WORKSPACE, "hgr_score_topk_splits_scatter_bounded: workspace %zu < %zu bytes", ws_bytes,
-                     umma_split_workspace_bytes(B, gr, K));
-  CUtensorMap mx, mb;
-  Params p{};
-  int rc = common_setup(X, bank, B, C, D, &mx, &mb, &p);
-  if (rc != HGR_OK) return rc;
-  const SplitPlan plan = split_plan(B, C, D, K, gr, group_splits, S, false, split_C_total);
-  p.sched = plan.sched;
-  p.groups = gr;
-  p.scale = scale;
-  p.stats = static_cast<unsigned int*>(ws);
-  const int KL = plan.KL;
-  p.KL = KL;
-  p.part_val = reinterpret_cast<float*>(static_cast<uint8_t*>(ws) + kWsHeaderBytes);
-  p.part_idx = reinterpret_cast<int32_t*>(p.part_val + static_cast<size_t>(p.sched.P) * B * KL);
-  rc = launch_pair_kernel(kEpiTopkGroups, KL, mx, mb, p, stream);
-  if (rc != HGR_OK) return rc;
-  SplitMergeArgs m{};
-  m.part_val = p.part_val;
-  m.part_idx = p.part_idx;
-  m.B = B;
-  m.C = C;
-  m.KL = KL;
-  m.K = K;
-  m.S = S;
-  m.sched = p.sched;
-  m.groups = gr;
-  for (int g = 0; g < gr.n; ++g) m.group_splits[g] = group_splits[g];
-  m.col_id = col_id;
-  m.id_base = id_base;
-  m.scale = scale;
-  m.scatter = scatter;
-  m.split_stride = split_stride;
-  return launch_topk_split_merge(m, stream);
 }
 
 // Row f1 without the dense matrix: X . bank_sorted^T on the tcgen05 loop, per-level arg-max in the epilogue.

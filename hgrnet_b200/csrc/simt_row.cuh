@@ -26,6 +26,12 @@ __device__ __forceinline__ float warp_sum_f32(float v) {
   return v;
 }
 
+__device__ __forceinline__ float warp_max_f32(float v) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));
+  return v;
+}
+
 // xr: the image row as D8 uint4 (8 bf16 each), readable by every lane (shared or global memory).
 template <int KL>
 __device__ __forceinline__ void scan_row_range(const uint4* xr, const uint4* __restrict__ bank4, int64_t c0,
@@ -59,26 +65,33 @@ __device__ __forceinline__ void scan_row_range(const uint4* xr, const uint4* __r
 // independent rows in flight), the image row is a warp-uniform broadcast load, and the 32 finished dot products
 // are offered to the replicated list in ascending row order.  ~10x the throughput of scan_row_range for one warp,
 // which waits a full memory round trip for every two rows.
-template <int KL>
+// `rows` (optional) keeps only the bank rows c with rows(c) true, tested before the row's operands are loaded; the
+// default takes every row and loads unconditionally (a lane past c1 re-reads row c0).
+struct EveryRow {
+  static constexpr bool kFilter = false;
+  __device__ __forceinline__ bool operator()(int64_t) const { return true; }
+};
+
+template <int KL, class Rows = EveryRow>
 __device__ __forceinline__ void scan_row_range_lanes(const uint4* __restrict__ xr, const uint4* __restrict__ bank4,
-                                                     int64_t c0, int64_t c1, int D8, int lane, SortedList<KL>& list) {
+                                                     int64_t c0, int64_t c1, int D8, int lane, SortedList<KL>& list,
+                                                     const Rows& rows = Rows()) {
   for (int64_t cb = c0; cb < c1; cb += 32) {
     const int64_t c = cb + lane;
-    const bool ok = c < c1;
+    const bool ok = c < c1 && rows(c);
     const uint4* b = bank4 + (ok ? c : c0) * D8;
     float a0 = 0.f, a1 = 0.f;
-    int idx = 0;
-    for (; idx + 1 < D8; idx += 2) {
-      const uint4 x0 = __ldg(xr + idx), x1 = __ldg(xr + idx + 1);
-      a0 = dot8_bf16(__ldg(b + idx), x0, a0);
-      a1 = dot8_bf16(__ldg(b + idx + 1), x1, a1);
+    if (ok || !Rows::kFilter) {
+      int idx = 0;
+      for (; idx + 1 < D8; idx += 2) {
+        const uint4 x0 = __ldg(xr + idx), x1 = __ldg(xr + idx + 1);
+        a0 = dot8_bf16(__ldg(b + idx), x0, a0);
+        a1 = dot8_bf16(__ldg(b + idx + 1), x1, a1);
+      }
+      if (idx < D8) a0 = dot8_bf16(__ldg(b + idx), __ldg(xr + idx), a0);
     }
-    if (idx < D8) a0 = dot8_bf16(__ldg(b + idx), __ldg(xr + idx), a0);
     const float v = ok ? a0 + a1 : -INFINITY;
-    float vmax = v;
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) vmax = fmaxf(vmax, __shfl_xor_sync(0xffffffffu, vmax, o));
-    if (vmax > list.thr()) {
+    if (warp_max_f32(v) > list.thr()) {
       for (int l = 0; l < 32; ++l) {
         const float vl = __shfl_sync(0xffffffffu, v, l);
         if (vl > list.thr()) list.insert(vl, static_cast<int32_t>(cb + l));

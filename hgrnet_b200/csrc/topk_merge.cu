@@ -6,16 +6,16 @@
 // multi-GPU head, the combination of the per-rank lists after the NCCL all-gather.
 //
 // One warp per row, kMergeWarps rows per CTA.  The CTA first stages all lists of its rows in
-// shared memory (coalesced), then each warp runs K rounds of a P-way merge: lane l owns lists
+// shared memory (coalesced), then each warp runs K rounds of a P-way merge (merge_heads): lane l owns lists
 // l, l+32, ...; per round the lane-local best head, a warp arg-max by (value desc, list asc),
 // and the winner advances its head (shared-memory read).  Heads compare by (value desc, item
 // asc), every list is itself sorted that way, so the result is ordered (value desc, bank row asc)
 // -- deterministic whatever way the producers interleave bank rows over lists.
 //
 // Speculative lists (KL < K, tcgen05 path): the row is CERTIFIED when every full list ends strictly
-// below the merged K-th value -- anything such a list dropped is <= its last entry, hence cannot
-// belong to (or tie with) the top-K.  An uncertified row is re-scanned exactly by its warp on the CUDA
-// cores (simt_row.cuh).  With randomly ordered bank rows this is a ~1e-8-per-row event.
+// below the merged K-th value (narrow_tails) -- anything such a list dropped is <= its last entry, hence
+// cannot belong to (or tie with) the top-K.  An uncertified row is re-scanned exactly by its warp on the
+// CUDA cores (repair_lists, simt_row.cuh).  With randomly ordered bank rows this is a ~1e-8-per-row event.
 #include "common.cuh"
 #include "simt_row.cuh"
 
@@ -26,122 +26,182 @@ constexpr int kMergeWarps = 4;
 
 constexpr int kDoubtWords = 10;  // bit per list, up to 320 lists per row
 
-// Exact repair of a row whose speculative lists could not all be certified.  Only the column ranges of the
-// DOUBTFUL lists are re-scanned on the CUDA cores (1 / lists-per-row of the bank each); the entries of the certified
-// lists are final as they are (whatever such a list dropped is below the old K-th value, which can only rise) and are
-// inserted as candidates.  Lists are visited in ascending column order and SortedList keeps the first of equal
-// values, so the result has the documented (value desc, bank row asc) order.  The list is replicated in every lane.
-// (Arguments by value: handing the kernel's whole MergeArgs to a non-inlined function would copy it to the stack of
-// every thread at kernel entry.)
-struct RepairArgs {
-  const float* part_val;
-  const int32_t* part_idx;
-  int64_t pstride, C;
-  const void* X;
-  const void* bank;
-  Sched sched;
-  int KL, D8;
-};
-__device__ __noinline__ void repair_row(const RepairArgs a, int64_t row, int lane, int cnt, const uint32_t* dmask,
-                                        SortedList<HGR_TOPK_MAX>& full) {
-  full.init();
-  const int KL = a.KL;
-  const int64_t pstride = a.pstride;
-  const int32_t mt = static_cast<int32_t>(row / a.sched.rows);
-  const int32_t w0 = a.sched.first_cta(mt);
-  for (int p = 0; p < cnt; ++p) {   // list p of the row = worker w0 + p
-    if ((dmask[p >> 5] >> (p & 31)) & 1u) {
-      // the worker's chunk of flattened units, clipped to this row tile -> bank rows [c0, c1)
-      const int64_t t0 = static_cast<int64_t>(mt) * a.sched.U;
-      int64_t u0 = a.sched.unit_begin(w0 + p) - t0, u1 = a.sched.unit_begin(w0 + p + 1) - t0;
-      u0 = u0 < 0 ? 0 : u0;
-      u1 = u1 > a.sched.U ? a.sched.U : u1;
-      int64_t c0 = u0 * kUnit, c1 = u1 * kUnit;
-      c1 = c1 > a.C ? a.C : c1;
-      if (c0 < c1)
-        scan_row_range_lanes<HGR_TOPK_MAX>(reinterpret_cast<const uint4*>(a.X) + row * a.D8,
-                                           reinterpret_cast<const uint4*>(a.bank), c0, c1, a.D8, lane, full);
-    } else {
-      for (int k = 0; k < KL; ++k) {
-        const int64_t g = p * pstride + row * KL + k;
-        const int32_t it = a.part_idx[g];
-        const float v = a.part_val[g];
-        if (it >= 0 && v > full.thr()) full.insert(v, it);
-      }
-    }
-  }
-}
-
-// Exact repair of a row of the class-sharded head whose GLOBAL certificate failed (hgr_topk_merge_certified): list p
-// is shard p's final local top-K (node ids, scaled values).  A doubtful shard (bit p of `dm`: its bound reaches the
-// merged K-th value) is re-scanned completely with the row's features -- over NVLink when the bank is a peer's --, its
-// exact local top-K mapped to node ids and scaled like the producer did; the lists of the other shards are final as
-// they are (what such a shard dropped is below the old K-th value, which can only rise).
-__device__ __noinline__ void repair_row_global(const float* part_val, const int32_t* part_idx, int64_t pstride,
-                                               int64_t row, int K, int P, unsigned dm, const uint4* xrow, int D8,
-                                               const hgr_shard_t* shards, float scale, int lane,
-                                               SortedList<HGR_TOPK_MAX>& full) {
-  full.init();
-  for (int p = 0; p < P; ++p) {
-    if ((dm >> p) & 1u) {
-      const hgr_shard_t sh = shards[p];
-      SortedList<HGR_TOPK_MAX> sub;
-      sub.init();
-      if (sh.C > 0)
-        scan_row_range_lanes<HGR_TOPK_MAX>(xrow, reinterpret_cast<const uint4*>(sh.bank), 0, sh.C, D8, lane, sub);
-#pragma unroll
-      for (int k = 0; k < HGR_TOPK_MAX; ++k) {
-        const int32_t it = sub.i[k];
-        const float v = sub.v[k] * scale;
-        if (it >= 0 && v > full.thr()) full.insert(v, sh.col_id ? sh.col_id[it] : sh.id_base + it);
-      }
-    } else {
-      for (int k = 0; k < K; ++k) {
-        const int64_t g = p * pstride + row * K + k;
-        const int32_t it = part_idx[g];
-        const float v = part_val[g];
-        if (it >= 0 && v > full.thr()) full.insert(v, it);
-      }
-    }
-  }
-}
-
-// Everything the rare repair paths need lives in the frame of this one cold function (two 32-entry lists), so that the
-// merge kernels themselves keep their register count and carry no stack.  `a` points at the kernel's __grid_constant__
-// parameter.  Returns rank `lane` of the repaired row.
-__device__ __noinline__ Cand repair_cold(const MergeArgs* a, int64_t row, int lane, int cnt, const uint32_t* dmask,
-                                         unsigned dm_global) {
-  SortedList<HGR_TOPK_MAX> full;
-  if (dm_global != 0u) {
-    if (lane == 0 && a->repair_count) atomicAdd(a->repair_count, 1u);
-    repair_row_global(a->part_val, a->part_idx, a->part_stride > 0 ? a->part_stride : a->B * a->K, row, a->K,
-                      static_cast<int>(a->P), dm_global, reinterpret_cast<const uint4*>(a->xrows) + row * a->xD8, a->xD8,
-                      a->shards, a->shard_scale, lane, full);
-  } else {
-    if (lane == 0 && a->rescan_count) atomicAdd(a->rescan_count, 1u);
-    RepairArgs ra;
-    ra.part_val = a->part_val;
-    ra.part_idx = a->part_idx;
-    ra.pstride = a->part_stride > 0 ? a->part_stride : a->B * a->KL;
-    ra.C = a->C;
-    ra.X = a->X;
-    ra.bank = a->bank;
-    ra.sched = a->sched;
-    ra.KL = a->KL;
-    ra.D8 = a->D8;
-    repair_row(ra, row, lane, cnt, dmask, full);
-  }
+// Rank `lane` of a list replicated in every lane.
+__device__ __forceinline__ Cand lane_entry(const SortedList<HGR_TOPK_MAX>& list, int lane) {
   Cand c;
   c.v = -INFINITY;
   c.i = -1;
 #pragma unroll
   for (int k = 0; k < HGR_TOPK_MAX; ++k) {
     if (lane == k) {
-      c.v = full.v[k];
-      c.i = full.i[k];
+      c.v = list.v[k];
+      c.i = list.i[k];
     }
   }
   return c;
+}
+
+// Offers the valid entries (item >= 0) of a list of n to `full`, in list order.
+__device__ __forceinline__ void insert_entries(SortedList<HGR_TOPK_MAX>& full, const float* val, const int32_t* idx, int n) {
+  for (int k = 0; k < n; ++k) {
+    const int32_t it = idx[k];
+    const float v = val[k];
+    if (it >= 0 && v > full.thr()) full.insert(v, it);
+  }
+}
+
+// The two exact repairs below (repair_lists, repair_shards) are written once and fill a replicated list `full`.  The
+// kernels reach them only through the cold __noinline__ repair_cold of their argument type, so that everything the
+// rare repair needs (two 32-entry lists) lives outside the merge kernels, which keep their register count.  repair_cold
+// takes a pointer to the kernel's __grid_constant__ parameter (handed over by value, the whole argument block would be
+// copied to the stack of every thread at kernel entry) and returns rank `lane` of the repaired row.
+
+// ---- exact repair of the scoring kernel's own lists (repair_lists) ----------------------------------------------
+// A row -- or split s of a row -- whose speculative lists could not all be certified.  Only the column ranges of the
+// DOUBTFUL lists (bits of `dmask`) are re-scanned on the CUDA cores (1 / lists-per-row of the bank each); the entries of
+// the certified lists are final as they are (whatever such a list dropped is below the old K-th value, which can only
+// rise) and are inserted as candidates.  Slots are visited in ascending column order and SortedList keeps the first of
+// equal values, so the result has the documented (value desc, bank row asc) order.
+// slot_cols: bank rows [c0, c1) of list slot p of row tile mt, and whether the slot takes part in split s.
+//  * MergeArgs: slot p is worker first_cta(mt) + p, its chunk of flattened units clipped to the tile; every slot counts.
+//  * SplitMergeArgs: slot p of the grouped schedule (group_slot_range); it counts when its group is in split s.
+__device__ __forceinline__ bool slot_cols(const MergeArgs& a, int32_t mt, int p, int, int64_t& c0, int64_t& c1) {
+  const int64_t t0 = static_cast<int64_t>(mt) * a.sched.U;
+  const int32_t w = a.sched.first_cta(mt) + p;
+  int64_t u0 = a.sched.unit_begin(w) - t0, u1 = a.sched.unit_begin(w + 1) - t0;
+  u0 = u0 < 0 ? 0 : u0;
+  u1 = u1 > a.sched.U ? a.sched.U : u1;
+  c0 = u0 * kUnit;
+  c1 = u1 * kUnit;
+  c1 = c1 > a.C ? a.C : c1;
+  return true;
+}
+__device__ __forceinline__ bool slot_cols(const SplitMergeArgs& a, int32_t mt, int p, int s, int64_t& c0, int64_t& c1) {
+  const int g = group_slot_range(a.sched, a.groups, mt, p, c0, c1);
+  return (a.group_splits[g] >> s) & 1u;
+}
+__device__ __forceinline__ int64_t list_stride(const MergeArgs& a) { return a.part_stride > 0 ? a.part_stride : a.B * a.KL; }
+__device__ __forceinline__ int64_t list_stride(const SplitMergeArgs& a) { return a.B * a.KL; }
+
+template <class Args>
+__device__ __forceinline__ void repair_lists(const Args* a, int64_t row, int lane, int cnt, int s, const uint32_t* dmask,
+                                             SortedList<HGR_TOPK_MAX>& full) {
+  const int KL = a->KL;
+  const int64_t pstride = list_stride(*a);
+  const int32_t mt = static_cast<int32_t>(row / a->sched.rows);
+  for (int p = 0; p < cnt; ++p) {
+    int64_t c0, c1;
+    if (!slot_cols(*a, mt, p, s, c0, c1)) continue;
+    if ((dmask[p >> 5] >> (p & 31)) & 1u)
+      scan_row_range_lanes<HGR_TOPK_MAX>(reinterpret_cast<const uint4*>(a->X) + row * a->D8,
+                                         reinterpret_cast<const uint4*>(a->bank), c0, c1, a->D8, lane, full);
+    else
+      insert_entries(full, a->part_val + p * pstride + row * KL, a->part_idx + p * pstride + row * KL, KL);
+  }
+}
+
+// ---- exact repair from the shard table (repair_shards) ----------------------------------------------------------
+// Owner side of the class-sharded head: list p of a row is class shard p's final local top-K (node ids, values scaled
+// by the producer).  A doubtful shard (bit p of `dm`: its bound reaches the merged K-th value) is re-scanned completely
+// with the row's features -- over NVLink when the bank is a peer's --, its exact local top-K mapped to node ids and
+// scaled like the producer did; the lists of the other shards are final as they are (what such a shard dropped is
+// below the old K-th value, which can only rise).  Shards are visited in ascending order and SortedList keeps the first
+// of equal values, so the tie order stays (value desc, shard asc, local row asc).  All HGR_TOPK_MAX entries of a
+// re-scanned shard are offered (an unrolled loop keeps its list in registers), but only ranks < K of the result are
+// kept, and those are the same as with K entries: the shard's entry of rank k >= K sorts behind K entries of its own
+// shard (values >= its own -- the scale keeps the order -- offered earlier), so it can only land at rank K or later.
+//  * MergeArgs (hgr_topk_merge_certified): every row of a shard; list p at p * part_stride + row * K.
+//  * SplitCertArgs (hgr_topk_merge_splits_certified), split s: the shard rows whose node has bit s in node_splits;
+//    list p at s * split_stride + p * part_stride + row * K.
+struct SplitRows {   // bank rows of a shard whose node is in split s
+  static constexpr bool kFilter = true;
+  const int32_t* col_id;
+  int32_t id_base;
+  const uint8_t* node_splits;
+  int64_t n_nodes;
+  int s;
+  __device__ __forceinline__ bool operator()(int64_t c) const {
+    const int64_t node = col_id ? col_id[c] : id_base + c;
+    return node >= 0 && node < n_nodes && ((node_splits[node] >> s) & 1u);
+  }
+};
+__device__ __forceinline__ EveryRow shard_rows(const MergeArgs&, const hgr_shard_t&, int) { return EveryRow(); }
+__device__ __forceinline__ SplitRows shard_rows(const SplitCertArgs& a, const hgr_shard_t& sh, int s) {
+  return SplitRows{sh.col_id, sh.id_base, a.node_splits, a.n_nodes, s};
+}
+__device__ __forceinline__ int64_t shard_list(const MergeArgs& a, int p, int64_t row, int) {
+  return p * (a.part_stride > 0 ? a.part_stride : a.B * a.K) + row * a.K;
+}
+__device__ __forceinline__ int64_t shard_list(const SplitCertArgs& a, int p, int64_t row, int s) {
+  return s * a.split_stride + p * a.part_stride + row * a.K;
+}
+__device__ __forceinline__ float shard_scale(const MergeArgs& a) { return a.shard_scale; }
+__device__ __forceinline__ float shard_scale(const SplitCertArgs& a) { return a.scale; }
+
+template <class Args>
+__device__ __forceinline__ void repair_shards(const Args* a, int64_t row, int lane, int s, unsigned dm,
+                                              SortedList<HGR_TOPK_MAX>& full) {
+  const int K = a->K;
+  const uint4* xr = reinterpret_cast<const uint4*>(a->xrows) + row * a->xD8;
+  for (int p = 0; p < static_cast<int>(a->P); ++p) {
+    if ((dm >> p) & 1u) {
+      const hgr_shard_t sh = a->shards[p];
+      SortedList<HGR_TOPK_MAX> sub;
+      sub.init();
+      scan_row_range_lanes<HGR_TOPK_MAX>(xr, reinterpret_cast<const uint4*>(sh.bank), 0, sh.C, a->xD8, lane, sub,
+                                         shard_rows(*a, sh, s));
+#pragma unroll
+      for (int k = 0; k < HGR_TOPK_MAX; ++k) {
+        const int32_t it = sub.i[k];
+        const float v = sub.v[k] * shard_scale(*a);
+        if (it >= 0 && v > full.thr()) full.insert(v, sh.col_id ? sh.col_id[it] : sh.id_base + it);
+      }
+    } else {
+      const int64_t l = shard_list(*a, p, row, s);
+      insert_entries(full, a->part_val + l, a->part_idx + l, K);
+    }
+  }
+}
+
+// MergeArgs (one call site for both repairs): from the shard table when the global certificate failed (dm_global != 0),
+// else of the row's own speculative lists.  The list lives in repair_cold's frame and the repairs run in functions of
+// their own: under the 72-register budget of these kernels a list held in registers would spill.
+__device__ __noinline__ void repair_row(const MergeArgs* a, int64_t row, int lane, int cnt, const uint32_t* dmask,
+                                        SortedList<HGR_TOPK_MAX>& full) {
+  repair_lists(a, row, lane, cnt, 0, dmask, full);
+}
+__device__ __noinline__ void repair_row_global(const MergeArgs* a, int64_t row, int lane, unsigned dm,
+                                               SortedList<HGR_TOPK_MAX>& full) {
+  repair_shards(a, row, lane, 0, dm, full);
+}
+__device__ __noinline__ Cand repair_cold(const MergeArgs* a, int64_t row, int lane, int cnt, const uint32_t* dmask,
+                                         unsigned dm_global) {
+  SortedList<HGR_TOPK_MAX> full;
+  full.init();
+  if (dm_global != 0u) {
+    if (lane == 0 && a->repair_count) atomicAdd(a->repair_count, 1u);
+    repair_row_global(a, row, lane, dm_global, full);
+  } else {
+    if (lane == 0 && a->rescan_count) atomicAdd(a->rescan_count, 1u);
+    repair_row(a, row, lane, cnt, dmask, full);
+  }
+  return lane_entry(full, lane);
+}
+// SplitMergeArgs (split s of a row) and SplitCertArgs (split s of an owned row of the class-sharded head).
+__device__ __noinline__ Cand repair_cold(const SplitMergeArgs* a, int64_t row, int lane, int cnt, int s,
+                                         const uint32_t* dmask) {
+  SortedList<HGR_TOPK_MAX> full;
+  full.init();
+  if (lane == 0 && a->rescan_count) atomicAdd(a->rescan_count, 1u);
+  repair_lists(a, row, lane, cnt, s, dmask, full);
+  return lane_entry(full, lane);
+}
+__device__ __noinline__ Cand repair_cold(const SplitCertArgs* a, int64_t row, int lane, int s, unsigned dm) {
+  if (lane == 0 && a->repair_count) atomicAdd(a->repair_count, 1u);
+  SortedList<HGR_TOPK_MAX> full;
+  full.init();
+  repair_shards(a, row, lane, s, dm, full);
+  return lane_entry(full, lane);
 }
 
 // Lists of a row: P, or -- for the scoring kernel's own lists -- one per worker of the row's tile.
@@ -178,10 +238,10 @@ __device__ __forceinline__ void rank_winners(unsigned long long* win, int ksel, 
 
 // Tail shared by both merge kernels.  Lane r holds rank r of the merged list (my_v, my_i = bank row or -1).
 // `dmask` (per-warp shared memory, one bit per list): full speculative lists that end at or above the merged K-th
-// value -> the row is repaired exactly (repair_row).  Then: bank row -> node id, scale, store (dense or row-block
+// value -> the row is repaired exactly (repair_cold).  Then: bank row -> node id, scale, store (dense or row-block
 // scatter), Hit@k.
-// `tailmax`: lane-local largest last entry of a FULL narrow list (-inf: none) -- what the producer of a class shard
-// reports as its bound when the certificate is left to the owner of the row (scatter.emit_bound).
+// `tailmax`: lane-local largest last entry of a FULL narrow list (-inf: none; narrow_tails) -- what the producer of a
+// class shard reports as its bound when the certificate is left to the owner of the row (scatter.emit_bound).
 __device__ __forceinline__ void finish_row(const MergeArgs& a, int64_t row, int lane, float my_v, int32_t my_i,
                                            bool doubt, const uint32_t* dmask, int cnt, int* s_hits,
                                            float tailmax = -INFINITY) {
@@ -216,9 +276,7 @@ __device__ __forceinline__ void finish_row(const MergeArgs& a, int64_t row, int 
     oi[orow * K + lane] = gid;
   }
   if (emit_bound) {
-    float b = a.KL < K ? tailmax : -INFINITY;   // K-entry lists drop nothing that could matter
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) b = fmaxf(b, __shfl_xor_sync(0xffffffffu, b, o));
+    const float b = warp_max_f32(a.KL < K ? tailmax : -INFINITY);   // K-entry lists drop nothing that could matter
     if (lane == 0) {
       const int64_t g = row / a.scatter.block_rows;
       a.scatter.bound[g][row - g * a.scatter.block_rows] = b * a.scale;
@@ -234,6 +292,103 @@ __device__ __forceinline__ void finish_row(const MergeArgs& a, int64_t row, int 
         if (pos < hit_cut(c)) atomicAdd(&s_hits[c], 1);
     }
   }
+}
+
+// ---- K rounds of the P-way merge of sorted lists in shared memory (merge_heads) ---------------------------------
+// lv / li: the warp's lists, [list][KL], each sorted (value desc, item asc).  Lane l owns lists l, l + 32, ...; live[q]
+// says whether list lane + 32 q takes part.  Per round the lane-local best head, a warp arg-max by (value desc, item
+// asc), and the lowest lane holding the winner advances that list.  Lane r gets rank r of the result in (my_v, my_i),
+// (-inf, -1) past the last candidate.  Returns the K-th value (-inf: fewer than K candidates).
+template <int kMaxListsPerLane>
+__device__ __forceinline__ float merge_heads(const float* lv, const int32_t* li, int KL, int K,
+                                             const bool (&live)[kMaxListsPerLane], int lane, float& my_v, int32_t& my_i) {
+  int head[kMaxListsPerLane];
+  float hv[kMaxListsPerLane];   // value of the current head of my q-th list (-inf: exhausted)
+  int32_t hi[kMaxListsPerLane]; // its item (bank row / node id)
+#pragma unroll
+  for (int q = 0; q < kMaxListsPerLane; ++q) {
+    const int p = lane + 32 * q;
+    head[q] = 0;
+    hi[q] = live[q] ? li[p * KL] : -1;
+    hv[q] = hi[q] >= 0 ? lv[p * KL] : -INFINITY;
+  }
+  my_v = -INFINITY;
+  my_i = -1;
+  float kth = -INFINITY;
+  for (int r = 0; r < K; ++r) {
+    // lane-local best head, then warp arg-max; order: value desc, item asc
+    float bv = hv[0];
+    int32_t bi = hi[0];
+#pragma unroll
+    for (int q = 1; q < kMaxListsPerLane; ++q) {
+      if (hv[q] > bv || (hv[q] == bv && hi[q] < bi && hi[q] >= 0)) {
+        bv = hv[q];
+        bi = hi[q];
+      }
+    }
+    const float lbv = bv;
+    const int32_t lbi = bi;
+    // warp arg-max with two REDUX instructions: max of an order-preserving integer image of the value, then
+    // the smallest item among the lanes that hold that value
+    const uint32_t lkey = order_key(lbv);
+    const uint32_t mkey = __reduce_max_sync(0xffffffffu, lkey);
+    const uint32_t mitem =
+        __reduce_min_sync(0xffffffffu, (lkey == mkey && lbi >= 0) ? static_cast<uint32_t>(lbi) : 0xFFFFFFFFu);
+    if (mitem == 0xFFFFFFFFu) {  // every list exhausted: fewer than K candidates, the rest stays (-inf, -1)
+      kth = -INFINITY;
+      break;
+    }
+    bv = order_key_value(mkey);
+    bi = static_cast<int32_t>(mitem);
+    kth = bv;
+    // the lowest lane holding the winner advances that list
+    const unsigned holders = __ballot_sync(0xffffffffu, lbv == bv && lbi == bi);
+    if (lane == __ffs(holders) - 1) {
+      bool done = false;
+#pragma unroll
+      for (int q = 0; q < kMaxListsPerLane; ++q) {
+        if (!done && hv[q] == bv && hi[q] == bi) {
+          const int p = lane + 32 * q;
+          const int h = ++head[q];
+          hi[q] = h < KL ? li[p * KL + h] : -1;
+          hv[q] = hi[q] >= 0 ? lv[p * KL + h] : -INFINITY;
+          done = true;
+        }
+      }
+    }
+    if (lane == r) {
+      my_v = bv;
+      my_i = bi;
+    }
+  }
+  return kth;
+}
+
+// ---- the tails of full narrow lists (narrow_tails) --------------------------------------------------------------
+// Speculative lists (KL < K): a FULL list whose last entry is at or above the merged K-th value `kth` may have dropped
+// members of (or ties with) the top-K.  Every such live list of the lane gets its bit in the warp's doubt mask `dmask`
+// (null: no marks) and sets `doubt`.  Returns the lane-local largest last entry of a full live list (-inf: none) --
+// what the producer of a class shard reports as its bound when the certificate is left to the owner of the row.
+// K-entry lists drop nothing that could matter: -inf, no marks.
+template <int kMaxListsPerLane>
+__device__ __forceinline__ float narrow_tails(const float* lv, const int32_t* li, int KL, int K,
+                                              const bool (&live)[kMaxListsPerLane], int lane, float kth, uint32_t* dmask,
+                                              bool& doubt) {
+  float tailmax = -INFINITY;
+  if (KL < K) {
+#pragma unroll
+    for (int q = 0; q < kMaxListsPerLane; ++q) {
+      const int p = lane + 32 * q;
+      if (live[q] && li[p * KL + KL - 1] >= 0) {
+        tailmax = fmaxf(tailmax, lv[p * KL + KL - 1]);
+        if (dmask && lv[p * KL + KL - 1] >= kth) {
+          doubt = true;
+          atomicOr(&dmask[p >> 5], 1u << (p & 31));
+        }
+      }
+    }
+  }
+  return tailmax;
 }
 
 // kMaxListsPerLane: 4 covers P <= 128 lists per row, 10 covers P <= 320 (one list per epilogue warp of
@@ -276,82 +431,14 @@ topk_merge_kernel(const __grid_constant__ MergeArgs a) {
     const float* lv = s_val + warp * slots * KL;
     const int32_t* li = s_idx + warp * slots * KL;
 
-    int head[kMaxListsPerLane];
-    float hv[kMaxListsPerLane];   // value of the current head of my q-th list (-inf: exhausted)
-    int32_t hi[kMaxListsPerLane]; // its item (bank row / node id)
+    bool live[kMaxListsPerLane];
 #pragma unroll
-    for (int q = 0; q < kMaxListsPerLane; ++q) {
-      const int p = lane + 32 * q;
-      head[q] = 0;
-      hi[q] = p < cnt ? li[p * KL] : -1;
-      hv[q] = hi[q] >= 0 ? lv[p * KL] : -INFINITY;
-    }
-    float my_v = -INFINITY;  // lane r keeps rank r of the result
-    int32_t my_i = -1;
-    float kth = -INFINITY;
-    for (int r = 0; r < K; ++r) {
-      // lane-local best head, then warp arg-max; order: value desc, item asc
-      float bv = hv[0];
-      int32_t bi = hi[0];
-#pragma unroll
-      for (int q = 1; q < kMaxListsPerLane; ++q) {
-        if (hv[q] > bv || (hv[q] == bv && hi[q] < bi && hi[q] >= 0)) {
-          bv = hv[q];
-          bi = hi[q];
-        }
-      }
-      const float lbv = bv;
-      const int32_t lbi = bi;
-      // warp arg-max with two REDUX instructions: max of an order-preserving integer image of the value, then
-      // the smallest item among the lanes that hold that value
-      const uint32_t lkey = order_key(lbv);
-      const uint32_t mkey = __reduce_max_sync(0xffffffffu, lkey);
-      const uint32_t mitem =
-          __reduce_min_sync(0xffffffffu, (lkey == mkey && lbi >= 0) ? static_cast<uint32_t>(lbi) : 0xFFFFFFFFu);
-      if (mitem == 0xFFFFFFFFu) {  // every list exhausted: fewer than K candidates, the rest stays (-inf, -1)
-        kth = -INFINITY;
-        break;
-      }
-      bv = order_key_value(mkey);
-      bi = static_cast<int32_t>(mitem);
-      kth = bv;
-      // the lowest lane holding the winner advances that list
-      const unsigned holders = __ballot_sync(0xffffffffu, lbv == bv && lbi == bi);
-      if (lane == __ffs(holders) - 1) {
-        bool done = false;
-#pragma unroll
-        for (int q = 0; q < kMaxListsPerLane; ++q) {
-          if (!done && hv[q] == bv && hi[q] == bi) {
-            const int p = lane + 32 * q;
-            const int h = ++head[q];
-            hi[q] = h < KL ? li[p * KL + h] : -1;
-            hv[q] = hi[q] >= 0 ? lv[p * KL + h] : -INFINITY;
-            done = true;
-          }
-        }
-      }
-      if (lane == r) {
-        my_v = bv;
-        my_i = bi;
-      }
-    }
-
+    for (int q = 0; q < kMaxListsPerLane; ++q) live[q] = lane + 32 * q < cnt;
+    float my_v;  // lane r keeps rank r of the result
+    int32_t my_i;
+    const float kth = merge_heads<kMaxListsPerLane>(lv, li, KL, K, live, lane, my_v, my_i);
     bool doubt = false;
-    float tailmax = -INFINITY;
-    if (KL < K) {
-      // certificate for speculative (narrow) lists
-#pragma unroll
-      for (int q = 0; q < kMaxListsPerLane; ++q) {
-        const int p = lane + 32 * q;
-        if (p < cnt && li[p * KL + KL - 1] >= 0) {
-          tailmax = fmaxf(tailmax, lv[p * KL + KL - 1]);
-          if (lv[p * KL + KL - 1] >= kth) {
-            doubt = true;
-            atomicOr(&s_dmask[warp][p >> 5], 1u << (p & 31));
-          }
-        }
-      }
-    }
+    const float tailmax = narrow_tails<kMaxListsPerLane>(lv, li, KL, K, live, lane, kth, s_dmask[warp], doubt);
     finish_row(a, row, lane, my_v, my_i, doubt, s_dmask[warp], cnt, s_hits, tailmax);
   }
   flush_hits(a, s_hits, threadIdx.x);
@@ -687,46 +774,35 @@ topk_merge_counts_kernel(const __grid_constant__ MergeArgs a) {
 // ---- per-split merge (hgr_score_topk_splits) --------------------------------------------------------------------
 // The lists of a row on the grouped schedule never cross a group, so the lists of the row's groups in split s cover
 // exactly the columns of s.  One warp per row stages all the row's lists in shared memory, then for every split runs
-// the K rounds of the P-way merge of topk_merge_kernel over that split's lists only, certifies the result against the
-// split's own K-th value and, for an uncertified (row, split), re-scans that split's doubtful lists exactly.
+// merge_heads over that split's lists only, certifies the result against the split's own K-th value (narrow_tails)
+// and, for an uncertified (row, split), re-scans that split's doubtful lists exactly (repair_lists).
 constexpr int kSplitDoubtWords = 4;   // bit per list, up to 128 lists per row
 
-// Exact repair of split s of a row (cold): the doubtful lists of s are re-scanned over their bank rows, the others of s
-// inserted as they are -- in column order, as repair_row does.  Returns rank `lane` of the repaired row.
-__device__ __noinline__ Cand split_repair_cold(const SplitMergeArgs* a, int64_t row, int lane, int cnt, int s,
-                                               const uint32_t* dmask) {
-  if (lane == 0 && a->rescan_count) atomicAdd(a->rescan_count, 1u);
-  SortedList<HGR_TOPK_MAX> full;
-  full.init();
-  const int32_t mt = static_cast<int32_t>(row / a->sched.rows);
-  const int KL = a->KL;
-  for (int p = 0; p < cnt; ++p) {
-    int64_t c0, c1;
-    const int g = group_slot_range(a->sched, a->groups, mt, p, c0, c1);
-    if (!((a->group_splits[g] >> s) & 1u)) continue;
-    if ((dmask[p >> 5] >> (p & 31)) & 1u) {
-      scan_row_range_lanes<HGR_TOPK_MAX>(reinterpret_cast<const uint4*>(a->X) + row * a->D8,
-                                         reinterpret_cast<const uint4*>(a->bank), c0, c1, a->D8, lane, full);
-    } else {
-      for (int k = 0; k < KL; ++k) {
-        const int64_t e = (p * a->B + row) * KL + k;
-        const int32_t it = a->part_idx[e];
-        const float v = a->part_val[e];
-        if (it >= 0 && v > full.thr()) full.insert(v, it);
-      }
-    }
-  }
-  Cand c;
-  c.v = -INFINITY;
-  c.i = -1;
+// Per-split Hit@k and row counters of a CTA: cnt[c] (= s_cnt[s][c]) counts Hit@hit_cut(c), cnt[HGR_NUM_HITS] the rows
+// whose label is a class of split s.  count_split_row: one such row, lane r holding rank r (node id `gid`, -1: none)
+// of its list of s.
+__device__ __forceinline__ void count_split_row(unsigned int* cnt, int lane, int K, int32_t gid, int32_t target) {
+  const unsigned m = __ballot_sync(0xffffffffu, lane < K && gid >= 0 && gid == target);
+  if (lane == 0) {
+    atomicAdd(&cnt[HGR_NUM_HITS], 1u);
+    if (m != 0) {
+      const int pos = __ffs(m) - 1;
 #pragma unroll
-  for (int k = 0; k < HGR_TOPK_MAX; ++k) {
-    if (lane == k) {
-      c.v = full.v[k];
-      c.i = full.i[k];
+      for (int c = 0; c < HGR_NUM_HITS; ++c)
+        if (pos < hit_cut(c)) atomicAdd(&cnt[c], 1u);
     }
   }
-  return c;
+}
+// The CTA's counters of the S splits into counts[S][HGR_NUM_HITS + 1] (null: none).  `tid` = threadIdx.x (flush_hits).
+__device__ __forceinline__ void flush_split_counts(const unsigned int (*s_cnt)[HGR_NUM_HITS + 1], int S, int64_t* counts,
+                                                   int tid) {
+  __syncthreads();
+  if (counts) {
+    for (int i = tid; i < S * (HGR_NUM_HITS + 1); i += blockDim.x) {
+      const unsigned int v = (&s_cnt[0][0])[i];
+      if (v) atomicAdd(reinterpret_cast<unsigned long long*>(counts) + i, static_cast<unsigned long long>(v));
+    }
+  }
 }
 
 // kScatter (hgr_score_topk_splits_scatter_bounded, producer of the class-sharded head): no local certificate or repair;
@@ -776,73 +852,19 @@ topk_split_merge_kernel(const __grid_constant__ SplitMergeArgs a) {
     const uint32_t tbits = (target >= 0 && target < a.n_nodes) ? a.node_splits[target] : 0u;
 
     for (int s = 0; s < a.S; ++s) {
-      int head[kMaxListsPerLane];
-      float hv[kMaxListsPerLane];
-      int32_t hi[kMaxListsPerLane];
+      bool live[kMaxListsPerLane];
 #pragma unroll
-      for (int q = 0; q < kMaxListsPerLane; ++q) {
-        const int p = lane + 32 * q;
-        head[q] = 0;
-        hi[q] = ((lmask[q] >> s) & 1u) ? li[p * KL] : -1;
-        hv[q] = hi[q] >= 0 ? lv[p * KL] : -INFINITY;
-      }
-      float my_v = -INFINITY;
-      int32_t my_i = -1;
-      float kth = -INFINITY;
-      for (int r = 0; r < K; ++r) {
-        float bv = hv[0];
-        int32_t bi = hi[0];
-#pragma unroll
-        for (int q = 1; q < kMaxListsPerLane; ++q) {
-          if (hv[q] > bv || (hv[q] == bv && hi[q] < bi && hi[q] >= 0)) {
-            bv = hv[q];
-            bi = hi[q];
-          }
-        }
-        const float lbv = bv;
-        const int32_t lbi = bi;
-        const uint32_t lkey = order_key(lbv);
-        const uint32_t mkey = __reduce_max_sync(0xffffffffu, lkey);
-        const uint32_t mitem =
-            __reduce_min_sync(0xffffffffu, (lkey == mkey && lbi >= 0) ? static_cast<uint32_t>(lbi) : 0xFFFFFFFFu);
-        if (mitem == 0xFFFFFFFFu) {   // the split's lists are exhausted: the rest stays (-inf, -1)
-          kth = -INFINITY;
-          break;
-        }
-        bv = order_key_value(mkey);
-        bi = static_cast<int32_t>(mitem);
-        kth = bv;
-        const unsigned holders = __ballot_sync(0xffffffffu, lbv == bv && lbi == bi);
-        if (lane == __ffs(holders) - 1) {
-          bool done = false;
-#pragma unroll
-          for (int q = 0; q < kMaxListsPerLane; ++q) {
-            if (!done && hv[q] == bv && hi[q] == bi) {
-              const int p = lane + 32 * q;
-              const int h = ++head[q];
-              hi[q] = h < KL ? li[p * KL + h] : -1;
-              hv[q] = hi[q] >= 0 ? lv[p * KL + h] : -INFINITY;
-              done = true;
-            }
-          }
-        }
-        if (lane == r) {
-          my_v = bv;
-          my_i = bi;
-        }
-      }
+      for (int q = 0; q < kMaxListsPerLane; ++q) live[q] = (lmask[q] >> s) & 1u;
+      float my_v;
+      int32_t my_i;
+      const float kth = merge_heads<kMaxListsPerLane>(lv, li, KL, K, live, lane, my_v, my_i);
+      // certificate against the split's own K-th value: a full narrow list of s that ends at or above it may hide
+      // members of the split's top-K (kScatter: the bound of what they dropped, no certificate)
+      bool doubt = false;
+      const float tailmax =
+          narrow_tails<kMaxListsPerLane>(lv, li, KL, K, live, lane, kth, kScatter ? nullptr : s_dmask[warp], doubt);
       if constexpr (kScatter) {
-        // bound of split s: the largest last entry of a full narrow list of s (K-entry lists drop nothing that matters)
-        float b = -INFINITY;
-        if (KL < K) {
-#pragma unroll
-          for (int q = 0; q < kMaxListsPerLane; ++q) {
-            const int p = lane + 32 * q;
-            if (((lmask[q] >> s) & 1u) && li[p * KL + KL - 1] >= 0) b = fmaxf(b, lv[p * KL + KL - 1]);
-          }
-        }
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) b = fmaxf(b, __shfl_xor_sync(0xffffffffu, b, o));
+        const float b = warp_max_f32(tailmax);
         const int64_t g = row / a.scatter.block_rows;
         const int64_t orow = row - g * a.scatter.block_rows;
         const int64_t so = s * a.split_stride;
@@ -853,22 +875,9 @@ topk_split_merge_kernel(const __grid_constant__ SplitMergeArgs a) {
         if (lane == 0) a.scatter.bound[g][so + orow] = b * a.scale;
         continue;
       }
-      // certificate against the split's own K-th value: a full narrow list of s that ends at or above it may hide
-      // members of the split's top-K
-      bool doubt = false;
-      if (KL < K) {
-#pragma unroll
-        for (int q = 0; q < kMaxListsPerLane; ++q) {
-          const int p = lane + 32 * q;
-          if (((lmask[q] >> s) & 1u) && li[p * KL + KL - 1] >= 0 && lv[p * KL + KL - 1] >= kth) {
-            doubt = true;
-            atomicOr(&s_dmask[warp][p >> 5], 1u << (p & 31));
-          }
-        }
-      }
       if (__any_sync(0xffffffffu, doubt)) {
         __syncwarp();
-        const Cand c = split_repair_cold(&a, row, lane, cnt, s, s_dmask[warp]);
+        const Cand c = repair_cold(&a, row, lane, cnt, s, s_dmask[warp]);
         my_v = c.v;
         my_i = c.i;
         __syncwarp();
@@ -882,27 +891,10 @@ topk_split_merge_kernel(const __grid_constant__ SplitMergeArgs a) {
         a.topk_val[o] = my_i >= 0 ? my_v * a.scale : -INFINITY;
         a.topk_idx[o] = gid;
       }
-      if (a.counts && ((tbits >> s) & 1u)) {   // the row's label is a class of split s
-        const unsigned m = __ballot_sync(0xffffffffu, lane < K && gid >= 0 && gid == target);
-        if (lane == 0) {
-          atomicAdd(&s_cnt[s][HGR_NUM_HITS], 1u);
-          if (m != 0) {
-            const int pos = __ffs(m) - 1;
-#pragma unroll
-            for (int c = 0; c < HGR_NUM_HITS; ++c)
-              if (pos < hit_cut(c)) atomicAdd(&s_cnt[s][c], 1u);
-          }
-        }
-      }
+      if (a.counts && ((tbits >> s) & 1u)) count_split_row(s_cnt[s], lane, K, gid, target);
     }
   }
-  __syncthreads();
-  if (a.counts) {
-    for (int i = threadIdx.x; i < a.S * (HGR_NUM_HITS + 1); i += blockDim.x) {
-      const unsigned int v = (&s_cnt[0][0])[i];
-      if (v) atomicAdd(reinterpret_cast<unsigned long long*>(a.counts) + i, static_cast<unsigned long long>(v));
-    }
-  }
+  flush_split_counts(s_cnt, a.S, a.counts, threadIdx.x);
 }
 
 // ---- per-split certified merge of the class-sharded head (hgr_topk_merge_splits_certified) -------------------------
@@ -910,89 +902,7 @@ topk_split_merge_kernel(const __grid_constant__ SplitMergeArgs a) {
 // in the order (value desc, shard asc, position in the list asc): each list is the shard's top-K of s in (value desc,
 // local bank row asc) order, so the result is the top-K of s's rows concatenated in rank-major order -- what score_topk
 // returns on that bank.  The merged K-th value must strictly beat every shard's bound of s; a doubtful (row, split,
-// shard) is re-scanned exactly from the shard table.
-
-// Exact local top-K of split s on one shard: its rows whose node has bit s in node_splits, in ascending row order (as
-// scan_row_range_lanes; membership is tested before the dot product).  Every lane holds the same list.
-__device__ __forceinline__ void scan_shard_split(const uint4* __restrict__ xr, const hgr_shard_t& sh, const uint8_t* node_splits,
-                                                 int64_t n_nodes, int s, int D8, int lane, SortedList<HGR_TOPK_MAX>& list) {
-  const uint4* bank4 = reinterpret_cast<const uint4*>(sh.bank);
-  for (int64_t cb = 0; cb < sh.C; cb += 32) {
-    const int64_t c = cb + lane;
-    bool ok = c < sh.C;
-    if (ok) {
-      const int64_t node = sh.col_id ? sh.col_id[c] : sh.id_base + c;
-      ok = node >= 0 && node < n_nodes && ((node_splits[node] >> s) & 1u);
-    }
-    float v = -INFINITY;
-    if (ok) {
-      const uint4* b = bank4 + c * D8;
-      float a0 = 0.f, a1 = 0.f;
-      int idx = 0;
-      for (; idx + 1 < D8; idx += 2) {
-        a0 = dot8_bf16(__ldg(b + idx), __ldg(xr + idx), a0);
-        a1 = dot8_bf16(__ldg(b + idx + 1), __ldg(xr + idx + 1), a1);
-      }
-      if (idx < D8) a0 = dot8_bf16(__ldg(b + idx), __ldg(xr + idx), a0);
-      v = a0 + a1;
-    }
-    const unsigned members = __ballot_sync(0xffffffffu, ok);
-    float vmax = v;
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) vmax = fmaxf(vmax, __shfl_xor_sync(0xffffffffu, vmax, o));
-    if (members != 0u && vmax > list.thr()) {
-      for (int l = 0; l < 32; ++l) {
-        const float vl = __shfl_sync(0xffffffffu, v, l);
-        if (((members >> l) & 1u) && vl > list.thr()) list.insert(vl, static_cast<int32_t>(cb + l));
-      }
-    }
-  }
-}
-
-// Exact repair of split s of a row (cold): the doubtful shards (bits of `dm`) are re-scanned, their exact top-K of s
-// mapped to node ids and scaled like the producer did; the lists of the other shards are final as they are (what such
-// a shard dropped is below the old K-th value, which can only rise).  Shards are visited in ascending order and
-// SortedList keeps the first of equal values, so the tie order stays (value desc, shard asc, local row asc).
-// Returns rank `lane` of the repaired row.
-__device__ __noinline__ Cand split_cert_repair_cold(const SplitCertArgs* a, int64_t row, int lane, int s, unsigned dm) {
-  if (lane == 0 && a->repair_count) atomicAdd(a->repair_count, 1u);
-  SortedList<HGR_TOPK_MAX> full;
-  full.init();
-  const int K = a->K;
-  const uint4* xr = reinterpret_cast<const uint4*>(a->xrows) + row * a->xD8;
-  for (int p = 0; p < static_cast<int>(a->P); ++p) {
-    if ((dm >> p) & 1u) {
-      const hgr_shard_t sh = a->shards[p];
-      SortedList<HGR_TOPK_MAX> sub;
-      sub.init();
-      scan_shard_split(xr, sh, a->node_splits, a->n_nodes, s, a->xD8, lane, sub);
-      for (int k = 0; k < K; ++k) {
-        const int32_t it = sub.i[k];
-        const float v = sub.v[k] * a->scale;
-        if (it >= 0 && v > full.thr()) full.insert(v, sh.col_id ? sh.col_id[it] : sh.id_base + it);
-      }
-    } else {
-      const int64_t base = s * a->split_stride + p * a->part_stride + row * K;
-      for (int k = 0; k < K; ++k) {
-        const int32_t it = a->part_idx[base + k];
-        const float v = a->part_val[base + k];
-        if (it >= 0 && v > full.thr()) full.insert(v, it);
-      }
-    }
-  }
-  Cand c;
-  c.v = -INFINITY;
-  c.i = -1;
-#pragma unroll
-  for (int k = 0; k < HGR_TOPK_MAX; ++k) {
-    if (lane == k) {
-      c.v = full.v[k];
-      c.i = full.i[k];
-    }
-  }
-  return c;
-}
-
+// shard) is re-scanned exactly from the shard table (repair_shards).
 // One warp per row; lane p holds the head of shard p's list.  Per output rank: the largest head value, the lowest lane
 // among equals, and that lane advances.
 __global__ void __launch_bounds__(kMergeWarps * 32)   // (a cap on the registers makes the merge spill around the call)
@@ -1042,7 +952,7 @@ topk_split_cert_kernel(const __grid_constant__ SplitCertArgs a) {
       const float bnd = lane < P ? a.part_bound[s * a.split_stride + lane * a.bound_stride + row] : -INFINITY;
       const unsigned dm = __ballot_sync(0xffffffffu, bnd > -INFINITY && bnd >= kth);
       if (dm != 0u) {
-        const Cand c = split_cert_repair_cold(&a, row, lane, s, dm);
+        const Cand c = repair_cold(&a, row, lane, s, dm);
         my_v = c.v;
         my_i = c.i;
       }
@@ -1051,27 +961,10 @@ topk_split_cert_kernel(const __grid_constant__ SplitCertArgs a) {
         a.topk_val[o] = my_i >= 0 ? my_v : -INFINITY;
         a.topk_idx[o] = my_i;
       }
-      if (a.counts && ((tbits >> s) & 1u)) {   // the row's label is a class of split s
-        const unsigned m = __ballot_sync(0xffffffffu, lane < K && my_i >= 0 && my_i == target);
-        if (lane == 0) {
-          atomicAdd(&s_cnt[s][HGR_NUM_HITS], 1u);
-          if (m != 0) {
-            const int pos = __ffs(m) - 1;
-#pragma unroll
-            for (int c = 0; c < HGR_NUM_HITS; ++c)
-              if (pos < hit_cut(c)) atomicAdd(&s_cnt[s][c], 1u);
-          }
-        }
-      }
+      if (a.counts && ((tbits >> s) & 1u)) count_split_row(s_cnt[s], lane, K, my_i, target);
     }
   }
-  __syncthreads();
-  if (a.counts) {
-    for (int i = threadIdx.x; i < a.S * (HGR_NUM_HITS + 1); i += blockDim.x) {
-      const unsigned int v = (&s_cnt[0][0])[i];
-      if (v) atomicAdd(reinterpret_cast<unsigned long long*>(a.counts) + i, static_cast<unsigned long long>(v));
-    }
-  }
+  flush_split_counts(s_cnt, a.S, a.counts, threadIdx.x);
 }
 
 // ---- cross-GPU sequencing of the peer-memory exchange ---------------------------------------------------------
