@@ -36,6 +36,7 @@ SIGNATURES = {
     "hgr_normalize_rows_dual": (c_int, [c_void_p, c_int, c_int64, c_int64, c_void_p, c_void_p, c_void_p, c_void_p]),
     "hgr_score_topk_workspace_bytes": (c_size_t, [c_int64, c_int64, c_int64, c_int]),
     "hgr_score_topk_plan": (c_int, [c_int64, c_int64, c_int64, c_int, c_void_p]),
+    "hgr_score_topk_footprint": (c_int, [c_int64, c_int64, c_int64, c_int, c_int, c_void_p]),
     "hgr_score_topk": (c_int, [c_void_p, c_void_p, c_void_p, c_int32, c_void_p, c_int64, c_int64, c_int64,
                                c_float, c_int, c_void_p, c_size_t, c_void_p, c_void_p, c_void_p, c_int,
                                c_void_p]),

@@ -11,7 +11,7 @@
 // is streamed once per gather), fp32 accumulators in registers, warp-shuffle reduction of the
 // squared norm, one 128-bit store per lane and vector.  Compulsory traffic per row:
 // nnz_row * D * sizeof(in) + D * sizeof(out) (+ CSR).
-#include "common.cuh"
+#include "placement.cuh"
 
 namespace hgr {
 namespace {
@@ -173,71 +173,56 @@ aggregate_normalize_kernel(const TIn* __restrict__ E, int D8, const int32_t* __r
 }
 
 // Identity CSR (row r = {src}, weight 1): the plain row normalise of update_classifier / forward.  No
-// accumulators besides the row itself, TWO rows per warp in flight, 2+ CTAs per SM: enough bytes in flight to
-// approach the HBM roofline on the 21,841-row bank.
+// accumulators besides the row itself, one row per warp, 3 CTAs per SM: 24 rows in flight per SM on the 21,841-row
+// bank, and at most 72 registers, so that a CTA of it fits on an SM beside a resident scoring CTA and a merge CTA
+// (DESIGN.md section 4).  (Two rows per warp in flight took 101-108 registers, and 85 with spills.)
 template <typename TIn, typename TOut, int MAXV>
-__global__ void __launch_bounds__(256, 2)
+__global__ void __launch_bounds__(256, 3)
 normalize_rows_kernel(const TIn* __restrict__ E, int D8, const int32_t* __restrict__ row_map, int64_t n_out,
                       TOut* __restrict__ out, float* __restrict__ out_norm, TOut* __restrict__ out2 = nullptr,
                       const int32_t* __restrict__ dst_map = nullptr) {
+  HGR_PLACE_ENTER();
   const int lane = threadIdx.x & 31;
   const int64_t warp0 = (static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
   const int64_t nwarps = (static_cast<int64_t>(gridDim.x) * blockDim.x) >> 5;
   const int64_t D = static_cast<int64_t>(D8) * 8;
-  for (int64_t row = warp0; row < n_out; row += 2 * nwarps) {
-    const int64_t row2 = row + nwarps;
-    const bool has2 = row2 < n_out;
-    const int64_t s1 = row_map ? row_map[row] : row;
-    const int64_t s2 = has2 ? (row_map ? row_map[row2] : row2) : s1;
-    float a[MAXV][8], b[MAXV][8];
+  for (int64_t row = warp0; row < n_out; row += nwarps) {
+    const int64_t src = row_map ? row_map[row] : row;
+    float a[MAXV][8];
 #pragma unroll
     for (int v = 0; v < MAXV; ++v) {
       const int idx = lane + 32 * v;
       if (idx < D8) {
-        Vec8<TIn>::load(E + s1 * D + idx * 8, a[v]);
-        Vec8<TIn>::load(E + s2 * D + idx * 8, b[v]);
+        Vec8<TIn>::load(E + src * D + idx * 8, a[v]);
       } else {
 #pragma unroll
-        for (int e = 0; e < 8; ++e) a[v][e] = b[v][e] = 0.f;
+        for (int e = 0; e < 8; ++e) a[v][e] = 0.f;
       }
     }
-    float ssa = 0.f, ssb = 0.f;
+    float ss = 0.f;
 #pragma unroll
     for (int v = 0; v < MAXV; ++v)
 #pragma unroll
-      for (int e = 0; e < 8; ++e) {
-        ssa = fmaf(a[v][e], a[v][e], ssa);
-        ssb = fmaf(b[v][e], b[v][e], ssb);
-      }
-    ssa = warp_sum(ssa);
-    ssb = warp_sum(ssb);
-    const float na = sqrtf(ssa), nb = sqrtf(ssb);
-    if (out_norm && lane == 0) {
-      out_norm[row] = na;
-      if (has2) out_norm[row2] = nb;
-    }
+      for (int e = 0; e < 8; ++e) ss = fmaf(a[v][e], a[v][e], ss);
+    ss = warp_sum(ss);
+    const float n = sqrtf(ss);
+    if (out_norm && lane == 0) out_norm[row] = n;
     // second destination (dual form): row r also lands at row dst_map[r] of out2 -- the test-class bank in its own
     // row order, written by the same pass that writes the all-node bank
-    const int64_t d1 = dst_map ? dst_map[row] : -1;
-    const int64_t d2 = (dst_map && has2) ? dst_map[row2] : -1;
+    const int64_t d = dst_map ? dst_map[row] : -1;
 #pragma unroll
     for (int v = 0; v < MAXV; ++v) {
       const int idx = lane + 32 * v;
       if (idx < D8) {
         float o[8];
 #pragma unroll
-        for (int e = 0; e < 8; ++e) o[e] = __fdiv_rn(a[v][e], na);
+        for (int e = 0; e < 8; ++e) o[e] = __fdiv_rn(a[v][e], n);
         Vec8<TOut>::store(out + row * D + idx * 8, o);
-        if (d1 >= 0) Vec8<TOut>::store(out2 + d1 * D + idx * 8, o);
-        if (has2) {
-#pragma unroll
-          for (int e = 0; e < 8; ++e) o[e] = __fdiv_rn(b[v][e], nb);
-          Vec8<TOut>::store(out + row2 * D + idx * 8, o);
-          if (d2 >= 0) Vec8<TOut>::store(out2 + d2 * D + idx * 8, o);
-        }
+        if (d >= 0) Vec8<TOut>::store(out2 + d * D + idx * 8, o);
       }
     }
   }
+  HGR_PLACE_LEAVE(kNormalize);
 }
 
 // Row normalise with BROADCAST stores: row r of the local block lands at row (row0 + r) of every destination
@@ -349,8 +334,8 @@ int dispatch(const void* E, int64_t D, const int32_t* rowptr, const int32_t* col
   const TIn* e = static_cast<const TIn*>(E);
   TOut* o = static_cast<TOut*>(out);
   if (rowptr == nullptr && D8 <= 128) {  // identity CSR: the specialised row normalise
-    const int64_t capn = static_cast<int64_t>(num_sms()) * 4;
-    const int64_t wantn = (n_out + 2 * rows_per_block - 1) / (2 * rows_per_block);
+    const int64_t capn = static_cast<int64_t>(num_sms()) * 3;   // one wave (launch bounds)
+    const int64_t wantn = (n_out + rows_per_block - 1) / rows_per_block;
     const int nb = static_cast<int>(wantn < capn ? (wantn < 1 ? 1 : wantn) : capn);
     if (D8 <= 32) normalize_rows_kernel<TIn, TOut, 1><<<nb, threads, 0, stream>>>(e, D8, row_map, n_out, o, out_norm);
     else if (D8 <= 64) normalize_rows_kernel<TIn, TOut, 2><<<nb, threads, 0, stream>>>(e, D8, row_map, n_out, o, out_norm);
@@ -418,8 +403,8 @@ static int dual_dispatch(const void* E, int64_t n_rows, int64_t D, __nv_bfloat16
   const int D8 = static_cast<int>(D / 8);
   const int threads = 256;
   const int64_t rows_per_block = threads / 32;
-  const int64_t capn = static_cast<int64_t>(num_sms()) * 4;
-  const int64_t wantn = (n_rows + 2 * rows_per_block - 1) / (2 * rows_per_block);
+  const int64_t capn = static_cast<int64_t>(num_sms()) * 3;   // one wave (launch bounds)
+  const int64_t wantn = (n_rows + rows_per_block - 1) / rows_per_block;
   const int nb = static_cast<int>(wantn < capn ? (wantn < 1 ? 1 : wantn) : capn);
   const TIn* e = static_cast<const TIn*>(E);
   if (D8 <= 32) normalize_rows_kernel<TIn, __nv_bfloat16, 1><<<nb, threads, 0, stream>>>(e, D8, nullptr, n_rows, out, nullptr, out2, dst_map);
@@ -429,6 +414,33 @@ static int dual_dispatch(const void* E, int64_t n_rows, int64_t D, __nv_bfloat16
   HGR_CHECK_LAUNCH();
   return HGR_OK;
 }
+
+template <typename TIn>
+static int normalize_footprint_of(int64_t D, int32_t* out) {
+  const int D8 = static_cast<int>(D / 8);
+  cudaFuncAttributes fa;
+  if (D8 <= 32) HGR_CHECK_CUDA(cudaFuncGetAttributes(&fa, normalize_rows_kernel<TIn, __nv_bfloat16, 1>));
+  else if (D8 <= 64) HGR_CHECK_CUDA(cudaFuncGetAttributes(&fa, normalize_rows_kernel<TIn, __nv_bfloat16, 2>));
+  else if (D8 <= 96) HGR_CHECK_CUDA(cudaFuncGetAttributes(&fa, normalize_rows_kernel<TIn, __nv_bfloat16, 3>));
+  else HGR_CHECK_CUDA(cudaFuncGetAttributes(&fa, normalize_rows_kernel<TIn, __nv_bfloat16, 4>));
+  out[0] = 256;
+  out[1] = fa.numRegs;
+  out[2] = static_cast<int32_t>(fa.sharedSizeBytes);
+  out[3] = 0;
+  return HGR_OK;
+}
+
+int normalize_rows_footprint(int e_dtype, int64_t D, int32_t* out) {
+  if (D < 8 || D % 8 != 0 || D > 1024) return set_error(HGR_ERR_UNSUPPORTED, "normalise footprint: D = %lld", (long long)D);
+  if (e_dtype == HGR_F32) return normalize_footprint_of<float>(D, out);
+  if (e_dtype == HGR_F16) return normalize_footprint_of<__half>(D, out);
+  if (e_dtype == HGR_BF16) return normalize_footprint_of<__nv_bfloat16>(D, out);
+  return set_error(HGR_ERR_UNSUPPORTED, "normalise footprint: dtype %d not supported", e_dtype);
+}
+
+#ifdef HGR_PLACEMENT
+int placement_attach_normalize(const place::Log& l) { return place::attach(l); }
+#endif
 
 int launch_normalize_dual(const void* E, int e_dtype, int64_t n_rows, int64_t D, void* out, const int32_t* dst_map,
                           void* out2, cudaStream_t stream) {

@@ -116,6 +116,9 @@ struct MergeArgs {
   unsigned int* repair_count = nullptr;
 };
 int launch_topk_merge(const MergeArgs& args, cudaStream_t stream);
+// {threads, registers per thread, static shared memory, dynamic shared memory} of the merge launch_topk_merge runs on
+// the scoring kernel's own P lists of KL entries per row (register merges only)
+int merge_kernel_footprint(int64_t P, int KL, int32_t* out);
 
 // Arguments of the per-split merge (hgr_score_topk_splits, topk_merge.cu): the scoring kernel's lists on the grouped
 // schedule, group_parts(mt) lists of length KL per row, list slot p of row tile mt covering the bank rows
@@ -185,6 +188,7 @@ int launch_logits_simt(const __nv_bfloat16* X, const __nv_bfloat16* bank, int64_
 size_t umma_score_workspace_bytes(int64_t B, int64_t C, int K);
 bool umma_supported(int64_t B, int64_t C, int64_t D, int K);
 void umma_plan(int64_t B, int64_t C, int64_t D, int K, int32_t* plan);
+int umma_footprint(int64_t B, int64_t C, int64_t D, int K, int32_t* out);
 // C_total > 0 (with scatter->emit_bound): the lists are sized for a row's GLOBAL stream of C_total classes, of which
 // this bank is one shard -- no local certificate / repair, the owner of the row certifies against the global K-th value
 int launch_score_topk_umma(const __nv_bfloat16* X, const __nv_bfloat16* bank, const int32_t* col_id,
@@ -238,6 +242,9 @@ int launch_hier_mistakes(const int32_t* topk_idx, int64_t B, int K, int64_t set_
                          const int32_t* chain_node, int64_t n_nodes, int64_t* counts, cudaStream_t stream);
 int launch_normalize_dual(const void* E, int e_dtype, int64_t n_rows, int64_t D, void* out, const int32_t* dst_map,
                           void* out2, cudaStream_t stream);
+// {threads, registers per thread, static shared memory, dynamic shared memory} of the row normalise of [*, D] rows
+// of type e_dtype into bf16 (hgr_aggregate_normalize with identity CSR)
+int normalize_rows_footprint(int e_dtype, int64_t D, int32_t* out);
 int launch_normalize_bcast(const void* E, int e_dtype, int64_t n_rows, int64_t D, int64_t row0, int n_dst,
                            void* const* dst, cudaStream_t stream);
 

@@ -295,6 +295,14 @@ int hgr_score_topk_plan(int64_t B, int64_t C, int64_t D, int K, int32_t* plan) {
   return HGR_OK;
 }
 
+int hgr_score_topk_footprint(int64_t B, int64_t C, int64_t D, int K, int x_dtype, int32_t* out) {
+  HGR_CHECK_ARG(out != nullptr, "hgr_score_topk_footprint: null out");
+  HGR_CHECK_ARG(K >= 1 && K <= HGR_TOPK_MAX, "hgr_score_topk_footprint: K = %d outside [1, %d]", K, HGR_TOPK_MAX);
+  if (!umma_supported(B, C, D, K)) return set_error(HGR_ERR_UNSUPPORTED, "hgr_score_topk_footprint: shape not supported by the tcgen05 kernel");
+  const int rc = normalize_rows_footprint(x_dtype, D, out);
+  return rc != HGR_OK ? rc : umma_footprint(B, C, D, K, out + 4);
+}
+
 int hgr_score_topk(const void* X, const void* bank, const int32_t* col_id, int32_t id_base, const int32_t* targets,
                    int64_t B, int64_t C, int64_t D, float scale, int K, void* workspace, size_t workspace_bytes,
                    float* topk_val, int32_t* topk_idx, int64_t* hits, int impl, void* stream) {

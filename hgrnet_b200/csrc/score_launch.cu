@@ -214,6 +214,15 @@ void umma_plan(int64_t B, int64_t C, int64_t D, int K, int32_t* plan) {
   plan[7] = static_cast<int32_t>((s.T + s.G - 1) / s.G * kUnit);
 }
 
+// The production scoring kernel and the merge behind it as launch_score_topk_umma runs them: {threads, registers per
+// thread, static shared memory, dynamic shared memory} of each.
+int umma_footprint(int64_t B, int64_t C, int64_t D, int K, int32_t* out) {
+  int32_t plan[8];
+  umma_plan(B, C, D, K, plan);
+  const int rc = pair_kernel_footprint(B, plan[4], out);
+  return rc != HGR_OK ? rc : merge_kernel_footprint(plan[3], plan[4], out + 4);
+}
+
 int launch_score_topk_umma(const __nv_bfloat16* X, const __nv_bfloat16* bank, const int32_t* col_id,
                            int32_t id_base, const int32_t* targets, int64_t B, int64_t C, int64_t D, float scale,
                            int K, void* ws, size_t ws_bytes, float* topk_val, int32_t* topk_idx, int64_t* hits,

@@ -18,6 +18,7 @@
 // .cta_group::2); the leader's single MMA thread commits with a cluster multicast to the `empty`
 // and `tmem_full` barriers of both CTAs; the epilogue warps of both CTAs arrive on the leader's
 // `tmem_empty`.  Epilogues: umma_common.cuh (deferred-insert lists), sketch_epi.cuh (floor sketch); work split: sched.cuh.
+#include "placement.cuh"
 #include "sketch_epi.cuh"
 #include "umma_common.cuh"
 
@@ -40,18 +41,20 @@ struct PairCtl {
 
 // What an epilogue needs of a CTA, read by the kernel (launch bounds, shared-memory carve-up, barrier counts) and by
 // its launcher (threads, dynamic shared memory, opt-in limit).
-template <int EPI>
+template <int EPI, int KL = 8>
 struct EpiRes {
   static constexpr bool kTopk = EPI == kEpiTopkDefer || EPI == kEpiTopkGroups;
+  static constexpr int kQueueLen = defer_queue_len<KL>();     // top-K epilogues: candidate queue entries per thread
   static constexpr bool kQueue = kTopk || EPI == kEpiSketch;   // a candidate queue per thread
   // one warp per TMEM lane quarter; the dense epilogue has two, which take alternate chunks of every sub-tile
   static constexpr int kWarps = EPI == kEpiDense ? 8 : 4;
   static constexpr int kThreads = 64 + 32 * kWarps;           // + the TMA and the MMA warp
   static constexpr int kStagingBytes = EPI == kEpiSketch ? kSkQueueBytes
-                                     : kTopk ? (kDeferQueue + 1) * kDeferStride
+                                     : kTopk ? (kQueueLen + 1) * kDeferStride
                                      : EPI == kEpiDense ? kWarps * kDenseTileFloats * 4 : 0;
   // Operand stages: as many 32 KB stages as fit beside the staging memory (measured: 4 stages cost ~2 us of main loop
-  // at cfg 2, and leaving room for co-resident small kernels bought nothing).
+  // at cfg 2, and leaving room for co-resident small kernels that way bought nothing).  With narrow lists the shorter
+  // queue (defer_queue_len) leaves room for a normalise and two merge CTAs beside a 5-stage CTA instead.
   static constexpr int kMaxStages = kQueue ? 5 : 6;
   static constexpr int kTmemEmptyArrivals = 2 * kWarps;       // every epilogue warp of both CTAs
   static constexpr size_t smem_bytes(int stages) {
@@ -292,8 +295,11 @@ __device__ __forceinline__ void epi_topk_defer(const Params& p, const EpiWarp& w
   SortedList<KL> list;
   list.init();
   float floor_thr = -INFINITY;   // warm-up floor of the segment
-  CandQueue cq;
+  CandQueue<defer_queue_len<KL>()> cq;
   cq.init(ptx::smem_u32(reinterpret_cast<uint2*>(staging) + epi_tid));
+#ifdef HGR_PLACEMENT
+  unsigned long long n_chunks = 0, n_crowded = 0;
+#endif
   int it = 0;
   EpiClock ck(p.timeline != nullptr && epi_tid == 0);
   while (walk.next(t)) {
@@ -315,7 +321,11 @@ __device__ __forceinline__ void epi_topk_defer(const Params& p, const EpiWarp& w
       ptx::tmem_ld_wait();
       ck.lap(ck.ld);
       const int nv = t.nvalid - c0;
-      const bool roomy = __reduce_max_sync(0xffffffffu, cq.count()) <= kDeferQueue - kChunk;
+      const bool roomy = __reduce_max_sync(0xffffffffu, cq.count()) <= cq.kEntries - kChunk;
+#ifdef HGR_PLACEMENT
+      ++n_chunks;
+      n_crowded += roomy ? 0 : 1;
+#endif
       // Long lists (many survivors per sub-tile) make room up front; short lists rarely pass half of the queue, and
       // when a lane does they take the saturating append below, so that only a queue that really fills up makes the
       // warp drain while it still holds the TMEM buffer (measured: KL = 8 -0.2 us, KL = 16 +7 us with the lazy rule).
@@ -373,6 +383,9 @@ __device__ __forceinline__ void epi_topk_defer(const Params& p, const EpiWarp& w
     ++it;
   }
   epi_done(p, ck, epi_tid);
+#ifdef HGR_PLACEMENT
+  if (w.lane == 0) place::count_chunks(n_chunks, n_crowded);
+#endif
 }
 
 // ===================== epilogue: floor sketch + candidate queue (sketch_epi.cuh) =====================
@@ -593,7 +606,8 @@ template <int EPI, int KL>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(EpiRes<EPI>::kThreads, 1)
 score_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constant__ CUtensorMap map_bank,
                        const Params p) {
-  using R = EpiRes<EPI>;
+  HGR_PLACE_ENTER();
+  using R = EpiRes<EPI, KL>;
   const int stages = p.stages;   // <= R::kMaxStages, chosen by the launcher (EpiRes::stages)
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -662,11 +676,12 @@ score_umma_pair_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_c
       atomicAdd(&p.stats[1], 1u);
     }
   }
+  HGR_PLACE_LEAVE(kScore);
 }
 
 template <int EPI, int KL>
 int launch_one(const CUtensorMap& mx, const CUtensorMap& mb, const Params& p, cudaStream_t stream) {
-  using R = EpiRes<EPI>;
+  using R = EpiRes<EPI, KL>;
   Params pp = p;
   pp.stages = R::stages(p.B);
   auto kern = score_umma_pair_kernel<EPI, KL>;
@@ -681,7 +696,42 @@ int launch_one(const CUtensorMap& mx, const CUtensorMap& mb, const Params& p, cu
 
 }  // namespace
 
+#ifdef HGR_PLACEMENT
+// Diagnostics builds only: log into `rec` (cap records, `n` counts them) and `chunks` from now on; null pointers stop.
+extern "C" int hgr_placement_attach(void* rec, void* n, unsigned int cap, void* chunks) {
+  const place::Log l{static_cast<place::Rec*>(rec), static_cast<unsigned int*>(n), cap,
+                     static_cast<unsigned long long*>(chunks)};
+  int rc = place::attach(l);
+  if (rc == HGR_OK) rc = placement_attach_normalize(l);
+  return rc == HGR_OK ? placement_attach_merge(l) : rc;
+}
+#endif
+
 int pair_ring_depth(int64_t B) { return EpiRes<kEpiTopkDefer>::stages(B); }
+
+template <int KL>
+int footprint_one(int64_t B, int32_t* out) {
+  using R = EpiRes<kEpiTopkDefer, KL>;
+  cudaFuncAttributes fa;
+  HGR_CHECK_CUDA(cudaFuncGetAttributes(&fa, score_umma_pair_kernel<kEpiTopkDefer, KL>));
+  out[0] = R::kThreads;
+  out[1] = fa.numRegs;
+  out[2] = static_cast<int32_t>(fa.sharedSizeBytes);
+  out[3] = static_cast<int32_t>(R::smem_bytes(R::stages(B)));   // what launch_one asks for
+  return HGR_OK;
+}
+
+int pair_kernel_footprint(int64_t B, int KL, int32_t* out) {
+  switch (KL) {
+    case 8: return footprint_one<8>(B, out);
+    case 10: return footprint_one<10>(B, out);
+    case 12: return footprint_one<12>(B, out);
+    case 16: return footprint_one<16>(B, out);
+    case 20: return footprint_one<20>(B, out);
+    case 32: return footprint_one<32>(B, out);
+  }
+  return set_error(HGR_ERR_UNSUPPORTED, "hgr_score_topk_footprint: list length %d", KL);
+}
 
 template <int EPI>
 int launch_topk(int KL, const CUtensorMap& mx, const CUtensorMap& mb, const Params& p, cudaStream_t stream) {

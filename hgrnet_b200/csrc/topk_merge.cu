@@ -17,6 +17,7 @@
 // cannot belong to (or tie with) the top-K.  An uncertified row is re-scanned exactly by its warp on the
 // CUDA cores (repair_lists, simt_row.cuh).  With randomly ordered bank rows this is a ~1e-8-per-row event.
 #include "common.cuh"
+#include "placement.cuh"
 #include "simt_row.cuh"
 
 namespace hgr {
@@ -454,6 +455,7 @@ topk_merge_kernel(const __grid_constant__ MergeArgs a) {
 template <int NPL>
 __global__ void __launch_bounds__(kMergeWarps * 32, 7)  // (the cold repair functions must not set the register count)
 topk_select_kernel(const __grid_constant__ MergeArgs a) {
+  HGR_PLACE_ENTER();
   __shared__ int s_hits[HGR_NUM_HITS];
   __shared__ unsigned long long s_win[kMergeWarps][32];
   __shared__ uint32_t s_dmask[kMergeWarps][kDoubtWords];
@@ -564,6 +566,7 @@ topk_select_kernel(const __grid_constant__ MergeArgs a) {
     finish_row(a, row, lane, my_v, my_i, doubt, s_dmask[warp], cnt, s_hits, tailmax);
   }
   flush_hits(a, s_hits, threadIdx.x);
+  HGR_PLACE_LEAVE(kMerge);
 }
 
 // ---- ranking merge (very few candidates per row) ------------------------------------------------------------------
@@ -1036,6 +1039,35 @@ int launch_peer_wait(const uint32_t* flags, int n, uint32_t* seq, cudaStream_t s
   return HGR_OK;
 }
 
+// The merge that holds a row's `cand` candidates (an upper bound) in registers, or nullptr when they do not fit and
+// the lists are merged from shared memory.
+using RegMerge = void (*)(MergeArgs);
+static RegMerge register_merge(int64_t cand, bool use_sched) {
+  // (only for the scoring kernel's own lists: bank rows, sorted (value desc, row asc) by construction -- lists handed
+  //  to hgr_topk_merge carry node ids, whose order among equal values is the caller's)
+#ifndef HGR_NO_RANK_KERNEL   // (kernel experiments: tools/build_variant.sh norank -DHGR_NO_RANK_KERNEL topk_merge.cu)
+  if (cand <= 96 && use_sched) return cand <= 64 ? topk_rank_kernel<2> : topk_rank_kernel<3>;
+#endif
+  if (cand <= 320) return cand <= 128 ? topk_select_kernel<4> : (cand <= 192 ? topk_select_kernel<6> : topk_select_kernel<10>);
+  return nullptr;
+}
+
+#ifdef HGR_PLACEMENT
+int placement_attach_merge(const place::Log& l) { return place::attach(l); }
+#endif
+
+int merge_kernel_footprint(int64_t P, int KL, int32_t* out) {
+  const RegMerge kern = register_merge(P * KL, true);
+  if (kern == nullptr) return set_error(HGR_ERR_UNSUPPORTED, "merge footprint: %lld x %d candidates per row", (long long)P, KL);
+  cudaFuncAttributes fa;
+  HGR_CHECK_CUDA(cudaFuncGetAttributes(&fa, kern));
+  out[0] = kMergeWarps * 32;
+  out[1] = fa.numRegs;
+  out[2] = static_cast<int32_t>(fa.sharedSizeBytes);
+  out[3] = 0;
+  return HGR_OK;
+}
+
 int launch_topk_merge(const MergeArgs& args, cudaStream_t stream) {
   if (args.B == 0 || args.K == 0) return HGR_OK;
   if (args.sk_part != nullptr) {
@@ -1056,21 +1088,8 @@ int launch_topk_merge(const MergeArgs& args, cudaStream_t stream) {
   if (args.KL < args.K && (args.X == nullptr || args.bank == nullptr || !args.use_sched))
     return set_error(HGR_ERR_BAD_ARG, "topk merge: speculative lists need X / bank / the schedule for the exact repair");
   const int blocks = static_cast<int>((args.B + kMergeWarps - 1) / kMergeWarps);
-  const int64_t cand = args.P * args.KL;  // candidates per row (upper bound)
-  // (only for the scoring kernel's own lists: bank rows, sorted (value desc, row asc) by construction -- lists handed
-  //  to hgr_topk_merge carry node ids, whose order among equal values is the caller's)
-#ifndef HGR_NO_RANK_KERNEL   // (kernel experiments: tools/build_variant.sh norank -DHGR_NO_RANK_KERNEL topk_merge.cu)
-  if (cand <= 96 && args.use_sched) {
-    if (cand <= 64) topk_rank_kernel<2><<<blocks, kMergeWarps * 32, 0, stream>>>(args);
-    else topk_rank_kernel<3><<<blocks, kMergeWarps * 32, 0, stream>>>(args);
-    HGR_CHECK_LAUNCH();
-    return HGR_OK;
-  }
-#endif
-  if (cand <= 320) {
-    if (cand <= 128) topk_select_kernel<4><<<blocks, kMergeWarps * 32, 0, stream>>>(args);
-    else if (cand <= 192) topk_select_kernel<6><<<blocks, kMergeWarps * 32, 0, stream>>>(args);
-    else topk_select_kernel<10><<<blocks, kMergeWarps * 32, 0, stream>>>(args);
+  if (const RegMerge kern = register_merge(args.P * args.KL, args.use_sched)) {
+    kern<<<blocks, kMergeWarps * 32, 0, stream>>>(args);
     HGR_CHECK_LAUNCH();
     return HGR_OK;
   }

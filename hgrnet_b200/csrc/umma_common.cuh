@@ -144,22 +144,31 @@ __device__ __forceinline__ float warmup_floor_pairs(uint32_t taddr, int nvalid) 
 // to a per-thread queue, the TMEM buffer is handed back to the MMA warp at once, and only then is the queue
 // drained into the list -- in lock-step over one dense batch per sub-tile, while the tensor core already works
 // two sub-tiles ahead.  The epilogue leaves the critical path of the MMAs entirely.
-constexpr int kDeferQueue = 64;                   // queue entries per thread (+1 dud slot)
+// Queue entries per thread (+1 dud slot) for lists of KL entries.  Narrow lists (KL <= 10) keep 56: the 8 KB this
+// frees beside 5 operand stages let a normalise and two merge CTAs share the SM with a resident scoring CTA
+// (DESIGN.md section 4, budget rule).  Measured at cfg 2 (tools/placement.py): 2.3 % of the chunks then find some
+// lane's queue too full for the roomy append (0.13 % with 64 entries) and take the saturating one; the scoring kernel
+// alone at full clock is unchanged (24.64 vs 24.69 us).  Wider lists keep 64.
+template <int KL>
+constexpr int defer_queue_len() { return KL <= 10 ? 56 : 64; }
 constexpr uint32_t kDeferStride = 128 * 8;        // one entry of each of the CTA's 128 epilogue threads
+template <int kLen>
 struct CandQueue {
+  static constexpr int kEntries = kLen;
   uint32_t base;  // shared-space byte address of entry 0 of this thread; entries are kDeferStride bytes apart
   uint32_t wr;    // next free entry
   __device__ __forceinline__ void init(uint32_t b) { base = wr = b; }
-  __device__ __forceinline__ uint32_t limit() const { return base + kDeferQueue * kDeferStride; }  // the dud slot
+  __device__ __forceinline__ uint32_t limit() const { return base + kLen * kDeferStride; }  // the dud slot
   __device__ __forceinline__ int count() const { return static_cast<int>((wr - base) / kDeferStride); }
 };
 
 // Branch-free append: every value is stored at the write cursor, the cursor only advances for survivors (the
 // next store overwrites a non-survivor) and saturates at the last slot, which therefore only ever holds duds.
 // (Inline-asm stores inside an `if` would be compiled as 32 divergent branches per chunk.)  The queue has
-// kDeferQueue + 1 entries per thread.  Returns false when some lane of the warp ran out of slots: the caller then
+// kLen + 1 entries per thread.  Returns false when some lane of the warp ran out of slots: the caller then
 // rewinds, drains and appends the same chunk again.
-__device__ __forceinline__ bool cand_append_chunk(CandQueue& q, const uint32_t (&r)[kChunk], int nv,
+template <int kLen>
+__device__ __forceinline__ bool cand_append_chunk(CandQueue<kLen>& q, const uint32_t (&r)[kChunk], int nv,
                                                   int col_chunk, float thr) {
   uint32_t wr = q.wr;
   const uint32_t lim = q.limit();
@@ -175,9 +184,9 @@ __device__ __forceinline__ bool cand_append_chunk(CandQueue& q, const uint32_t (
 }
 
 // Same without the per-value saturation (one op less on the cursor's dependency chain): the caller guarantees
-// room for a whole chunk (count <= kDeferQueue - 32 in every lane).
-template <bool FULL>
-__device__ __forceinline__ void cand_append_chunk_roomy(CandQueue& q, const uint32_t (&r)[kChunk],
+// room for a whole chunk (count <= kLen - 32 in every lane).
+template <bool FULL, int kLen>
+__device__ __forceinline__ void cand_append_chunk_roomy(CandQueue<kLen>& q, const uint32_t (&r)[kChunk],
                                                         int nv, int col_chunk, float thr) {
   uint32_t wr = q.wr;
   // store-all / advance-on-pass: every value is written at the cursor and the next store overwrites a
@@ -192,13 +201,13 @@ __device__ __forceinline__ void cand_append_chunk_roomy(CandQueue& q, const uint
   q.wr = wr;
 }
 
-template <int KL>
-__device__ __forceinline__ void cand_drain(SortedList<KL>& list, CandQueue& q) {
+template <int KL, int kLen>
+__device__ __forceinline__ void cand_drain(SortedList<KL>& list, CandQueue<kLen>& q) {
   const int cnt = q.count();
   const int maxc = __reduce_max_sync(0xffffffffu, cnt);
   uint32_t rd = q.base;
   // the next entry is fetched while the current one is inserted (one warp per scheduler: nothing else would hide
-  // the shared-memory latency); reading one entry past a lane's count stays inside its kDeferQueue + 1 slots
+  // the shared-memory latency); reading one entry past a lane's count stays inside its kLen + 1 slots
   uint32_t xb, col;
   ptx::ld_shared_v2(rd, xb, col);
   for (int e = 0; e < maxc; ++e) {
@@ -213,6 +222,9 @@ __device__ __forceinline__ void cand_drain(SortedList<KL>& list, CandQueue& q) {
 
 // score_pair.cu
 int pair_ring_depth(int64_t B);   // operand stages of the production (deferred-insert) kernel for a batch size
+// {threads, registers per thread, static shared memory, dynamic shared memory} of the production kernel as
+// launch_pair_kernel launches it for B rows and lists of KL entries
+int pair_kernel_footprint(int64_t B, int KL, int32_t* out);
 int launch_pair_kernel(int epi, int KL, const CUtensorMap& mx, const CUtensorMap& mb, const Params& p,
                        cudaStream_t stream);
 

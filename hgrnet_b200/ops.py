@@ -239,6 +239,16 @@ def score_topk_plan(B: int, C: int, D: int, K: int = 20) -> dict:
     return dict(zip(keys, list(plan)))
 
 
+def score_topk_footprint(B: int, C: int, D: int, K: int = 20, x_dtype=torch.bfloat16) -> dict:
+    """What one batch of ``normalize_rows`` + ``score_topk`` asks of an SM, per kernel (``normalize``, ``score``,
+    ``merge``): ``{threads, registers, static_smem, dynamic_smem}`` (registers per thread, bytes).  Needs a device."""
+    import ctypes
+    out = (ctypes.c_int32 * 12)()
+    _cabi.check(_cabi.load().hgr_score_topk_footprint(B, C, D, K, _DTYPE_CODE[x_dtype], out))
+    keys = ("threads", "registers", "static_smem", "dynamic_smem")
+    return {name: dict(zip(keys, list(out)[4 * i:4 * i + 4])) for i, name in enumerate(("normalize", "score", "merge"))}
+
+
 def topk_merge(part_val: torch.Tensor, part_idx: torch.Tensor, *, targets: Optional[torch.Tensor] = None,
                hits: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
     """Merge ``[P, B, K]`` partial lists (node ids) into the final ``[B, K]`` top-K + hits.

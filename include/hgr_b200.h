@@ -123,6 +123,10 @@ size_t hgr_score_topk_workspace_bytes(int64_t B, int64_t C, int64_t D, int K);
  * per row tile, partial lists per row, entries per list (< K: speculative), epilogue warps per TMEM quarter, operand
  * ring depth, bank rows streamed per worker}. */
 int hgr_score_topk_plan(int64_t B, int64_t C, int64_t D, int K, int32_t* plan /* [8] */);
+/* What one batch of hgr_score_topk asks of an SM, for checking which of its kernels can share one: {threads, registers
+ * per thread, static shared memory, dynamic shared memory} of (0) the row normalise of x_dtype [B, D] features into
+ * bf16, (1) the tcgen05 scoring kernel, (2) the merge of its partial lists.  Needs a device. */
+int hgr_score_topk_footprint(int64_t B, int64_t C, int64_t D, int K, int x_dtype, int32_t* out /* [12] */);
 int hgr_score_topk(const void* X, const void* bank, const int32_t* col_id, int32_t id_base,
                    const int32_t* targets, int64_t B, int64_t C, int64_t D, float scale, int K,
                    void* workspace, size_t workspace_bytes, float* topk_val, int32_t* topk_idx,
