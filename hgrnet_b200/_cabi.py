@@ -65,20 +65,17 @@ SIGNATURES = {
     "hgr_logits_dense": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int64, c_float, c_void_p, c_int64,
                                  c_int, c_void_p]),
     "hgr_hier_metrics_fused_rows": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int64, c_void_p, c_int, c_void_p,
-                                            c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t,
-                                            c_void_p, c_void_p, c_void_p, c_void_p]),
+                                            c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_int,
+                                            c_void_p, c_size_t, c_void_p, c_void_p, c_void_p, c_void_p]),
     "hgr_score_topk_splits_workspace_bytes": (c_size_t, [c_int64, c_int64, c_int64, c_int, c_int, c_void_p]),
     "hgr_score_topk_splits": (c_int, [c_void_p, c_void_p, c_void_p, c_int32, c_void_p, c_void_p, c_int64, c_int64, c_int64,
                                       c_int64, c_float, c_int, c_int, c_void_p, c_void_p, c_int, c_void_p, c_size_t,
                                       c_void_p, c_void_p, c_void_p, c_int, c_void_p]),
-    "hgr_hier_metrics_fused_rows_splits": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int64, c_void_p, c_int, c_void_p,
-                                                   c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_int,
-                                                   c_void_p, c_size_t, c_void_p, c_void_p]),
     "hgr_hier_level_scatter": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int64, c_void_p, c_int, c_int64, c_void_p,
                                        c_size_t, c_int64, c_int, c_void_p, c_void_p]),
     "hgr_hier_finish_rows_gathered": (c_int, [c_void_p, c_int, c_int64, c_int64, c_int64, c_int, c_void_p, c_void_p,
-                                              c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
-                                              c_void_p]),
+                                              c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p,
+                                              c_void_p, c_void_p, c_void_p]),
     "hgr_score_topk_splits_scatter_bounded_workspace_bytes": (c_size_t, [c_int64, c_int64, c_int64, c_int, c_int, c_void_p]),
     "hgr_score_topk_splits_global_list_len": (c_int, [c_int64, c_int64, c_int64, c_int, c_int, c_void_p, c_void_p, c_int,
                                                       c_void_p]),
@@ -89,9 +86,6 @@ SIGNATURES = {
     "hgr_topk_merge_splits_certified": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int, c_int, c_int64,
                                                 c_int64, c_int64, c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p,
                                                 c_void_p, c_int64, c_void_p, c_float, c_void_p, c_void_p]),
-    "hgr_hier_finish_rows_gathered_splits": (c_int, [c_void_p, c_int, c_int64, c_int64, c_int64, c_int, c_void_p, c_void_p,
-                                                     c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_int,
-                                                     c_void_p, c_void_p]),
     "hgr_hier_mistakes": (c_int, [c_void_p, c_int64, c_int, c_int64, c_int, c_void_p, c_void_p, c_void_p, c_void_p,
                                   c_int64, c_void_p, c_void_p]),
     "hgr_masked_ce_workspace_bytes":(c_size_t, [c_int64, c_int64, c_int64]),

@@ -213,30 +213,20 @@ int umma_split_global_list_len(int64_t B, int64_t C, int64_t D, int K, const Gro
 
 int launch_level_argmax_umma(const __nv_bfloat16* X, const __nv_bfloat16* bank_sorted, int64_t B, int64_t M, int64_t D,
                              const int32_t* level_end, int n_levels, unsigned long long* lvl_best, cudaStream_t stream);
+// TOR / POR finish: node_splits NULL -> counts [HGR_HIER_MAX_CHAIN + 1][4]; otherwise counts [n_sets][...], a row
+// added to set s for every bit s of node_splits[targets[row]]
 int launch_hier_finish_rows(unsigned long long* lvl_best, int64_t B, int64_t M, int n_levels, const int32_t* sorted_to_pos,
                             const int32_t* first_out, const int32_t* targets, int64_t n_nodes, const int32_t* chain_ptr,
-                            const int32_t* chain_pos, const int32_t* chain_level, int32_t* lvl_idx, int32_t* top1,
-                            int64_t* counts, cudaStream_t stream);
+                            const int32_t* chain_pos, const int32_t* chain_level, const uint8_t* node_splits, int n_sets,
+                            int32_t* lvl_idx, int32_t* top1, int64_t* counts, cudaStream_t stream);
 // class-sharded TOR / POR (hgr_hier_level_scatter / hgr_hier_finish_rows_gathered)
 int launch_hier_push(unsigned long long* lvl_best, int64_t B, int n_levels, int64_t row_base, int64_t block_rows,
                      int n_blocks, unsigned long long* const* dst, cudaStream_t stream);
 int launch_hier_finish_gathered(const unsigned long long* parts, int n_parts, int64_t part_stride, int64_t B, int64_t M,
                                 int n_levels, const int32_t* sorted_to_pos, const int32_t* first_out,
                                 const int32_t* targets, int64_t n_nodes, const int32_t* chain_ptr,
-                                const int32_t* chain_pos, const int32_t* chain_level, int32_t* lvl_idx, int32_t* top1,
-                                int64_t* counts, cudaStream_t stream);
-// hgr_hier_metrics_fused_rows_splits: counts [n_splits][HGR_HIER_MAX_CHAIN + 1][4], a row in every split of its label
-int launch_hier_finish_rows_splits(unsigned long long* lvl_best, int64_t B, int64_t M, int n_levels,
-                                   const int32_t* sorted_to_pos, const int32_t* first_out, const int32_t* targets,
-                                   int64_t n_nodes, const int32_t* chain_ptr, const int32_t* chain_pos,
-                                   const int32_t* chain_level, const uint8_t* node_splits, int n_splits,
-                                   int64_t* counts, cudaStream_t stream);
-// hgr_hier_finish_rows_gathered_splits: the gathered words, counted per split as above
-int launch_hier_finish_gathered_splits(const unsigned long long* parts, int n_parts, int64_t part_stride, int64_t B,
-                                       int64_t M, int n_levels, const int32_t* sorted_to_pos, const int32_t* first_out,
-                                       const int32_t* targets, int64_t n_nodes, const int32_t* chain_ptr,
-                                       const int32_t* chain_pos, const int32_t* chain_level, const uint8_t* node_splits,
-                                       int n_splits, int64_t* counts, cudaStream_t stream);
+                                const int32_t* chain_pos, const int32_t* chain_level, const uint8_t* node_splits,
+                                int n_sets, int32_t* lvl_idx, int32_t* top1, int64_t* counts, cudaStream_t stream);
 int launch_hier_mistakes(const int32_t* topk_idx, int64_t B, int K, int64_t set_stride, int n_sets,
                          const int32_t* targets, const uint8_t* node_splits, const int32_t* chain_ptr,
                          const int32_t* chain_node, int64_t n_nodes, int64_t* counts, cudaStream_t stream);

@@ -669,14 +669,17 @@ int hgr_hier_metrics_fused_rows(const void* X, const void* bank_sorted, int64_t 
                                 const int32_t* level_end, int n_levels, const int32_t* sorted_to_pos,
                                 const int32_t* first_out, const int32_t* targets, int64_t n_nodes,
                                 const int32_t* chain_ptr, const int32_t* chain_pos, const int32_t* chain_level,
-                                void* workspace, size_t workspace_bytes, int32_t* lvl_idx, int32_t* top1,
-                                int64_t* counts, void* stream) {
+                                const uint8_t* node_splits, int n_sets, void* workspace, size_t workspace_bytes,
+                                int32_t* lvl_idx, int32_t* top1, int64_t* counts, void* stream) {
   HGR_CHECK_ARG(B >= 0 && M > 0 && M <= (int64_t(1) << 31) - 512, "hgr_hier_metrics_fused_rows: bad sizes B=%lld M=%lld",
                 (long long)B, (long long)M);
   HGR_CHECK_ARG(D > 0 && D % 8 == 0, "hgr_hier_metrics_fused_rows: D = %lld must be a positive multiple of 8", (long long)D);
   HGR_CHECK_ARG(n_nodes > 0 && n_nodes < (int64_t(1) << 31) - 1, "hgr_hier_metrics_fused_rows: n_nodes = %lld",
                 (long long)n_nodes);
   HGR_CHECK_ARG(n_levels >= 1 && n_levels <= 32, "hgr_hier_metrics_fused_rows: %d levels outside [1, 32]", n_levels);
+  HGR_CHECK_ARG(n_sets >= 1 && n_sets <= (node_splits ? kMaxSplits : 1),
+                "hgr_hier_metrics_fused_rows: %d counter sets outside [1, %d] (%s node_splits)", n_sets,
+                node_splits ? kMaxSplits : 1, node_splits ? "with" : "without");
   if (B == 0) return HGR_OK;
   HGR_CHECK_ARG(X && bank_sorted && level_end && sorted_to_pos && first_out && targets && chain_ptr && chain_pos &&
                     chain_level && counts && workspace,
@@ -693,42 +696,7 @@ int hgr_hier_metrics_fused_rows(const void* X, const void* bank_sorted, int64_t 
                                           D, level_end, n_levels, best, s);
   if (rc != HGR_OK) return rc;
   return launch_hier_finish_rows(best, B, M, n_levels, sorted_to_pos, first_out, targets, n_nodes, chain_ptr, chain_pos,
-                                 chain_level, lvl_idx, top1, counts, s);
-}
-
-// main.py:143,152-191 run once per split: hgr_hier_metrics_fused_rows with the counters binned per split of the label.
-int hgr_hier_metrics_fused_rows_splits(const void* X, const void* bank_sorted, int64_t B, int64_t M, int64_t D,
-                                       const int32_t* level_end, int n_levels, const int32_t* sorted_to_pos,
-                                       const int32_t* first_out, const int32_t* targets, int64_t n_nodes,
-                                       const int32_t* chain_ptr, const int32_t* chain_pos, const int32_t* chain_level,
-                                       const uint8_t* node_splits, int n_splits, void* workspace, size_t workspace_bytes,
-                                       int64_t* counts, void* stream) {
-  HGR_CHECK_ARG(B >= 0 && M > 0 && M <= (int64_t(1) << 31) - 512, "hgr_hier_metrics_fused_rows_splits: bad sizes B=%lld M=%lld",
-                (long long)B, (long long)M);
-  HGR_CHECK_ARG(D > 0 && D % 8 == 0, "hgr_hier_metrics_fused_rows_splits: D = %lld must be a positive multiple of 8", (long long)D);
-  HGR_CHECK_ARG(n_nodes > 0 && n_nodes < (int64_t(1) << 31) - 1, "hgr_hier_metrics_fused_rows_splits: n_nodes = %lld",
-                (long long)n_nodes);
-  HGR_CHECK_ARG(n_levels >= 1 && n_levels <= 32, "hgr_hier_metrics_fused_rows_splits: %d levels outside [1, 32]", n_levels);
-  HGR_CHECK_ARG(n_splits >= 1 && n_splits <= kMaxSplits, "hgr_hier_metrics_fused_rows_splits: %d splits outside [1, %d]",
-                n_splits, kMaxSplits);
-  if (B == 0) return HGR_OK;
-  HGR_CHECK_ARG(X && bank_sorted && level_end && sorted_to_pos && first_out && targets && chain_ptr && chain_pos &&
-                    chain_level && node_splits && counts && workspace,
-                "hgr_hier_metrics_fused_rows_splits: null pointer");
-  HGR_CHECK_ARG(aligned16(X) && aligned16(bank_sorted) && aligned16(workspace),
-                "hgr_hier_metrics_fused_rows_splits: X / bank / workspace must be 16-byte aligned");
-  HGR_CHECK_ARG(workspace_bytes >= static_cast<size_t>(B) * n_levels * 8,
-                "hgr_hier_metrics_fused_rows_splits: workspace %zu < %zu bytes", workspace_bytes,
-                static_cast<size_t>(B) * n_levels * 8);
-  if (!umma_supported(B, M, D, 1))
-    return set_error(HGR_ERR_UNSUPPORTED, "hgr_hier_metrics_fused_rows_splits: shape not supported by the tcgen05 kernel");
-  cudaStream_t s = static_cast<cudaStream_t>(stream);
-  unsigned long long* best = static_cast<unsigned long long*>(workspace);
-  const int rc = launch_level_argmax_umma(static_cast<const __nv_bfloat16*>(X), static_cast<const __nv_bfloat16*>(bank_sorted), B, M,
-                                          D, level_end, n_levels, best, s);
-  if (rc != HGR_OK) return rc;
-  return launch_hier_finish_rows_splits(best, B, M, n_levels, sorted_to_pos, first_out, targets, n_nodes, chain_ptr,
-                                        chain_pos, chain_level, node_splits, n_splits, counts, s);
+                                 chain_level, node_splits, n_sets, lvl_idx, top1, counts, s);
 }
 
 int hgr_hier_level_scatter(const void* X, const void* bank_shard, int64_t B, int64_t M_r, int64_t D,
@@ -771,8 +739,8 @@ int hgr_hier_level_scatter(const void* X, const void* bank_shard, int64_t B, int
 int hgr_hier_finish_rows_gathered(const uint64_t* parts, int n_parts, int64_t part_stride, int64_t n_rows, int64_t M,
                                   int n_levels, const int32_t* sorted_to_pos, const int32_t* first_out,
                                   const int32_t* targets, int64_t n_nodes, const int32_t* chain_ptr,
-                                  const int32_t* chain_pos, const int32_t* chain_level, int32_t* lvl_idx, int32_t* top1,
-                                  int64_t* counts, void* stream) {
+                                  const int32_t* chain_pos, const int32_t* chain_level, const uint8_t* node_splits,
+                                  int n_sets, int32_t* lvl_idx, int32_t* top1, int64_t* counts, void* stream) {
   HGR_CHECK_ARG(n_rows >= 0 && M > 0 && M <= (int64_t(1) << 31) - 512, "hgr_hier_finish_rows_gathered: bad sizes n_rows=%lld M=%lld",
                 (long long)n_rows, (long long)M);
   HGR_CHECK_ARG(n_nodes > 0 && n_nodes < (int64_t(1) << 31) - 1, "hgr_hier_finish_rows_gathered: n_nodes = %lld",
@@ -780,6 +748,9 @@ int hgr_hier_finish_rows_gathered(const uint64_t* parts, int n_parts, int64_t pa
   HGR_CHECK_ARG(n_levels >= 1 && n_levels <= 32, "hgr_hier_finish_rows_gathered: %d levels outside [1, 32]", n_levels);
   HGR_CHECK_ARG(n_parts >= 1 && n_parts <= kMaxScatterBlocks, "hgr_hier_finish_rows_gathered: n_parts = %d outside [1, %d]",
                 n_parts, kMaxScatterBlocks);
+  HGR_CHECK_ARG(n_sets >= 1 && n_sets <= (node_splits ? kMaxSplits : 1),
+                "hgr_hier_finish_rows_gathered: %d counter sets outside [1, %d] (%s node_splits)", n_sets,
+                node_splits ? kMaxSplits : 1, node_splits ? "with" : "without");
   HGR_CHECK_ARG(part_stride >= n_rows * n_levels, "hgr_hier_finish_rows_gathered: part_stride < n_rows * n_levels");
   if (n_rows == 0) return HGR_OK;
   HGR_CHECK_ARG(parts && sorted_to_pos && first_out && targets && chain_ptr && chain_pos && chain_level && counts,
@@ -787,34 +758,7 @@ int hgr_hier_finish_rows_gathered(const uint64_t* parts, int n_parts, int64_t pa
   HGR_CHECK_ARG((reinterpret_cast<uintptr_t>(parts) & 7u) == 0, "hgr_hier_finish_rows_gathered: parts must be 8-byte aligned");
   return launch_hier_finish_gathered(reinterpret_cast<const unsigned long long*>(parts), n_parts, part_stride, n_rows, M,
                                      n_levels, sorted_to_pos, first_out, targets, n_nodes, chain_ptr, chain_pos, chain_level,
-                                     lvl_idx, top1, counts, static_cast<cudaStream_t>(stream));
-}
-
-int hgr_hier_finish_rows_gathered_splits(const uint64_t* parts, int n_parts, int64_t part_stride, int64_t n_rows,
-                                         int64_t M, int n_levels, const int32_t* sorted_to_pos, const int32_t* first_out,
-                                         const int32_t* targets, int64_t n_nodes, const int32_t* chain_ptr,
-                                         const int32_t* chain_pos, const int32_t* chain_level, const uint8_t* node_splits,
-                                         int n_splits, int64_t* counts, void* stream) {
-  HGR_CHECK_ARG(n_rows >= 0 && M > 0 && M <= (int64_t(1) << 31) - 512,
-                "hgr_hier_finish_rows_gathered_splits: bad sizes n_rows=%lld M=%lld", (long long)n_rows, (long long)M);
-  HGR_CHECK_ARG(n_nodes > 0 && n_nodes < (int64_t(1) << 31) - 1, "hgr_hier_finish_rows_gathered_splits: n_nodes = %lld",
-                (long long)n_nodes);
-  HGR_CHECK_ARG(n_levels >= 1 && n_levels <= 32, "hgr_hier_finish_rows_gathered_splits: %d levels outside [1, 32]", n_levels);
-  HGR_CHECK_ARG(n_parts >= 1 && n_parts <= kMaxScatterBlocks,
-                "hgr_hier_finish_rows_gathered_splits: n_parts = %d outside [1, %d]", n_parts, kMaxScatterBlocks);
-  HGR_CHECK_ARG(n_splits >= 1 && n_splits <= kMaxSplits, "hgr_hier_finish_rows_gathered_splits: %d splits outside [1, %d]",
-                n_splits, kMaxSplits);
-  HGR_CHECK_ARG(part_stride >= n_rows * n_levels, "hgr_hier_finish_rows_gathered_splits: part_stride < n_rows * n_levels");
-  if (n_rows == 0) return HGR_OK;
-  HGR_CHECK_ARG(parts && sorted_to_pos && first_out && targets && chain_ptr && chain_pos && chain_level && node_splits &&
-                    counts,
-                "hgr_hier_finish_rows_gathered_splits: null pointer");
-  HGR_CHECK_ARG((reinterpret_cast<uintptr_t>(parts) & 7u) == 0,
-                "hgr_hier_finish_rows_gathered_splits: parts must be 8-byte aligned");
-  return launch_hier_finish_gathered_splits(reinterpret_cast<const unsigned long long*>(parts), n_parts, part_stride,
-                                            n_rows, M, n_levels, sorted_to_pos, first_out, targets, n_nodes, chain_ptr,
-                                            chain_pos, chain_level, node_splits, n_splits, counts,
-                                            static_cast<cudaStream_t>(stream));
+                                     node_splits, n_sets, lvl_idx, top1, counts, static_cast<cudaStream_t>(stream));
 }
 
 // main.py:135-148 extended from "label in the first k" to the hierarchy distance of the first k (hier_mistakes.cu).

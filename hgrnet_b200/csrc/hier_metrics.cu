@@ -109,18 +109,19 @@ __device__ __forceinline__ RowCounts finish_row(const Words& words, int64_t row,
 constexpr int kRowsPerBlock = 8;
 constexpr int kHistWords = (HGR_HIER_MAX_CHAIN + 1) * 4;
 
-// kSplits (hgr_hier_metrics_fused_rows_splits): counter set s ([s][kHistWords]) takes the rows whose label has bit s in
-// node_splits -- a row in several splits is added to each of them.
-template <class Words, bool kSplits = false>
+// kSplits (node_splits != NULL): counter set s ([s][kHistWords]) takes the rows whose label has bit s in node_splits --
+// a row in several splits is added to each of them.  Without splits there is one set and a 528-byte histogram.
+template <bool kSplits, class Words>
 __device__ __forceinline__ void finish_rows_block(const Words& words, int64_t B, int64_t M, int n_levels,
                                                   const int32_t* __restrict__ sorted_to_pos,
                                                   const int32_t* __restrict__ first_out,
                                                   const int32_t* __restrict__ targets, int64_t n_nodes,
                                                   const int32_t* __restrict__ chain_ptr,
                                                   const int32_t* __restrict__ chain_pos,
-                                                  const int32_t* __restrict__ chain_level, int32_t* __restrict__ lvl_idx,
-                                                  int32_t* __restrict__ top1, unsigned long long* counts,
-                                                  const uint8_t* __restrict__ node_splits = nullptr, int n_splits = 1) {
+                                                  const int32_t* __restrict__ chain_level,
+                                                  const uint8_t* __restrict__ node_splits, int n_sets,
+                                                  int32_t* __restrict__ lvl_idx, int32_t* __restrict__ top1,
+                                                  unsigned long long* counts) {
   constexpr int kSets = kSplits ? kMaxSplits : 1;
   __shared__ unsigned int s_cnt[kSets * kHistWords];   // <= kRowsPerBlock * HGR_HIER_MAX_CHAIN per word: 32 bits suffice
   for (int i = threadIdx.x; i < kSets * kHistWords; i += blockDim.x) s_cnt[i] = 0u;
@@ -157,29 +158,20 @@ __device__ __forceinline__ void finish_rows_block(const Words& words, int64_t B,
     }
   }
   __syncthreads();
-  for (int i = threadIdx.x; i < (kSplits ? n_splits : 1) * kHistWords; i += blockDim.x)
+  for (int i = threadIdx.x; i < (kSplits ? n_sets : 1) * kHistWords; i += blockDim.x)
     if (s_cnt[i]) atomicAdd(counts + i, static_cast<unsigned long long>(s_cnt[i]));
 }
 
+template <bool kSplits>
 __global__ void __launch_bounds__(kRowsPerBlock * 32)
 hier_finish_rows_kernel(unsigned long long* __restrict__ lvl_best, int64_t B, int64_t M, int n_levels,
                         const int32_t* __restrict__ sorted_to_pos, const int32_t* __restrict__ first_out,
                         const int32_t* __restrict__ targets, int64_t n_nodes, const int32_t* __restrict__ chain_ptr,
                         const int32_t* __restrict__ chain_pos, const int32_t* __restrict__ chain_level,
-                        int32_t* __restrict__ lvl_idx, int32_t* __restrict__ top1, unsigned long long* counts) {
-  finish_rows_block(WsWords{lvl_best}, B, M, n_levels, sorted_to_pos, first_out, targets, n_nodes, chain_ptr, chain_pos,
-                    chain_level, lvl_idx, top1, counts);
-}
-
-__global__ void __launch_bounds__(kRowsPerBlock * 32)
-hier_finish_rows_splits_kernel(unsigned long long* __restrict__ lvl_best, int64_t B, int64_t M, int n_levels,
-                               const int32_t* __restrict__ sorted_to_pos, const int32_t* __restrict__ first_out,
-                               const int32_t* __restrict__ targets, int64_t n_nodes,
-                               const int32_t* __restrict__ chain_ptr, const int32_t* __restrict__ chain_pos,
-                               const int32_t* __restrict__ chain_level, const uint8_t* __restrict__ node_splits,
-                               int n_splits, unsigned long long* counts) {
-  finish_rows_block<WsWords, true>(WsWords{lvl_best}, B, M, n_levels, sorted_to_pos, first_out, targets, n_nodes,
-                                   chain_ptr, chain_pos, chain_level, nullptr, nullptr, counts, node_splits, n_splits);
+                        const uint8_t* __restrict__ node_splits, int n_sets, int32_t* __restrict__ lvl_idx,
+                        int32_t* __restrict__ top1, unsigned long long* counts) {
+  finish_rows_block<kSplits>(WsWords{lvl_best}, B, M, n_levels, sorted_to_pos, first_out, targets, n_nodes, chain_ptr,
+                             chain_pos, chain_level, node_splits, n_sets, lvl_idx, top1, counts);
 }
 
 // ---- class-sharded form (hgr_hier_level_scatter / hgr_hier_finish_rows_gathered) -------------------------------------
@@ -205,28 +197,17 @@ struct GatheredWords {
   }
 };
 
+template <bool kSplits>
 __global__ void __launch_bounds__(kRowsPerBlock * 32)
 hier_finish_gathered_kernel(const unsigned long long* __restrict__ parts, int n_parts, int64_t part_stride, int64_t B,
                             int64_t M, int n_levels, const int32_t* __restrict__ sorted_to_pos,
                             const int32_t* __restrict__ first_out, const int32_t* __restrict__ targets, int64_t n_nodes,
                             const int32_t* __restrict__ chain_ptr, const int32_t* __restrict__ chain_pos,
-                            const int32_t* __restrict__ chain_level, int32_t* __restrict__ lvl_idx,
-                            int32_t* __restrict__ top1, unsigned long long* counts) {
-  finish_rows_block(GatheredWords{parts, n_parts, part_stride}, B, M, n_levels, sorted_to_pos, first_out, targets,
-                    n_nodes, chain_ptr, chain_pos, chain_level, lvl_idx, top1, counts);
-}
-
-// hgr_hier_finish_rows_gathered_splits: the gathered words, counted per split of the row's label
-__global__ void __launch_bounds__(kRowsPerBlock * 32)
-hier_finish_gathered_splits_kernel(const unsigned long long* __restrict__ parts, int n_parts, int64_t part_stride,
-                                   int64_t B, int64_t M, int n_levels, const int32_t* __restrict__ sorted_to_pos,
-                                   const int32_t* __restrict__ first_out, const int32_t* __restrict__ targets,
-                                   int64_t n_nodes, const int32_t* __restrict__ chain_ptr,
-                                   const int32_t* __restrict__ chain_pos, const int32_t* __restrict__ chain_level,
-                                   const uint8_t* __restrict__ node_splits, int n_splits, unsigned long long* counts) {
-  finish_rows_block<GatheredWords, true>(GatheredWords{parts, n_parts, part_stride}, B, M, n_levels, sorted_to_pos,
-                                         first_out, targets, n_nodes, chain_ptr, chain_pos, chain_level, nullptr, nullptr,
-                                         counts, node_splits, n_splits);
+                            const int32_t* __restrict__ chain_level, const uint8_t* __restrict__ node_splits, int n_sets,
+                            int32_t* __restrict__ lvl_idx, int32_t* __restrict__ top1, unsigned long long* counts) {
+  finish_rows_block<kSplits>(GatheredWords{parts, n_parts, part_stride}, B, M, n_levels, sorted_to_pos, first_out,
+                             targets, n_nodes, chain_ptr, chain_pos, chain_level, node_splits, n_sets, lvl_idx, top1,
+                             counts);
 }
 
 struct HierDst {
@@ -267,55 +248,28 @@ int launch_hier_push(unsigned long long* lvl_best, int64_t B, int n_levels, int6
 int launch_hier_finish_gathered(const unsigned long long* parts, int n_parts, int64_t part_stride, int64_t B, int64_t M,
                                 int n_levels, const int32_t* sorted_to_pos, const int32_t* first_out,
                                 const int32_t* targets, int64_t n_nodes, const int32_t* chain_ptr,
-                                const int32_t* chain_pos, const int32_t* chain_level, int32_t* lvl_idx, int32_t* top1,
-                                int64_t* counts, cudaStream_t stream) {
+                                const int32_t* chain_pos, const int32_t* chain_level, const uint8_t* node_splits,
+                                int n_sets, int32_t* lvl_idx, int32_t* top1, int64_t* counts, cudaStream_t stream) {
   const int blocks = static_cast<int>((B + kRowsPerBlock - 1) / kRowsPerBlock);     // one warp per image row
-  hier_finish_gathered_kernel<<<blocks, kRowsPerBlock * 32, 0, stream>>>(
-      parts, n_parts, part_stride, B, M, n_levels, sorted_to_pos, first_out, targets, n_nodes, chain_ptr, chain_pos,
-      chain_level, lvl_idx, top1, reinterpret_cast<unsigned long long*>(counts));
+  auto kernel = node_splits ? hier_finish_gathered_kernel<true> : hier_finish_gathered_kernel<false>;
+  kernel<<<blocks, kRowsPerBlock * 32, 0, stream>>>(parts, n_parts, part_stride, B, M, n_levels, sorted_to_pos, first_out,
+                                                    targets, n_nodes, chain_ptr, chain_pos, chain_level, node_splits,
+                                                    n_sets, lvl_idx, top1, reinterpret_cast<unsigned long long*>(counts));
   HGR_CHECK_LAUNCH();
   return HGR_OK;
 }
 
 int launch_hier_finish_rows(unsigned long long* lvl_best, int64_t B, int64_t M, int n_levels, const int32_t* sorted_to_pos,
                             const int32_t* first_out, const int32_t* targets, int64_t n_nodes, const int32_t* chain_ptr,
-                            const int32_t* chain_pos, const int32_t* chain_level, int32_t* lvl_idx, int32_t* top1,
-                            int64_t* counts, cudaStream_t stream) {
+                            const int32_t* chain_pos, const int32_t* chain_level, const uint8_t* node_splits, int n_sets,
+                            int32_t* lvl_idx, int32_t* top1, int64_t* counts, cudaStream_t stream) {
   if (n_levels < 1 || n_levels > kMaxLevels)
     return set_error(HGR_ERR_UNSUPPORTED, "hgr_hier_metrics_fused_rows: %d levels outside [1, %d]", n_levels, kMaxLevels);
   const int blocks = static_cast<int>((B + kRowsPerBlock - 1) / kRowsPerBlock);     // one warp per image row
-  hier_finish_rows_kernel<<<blocks, kRowsPerBlock * 32, 0, stream>>>(
-      lvl_best, B, M, n_levels, sorted_to_pos, first_out, targets, n_nodes, chain_ptr, chain_pos, chain_level, lvl_idx,
-      top1, reinterpret_cast<unsigned long long*>(counts));
-  HGR_CHECK_LAUNCH();
-  return HGR_OK;
-}
-
-int launch_hier_finish_rows_splits(unsigned long long* lvl_best, int64_t B, int64_t M, int n_levels,
-                                   const int32_t* sorted_to_pos, const int32_t* first_out, const int32_t* targets,
-                                   int64_t n_nodes, const int32_t* chain_ptr, const int32_t* chain_pos,
-                                   const int32_t* chain_level, const uint8_t* node_splits, int n_splits,
-                                   int64_t* counts, cudaStream_t stream) {
-  if (n_levels < 1 || n_levels > kMaxLevels)
-    return set_error(HGR_ERR_UNSUPPORTED, "hgr_hier_metrics_fused_rows_splits: %d levels outside [1, %d]", n_levels,
-                     kMaxLevels);
-  const int blocks = static_cast<int>((B + kRowsPerBlock - 1) / kRowsPerBlock);     // one warp per image row
-  hier_finish_rows_splits_kernel<<<blocks, kRowsPerBlock * 32, 0, stream>>>(
-      lvl_best, B, M, n_levels, sorted_to_pos, first_out, targets, n_nodes, chain_ptr, chain_pos, chain_level,
-      node_splits, n_splits, reinterpret_cast<unsigned long long*>(counts));
-  HGR_CHECK_LAUNCH();
-  return HGR_OK;
-}
-
-int launch_hier_finish_gathered_splits(const unsigned long long* parts, int n_parts, int64_t part_stride, int64_t B,
-                                       int64_t M, int n_levels, const int32_t* sorted_to_pos, const int32_t* first_out,
-                                       const int32_t* targets, int64_t n_nodes, const int32_t* chain_ptr,
-                                       const int32_t* chain_pos, const int32_t* chain_level, const uint8_t* node_splits,
-                                       int n_splits, int64_t* counts, cudaStream_t stream) {
-  const int blocks = static_cast<int>((B + kRowsPerBlock - 1) / kRowsPerBlock);     // one warp per image row
-  hier_finish_gathered_splits_kernel<<<blocks, kRowsPerBlock * 32, 0, stream>>>(
-      parts, n_parts, part_stride, B, M, n_levels, sorted_to_pos, first_out, targets, n_nodes, chain_ptr, chain_pos,
-      chain_level, node_splits, n_splits, reinterpret_cast<unsigned long long*>(counts));
+  auto kernel = node_splits ? hier_finish_rows_kernel<true> : hier_finish_rows_kernel<false>;
+  kernel<<<blocks, kRowsPerBlock * 32, 0, stream>>>(lvl_best, B, M, n_levels, sorted_to_pos, first_out, targets, n_nodes,
+                                                    chain_ptr, chain_pos, chain_level, node_splits, n_sets, lvl_idx, top1,
+                                                    reinterpret_cast<unsigned long long*>(counts));
   HGR_CHECK_LAUNCH();
   return HGR_OK;
 }

@@ -25,6 +25,7 @@ import torch
 import torch.distributed as dist
 
 from . import ops
+from .evaluate import EvalCounters
 
 
 def shard_bounds(C: int, world: int) -> List[Tuple[int, int]]:
@@ -475,7 +476,7 @@ class PeerExchange:
         ``hier_out = (lvl_idx [n, n_levels], top1 [n])`` int32 receives their per-level winners and top-1.
         ``splits`` after a ``scatter(splits=...)`` (needs ``certify``): per split the certified top-K of my rows
         (``[S, n, K]``), Hit@k and rows counted into ``split_counts`` ``[S, HGR_NUM_HITS + 1]``; with ``hier``, ``counts``
-        holds the per-split TOR / POR counters ``[S, HGR_HIER_MAX_CHAIN + 1, 4]``."""
+        holds the per-split TOR / POR counters ``[S, HGR_HIER_MAX_CHAIN + 1, 4]`` (``ops.new_hier_counts(device, S)``)."""
         ops.peer_wait(self.bases[self.rank], self.world, self.seq[1:2])
         n = self.hi - self.lo
         if n <= 0:
@@ -488,13 +489,7 @@ class PeerExchange:
                                                   self.block_rows, self.split_stride, x_norm[self.lo:self.hi], table,
                                                   splits.node_splits, self.device, targets=t, counts=split_counts,
                                                   repair_count=repairs, out=out)
-            if hier is not None:
-                parts, part_stride = self.local_hier(slot)
-                ops.hier_finish_rows_gathered_splits(parts, self.world, part_stride, n, hier.M, hier.n_levels,
-                                                     hier.sorted_to_pos, hier.first_out, t, hier.chain_ptr, hier.chain_pos,
-                                                     hier.chain_level, splits.node_splits, counts)
-            return res
-        if certify is not None:
+        elif certify is not None:
             x_norm, table, repairs = certify
             res = ops.topk_merge_certified(pv, pi, self.local_bounds(slot), self.world, n, self.K, stride, self.block_rows,
                                            x_norm[self.lo:self.hi], table, self.device, targets=t, hits=hits,
@@ -506,7 +501,8 @@ class PeerExchange:
             lvl_idx, top1 = hier_out if hier_out is not None else (None, None)
             ops.hier_finish_rows_gathered(parts, self.world, part_stride, n, hier.M, hier.n_levels, hier.sorted_to_pos,
                                           hier.first_out, t, hier.chain_ptr, hier.chain_pos, hier.chain_level, counts,
-                                          lvl_idx=lvl_idx, top1=top1)
+                                          node_splits=None if splits is None else splits.node_splits, lvl_idx=lvl_idx,
+                                          top1=top1)
         return res
 
     def close(self) -> None:
@@ -553,9 +549,10 @@ class ShardedEvalStream:
     against the rank's part of several test splits instead of ``bank_shard``, in one pass, as ``EvalStream(splits=...)``
     does on one GPU.  ``val`` / ``idx`` are ``[S, rows, K]``; the per-split Hit@k / row counters ``split_counts``
     ``[S, HGR_NUM_HITS + 1]`` and, when the ``SplitShard`` has ``hier``, the per-split TOR / POR counters
-    ``split_hier_counts`` live in ``counters`` too.  ``split_hit_counts()`` / ``split_ratios()`` / ``split_lines()`` sum
-    them over ranks.  With ``splits`` the stream scores nothing against ``bank_shard`` / ``id_base``: ``bank_shard`` only
-    has to agree with the ``SplitShard`` on D and device (pass e.g. ``split_eval.bank()``), and ``id_base`` is unused.
+    ``hier_counts`` ``[S, HGR_HIER_MAX_CHAIN + 1, 4]`` live in ``counters`` too.  ``split_hit_counts()`` /
+    ``split_ratios()`` / ``split_lines()`` sum them over ranks.  With ``splits`` the stream scores nothing against
+    ``bank_shard`` / ``id_base``: ``bank_shard`` only has to agree with the ``SplitShard`` on D and device (pass e.g.
+    ``split_eval.bank()``), and ``id_base`` is unused.
 
     ``mistakes`` (a ``MistakeShard`` of this rank, peer exchange only, with or without ``splits``): after the merge the
     row owner counts the mistake severity and LCA distance@k of its merged lists against each row's own label
@@ -623,26 +620,16 @@ class ShardedEvalStream:
         if not host_io:
             self.dev_feats = [torch.empty((batch, D), dtype=feat_dtype, device=self.device) for _ in range(steps)]
             self.dev_labels = [torch.zeros((batch,), dtype=torch.int32, device=self.device) for _ in range(steps)]
-        # hit counters, then (with hier) the per-chain-length TOR / POR counters: one buffer, one D2H copy per batch
+        # every counter of the stream in one device buffer (evaluate.EvalCounters): one D2H copy per batch
         self.hier = hier
-        n_hier = 0 if hier is None else (ops.HGR_HIER_MAX_CHAIN + 1) * 4
         S = 0 if splits is None else splits.S
-        n_split = S * (ops.HGR_NUM_HITS + 1)
-        n_split_hier = 0 if splits is None or splits.hier is None else S * (ops.HGR_HIER_MAX_CHAIN + 1) * 4
         self.mistakes = mistakes
-        n_mist = 0 if mistakes is None else max(S, 1) * ops.HGR_MISTAKE_COUNTERS
-        n_counters = ops.HGR_NUM_HITS + n_hier + n_split + n_split_hier + n_mist
-        self.counters = torch.zeros(n_counters, dtype=torch.int64, device=self.device)
-        self.hits = self.counters[:ops.HGR_NUM_HITS]
-        o = ops.HGR_NUM_HITS
-        self.hier_counts = None if hier is None else self.counters[o:o + n_hier].view(ops.HGR_HIER_MAX_CHAIN + 1, 4)
-        o += n_hier
-        self.split_counts = None if splits is None else self.counters[o:o + n_split].view(S, ops.HGR_NUM_HITS + 1)
-        o += n_split
-        self.split_hier_counts = (self.counters[o:o + n_split_hier].view(S, ops.HGR_HIER_MAX_CHAIN + 1, 4)
-                                  if n_split_hier else None)
-        o += n_split_hier
-        self.mistake_counts = self.counters[o:o + n_mist].view(-1, ops.HGR_MISTAKE_COUNTERS) if n_mist else None
+        self.tally = EvalCounters(self.device, n_splits=S, hier=self._hier_shard() is not None,
+                                  mistakes=mistakes is not None, K=K, read=self._read_counters)
+        self.counters, self.hits = self.tally.counters, self.tally.hits
+        self.split_counts, self.hier_counts = self.tally.split_counts, self.tally.hier_counts
+        self.mistake_counts = self.tally.mistake_counts
+        n_counters = self.counters.numel()
         self.val = [None] * steps
         self.idx = [None] * steps
         self.row_lo, self.row_hi = 0, batch
@@ -658,7 +645,7 @@ class ShardedEvalStream:
             if steps < 2:
                 raise ValueError("ShardedEvalStream needs steps >= 2 (two batches per exchange channel and replay)")
             self.channels = max(1, min(channels, steps // 2))
-            hs = hier if splits is None else splits.hier
+            hs = self._hier_shard()
             self.pxs = [PeerExchange(batch, K, self.device, group=group, slots=self.slots, D=D if host_io else 0,
                                      n_levels=0 if hs is None else hs.n_levels, n_splits=S)
                         for _ in range(self.channels)]
@@ -753,9 +740,8 @@ class ShardedEvalStream:
                 cert = (self._x[s], self.pbanks[s % len(self.pbanks)].table, self.repairs)
             self.pxs[s % self.channels].merge((s // self.channels) % self._ring[s % self.channels], self.dev_labels[s], self.hits,
                                               out=(self.val[s], self.idx[s]), targets_local=self.host_io, certify=cert,
-                                              hier=self._hier_shard(),
-                                              counts=self.hier_counts if self.splits is None else self.split_hier_counts,
-                                              splits=self.splits, split_counts=self.split_counts)
+                                              hier=self._hier_shard(), counts=self.hier_counts, splits=self.splits,
+                                              split_counts=self.split_counts)
             if self.mistakes is not None and self.row_hi > self.row_lo:     # the owner's merged lists, after the merge
                 t = self.dev_labels[s] if self.host_io else self.dev_labels[s][self.row_lo:self.row_hi]
                 ops.hier_mistakes(self.idx[s], t, counts=self.mistake_counts,
@@ -829,88 +815,42 @@ class ShardedEvalStream:
             dist.all_reduce(h, group=self.group)
         return h
 
+    # ------------------------------------------------------------------ readout (evaluate.EvalCounters)
+    # Every readout is a collective (one all_reduce of the counters): call it on every rank.
+    def _read_counters(self, counters):
+        torch.cuda.synchronize(self.device)
+        if self.world == 1:
+            return counters
+        c = counters.clone()
+        dist.all_reduce(c, group=self.group)
+        return c
+
     def hier_ratios(self):
         """``(hit_ratio, path_ratio, point_ratio)`` in percent -- the TOR / POR of the reference's ``test()`` line -- over
-        the rows of all ranks scored so far whose label lies in the hierarchy.  A collective (one ``all_reduce`` of the
-        per-chain-length counters): call it on every rank.  Needs ``hier``."""
-        if self.hier is None:
-            raise RuntimeError("ShardedEvalStream was built without hier metrics (pass hier=HierShard(...))")
-        from .evaluate import hier_totals
-        torch.cuda.synchronize(self.device)
-        c = self.hier_counts.clone()
-        if self.world > 1:
-            dist.all_reduce(c, group=self.group)
-        rows, hits, point, path = hier_totals(c).tolist()
-        if rows == 0:
-            return 0.0, 0.0, 0.0
-        return hits / rows * 100.0, path / rows * 100.0, point / rows * 100.0
+        the rows of all ranks scored so far whose label lies in the hierarchy.  Needs ``hier``."""
+        return self.tally.hier_ratios()
 
     def split_hit_counts(self):
         """Per split ``[Hit@1, @2, @5, @10, @20, rows]`` over the rows of all ranks scored so far, in the order of
-        ``splits.names``.  A collective (one ``all_reduce`` of the integer counters): call it on every rank.  Needs
-        ``splits``."""
-        if self.splits is None:
-            raise RuntimeError("ShardedEvalStream was built without splits (pass splits=SplitShard(...))")
-        torch.cuda.synchronize(self.device)
-        c = self.split_counts.clone()
-        if self.world > 1:
-            dist.all_reduce(c, group=self.group)
-        return c.tolist()
-
-    def _split_hier_totals(self):
-        from .evaluate import hier_totals
-        torch.cuda.synchronize(self.device)
-        c = self.split_hier_counts.clone()
-        if self.world > 1:
-            dist.all_reduce(c, group=self.group)
-        return [hier_totals(x).tolist() for x in c]
+        ``splits.names``.  Needs ``splits``."""
+        return self.tally.split_hit_counts()
 
     def split_ratios(self):
         """Per split ``(hit_ratio, path_ratio, point_ratio)`` in percent over the rows of all ranks whose label is in the
-        split.  A collective (one ``all_reduce``): call it on every rank.  Needs a ``SplitShard`` with ``hier``."""
-        if self.split_hier_counts is None:
-            raise RuntimeError("ShardedEvalStream was built without per-split TOR / POR (a SplitShard with hier)")
-        return [(0.0, 0.0, 0.0) if rows == 0 else (hits / rows * 100.0, path / rows * 100.0, point / rows * 100.0)
-                for rows, hits, point, path in self._split_hier_totals()]
+        split.  Needs a ``SplitShard`` with ``hier``."""
+        return self.tally.split_ratios()
 
     def split_lines(self):
         """One ``evaluate.split_line`` per split (Hit@k, plus TOR / POR when the ``SplitShard`` has ``hier`` and the
-        mistake metrics with ``mistakes``).  A collective: call it on every rank."""
-        from .evaluate import split_line
-        counts = self.split_hit_counts()
-        hier = self._split_hier_totals() if self.split_hier_counts is not None else None
-        mist = self.split_mistake_summary() if self.mistake_counts is not None else [None] * self.splits.S
-        out = []
-        for s, name in enumerate(self.splits.names):
-            rows = counts[s][ops.HGR_NUM_HITS]
-            h = None
-            if hier is not None:
-                r, tor, point, path = hier[s]
-                h = (tor, point, path, r)
-            out.append(split_line(name, counts[s][:ops.HGR_NUM_HITS], max(rows, 1), h, mist[s]))
-        return out
-
-    def _mistake_totals(self):
-        if self.mistake_counts is None:
-            raise RuntimeError("ShardedEvalStream was built without mistake metrics (pass mistakes=MistakeShard(...))")
-        torch.cuda.synchronize(self.device)
-        c = self.mistake_counts.clone()
-        if self.world > 1:
-            dist.all_reduce(c, group=self.group)
-        return c
+        mistake metrics with ``mistakes``)."""
+        return self.tally.split_lines(self.splits.names)
 
     def mistake_summary(self):
-        """``evaluate.mistake_summary`` over the rows of all ranks scored so far.  A collective (one ``all_reduce``):
-        call it on every rank.  Needs ``mistakes`` without ``splits``."""
-        from .evaluate import mistake_summary
-        if self.splits is not None:
-            raise RuntimeError("ShardedEvalStream has splits: use split_mistake_summary()")
-        return mistake_summary(self._mistake_totals()[0], self.K)
+        """``evaluate.mistake_summary`` over the rows of all ranks scored so far.  Needs ``mistakes`` without
+        ``splits``."""
+        return self.tally.mistake_summary()
 
     def split_mistake_summary(self):
-        """Per split ``evaluate.mistake_summary`` over the rows of all ranks whose label is in the split.  A collective
-        (one ``all_reduce``): call it on every rank.  Needs ``mistakes`` and ``splits``."""
-        from .evaluate import mistake_summary
-        if self.splits is None:
-            raise RuntimeError("ShardedEvalStream was built without splits: use mistake_summary()")
-        return [mistake_summary(c, self.K) for c in self._mistake_totals()]
+        """Per split ``evaluate.mistake_summary`` over the rows of all ranks whose label is in the split.  Needs
+        ``mistakes`` and ``splits``."""
+        return self.tally.split_mistake_summary()

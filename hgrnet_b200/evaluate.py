@@ -69,32 +69,33 @@ def hier_totals(counts: torch.Tensor) -> torch.Tensor:
     """Per-chain-length counters (``ops.new_hier_counts``: bin L = {rows, TOR hits, points, edges}) -> float64 ``[4]``
     ``(rows, hits, point, path)`` on the counters' device: the sums the reference adds to ``path_all_count``,
     ``hits_all``, ``point_all`` and ``path_all`` (main.py:158-191), with ``point = sum_L points_L / L`` and
-    ``path = sum_L edges_L / max(L - 1, 1)``.  No host synchronisation."""
+    ``path = sum_L edges_L / max(L - 1, 1)``.  ``[S, L, 4]`` counters give ``[S, 4]``.  No host synchronisation."""
     div = _TOTALS_DIV.get(counts.device)
-    if div is None or div.shape[0] != counts.shape[0]:
-        L = torch.arange(counts.shape[0], dtype=torch.float64)
+    if div is None or div.shape[0] != counts.shape[-2]:
+        L = torch.arange(counts.shape[-2], dtype=torch.float64)
         one = torch.ones_like(L)
         div = torch.stack([one, one, L.clamp(min=1), (L - 1).clamp(min=1)], 1).to(counts.device)
         _TOTALS_DIV[counts.device] = div
-    return (counts.double() / div).sum(0)
+    return (counts.double() / div).sum(-2)
+
+
+def hier_line(hit_ratio: float, path_ratio: float, point_ratio: float) -> str:
+    """The TOR / POR suffix of the reference's ``test()`` line (main.py:205-214), ratios in percent."""
+    return " hit_ratio(%):{:.2f} path_ratio(%):{:.2f} point_ratio(%):{:.2f}".format(hit_ratio, path_ratio, point_ratio)
 
 
 class HierMetrics:
-    """TOR / POR accumulators (main.py:123-127,152-191).  One fused call per batch (``hgr_hier_metrics_fused_rows``):
+    """TOR / POR counters (main.py:123-127,152-191).  One fused call per batch (``hgr_hier_metrics_fused_rows``):
     per-level arg-max over the train classes in the epilogue of the GEMM against the level-sorted train bank, then
-    chain matching and counting on the device into integer counters per chain length; the divisions by the chain
-    length stay device-side float ops, nothing is copied to the host before the ratios are printed.
+    chain matching and counting on the device into integer counters per chain length (``counts``), incremented in
+    place; nothing is copied to the host before the ratios are printed.
 
     ``update_rows`` scores every row against its own label and needs no host work per batch."""
 
     def __init__(self, model):
         self.model = model
         dev = model.device
-        # (rows, hits, point, path) -- the order of hier_totals: update_rows folds a batch in with one add
-        self._acc = torch.zeros(4, dtype=torch.float64, device=dev)
-        self.hits_all = self._acc[1]
-        self.point_all = self._acc[2]
-        self.path_all = self._acc[3]
+        self.counts = ops.new_hier_counts(dev)
         depth = torch.from_numpy(model.hierarchy.depth).to(torch.int64)
         self.n_levels = int(depth.max()) + 1 if depth.numel() else 1
         # Only the TRAIN columns enter TOR / POR (main.py:143,155,174): the GEMM runs against the train rows of the bank
@@ -118,12 +119,11 @@ class HierMetrics:
         self._bank_version = None
         self._train_ids = train.tolist()
         self._chains = None           # chain table of update_rows, built on first use
-        self._counts = None
 
     @property
     def path_all_count(self) -> int:
         """Rows scored so far (synchronises)."""
-        return int(self._acc[0])
+        return int(self.counts[:, 0].sum())
 
     def sorted_bank(self) -> torch.Tensor:
         """The train rows of the bank sorted by level; re-sorted when ``model.bank_train`` was refreshed (new tensor or
@@ -147,20 +147,20 @@ class HierMetrics:
         return dict(bank_sorted=self.sorted_bank(), level_end=self._level_end, sorted_to_pos=self._sorted_to_pos,
                     first_out=self._first_out, chain_ptr=chain_ptr, chain_pos=chain_pos, chain_level=chain_level)
 
-    def update_rows(self, x_norm: torch.Tensor, targets: torch.Tensor):
+    def update_rows(self, x_norm: torch.Tensor, targets: torch.Tensor, node_splits: Optional[torch.Tensor] = None,
+                    counts: Optional[torch.Tensor] = None):
         """Score a batch: ``x_norm`` [B, D] bf16 normalised image features, row i scored against the chain of node
         ``targets[i]``, so a batch may mix classes.  Rows whose target lies outside ``[0, n_nodes)`` are skipped
-        (padding).  No host work per batch and no synchronisation."""
-        if self._counts is None:
-            self._counts = ops.new_hier_counts(x_norm.device)
-        else:
-            self._counts.zero_()
-        ops.hier_metrics_fused_rows(x_norm, targets=targets.to(torch.int32), counts=self._counts, **self.rows_args())
-        self._acc += hier_totals(self._counts)
+        (padding).  Into ``counts`` (default: the object's own); with ``node_splits``, ``counts`` ``[S, 33, 4]`` takes
+        one set per split (``ops.hier_metrics_fused_rows``).  No host work per batch and no synchronisation."""
+        ops.hier_metrics_fused_rows(x_norm, targets=targets.to(torch.int32), node_splits=node_splits,
+                                    counts=self.counts if counts is None else counts, **self.rows_args())
 
     def ratios(self, num_sample):
-        return (float(self.hits_all) / num_sample * 100.0, float(self.path_all) / self.path_all_count * 100.0,
-                float(self.point_all) / num_sample * 100.0)
+        """``(hit_ratio, path_ratio, point_ratio)`` of the reference's line: TOR and POR over all ``num_sample`` rows,
+        the path ratio over the rows in the hierarchy (synchronises)."""
+        rows, hits, point, path = hier_totals(self.counts).tolist()
+        return hits / num_sample * 100.0, path / rows * 100.0, point / num_sample * 100.0
 
 
 def mistake_summary(counts, K: int = 20) -> dict:
@@ -196,15 +196,17 @@ class MistakeMetrics:
     the top-K lists of every batch: how far from the label in the hierarchy the predictions are, not only whether the
     label is among them (main.py:135-148).  Holds the chain table (``chain_csr`` of ``model.c2p``, on the device) and
     the counters, one set per list set; ``update`` counts a batch on the device (``ops.hier_mistakes``) with no host
-    synchronisation.  ``n_sets`` > 1 counts ``[n_sets, B, K]`` lists of several test splits (``SplitEval``)."""
+    synchronisation.  ``n_sets`` > 1 counts ``[n_sets, B, K]`` lists of several test splits (``SplitEval``).
+    ``counts``: the ``[n_sets, HGR_MISTAKE_COUNTERS]`` counters to own (default: new ones), e.g. a view of an
+    ``EvalCounters`` block."""
 
-    def __init__(self, model, n_sets: int = 1, K: int = 20):
+    def __init__(self, model, n_sets: int = 1, K: int = 20, counts: Optional[torch.Tensor] = None):
         dev = model.device
         ptr, nodes = chain_csr(model.c2p)
         self.chain_ptr = torch.from_numpy(ptr.astype(np.int32)).to(dev)
         self.chain_node = torch.from_numpy(nodes.astype(np.int32)).to(dev)
         self.n_sets, self.K = n_sets, K
-        self.counts = ops.new_mistake_counts(dev, n_sets)
+        self.counts = ops.new_mistake_counts(dev, n_sets) if counts is None else counts
 
     def args(self) -> dict:
         """The chain table arguments of ``ops.hier_mistakes``."""
@@ -261,20 +263,91 @@ def split_line(name, hits, rows, hier=None, mistakes=None):
     out_str, _ = count_acc(dict(zip(HIT_CUTS, hits)), rows)
     if hier is not None:
         tor, point, path, path_rows = hier
-        out_str += " hit_ratio(%):{:.2f}".format(tor / rows * 100.0)
-        out_str += " path_ratio(%):{:.2f}".format(path / path_rows * 100.0 if path_rows else 0.0)
-        out_str += " point_ratio(%):{:.2f}".format(point / rows * 100.0)
+        out_str += hier_line(tor / rows * 100.0, path / path_rows * 100.0 if path_rows else 0.0, point / rows * 100.0)
     if mistakes is not None:
         out_str += mistake_line(mistakes)
     return "{}: {}".format(name, out_str)
 
 
+class EvalCounters:
+    """The integer counters of one evaluator in ONE int64 device buffer (``counters``), and every value reported from
+    them.  Layout: ``hits [HGR_NUM_HITS]`` (Hit@{1,2,5,10,20}); with S splits ``split_counts [S, HGR_NUM_HITS + 1]``
+    (per split Hit@k and rows); with ``hier`` ``hier_counts [n, HGR_HIER_MAX_CHAIN + 1, 4]`` (TOR / POR per chain
+    length); with ``mistakes`` ``mistake_counts [n, HGR_MISTAKE_COUNTERS]`` -- n = S, or 1 without splits.  The
+    kernels increment the views in place, so nothing is zeroed per batch and a stream mirrors everything to the host
+    with one copy.  ``read(counters)`` gives the counters the readout reports, in the same layout (default: the
+    buffer itself): a stream synchronises its streams first, a class-sharded stream also sums them over ranks."""
+
+    def __init__(self, device, n_splits: int = 0, hier: bool = False, mistakes: bool = False, K: int = 20, read=None):
+        n = max(n_splits, 1)
+        self.S, self.K = n_splits, K
+        self._shapes = [(ops.HGR_NUM_HITS,), (n_splits, ops.HGR_NUM_HITS + 1),
+                        (n if hier else 0, HGR_HIER_MAX_CHAIN + 1, 4), (n if mistakes else 0, HGR_MISTAKE_COUNTERS)]
+        self.counters = torch.zeros(sum(int(np.prod(sh)) for sh in self._shapes), dtype=torch.int64, device=device)
+        self.hits, self.split_counts, self.hier_counts, self.mistake_counts = self._views(self.counters)
+        self._read = read
+
+    def _views(self, counters: torch.Tensor):
+        parts = torch.split(counters, [int(np.prod(sh)) for sh in self._shapes])
+        return tuple(p.view(sh) if p.numel() else None for p, sh in zip(parts, self._shapes))
+
+    def read(self):
+        """``(hits, split_counts, hier_counts, mistake_counts)`` to report, after the read step."""
+        return self._views(self.counters if self._read is None else self._read(self.counters))
+
+    def _need(self, what: str, have: bool):
+        if not have:
+            raise RuntimeError("the evaluator was built without %s" % what)
+
+    def hit_counts(self):
+        """Hit@{1,2,5,10,20} so far."""
+        return self.read()[0].tolist()
+
+    def split_hit_counts(self):
+        """Per split ``[Hit@1, @2, @5, @10, @20, rows]`` so far, in split order."""
+        self._need("splits", self.S > 0)
+        return self.read()[1].tolist()
+
+    def split_ratios(self):
+        """Per counter set ``(hit_ratio, path_ratio, point_ratio)`` in percent -- the TOR / POR of the reference's
+        ``test()`` line -- over the rows of the set whose label lies in the hierarchy (0 without rows)."""
+        self._need("TOR / POR counters", self.hier_counts is not None)
+        return [(0.0, 0.0, 0.0) if rows == 0 else (hits / rows * 100.0, path / rows * 100.0, point / rows * 100.0)
+                for rows, hits, point, path in hier_totals(self.read()[2]).tolist()]
+
+    def hier_ratios(self):
+        """``split_ratios`` of the one set without splits."""
+        self._need("TOR / POR counters without splits", self.S == 0)
+        return self.split_ratios()[0]
+
+    def mistake_summary(self):
+        """``mistake_summary`` of the one set without splits."""
+        self._need("mistake counters without splits", self.mistake_counts is not None and self.S == 0)
+        return mistake_summary(self.read()[3][0], self.K)
+
+    def split_mistake_summary(self):
+        """Per split ``mistake_summary`` over the rows whose label is in the split."""
+        self._need("per-split mistake counters", self.mistake_counts is not None and self.S > 0)
+        return [mistake_summary(c, self.K) for c in self.read()[3]]
+
+    def split_lines(self, names):
+        """One ``split_line`` per split: Hit@k, plus TOR / POR and the mistake metrics when counted."""
+        self._need("splits", self.S > 0)
+        _, counts, hier, mist = self.read()
+        hier = [None] * self.S if hier is None else [(tor, point, path, rows)
+                                                     for rows, tor, point, path in hier_totals(hier).tolist()]
+        mist = [None] * self.S if mist is None else [mistake_summary(c, self.K) for c in mist.tolist()]
+        return [split_line(name, c[:ops.HGR_NUM_HITS], max(c[ops.HGR_NUM_HITS], 1), h, m)
+                for name, c, h, m in zip(names, counts.tolist(), hier, mist)]
+
+
 class SplitEval:
     """Several test splits of one hierarchy scored in ONE pass per batch (``hgr_score_topk_splits``): the union bank is
-    built from ``model.zsl_weights`` in the group layout of ``split_groups`` and rebuilt after a bank refresh; the hit
-    counters of every split stay on the device.  With ``hier=True`` the TOR / POR counters of every split follow from
-    one level GEMM per batch (``hgr_hier_metrics_fused_rows_splits``).  With ``mistakes=True`` the mistake severity and
-    LCA distance@k of every split are counted from the ``[S, B, K]`` lists (``MistakeMetrics``, one set per split).
+    built from ``model.zsl_weights`` in the group layout of ``split_groups`` and rebuilt after a bank refresh; the
+    counters of every split stay on the device (``EvalCounters``: ``split_counts``, ``hier_counts``,
+    ``mistake_counts``).  With ``hier=True`` the TOR / POR counters of every split follow from one level GEMM per batch
+    (``HierMetrics.update_rows`` with ``node_splits``).  With ``mistakes=True`` the mistake severity and LCA
+    distance@k of every split are counted from the ``[S, B, K]`` lists (``MistakeMetrics``, one set per split).
     ``lines()`` gives one line per split."""
 
     def __init__(self, model, splits, hier: bool = True, K: int = 20, mistakes: bool = False):
@@ -287,11 +360,11 @@ class SplitEval:
         self._bank_nodes = torch.from_numpy(bank_nodes).to(dev)
         self.col_id = self._bank_nodes.to(torch.int32)
         self.node_splits = torch.from_numpy(node_splits).to(dev)
-        self.counts = torch.zeros((self.S, ops.HGR_NUM_HITS + 1), dtype=torch.int64, device=dev)
+        self.tally = EvalCounters(dev, n_splits=self.S, hier=hier, mistakes=mistakes, K=K)
+        self.split_counts, self.hier_counts = self.tally.split_counts, self.tally.hier_counts
+        self.mistake_counts = self.tally.mistake_counts
         self.hier = HierMetrics(model) if hier else None
-        self._hier_counts = None
-        self._hier_acc = torch.zeros((self.S, 4), dtype=torch.float64, device=dev)   # (rows, hits, point, path)
-        self.mistakes = MistakeMetrics(model, n_sets=self.S, K=K) if mistakes else None
+        self.mistakes = MistakeMetrics(model, n_sets=self.S, K=K, counts=self.mistake_counts) if mistakes else None
         self._bank = None
         self._bank_version = None
 
@@ -313,40 +386,22 @@ class SplitEval:
         the splits its label belongs to).  TOR / POR match row i against ``hier_targets[i]`` (default: ``targets``).
         Returns ``(val [S,B,K], idx [S,B,K])``.  No host synchronisation."""
         t = targets.to(torch.int32)
-        out = ops.score_topk_splits(x_norm, targets=t, counts=self.counts, **self.score_args())
+        out = ops.score_topk_splits(x_norm, targets=t, counts=self.split_counts, **self.score_args())
         if self.hier is not None:
-            if self._hier_counts is None:
-                self._hier_counts = torch.zeros((self.S, HGR_HIER_MAX_CHAIN + 1, 4), dtype=torch.int64,
-                                                device=x_norm.device)
-            else:
-                self._hier_counts.zero_()
-            ht = t if hier_targets is None else hier_targets.to(torch.int32)
-            ops.hier_metrics_fused_rows_splits(x_norm, targets=ht, node_splits=self.node_splits,
-                                               counts=self._hier_counts, **self.hier.rows_args())
-            self._hier_acc += torch.stack([hier_totals(c) for c in self._hier_counts])
+            self.hier.update_rows(x_norm, t if hier_targets is None else hier_targets, node_splits=self.node_splits,
+                                  counts=self.hier_counts)
         if self.mistakes is not None:
             self.mistakes.update(out[1], t, node_splits=self.node_splits)
         return out
 
     def hit_counts(self):
         """Per split ``[Hit@1, @2, @5, @10, @20, rows]`` so far (synchronises)."""
-        return self.counts.tolist()
+        return self.tally.split_hit_counts()
 
     def lines(self):
         """One line per split: ``name: Top@1(%):..., ... .`` plus TOR / POR with ``hier`` and the mistake metrics with
         ``mistakes`` (synchronises)."""
-        counts = self.counts.tolist()
-        acc = self._hier_acc.tolist()
-        mist = self.mistakes.summary() if self.mistakes is not None else [None] * self.S
-        out = []
-        for s, name in enumerate(self.names):
-            rows = counts[s][ops.HGR_NUM_HITS]
-            h = None
-            if self.hier is not None:
-                r, tor, point, path = acc[s]
-                h = (tor, point, path, r)
-            out.append(split_line(name, counts[s][:ops.HGR_NUM_HITS], max(rows, 1), h, mist[s]))
-        return out
+        return self.tally.split_lines(self.names)
 
 
 def test(opts, model, device, splits=None, loader: Optional[Iterable] = None, log: bool = True):
@@ -390,11 +445,7 @@ def test(opts, model, device, splits=None, loader: Optional[Iterable] = None, lo
     out_str = _format(hits, num_sample, hier, mist)
     print(out_str, flush=True)
     if log:
-        with open(model.save_path + "arugements.log", "a") as f:       # [sic] main.py:217
-            f.writelines(out_str + "\n")
-        with open("{}.txt".format(opts.weights), "a") as f:            # main.py:219-222
-            method = "{},{},{}:".format(opts.weights, opts.out_ratio, opts.in_ratio)
-            f.writelines(method + "\n" + out_str + "\n")
+        _log(opts, model, out_str)
     return out_str
 
 
@@ -416,25 +467,23 @@ def _test_splits(opts, model, device, splits, split_keys, loader, log):
     out_str = "\n" + "\n".join(se.lines())
     print(out_str, flush=True)
     if log:
-        with open(model.save_path + "arugements.log", "a") as f:       # [sic] main.py:217
-            f.writelines(out_str + "\n")
-        with open("{}.txt".format(opts.weights), "a") as f:            # main.py:219-222
-            method = "{},{},{}:".format(opts.weights, opts.out_ratio, opts.in_ratio)
-            f.writelines(method + "\n" + out_str + "\n")
+        _log(opts, model, out_str)
     return out_str
 
 
+def _log(opts, model, out_str):
+    with open(model.save_path + "arugements.log", "a") as f:           # [sic] main.py:217
+        f.writelines(out_str + "\n")
+    with open("{}.txt".format(opts.weights), "a") as f:                # main.py:219-222
+        method = "{},{},{}:".format(opts.weights, opts.out_ratio, opts.in_ratio)
+        f.writelines(method + "\n" + out_str + "\n")
+
+
 def _format(hits, num_sample, hier, mist=None):
-    h = hits.tolist()
-    hits_dict = dict(zip(HIT_CUTS, h))
-    out_str = "\n"
-    tmp_str, _ = count_acc(hits_dict, num_sample)
-    out_str += tmp_str
+    out_str, _ = count_acc(dict(zip(HIT_CUTS, hits.tolist())), num_sample)
+    out_str = "\n" + out_str
     if hier is not None:
-        hit_ratio, path_ratio, point_ratio = hier.ratios(num_sample)
-        out_str += " hit_ratio(%):{:.2f}".format(hit_ratio)
-        out_str += " path_ratio(%):{:.2f}".format(path_ratio)
-        out_str += " point_ratio(%):{:.2f}".format(point_ratio)
+        out_str += hier_line(*hier.ratios(num_sample))
     if mist is not None:
         out_str += mistake_line(mist.summary())
     return out_str

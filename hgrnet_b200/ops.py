@@ -551,24 +551,53 @@ def _hier_workspace(nbytes: int, device) -> torch.Tensor:
     return ws
 
 
-def new_hier_counts(device) -> torch.Tensor:
-    """Zeroed per-chain-length counters of ``hier_metrics_fused_rows``: int64 ``[HGR_HIER_MAX_CHAIN + 1, 4]``, bin L =
-    ``{rows, TOR hits, points, edges}`` of the rows whose label chain has L entries."""
-    return torch.zeros((HGR_HIER_MAX_CHAIN + 1, 4), dtype=torch.int64, device=device)
+def new_hier_counts(device, n_sets: Optional[int] = None) -> torch.Tensor:
+    """Zeroed per-chain-length counters of ``hier_metrics_fused_rows``: int64 ``[HGR_HIER_MAX_CHAIN + 1, 4]``, or
+    ``[n_sets, HGR_HIER_MAX_CHAIN + 1, 4]`` with ``n_sets``; bin L = ``{rows, TOR hits, points, edges}`` of the rows whose
+    label chain has L entries."""
+    shape = (HGR_HIER_MAX_CHAIN + 1, 4)
+    return torch.zeros(shape if n_sets is None else (n_sets, *shape), dtype=torch.int64, device=device)
+
+
+def _hier_sets(counts: torch.Tensor, node_splits: Optional[torch.Tensor], n_nodes: int):
+    """The counter sets of a TOR / POR call: ``counts`` ``[33, 4]`` or ``[S, 33, 4]`` (``new_hier_counts``), S > 1 only
+    with ``node_splits`` (uint8 per node).  Returns ``(S, node_splits)``."""
+    if not counts.is_cuda:
+        raise ValueError("counts must be a CUDA tensor: hgrnet_b200 has no CPU path")
+    if counts.dtype != torch.int64 or counts.dim() not in (2, 3) or tuple(counts.shape[-2:]) != (HGR_HIER_MAX_CHAIN + 1, 4) \
+            or not counts.is_contiguous():
+        raise ValueError("counts must be a contiguous int64 [%d, 4] or [S, %d, 4] tensor (new_hier_counts)"
+                         % (HGR_HIER_MAX_CHAIN + 1, HGR_HIER_MAX_CHAIN + 1))
+    S = counts.shape[0] if counts.dim() == 3 else 1
+    if node_splits is not None:
+        node_splits = _require(node_splits, "node_splits", torch.uint8)
+        if node_splits.numel() != n_nodes:
+            raise ValueError("node_splits must have one entry per node")
+    elif S != 1:
+        raise ValueError("%d counter sets need node_splits" % S)
+    return S, node_splits
+
+
+def _check_rows_out(lvl_idx, top1, B: int, n_levels: int) -> None:
+    for name, t, shape in (("lvl_idx", lvl_idx, (B, n_levels)), ("top1", top1, (B,))):
+        if t is not None and (t.dtype != torch.int32 or tuple(t.shape) != shape or not t.is_contiguous() or not t.is_cuda):
+            raise ValueError("%s must be a contiguous CUDA int32 %s tensor" % (name, list(shape)))
 
 
 def hier_metrics_fused_rows(x_norm: torch.Tensor, bank_sorted: torch.Tensor, level_end, sorted_to_pos: torch.Tensor,
                             first_out: torch.Tensor, targets: torch.Tensor, chain_ptr: torch.Tensor,
                             chain_pos: torch.Tensor, chain_level: torch.Tensor, counts: torch.Tensor,
-                            lvl_idx: Optional[torch.Tensor] = None, top1: Optional[torch.Tensor] = None) -> None:
+                            node_splits: Optional[torch.Tensor] = None, lvl_idx: Optional[torch.Tensor] = None,
+                            top1: Optional[torch.Tensor] = None) -> None:
     """TOR / POR counters (main.py:143,152-191) of one batch without the dense logits: ``bank_sorted`` holds the train
     rows of the bank sorted by level (``level_end``: host list of exclusive ends), the per-level arg-max runs in the
     epilogue of the tcgen05 GEMM.  Row i is matched against the chain of node ``targets[i]``, read from the chain table
     ``chain_ptr [n_nodes + 1]`` / ``chain_pos`` / ``chain_level`` (``evaluate.chain_table``).  Positions (chain_pos,
     first_out, lvl_idx, top1) are positions in ``train_index``.  ``counts`` (``new_hier_counts``) is incremented per
-    chain length; rows whose target is outside ``[0, n_nodes)`` are counted nowhere.  No host work depends on the
-    batch's contents, so the call can be captured in a CUDA graph.  See ``hgr_hier_metrics_fused_rows`` in the
-    header."""
+    chain length; rows whose target is outside ``[0, n_nodes)`` are counted nowhere.  With ``node_splits`` (uint8 per
+    node) ``counts`` may be ``[S, 33, 4]``: a row is added to set s for every bit s of ``node_splits[targets[row]]``,
+    from one GEMM whatever S is.  No host work depends on the batch's contents, so the call can be captured in a CUDA
+    graph.  See ``hgr_hier_metrics_fused_rows`` in the header."""
     import ctypes
     lib = _cabi.load()
     x_norm = _require(x_norm, "x_norm", torch.bfloat16)
@@ -579,64 +608,22 @@ def hier_metrics_fused_rows(x_norm: torch.Tensor, bank_sorted: torch.Tensor, lev
     chain_ptr = _require(chain_ptr, "chain_ptr", torch.int32)
     chain_pos = _require(chain_pos, "chain_pos", torch.int32)
     chain_level = _require(chain_level, "chain_level", torch.int32)
-    if not counts.is_cuda:
-        raise ValueError("counts must be a CUDA tensor: hgrnet_b200 has no CPU path")
-    if counts.dtype != torch.int64 or counts.numel() != (HGR_HIER_MAX_CHAIN + 1) * 4 or not counts.is_contiguous():
-        raise ValueError("counts must be a contiguous int64 [%d, 4] tensor (new_hier_counts)" % (HGR_HIER_MAX_CHAIN + 1))
+    n_nodes = chain_ptr.numel() - 1
+    S, node_splits = _hier_sets(counts, node_splits, n_nodes)
     B, D = x_norm.shape
     M = bank_sorted.shape[0]
     n_levels = len(level_end)
-    n_nodes = chain_ptr.numel() - 1
     if sorted_to_pos.numel() != M or first_out.numel() != n_levels or targets.numel() != B \
             or chain_pos.numel() != chain_level.numel():
         raise ValueError("hier_metrics_fused_rows: inconsistent sizes")
-    for name, t, shape in (("lvl_idx", lvl_idx, (B, n_levels)), ("top1", top1, (B,))):
-        if t is not None and (t.dtype != torch.int32 or tuple(t.shape) != shape or not t.is_contiguous() or not t.is_cuda):
-            raise ValueError("%s must be a contiguous CUDA int32 %s tensor" % (name, list(shape)))
+    _check_rows_out(lvl_idx, top1, B, n_levels)
     ends = (ctypes.c_int32 * n_levels)(*[int(e) for e in level_end])
     ws = _hier_workspace(B * n_levels * 8, x_norm.device)
     _cabi.check(lib.hgr_hier_metrics_fused_rows(_ptr(x_norm), _ptr(bank_sorted), B, M, D, ends, n_levels,
                                                 _ptr(sorted_to_pos), _ptr(first_out), _ptr(targets), n_nodes,
-                                                _ptr(chain_ptr), _ptr(chain_pos), _ptr(chain_level), _ptr(ws), ws.numel(),
-                                                _ptr(lvl_idx), _ptr(top1), _ptr(counts), _stream()))
-
-
-def hier_metrics_fused_rows_splits(x_norm: torch.Tensor, bank_sorted: torch.Tensor, level_end, sorted_to_pos: torch.Tensor,
-                                   first_out: torch.Tensor, targets: torch.Tensor, chain_ptr: torch.Tensor,
-                                   chain_pos: torch.Tensor, chain_level: torch.Tensor, node_splits: torch.Tensor,
-                                   counts: torch.Tensor) -> None:
-    """``hier_metrics_fused_rows`` with one counter set per split (``hgr_hier_metrics_fused_rows_splits``): ``counts``
-    int64 ``[S, HGR_HIER_MAX_CHAIN + 1, 4]``; a row is added to set s for every bit s of ``node_splits[targets[row]]``
-    (uint8 per node).  One GEMM per batch whatever S is."""
-    import ctypes
-    lib = _cabi.load()
-    x_norm = _require(x_norm, "x_norm", torch.bfloat16)
-    bank_sorted = _require(bank_sorted, "bank_sorted", torch.bfloat16)
-    sorted_to_pos = _require(sorted_to_pos, "sorted_to_pos", torch.int32)
-    first_out = _require(first_out, "first_out", torch.int32)
-    targets = _require(targets, "targets", torch.int32)
-    chain_ptr = _require(chain_ptr, "chain_ptr", torch.int32)
-    chain_pos = _require(chain_pos, "chain_pos", torch.int32)
-    chain_level = _require(chain_level, "chain_level", torch.int32)
-    node_splits = _require(node_splits, "node_splits", torch.uint8)
-    S = counts.shape[0] if counts.dim() == 3 else -1
-    if not counts.is_cuda or counts.dtype != torch.int64 or tuple(counts.shape[1:]) != (HGR_HIER_MAX_CHAIN + 1, 4) \
-            or not counts.is_contiguous():
-        raise ValueError("counts must be a contiguous CUDA int64 [S, %d, 4] tensor" % (HGR_HIER_MAX_CHAIN + 1))
-    B, D = x_norm.shape
-    M = bank_sorted.shape[0]
-    n_levels = len(level_end)
-    n_nodes = chain_ptr.numel() - 1
-    if sorted_to_pos.numel() != M or first_out.numel() != n_levels or targets.numel() != B \
-            or chain_pos.numel() != chain_level.numel() or node_splits.numel() != n_nodes:
-        raise ValueError("hier_metrics_fused_rows_splits: inconsistent sizes")
-    ends = (ctypes.c_int32 * n_levels)(*[int(e) for e in level_end])
-    ws = _hier_workspace(B * n_levels * 8, x_norm.device)
-    _cabi.check(lib.hgr_hier_metrics_fused_rows_splits(_ptr(x_norm), _ptr(bank_sorted), B, M, D, ends, n_levels,
-                                                       _ptr(sorted_to_pos), _ptr(first_out), _ptr(targets), n_nodes,
-                                                       _ptr(chain_ptr), _ptr(chain_pos), _ptr(chain_level),
-                                                       _ptr(node_splits), S, _ptr(ws), ws.numel(), _ptr(counts),
-                                                       _stream()))
+                                                _ptr(chain_ptr), _ptr(chain_pos), _ptr(chain_level), _ptr(node_splits),
+                                                S, _ptr(ws), ws.numel(), _ptr(lvl_idx), _ptr(top1), _ptr(counts),
+                                                _stream()))
 
 
 def hier_level_scatter(x_norm: torch.Tensor, bank_shard: torch.Tensor, level_end_local, row_base: int, dst_block_ptrs,
@@ -666,12 +653,13 @@ def hier_level_scatter(x_norm: torch.Tensor, bank_shard: torch.Tensor, level_end
 def hier_finish_rows_gathered(parts_ptr: int, n_parts: int, part_stride: int, n_rows: int, M: int, n_levels: int,
                               sorted_to_pos: torch.Tensor, first_out: torch.Tensor, targets: torch.Tensor,
                               chain_ptr: torch.Tensor, chain_pos: torch.Tensor, chain_level: torch.Tensor,
-                              counts: torch.Tensor, lvl_idx: Optional[torch.Tensor] = None,
-                              top1: Optional[torch.Tensor] = None) -> None:
+                              counts: torch.Tensor, node_splits: Optional[torch.Tensor] = None,
+                              lvl_idx: Optional[torch.Tensor] = None, top1: Optional[torch.Tensor] = None) -> None:
     """Owner half of class-sharded TOR / POR (``hgr_hier_finish_rows_gathered``): for ``n_rows`` rows, the max over the
     ``n_parts`` shards' winner words at ``parts_ptr`` (``part_stride`` words apart, e.g. a peer-exchange slot), then
     what ``hier_metrics_fused_rows`` does with its own words.  ``targets`` / ``lvl_idx`` / ``top1`` cover these rows;
-    ``M``, ``sorted_to_pos``, ``first_out`` and the chain table are the global ones."""
+    ``M``, ``sorted_to_pos``, ``first_out`` and the chain table are the global ones; ``counts`` / ``node_splits`` as in
+    ``hier_metrics_fused_rows``."""
     lib = _cabi.load()
     sorted_to_pos = _require(sorted_to_pos, "sorted_to_pos", torch.int32)
     first_out = _require(first_out, "first_out", torch.int32)
@@ -679,46 +667,16 @@ def hier_finish_rows_gathered(parts_ptr: int, n_parts: int, part_stride: int, n_
     chain_ptr = _require(chain_ptr, "chain_ptr", torch.int32)
     chain_pos = _require(chain_pos, "chain_pos", torch.int32)
     chain_level = _require(chain_level, "chain_level", torch.int32)
-    if not counts.is_cuda or counts.dtype != torch.int64 or counts.numel() != (HGR_HIER_MAX_CHAIN + 1) * 4 \
-            or not counts.is_contiguous():
-        raise ValueError("counts must be a contiguous CUDA int64 [%d, 4] tensor (new_hier_counts)" % (HGR_HIER_MAX_CHAIN + 1))
+    n_nodes = chain_ptr.numel() - 1
+    S, node_splits = _hier_sets(counts, node_splits, n_nodes)
     if sorted_to_pos.numel() != M or first_out.numel() != n_levels or targets.numel() != n_rows \
             or chain_pos.numel() != chain_level.numel():
         raise ValueError("hier_finish_rows_gathered: inconsistent sizes")
-    for name, t, shape in (("lvl_idx", lvl_idx, (n_rows, n_levels)), ("top1", top1, (n_rows,))):
-        if t is not None and (t.dtype != torch.int32 or tuple(t.shape) != shape or not t.is_contiguous() or not t.is_cuda):
-            raise ValueError("%s must be a contiguous CUDA int32 %s tensor" % (name, list(shape)))
+    _check_rows_out(lvl_idx, top1, n_rows, n_levels)
     _cabi.check(lib.hgr_hier_finish_rows_gathered(parts_ptr, n_parts, part_stride, n_rows, M, n_levels, _ptr(sorted_to_pos),
-                                                  _ptr(first_out), _ptr(targets), chain_ptr.numel() - 1, _ptr(chain_ptr),
-                                                  _ptr(chain_pos), _ptr(chain_level), _ptr(lvl_idx), _ptr(top1),
-                                                  _ptr(counts), _stream()))
-
-
-def hier_finish_rows_gathered_splits(parts_ptr: int, n_parts: int, part_stride: int, n_rows: int, M: int, n_levels: int,
-                                     sorted_to_pos: torch.Tensor, first_out: torch.Tensor, targets: torch.Tensor,
-                                     chain_ptr: torch.Tensor, chain_pos: torch.Tensor, chain_level: torch.Tensor,
-                                     node_splits: torch.Tensor, counts: torch.Tensor) -> None:
-    """``hier_finish_rows_gathered`` with one counter set per split (``hgr_hier_finish_rows_gathered_splits``):
-    ``counts`` int64 ``[S, HGR_HIER_MAX_CHAIN + 1, 4]`` as in ``hier_metrics_fused_rows_splits``."""
-    lib = _cabi.load()
-    sorted_to_pos = _require(sorted_to_pos, "sorted_to_pos", torch.int32)
-    first_out = _require(first_out, "first_out", torch.int32)
-    targets = _require(targets, "targets", torch.int32)
-    chain_ptr = _require(chain_ptr, "chain_ptr", torch.int32)
-    chain_pos = _require(chain_pos, "chain_pos", torch.int32)
-    chain_level = _require(chain_level, "chain_level", torch.int32)
-    node_splits = _require(node_splits, "node_splits", torch.uint8)
-    if not counts.is_cuda or counts.dtype != torch.int64 or counts.dim() != 3 \
-            or tuple(counts.shape[1:]) != (HGR_HIER_MAX_CHAIN + 1, 4) or not counts.is_contiguous():
-        raise ValueError("counts must be a contiguous CUDA int64 [S, %d, 4] tensor" % (HGR_HIER_MAX_CHAIN + 1))
-    n_nodes = chain_ptr.numel() - 1
-    if sorted_to_pos.numel() != M or first_out.numel() != n_levels or targets.numel() != n_rows \
-            or chain_pos.numel() != chain_level.numel() or node_splits.numel() != n_nodes:
-        raise ValueError("hier_finish_rows_gathered_splits: inconsistent sizes")
-    _cabi.check(lib.hgr_hier_finish_rows_gathered_splits(parts_ptr, n_parts, part_stride, n_rows, M, n_levels,
-                                                         _ptr(sorted_to_pos), _ptr(first_out), _ptr(targets), n_nodes,
-                                                         _ptr(chain_ptr), _ptr(chain_pos), _ptr(chain_level),
-                                                         _ptr(node_splits), counts.shape[0], _ptr(counts), _stream()))
+                                                  _ptr(first_out), _ptr(targets), n_nodes, _ptr(chain_ptr),
+                                                  _ptr(chain_pos), _ptr(chain_level), _ptr(node_splits), S,
+                                                  _ptr(lvl_idx), _ptr(top1), _ptr(counts), _stream()))
 
 
 def new_mistake_counts(device, n_sets: int = 1) -> torch.Tensor:

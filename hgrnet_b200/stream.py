@@ -41,7 +41,7 @@ from typing import Optional
 import torch
 
 from . import ops
-from ._cabi import HGR_HIER_MAX_CHAIN
+from .evaluate import EvalCounters
 
 
 class EvalStream:
@@ -75,35 +75,27 @@ class EvalStream:
 
         self.dev_pack = [torch.zeros(nbytes, dtype=torch.uint8, device=self.device) for _ in range(slots)]
         self.dev_feats, self.dev_labels = map(list, zip(*[views(p) for p in self.dev_pack]))
-        # hit counters, then (with hier) the per-chain-length TOR / POR counters: one buffer, one D2H copy per step
+        # every counter of the stream in one device buffer (evaluate.EvalCounters): one D2H copy per step
+        if hier is not None and splits is not None:
+            raise ValueError("splits and hier together: the splits' TOR / POR come with the SplitEval's hier")
         self.hier = hier
-        self._hier_args = hier.rows_args() if hier is not None else None
         self.splits = splits
-        self._split_args = splits.score_args() if splits is not None else None
-        self._split_hier_args = splits.hier.rows_args() if splits is not None and splits.hier is not None else None
-        n_hier = 0 if hier is None else (HGR_HIER_MAX_CHAIN + 1) * 4
-        n_split = 0 if splits is None else splits.S * (ops.HGR_NUM_HITS + 1)
-        n_split_hier = 0 if self._split_hier_args is None else splits.S * (HGR_HIER_MAX_CHAIN + 1) * 4
         self.mistakes = mistakes
+        self._split_args = splits.score_args() if splits is not None else None
+        hier = hier if splits is None else splits.hier
+        self._hier_args = hier.rows_args() if hier is not None else None
         self._mistake_args = mistakes.args() if mistakes is not None else None
-        n_mist = 0 if mistakes is None else (1 if splits is None else splits.S) * ops.HGR_MISTAKE_COUNTERS
-        n_counters = ops.HGR_NUM_HITS + n_hier + n_split + n_split_hier + n_mist
+        self._node_splits = None if splits is None else splits.node_splits
+        self.tally = EvalCounters(self.device, n_splits=0 if splits is None else splits.S, hier=hier is not None,
+                                  mistakes=mistakes is not None, K=K, read=self._read_counters)
+        self.counters, self.hits = self.tally.counters, self.tally.hits
+        self.split_counts, self.hier_counts = self.tally.split_counts, self.tally.hier_counts
+        self.mistake_counts = self.tally.mistake_counts
         if host_io:
             self.host_pack = [torch.zeros(nbytes, dtype=torch.uint8).pin_memory() for _ in range(slots)]
             self.host_feats, self.host_labels = map(list, zip(*[views(p) for p in self.host_pack]))
-            self.host_counters = torch.zeros(n_counters, dtype=torch.int64).pin_memory()
+            self.host_counters = torch.zeros(self.counters.numel(), dtype=torch.int64).pin_memory()
             self.host_hits = self.host_counters[:ops.HGR_NUM_HITS]
-        self.counters = torch.zeros(n_counters, dtype=torch.int64, device=self.device)
-        self.hits = self.counters[:ops.HGR_NUM_HITS]
-        o = ops.HGR_NUM_HITS
-        self.hier_counts = self.counters[o:o + n_hier].view(HGR_HIER_MAX_CHAIN + 1, 4) if hier is not None else None
-        o += n_hier
-        self.split_counts = self.counters[o:o + n_split].view(-1, ops.HGR_NUM_HITS + 1) if n_split else None
-        o += n_split
-        self.split_hier_counts = (self.counters[o:o + n_split_hier].view(-1, HGR_HIER_MAX_CHAIN + 1, 4)
-                                  if n_split_hier else None)
-        o += n_split_hier
-        self.mistake_counts = self.counters[o:o + n_mist].view(-1, ops.HGR_MISTAKE_COUNTERS) if n_mist else None
         self.val = [None] * slots
         self.idx = [None] * slots
         self.streams = [torch.cuda.Stream(device=self.device) for _ in range(max(1, min(streams, slots)))]
@@ -125,14 +117,12 @@ class EvalStream:
         else:                                                                        # the same, once per test split
             self.val[s], self.idx[s] = ops.score_topk_splits(x, targets=self.dev_labels[s], counts=self.split_counts,
                                                              **self._split_args)
-            if self._split_hier_args is not None:
-                ops.hier_metrics_fused_rows_splits(x, targets=self.dev_labels[s], node_splits=self.splits.node_splits,
-                                                   counts=self.split_hier_counts, **self._split_hier_args)
         if self._hier_args is not None:                                              # main.py:143,152-191
-            ops.hier_metrics_fused_rows(x, targets=self.dev_labels[s], counts=self.hier_counts, **self._hier_args)
+            ops.hier_metrics_fused_rows(x, targets=self.dev_labels[s], counts=self.hier_counts,
+                                        node_splits=self._node_splits, **self._hier_args)
         if self._mistake_args is not None:                                           # main.py:135-148, hierarchy distance
-            ops.hier_mistakes(self.idx[s], self.dev_labels[s], counts=self.mistake_counts,
-                              node_splits=None if self.splits is None else self.splits.node_splits, **self._mistake_args)
+            ops.hier_mistakes(self.idx[s], self.dev_labels[s], counts=self.mistake_counts, node_splits=self._node_splits,
+                              **self._mistake_args)
         if self.host_io:
             self.host_counters.copy_(self.counters, non_blocking=True)
 
@@ -180,61 +170,37 @@ class EvalStream:
         for st in self.streams:
             st.synchronize()
 
+    # ------------------------------------------------------------------ readout (evaluate.EvalCounters)
+    def _read_counters(self, counters):
+        # the per-step D2H copies of several streams land in the same bytes in no particular order: read the device
+        # counters once every stream is idle
+        self.synchronize()
+        return counters
+
     def hit_counts(self):
         """Hit@{1,2,5,10,20} so far (synchronises)."""
-        self.synchronize()
-        # (the per-step D2H copies of several streams land in the same 40 bytes in no particular order: read the
-        # counters once more now that every stream is idle)
-        return self.hits.tolist()
+        return self.tally.hit_counts()
 
     def hier_ratios(self):
         """``(hit_ratio, path_ratio, point_ratio)`` in percent -- the TOR / POR of the reference's ``test()`` line -- over
         the rows scored so far whose label lies in the hierarchy (synchronises).  Needs ``hier``."""
-        if self.hier is None:
-            raise RuntimeError("EvalStream was built without hier metrics (pass hier=HierMetrics(model))")
-        from .evaluate import hier_totals
-        self.synchronize()
-        rows, hits, point, path = hier_totals(self.hier_counts).tolist()
-        if rows == 0:
-            return 0.0, 0.0, 0.0
-        return hits / rows * 100.0, path / rows * 100.0, point / rows * 100.0
+        return self.tally.hier_ratios()
 
     def split_hit_counts(self):
-        """Per split ``[Hit@1, @2, @5, @10, @20, rows]`` so far, in the order of ``splits.names`` (synchronises).
-        Needs ``splits``."""
-        if self.splits is None:
-            raise RuntimeError("EvalStream was built without splits (pass splits=SplitEval(model, {...}))")
-        self.synchronize()
-        return self.split_counts.tolist()
+        """Per split ``[Hit@1, @2, @5, @10, @20, rows]`` so far, in the order of ``splits.names`` (synchronises)."""
+        return self.tally.split_hit_counts()
 
     def split_ratios(self):
         """Per split ``(hit_ratio, path_ratio, point_ratio)`` in percent over the rows whose label is in the split
         (synchronises).  Needs ``splits`` with TOR / POR."""
-        if self.split_hier_counts is None:
-            raise RuntimeError("EvalStream was built without per-split TOR / POR (SplitEval(..., hier=True))")
-        from .evaluate import hier_totals
-        self.synchronize()
-        out = []
-        for c in self.split_hier_counts:
-            rows, hits, point, path = hier_totals(c).tolist()
-            out.append((0.0, 0.0, 0.0) if rows == 0 else (hits / rows * 100.0, path / rows * 100.0, point / rows * 100.0))
-        return out
+        return self.tally.split_ratios()
 
     def mistake_summary(self):
         """``evaluate.mistake_summary`` of the rows scored so far (synchronises).  Needs ``mistakes`` without
         ``splits``."""
-        if self.mistake_counts is None or self.splits is not None:
-            raise RuntimeError("EvalStream was built without mistakes=MistakeMetrics(model), or with splits "
-                               "(use split_mistake_summary)")
-        from .evaluate import mistake_summary
-        self.synchronize()
-        return mistake_summary(self.mistake_counts[0], self.K)
+        return self.tally.mistake_summary()
 
     def split_mistake_summary(self):
         """Per split ``evaluate.mistake_summary`` over the rows whose label is in the split, in the order of
         ``splits.names`` (synchronises).  Needs ``mistakes`` and ``splits``."""
-        if self.mistake_counts is None or self.splits is None:
-            raise RuntimeError("EvalStream was built without per-split mistake metrics (pass splits= and mistakes=)")
-        from .evaluate import mistake_summary
-        self.synchronize()
-        return [mistake_summary(c, self.K) for c in self.mistake_counts]
+        return self.tally.split_mistake_summary()

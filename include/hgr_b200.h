@@ -294,6 +294,9 @@ int hgr_logits_dense(const void* X, const void* bank, int64_t B, int64_t C, int6
  *               chain[k]}), points (#{k: lvl[chain_level[k]] == chain[k]}), edges (#{k: matches at k and k+1}; L == 1:
  *               match[0])} of the rows whose chain has L entries (bin 0 stays zero).  The reference's totals follow on
  *               the host: hits = sum_L tor_L, path = sum_L edges_L / max(L-1, 1), point = sum_L points_L / L.
+ *  node_splits  NULL: n_sets must be 1 and counts is as above.  Otherwise [n_nodes] uint8 and 1 <= n_sets <= 8: counts
+ *               is [n_sets][HGR_HIER_MAX_CHAIN + 1][4] and a row is added to set s for every bit s of
+ *               node_splits[targets[row]] (main.py:143,152-191 run once per test split, from one GEMM per batch)
  * A row whose target lies outside [0, n_nodes), or whose chain length lies outside [1, HGR_HIER_MAX_CHAIN], is counted
  * nowhere (its lvl_idx / top1 are still written): callers pad a fixed-shape batch with target -1.
  * Ties: first position in train_index (the CPU arg-max rule; torch's CUDA top-k leaves it unspecified).
@@ -303,8 +306,8 @@ int hgr_hier_metrics_fused_rows(const void* X, const void* bank_sorted, int64_t 
                                 const int32_t* level_end, int n_levels, const int32_t* sorted_to_pos,
                                 const int32_t* first_out, const int32_t* targets, int64_t n_nodes,
                                 const int32_t* chain_ptr, const int32_t* chain_pos, const int32_t* chain_level,
-                                void* workspace, size_t workspace_bytes, int32_t* lvl_idx, int32_t* top1,
-                                int64_t* counts, void* stream);
+                                const uint8_t* node_splits, int n_sets, void* workspace, size_t workspace_bytes,
+                                int32_t* lvl_idx, int32_t* top1, int64_t* counts, void* stream);
 
 /*
  * Several test splits of one hierarchy in ONE scoring pass (the reference prints one line per run of main.py:104-222
@@ -335,19 +338,6 @@ int hgr_score_topk_splits(const void* X, const void* bank, const int32_t* col_id
                           int impl, void* stream);
 
 /*
- * hgr_hier_metrics_fused_rows with the counters of every split (main.py:143,152-191 run once per split): the same GEMM
- * and row decoding, once per batch, and each row is added to counter set s for every bit s of node_splits[targets[row]]
- * (a row outside the hierarchy nowhere).  counts [n_splits][HGR_HIER_MAX_CHAIN + 1][4] int64, incremented; n_splits
- * <= 8.  workspace as hgr_hier_metrics_fused_rows.
- */
-int hgr_hier_metrics_fused_rows_splits(const void* X, const void* bank_sorted, int64_t B, int64_t M, int64_t D,
-                                       const int32_t* level_end, int n_levels, const int32_t* sorted_to_pos,
-                                       const int32_t* first_out, const int32_t* targets, int64_t n_nodes,
-                                       const int32_t* chain_ptr, const int32_t* chain_pos, const int32_t* chain_level,
-                                       const uint8_t* node_splits, int n_splits, void* workspace, size_t workspace_bytes,
-                                       int64_t* counts, void* stream);
-
-/*
  * hgr_hier_metrics_fused_rows for the CLASS-SHARDED head (main.py:143,152-191): the level-sorted train bank [M, D] is
  * cut into contiguous row ranges, one per rank, and image rows are owned block-wise as in hgr_score_topk_scatter.  The
  * result is bit-identical to hgr_hier_metrics_fused_rows on the whole batch on one GPU: a winner word is
@@ -368,7 +358,8 @@ int hgr_hier_metrics_fused_rows_splits(const void* X, const void* bank_sorted, i
  *                                 part_stride + row * n_levels + level] (part_stride in words), then the decode, -1
  *                                 rule, tie rule and chain matching of hgr_hier_metrics_fused_rows.  targets, lvl_idx,
  *                                 top1 cover the owner's rows; M, sorted_to_pos, first_out and the chain table are the
- *                                 GLOBAL ones; counts as hgr_hier_metrics_fused_rows.  parts is only read.
+ *                                 GLOBAL ones; node_splits / n_sets / counts as hgr_hier_metrics_fused_rows.  parts
+ *                                 is only read.
  */
 int hgr_hier_level_scatter(const void* X, const void* bank_shard, int64_t B, int64_t M_r, int64_t D,
                            const int32_t* level_end_local, int n_levels, int64_t row_base, void* workspace,
@@ -377,8 +368,8 @@ int hgr_hier_level_scatter(const void* X, const void* bank_shard, int64_t B, int
 int hgr_hier_finish_rows_gathered(const uint64_t* parts, int n_parts, int64_t part_stride, int64_t n_rows, int64_t M,
                                   int n_levels, const int32_t* sorted_to_pos, const int32_t* first_out,
                                   const int32_t* targets, int64_t n_nodes, const int32_t* chain_ptr,
-                                  const int32_t* chain_pos, const int32_t* chain_level, int32_t* lvl_idx, int32_t* top1,
-                                  int64_t* counts, void* stream);
+                                  const int32_t* chain_pos, const int32_t* chain_level, const uint8_t* node_splits,
+                                  int n_sets, int32_t* lvl_idx, int32_t* top1, int64_t* counts, void* stream);
 
 /*
  * Several test splits in one scoring pass on the CLASS-SHARDED head (main.py:104-222 run once per split, as
@@ -414,9 +405,6 @@ int hgr_hier_finish_rows_gathered(const uint64_t* parts, int n_parts, int64_t pa
  *                                 in hgr_score_topk_splits (optional); *repair_count (optional) counts (row, split) pairs
  *                                 repaired.  split_stride >= 2 * P * part_stride + P * bound_stride: a split's
  *                                 value lists, id lists and bounds all sit at + s * split_stride.
- * hgr_hier_finish_rows_gathered_splits   hgr_hier_finish_rows_gathered with the counters of every split: counts
- *                                 [n_splits][HGR_HIER_MAX_CHAIN + 1][4], a row added to set s for every bit s of
- *                                 node_splits[targets[row]] (hgr_hier_metrics_fused_rows_splits); no lvl_idx / top1.
  */
 size_t hgr_score_topk_splits_scatter_bounded_workspace_bytes(int64_t B, int64_t C, int64_t D, int K, int n_groups,
                                                              const int32_t* group_end);
@@ -435,11 +423,6 @@ int hgr_topk_merge_splits_certified(const float* part_val, const int32_t* part_i
                                     int64_t n_nodes, float* topk_val, int32_t* topk_idx, int64_t* counts, const void* X,
                                     int64_t D, const hgr_shard_t* shards, float scale, unsigned int* repair_count,
                                     void* stream);
-int hgr_hier_finish_rows_gathered_splits(const uint64_t* parts, int n_parts, int64_t part_stride, int64_t n_rows,
-                                         int64_t M, int n_levels, const int32_t* sorted_to_pos, const int32_t* first_out,
-                                         const int32_t* targets, int64_t n_nodes, const int32_t* chain_ptr,
-                                         const int32_t* chain_pos, const int32_t* chain_level, const uint8_t* node_splits,
-                                         int n_splits, int64_t* counts, void* stream);
 
 /*
  * Hierarchical mistake severity and LCA distance@k (Bertinetto et al., "Making Better Mistakes", CVPR 2020) of top-K

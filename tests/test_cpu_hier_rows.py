@@ -2,6 +2,7 @@
 the per-batch Python chain, and the per-chain-length counters -> reference totals arithmetic."""
 from __future__ import annotations
 
+import ctypes
 import os
 import re
 import time
@@ -102,9 +103,62 @@ def test_hier_max_chain_matches_header():
     assert int(re.search(r"#define HGR_HIER_MAX_CHAIN (\d+)", header).group(1)) == _cabi.HGR_HIER_MAX_CHAIN == 32
 
 
+@pytest.mark.parametrize("node_splits, n_sets", [(None, 0), (None, 2), (0x60000, 0), (0x60000, 9)])
+def test_hier_rows_rejects_bad_counter_sets(node_splits, n_sets):
+    """One counter set without node_splits, 1..8 with them: refused before any CUDA call (fake device pointers)."""
+    from hgrnet_b200 import _cabi
+    lib = _cabi.load()
+    p = 0x10000
+    ends = (ctypes.c_int32 * 2)(10, 40)
+    assert lib.hgr_hier_metrics_fused_rows(p, p, 64, 40, 128, ends, 2, p, p, p, 600, p, p, p, node_splits, n_sets, p,
+                                           64 * 2 * 8, None, None, p, None) == -1
+    assert "counter sets" in lib.hgr_last_error().decode()
+
+
+def test_new_hier_counts_shapes():
+    from hgrnet_b200 import ops
+    assert tuple(ops.new_hier_counts("cpu").shape) == (ops.HGR_HIER_MAX_CHAIN + 1, 4)
+    assert tuple(ops.new_hier_counts("cpu", 3).shape) == (3, ops.HGR_HIER_MAX_CHAIN + 1, 4)
+
+
 def test_hier_rows_refuses_cpu_tensors():
     from hgrnet_b200 import ops
     z = lambda *s, dt=torch.int32: torch.zeros(*s, dtype=dt)
     with pytest.raises(ValueError, match="no CPU path"):
         ops.hier_metrics_fused_rows(z(4, 64, dt=torch.bfloat16), z(8, 64, dt=torch.bfloat16), [8], z(8), z(1), z(4),
                                     z(9), z(8), z(8), ops.new_hier_counts("cpu"))
+
+
+def test_eval_counters_layout_and_readout():
+    """``EvalCounters``: hits, then per-split hits, then TOR / POR sets, then mistake sets in one int64 buffer (the
+    byte layout the streams mirror to the host), and the ratios / lines derived from it."""
+    from hgrnet_b200 import ops
+    from hgrnet_b200.evaluate import EvalCounters, hier_line, split_line
+    H, NH, MC = (ops.HGR_HIER_MAX_CHAIN + 1) * 4, ops.HGR_NUM_HITS, ops.HGR_MISTAKE_COUNTERS
+    one = EvalCounters("cpu", hier=True, mistakes=True)
+    assert one.counters.numel() == NH + H + MC and one.split_counts is None
+    assert one.hier_counts.shape == (1, ops.HGR_HIER_MAX_CHAIN + 1, 4) and one.mistake_counts.shape == (1, MC)
+    assert one.hier_counts.data_ptr() == one.counters[NH:].data_ptr()
+    one.hier_counts[0, 3] = torch.tensor([4, 2, 6, 4])             # 4 rows with 3-entry chains
+    assert one.hier_ratios() == (50.0, 50.0, 50.0)
+    assert EvalCounters("cpu", hier=True).hier_ratios() == (0.0, 0.0, 0.0)
+    with pytest.raises(RuntimeError):
+        one.split_hit_counts()
+    S = 3
+    read = []
+    c = EvalCounters("cpu", n_splits=S, hier=True, read=lambda x: read.append(1) or 2 * x)
+    assert c.counters.numel() == NH + S * (NH + 1) + S * H and c.mistake_counts is None
+    assert c.split_counts.data_ptr() == c.counters[NH:].data_ptr()
+    assert c.hier_counts.data_ptr() == c.counters[NH + S * (NH + 1):].data_ptr()
+    c.split_counts[1] = torch.tensor([1, 2, 3, 4, 5, 10])
+    c.hier_counts[1, 1] = torch.tensor([5, 1, 2, 3])               # single-node chains: path = edges
+    assert c.split_hit_counts()[1] == [2, 4, 6, 8, 10, 20]         # through the read step
+    assert c.split_ratios()[1] == (20.0, 60.0, 40.0) and c.split_ratios()[0] == (0.0, 0.0, 0.0)
+    lines = c.split_lines(["a", "b", "c"])
+    assert lines[1] == split_line("b", [2, 4, 6, 8, 10], 20, (2.0, 4.0, 6.0, 10.0))
+    assert lines[1].endswith(hier_line(10.0, 60.0, 20.0)) and lines[0].startswith("a: Top@1(%):0.00")
+    with pytest.raises(RuntimeError):
+        c.hier_ratios()
+    with pytest.raises(RuntimeError):
+        c.split_mistake_summary()
+    assert len(read) == 4                                           # one read step per readout

@@ -125,19 +125,24 @@ def test_level_scatter_empty_shard_needs_no_bank():
 
 def _finish_call(**kw):
     from hgrnet_b200 import _cabi
-    a = dict(parts=0x10000, n_parts=4, stride=16 * 12, n_rows=16, M=500, n_levels=12, nodes=600)
+    a = dict(parts=0x10000, n_parts=4, stride=16 * 12, n_rows=16, M=500, n_levels=12, nodes=600, node_splits=None,
+             n_sets=1)
     a.update(kw)
     p = 0x50000
     return _cabi.load().hgr_hier_finish_rows_gathered(a["parts"], a["n_parts"], a["stride"], a["n_rows"], a["M"],
-                                                        a["n_levels"], p, p, p, a["nodes"], p, p, p, None, None, p, None)
+                                                        a["n_levels"], p, p, p, a["nodes"], p, p, p, a["node_splits"],
+                                                        a["n_sets"], None, None, p, None)
 
 
 @pytest.mark.parametrize("bad", [dict(n_parts=0), dict(n_parts=17), dict(stride=16 * 12 - 1), dict(n_levels=0),
                                  dict(n_levels=33), dict(M=0), dict(nodes=0), dict(parts=None), dict(parts=0x10004),
-                                 dict(n_rows=-1)])
-def test_finish_gathered_rejects_bad_arguments(bad):
+                                 dict(n_rows=-1), dict(n_sets=0), dict(n_sets=2),
+                                 dict(node_splits=0x60000, n_sets=0), dict(node_splits=0x60000, n_sets=9),
+                                 dict(node_splits=0x60000, n_sets=3, n_rows=-1)])
+def test_finish_gathered_rejects_bad_arguments_and_counter_sets(bad):
     assert _finish_call(**bad) == HGR_ERR_BAD_ARG
 
 
-def test_finish_gathered_zero_rows_is_a_no_op():
+def test_finish_gathered_zero_rows_is_a_no_op_for_any_counter_sets():
     assert _finish_call(n_rows=0, parts=None) == 0
+    assert _finish_call(n_rows=0, parts=None, node_splits=0x60000, n_sets=8) == 0

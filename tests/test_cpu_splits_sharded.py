@@ -143,13 +143,18 @@ def test_split_global_list_len_cfg5():
         4096, 2731, 1024, 20, 21841)
 
 
-def test_new_symbols_are_exported():
+def test_split_symbols_are_exported_and_tor_por_merged():
     from hgrnet_b200 import _cabi
     lib = _cabi.load()
     for name in ("hgr_score_topk_splits_scatter_bounded", "hgr_score_topk_splits_scatter_bounded_workspace_bytes",
                  "hgr_score_topk_splits_global_list_len", "hgr_topk_merge_splits_certified",
-                 "hgr_hier_finish_rows_gathered_splits"):
+                 "hgr_hier_finish_rows_gathered", "hgr_hier_metrics_fused_rows"):
         assert hasattr(lib, name) and name in _cabi.SIGNATURES
+    # one list set and several are the two modes of one TOR / POR entry point (node_splits, n_sets)
+    for name in ("hgr_hier_finish_rows_gathered_splits", "hgr_hier_metrics_fused_rows_splits"):
+        assert not hasattr(lib, name) and name not in _cabi.SIGNATURES
+    assert len(_cabi.SIGNATURES["hgr_hier_finish_rows_gathered"][1]) == 19
+    assert len(_cabi.SIGNATURES["hgr_hier_metrics_fused_rows"][1]) == 22
     assert lib.hgr_version() == 1
 
 

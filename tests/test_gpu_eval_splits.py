@@ -1,4 +1,4 @@
-"""Several test splits in one scoring pass (``hgr_score_topk_splits`` / ``hgr_hier_metrics_fused_rows_splits`` /
+"""Several test splits in one scoring pass (``hgr_score_topk_splits`` / ``hgr_hier_metrics_fused_rows`` with ``node_splits`` /
 ``evaluate.SplitEval``): per split the same top-K, hits and row counts as ``score_topk`` on that split's rows of the
 union bank, the fp32 oracle under the tie-aware comparison, exact repairs on a hierarchy-ordered bank, per-split TOR /
 POR counters, and the multi-split CLI path."""
@@ -121,7 +121,7 @@ def test_one_split_equals_score_topk():
     assert torch.equal(i[0], i1) and torch.equal(v[0], v1)
 
 
-def test_tor_por_per_split():
+def test_tor_por_split_sets_match_single_set_calls():
     from hgrnet_b200 import ops
     from tests.test_gpu_hier_rows import _setup
     h, x, train_index, n_levels, args, table, _ = _setup((4, 20, 160, 900), 300, 256, 2)
@@ -129,8 +129,8 @@ def test_tor_por_per_split():
     g = torch.Generator().manual_seed(4)
     targets = torch.randint(-1, N, (x.shape[0],), generator=g).to(torch.int32).to(DEV)
     node_splits = torch.randint(0, 8, (N,), generator=g).to(torch.uint8).to(DEV)   # three splits, any overlap
-    counts = torch.zeros((3, ops.HGR_HIER_MAX_CHAIN + 1, 4), dtype=torch.int64, device=DEV)
-    ops.hier_metrics_fused_rows_splits(x, targets=targets, node_splits=node_splits, counts=counts, **args, **table)
+    counts = ops.new_hier_counts(DEV, 3)
+    ops.hier_metrics_fused_rows(x, targets=targets, node_splits=node_splits, counts=counts, **args, **table)
     for s in range(3):
         in_s = (targets >= 0) & ((node_splits[targets.clamp(min=0).long()] >> s) & 1).bool()
         ref = ops.new_hier_counts(DEV)
@@ -184,11 +184,11 @@ def _stream_model(tmp_path):
     return spec, model, h
 
 
-def test_eval_stream_splits_match_eager(tmp_path):
+def test_eval_stream_splits_match_eager_counter_block(tmp_path):
     """A captured ``EvalStream(splits=...)``, replayed over several slots and streams, gives the counters of the eager
     ``SplitEval.update`` calls: per split hits / rows and TOR / POR."""
     from hgrnet_b200 import ops
-    from hgrnet_b200.evaluate import SplitEval
+    from hgrnet_b200.evaluate import SplitEval, hier_totals
     spec, model, h = _stream_model(tmp_path)
     N, B, slots = len(h), spec["B"], 4
     ids = np.random.default_rng(1).permutation(N)
@@ -217,7 +217,8 @@ def test_eval_stream_splits_match_eager(tmp_path):
     assert es.split_hit_counts() == want
     assert es.host_counters[ops.HGR_NUM_HITS:].tolist() == es.counters[ops.HGR_NUM_HITS:].tolist()
     assert all(w[ops.HGR_NUM_HITS] > 0 for w in want)
-    acc = se._hier_acc.tolist()
+    assert torch.equal(es.hier_counts, se.hier_counts)
+    acc = hier_totals(se.hier_counts).tolist()
     for (hr, pr, por), (rows, tor, point, path) in zip(es.split_ratios(), acc):
         assert rows > 0
         assert abs(hr - tor / rows * 100.0) < 1e-9 and abs(pr - path / rows * 100.0) < 1e-9

@@ -245,7 +245,7 @@ def test_eval_stream_hier_matches_eager(tmp_path):
     assert want[0] > 0 and want[1] > 0 and want[2] > 0
 
 
-def test_hier_rows_rejects_bad_arguments():
+def test_hier_rows_rejects_bad_arguments_and_counter_sets():
     from hgrnet_b200 import _cabi, ops
     from hgrnet_b200._cabi import HgrError
     h, x, train_index, n_levels, args, table, _ = _setup((4, 20, 200), 64, 128, 1)
@@ -260,7 +260,7 @@ def test_hier_rows_rejects_bad_arguments():
         return lib.hgr_hier_metrics_fused_rows(p(x), p(args["bank_sorted"]), 64, args["bank_sorted"].shape[0], 128,
                                                level_end, n_lv, p(args["sorted_to_pos"]), p(args["first_out"]), p(t),
                                                len(h), chain_ptr, p(table["chain_pos"]), p(table["chain_level"]),
-                                               workspace, 64 * n_levels * 8, None, None, p(counts), None)
+                                               None, 1, workspace, 64 * n_levels * 8, None, None, p(counts), None)
 
     for bad in (dict(chain_ptr=None), dict(workspace=p(ws) + 4)):
         with pytest.raises(HgrError):
@@ -274,6 +274,8 @@ def test_hier_rows_rejects_bad_arguments():
         ops.hier_metrics_fused_rows(x, targets=t, counts=counts, **args33, **table)
     assert counts.sum().item() == 0                              # nothing ran
     torch.cuda.synchronize()
+    with pytest.raises(ValueError, match="need node_splits"):     # several counter sets, one per split
+        ops.hier_metrics_fused_rows(x, targets=t, counts=ops.new_hier_counts(DEV, 2), **args, **table)
     cpu = {k: v.cpu() for k, v in table.items()}
     with pytest.raises(ValueError, match="no CPU path"):
         ops.hier_metrics_fused_rows(x, targets=t, counts=counts, **args, **cpu)

@@ -207,7 +207,7 @@ class _Rows:
 
 
 @pytest.mark.parametrize("host_io", [False, True])
-def test_sharded_eval_stream_single_rank(host_io):
+def test_sharded_eval_stream_single_rank_counter_block(host_io):
     from hgrnet_b200 import ops
     from hgrnet_b200.dist import HierShard, ShardedEvalStream
     from hgrnet_b200.hierarchy import synthetic_hierarchy
@@ -236,7 +236,7 @@ def test_sharded_eval_stream_single_rank(host_io):
     want = ops.new_hier_counts(DEV)
     for s in range(8):
         ops.hier_metrics_fused_rows(ops.normalize_rows(feats[s].to(DEV)), targets=labels[s].to(DEV), counts=want, **args)
-    assert torch.equal(on.hier_counts, 2 * want)
+    assert torch.equal(on.hier_counts[0], 2 * want)
     if host_io:
         snaps = torch.stack(on.host_counters)                    # the batch that finished last has seen every batch
         assert torch.equal(snaps.max(dim=0).values, on.counters.cpu())
@@ -307,7 +307,7 @@ def _worker(rank, world, port, out):
         c1, _, _ = _single(x, t, args)
         h1 = ops.new_hits(dev)
         rv, ri = ops.score_topk(x, w.to(dev), targets=t, K=K, hits=h1)
-        c = ses.hier_counts.clone()
+        c = ses.hier_counts[0].clone()
         dist.all_reduce(c)
         assert torch.equal(c, 16 * c1), "all-reduced TOR / POR counters differ from the single-GPU call"
         assert ses.all_reduce_hits().tolist() == [16 * v for v in h1.tolist()]

@@ -1,5 +1,5 @@
 """Several test splits in one scoring pass on the class-sharded head (``hgr_score_topk_splits_scatter_bounded`` /
-``hgr_topk_merge_splits_certified`` / ``hgr_hier_finish_rows_gathered_splits``, main.py:104-222 once per split): G
+``hgr_topk_merge_splits_certified`` / ``hgr_hier_finish_rows_gathered`` with ``node_splits``, main.py:104-222 once per split): G
 logical ranks inside one process on one GPU, as tests/test_gpu_peer.py does.  For every split the owners' result is
 ``ops.score_topk`` (exact lists) on that split's rows of the ranks' banks in rank-major order -- values, ids, order and
 hits bit for bit when no owner repaired a row, rows always; then per-split TOR / POR, ``ShardedEvalStream(splits=...)`` against
@@ -73,8 +73,7 @@ def _run_sharded(u, x, targets, G, reps=1):
         table = ops.shard_table([(sh.bank.data_ptr() if sh.C else 0, sh.col_id.data_ptr() if sh.C else 0, sh.C, 0)
                                  for sh in shards], DEV)
         counts = torch.zeros((u.S, ops.HGR_NUM_HITS + 1), dtype=torch.int64, device=DEV)
-        hier_counts = (torch.zeros((u.S, ops.HGR_HIER_MAX_CHAIN + 1, 4), dtype=torch.int64, device=DEV)
-                       if n_levels else None)
+        hier_counts = ops.new_hier_counts(DEV, u.S) if n_levels else None
         repairs = torch.zeros(1, dtype=torch.int32, device=DEV)
         for rep in range(reps):
             slot = rep % 4
@@ -233,7 +232,7 @@ def test_clustered_bank_is_repaired_exactly():
 
 @pytest.mark.parametrize("split", ["all", "real"])
 @pytest.mark.parametrize("G", [2, 8])
-def test_per_split_tor_por_equal_single_gpu(split, G):
+def test_per_split_tor_por_gathered_equal_single_gpu(split, G):
     from hgrnet_b200 import ops
     from tests.test_gpu_hier_sharded import _hierarchy, _rows_args, _split, _targets
     h = _hierarchy("cfg5")
@@ -246,8 +245,8 @@ def test_per_split_tor_por_equal_single_gpu(split, G):
     t[:B // 2] = torch.from_numpy(nodes[np.arange(B // 2) % 3000]).to(torch.int32).to(DEV)   # rows in every split
     x = ops.normalize_rows(torch.randn(B, D, generator=torch.Generator().manual_seed(3)).to(DEV))
     _, _, _, hier_counts, _, _ = _run_sharded(u, x, t, G)
-    want = torch.zeros((u.S, ops.HGR_HIER_MAX_CHAIN + 1, 4), dtype=torch.int64, device=DEV)
-    ops.hier_metrics_fused_rows_splits(x, targets=t, node_splits=u.node_splits, counts=want, **args)
+    want = ops.new_hier_counts(DEV, u.S)
+    ops.hier_metrics_fused_rows(x, targets=t, node_splits=u.node_splits, counts=want, **args)
     assert torch.equal(hier_counts, want)
     assert all(int(want[s, :, 0].sum()) > 0 for s in range(u.S))
 
