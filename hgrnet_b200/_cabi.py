@@ -88,6 +88,8 @@ SIGNATURES = {
                                                 c_void_p, c_int64, c_void_p, c_float, c_void_p, c_void_p]),
     "hgr_hier_mistakes": (c_int, [c_void_p, c_int64, c_int, c_int64, c_int, c_void_p, c_void_p, c_void_p, c_void_p,
                                   c_int64, c_void_p, c_void_p]),
+    "hgr_class_hits": (c_int, [c_void_p, c_int64, c_int, c_int64, c_int, c_void_p, c_void_p, c_int64, c_void_p,
+                               c_void_p]),
     "hgr_masked_ce_workspace_bytes":(c_size_t, [c_int64, c_int64, c_int64]),
     "hgr_om_backward_workspace_bytes": (c_size_t, [c_int64, c_int64, c_int64]),
     "hgr_om_backward": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int64, c_int64, c_void_p, c_void_p, c_void_p,

@@ -19,7 +19,8 @@ LIB = os.path.join(LIBDIR, "libhgr_b200.so")
 INCLUDE = os.path.join(os.path.dirname(HERE), "include")
 
 SOURCES = ["hgr_abi.cu", "aggregate_norm.cu", "topk_merge.cu", "score_simt.cu", "score_launch.cu", "score_pair.cu",
-           "masked_ce.cu", "om_backward.cu", "hier_metrics.cu", "hier_mistakes.cu"]
+           "masked_ce.cu", "om_backward.cu", "hier_metrics.cu", "hier_mistakes.cu",
+           "class_hits.cu"]
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 NVCC_FLAGS = ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr",
               "-Xptxas", "-v"]

@@ -230,6 +230,9 @@ int launch_hier_finish_gathered(const unsigned long long* parts, int n_parts, in
 int launch_hier_mistakes(const int32_t* topk_idx, int64_t B, int K, int64_t set_stride, int n_sets,
                          const int32_t* targets, const uint8_t* node_splits, const int32_t* chain_ptr,
                          const int32_t* chain_node, int64_t n_nodes, int64_t* counts, cudaStream_t stream);
+// per-class Hit@k: counts [n_sets][n_nodes][HGR_NUM_HITS + 1] (class_hits.cu)
+int launch_class_hits(const int32_t* topk_idx, int64_t B, int K, int64_t set_stride, int n_sets, const int32_t* targets,
+                      const uint8_t* node_splits, int64_t n_nodes, int64_t* counts, cudaStream_t stream);
 int launch_normalize_dual(const void* E, int e_dtype, int64_t n_rows, int64_t D, void* out, const int32_t* dst_map,
                           void* out2, cudaStream_t stream);
 // {threads, registers per thread, static shared memory, dynamic shared memory} of the row normalise of [*, D] rows

@@ -780,6 +780,24 @@ int hgr_hier_mistakes(const int32_t* topk_idx, int64_t B, int K, int64_t set_str
                               counts, static_cast<cudaStream_t>(stream));
 }
 
+// main.py:135-148 counted per label: the table behind class-averaged Hit@k (class_hits.cu).
+int hgr_class_hits(const int32_t* topk_idx, int64_t B, int K, int64_t set_stride, int n_sets, const int32_t* targets,
+                   const uint8_t* node_splits, int64_t n_nodes, int64_t* counts, void* stream) {
+  HGR_CHECK_ARG(B >= 0 && B <= (int64_t(1) << 31) - 1, "hgr_class_hits: bad size B=%lld", (long long)B);
+  HGR_CHECK_ARG(K >= 1 && K <= HGR_TOPK_MAX, "hgr_class_hits: K = %d outside [1, %d]", K, HGR_TOPK_MAX);
+  HGR_CHECK_ARG(n_nodes > 0 && n_nodes < (int64_t(1) << 31) - 1, "hgr_class_hits: n_nodes = %lld", (long long)n_nodes);
+  HGR_CHECK_ARG(n_sets >= 1 && n_sets <= (node_splits ? kMaxSplits : 1),
+                "hgr_class_hits: %d list sets outside [1, %d] (%s node_splits)", n_sets, node_splits ? kMaxSplits : 1,
+                node_splits ? "with" : "without");
+  HGR_CHECK_ARG(n_sets == 1 || set_stride >= B * K, "hgr_class_hits: set_stride %lld < B * K = %lld",
+                (long long)set_stride, (long long)(B * K));
+  if (B == 0) return HGR_OK;
+  HGR_CHECK_ARG(topk_idx && targets && counts, "hgr_class_hits: null pointer");
+  HGR_CHECK_ARG((reinterpret_cast<uintptr_t>(counts) & 7u) == 0, "hgr_class_hits: counts must be 8-byte aligned");
+  return launch_class_hits(topk_idx, B, K, set_stride, n_sets, targets, node_splits, n_nodes, counts,
+                           static_cast<cudaStream_t>(stream));
+}
+
 size_t hgr_masked_ce_workspace_bytes(int64_t B, int64_t U, int64_t T) { return masked_ce_workspace_bytes(B, U, T) + 16; }
 
 int hgr_masked_ce(const float* logits, int64_t ldl, int64_t B, int64_t U, const int32_t* set_ptr, const int32_t* set_col,

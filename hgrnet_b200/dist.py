@@ -558,13 +558,19 @@ class ShardedEvalStream:
     row owner counts the mistake severity and LCA distance@k of its merged lists against each row's own label
     (``ops.hier_mistakes``; one counter set per split with ``splits``).  No exchange data and no flag is added; the
     counters sit in ``counters``, and ``mistake_summary()`` / ``split_mistake_summary()`` sum them over ranks.
+
+    ``classes`` (an ``evaluate.ClassHits``, peer exchange only, with or without ``splits``): after the merge the row
+    owner counts Hit@k per class of its merged lists against each row's own label (``ops.class_hits``; one table per
+    split with ``splits``).  No exchange data and no flag is added.  The table is a device buffer of its own
+    (``class_counts``), outside ``counters``, so the per-batch ``host_counters`` copy keeps its size; ``class_table()`` /
+    ``class_summary()`` / ``split_class_summary()`` sum it over ranks.
     """
 
     def __init__(self, bank_shard: torch.Tensor, id_base: int, *, batch: int, K: int = 20, steps: int = 8,
                  feat_dtype=torch.float32, banks=None, group=None, use_graph: bool = True, exchange: str = "p2p",
                  channels: int = 4, host_io: bool = False, col_id: Optional[torch.Tensor] = None,
                  certify: str = "global", hier: Optional[HierShard] = None, splits: Optional[SplitShard] = None,
-                 mistakes: Optional[MistakeShard] = None):
+                 mistakes: Optional[MistakeShard] = None, classes=None):
         if exchange not in ("p2p", "nccl"):
             raise ValueError("exchange must be 'p2p' or 'nccl'")
         if splits is not None:
@@ -585,6 +591,12 @@ class ShardedEvalStream:
             if mistakes.chain_ptr.device != bank_shard.device:
                 raise ValueError("mistakes: the chain table is on %s, the bank on %s" % (mistakes.chain_ptr.device,
                                                                                        bank_shard.device))
+        if classes is not None:
+            if exchange != "p2p":
+                raise ValueError("classes (class-sharded per-class Hit@k) need the peer-memory exchange")
+            if classes.counts.device != bank_shard.device:
+                raise ValueError("classes: the counters are on %s, the bank on %s" % (classes.counts.device,
+                                                                                    bank_shard.device))
         if hier is not None and exchange != "p2p":
             raise ValueError("hier (class-sharded TOR / POR) needs the peer-memory exchange")
         if hier is not None and hier.D != bank_shard.shape[1]:
@@ -625,10 +637,12 @@ class ShardedEvalStream:
         S = 0 if splits is None else splits.S
         self.mistakes = mistakes
         self.tally = EvalCounters(self.device, n_splits=S, hier=self._hier_shard() is not None,
-                                  mistakes=mistakes is not None, K=K, read=self._read_counters)
+                                  mistakes=mistakes is not None, K=K, read=self._read_counters,
+                                  classes=0 if classes is None else classes.n_nodes)
         self.counters, self.hits = self.tally.counters, self.tally.hits
         self.split_counts, self.hier_counts = self.tally.split_counts, self.tally.hier_counts
         self.mistake_counts = self.tally.mistake_counts
+        self.class_counts = self.tally.class_counts
         n_counters = self.counters.numel()
         self.val = [None] * steps
         self.idx = [None] * steps
@@ -690,7 +704,7 @@ class ShardedEvalStream:
         with torch.cuda.stream(self.stream):
             self._issue()                      # warm-up: NCCL communicator, workspaces
             self.stream.synchronize()
-            self.counters.zero_()
+            self.tally.zero_()
             if use_graph:
                 try:
                     g = torch.cuda.CUDAGraph()
@@ -701,7 +715,7 @@ class ShardedEvalStream:
                     print("ShardedEvalStream: graph capture of the NCCL pipeline failed (%r); running eagerly" % (e,))
                     self.graph = None
         torch.cuda.synchronize(self.device)
-        self.counters.zero_()
+        self.tally.zero_()
 
     def _local(self, s: int):
         bank = self.banks[s % len(self.banks)]
@@ -742,11 +756,13 @@ class ShardedEvalStream:
                                               out=(self.val[s], self.idx[s]), targets_local=self.host_io, certify=cert,
                                               hier=self._hier_shard(), counts=self.hier_counts, splits=self.splits,
                                               split_counts=self.split_counts)
+            t = self.dev_labels[s] if self.host_io else self.dev_labels[s][self.row_lo:self.row_hi]
+            node_splits = None if self.splits is None else self.splits.node_splits
             if self.mistakes is not None and self.row_hi > self.row_lo:     # the owner's merged lists, after the merge
-                t = self.dev_labels[s] if self.host_io else self.dev_labels[s][self.row_lo:self.row_hi]
-                ops.hier_mistakes(self.idx[s], t, counts=self.mistake_counts,
-                                  node_splits=None if self.splits is None else self.splits.node_splits,
+                ops.hier_mistakes(self.idx[s], t, counts=self.mistake_counts, node_splits=node_splits,
                                   **self.mistakes.args())
+            if self.class_counts is not None and self.row_hi > self.row_lo:
+                ops.class_hits(self.idx[s], t, self.class_counts, node_splits=node_splits)
             if self.host_io:
                 self.host_counters[s].copy_(self.counters, non_blocking=True)
             return
@@ -842,7 +858,7 @@ class ShardedEvalStream:
 
     def split_lines(self):
         """One ``evaluate.split_line`` per split (Hit@k, plus TOR / POR when the ``SplitShard`` has ``hier`` and the
-        mistake metrics with ``mistakes``)."""
+        mistake metrics with ``mistakes`` and the class-averaged Hit@k with ``classes``)."""
         return self.tally.split_lines(self.splits.names)
 
     def mistake_summary(self):
@@ -854,3 +870,17 @@ class ShardedEvalStream:
         """Per split ``evaluate.mistake_summary`` over the rows of all ranks whose label is in the split.  Needs
         ``mistakes`` and ``splits``."""
         return self.tally.split_mistake_summary()
+
+    def class_table(self) -> torch.Tensor:
+        """The per-class table over the rows of all ranks scored so far, host int64 ``[n_nodes, 6]`` (``[S, n_nodes,
+        6]`` with ``splits``).  Needs ``classes``."""
+        return self.tally.class_table()
+
+    def class_summary(self):
+        """``evaluate.class_summary`` over the rows of all ranks scored so far.  Needs ``classes`` without ``splits``."""
+        return self.tally.class_summary()
+
+    def split_class_summary(self):
+        """Per split ``evaluate.class_summary`` over the rows of all ranks whose label is in the split.  Needs
+        ``classes`` and ``splits``."""
+        return self.tally.split_class_summary()

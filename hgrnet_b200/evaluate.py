@@ -226,6 +226,63 @@ class MistakeMetrics:
         return out[0] if self.n_sets == 1 else out
 
 
+def class_summary(table) -> dict:
+    """The class-averaged Hit@k of one set's per-class table (``[n_nodes, HGR_NUM_HITS + 1]`` int64 rows
+    ``[Hit@1, Hit@2, Hit@5, Hit@10, Hit@20, rows]``, tensor or array), as floats: ``classes`` = the number of classes
+    with at least one row, and ``mean@k`` for k in ``HIT_CUTS`` = the mean over those classes of Hit@k / rows (every
+    class weighs the same, whatever its row count).  All zero without rows."""
+    t = np.asarray(table.cpu() if hasattr(table, "cpu") else table, dtype=np.int64)
+    if t.ndim != 2 or t.shape[1] != len(HIT_CUTS) + 1:
+        raise ValueError("one set of per-class counters [n_nodes, %d] expected, got %s" % (len(HIT_CUTS) + 1,
+                                                                                           list(t.shape)))
+    rows = t[:, -1]
+    seen = rows > 0
+    n = int(seen.sum())
+    mean = (t[seen, :-1] / rows[seen, None]).mean(0) if n else np.zeros(len(HIT_CUTS))
+    out = {"classes": float(n)}
+    for k, m in zip(HIT_CUTS, mean.tolist()):
+        out["mean@%d" % k] = float(m)
+    return out
+
+
+def class_line(summary: dict) -> str:
+    """The suffix ``test()`` appends to its line with ``--hgr_class_metrics``, in percent:
+    ``" class_mean Top@1(%):xx.xx, Top@2(%):xx.xx, Top@5(%):xx.xx, Top@10(%):xx.xx, Top@20(%):xx.xx over N classes"``."""
+    return " class_mean " + ", ".join("Top@{}(%):{:.2f}".format(k, summary["mean@%d" % k] * 100.0) for k in HIT_CUTS) \
+        + " over {} classes".format(int(summary["classes"]))
+
+
+class ClassHits:
+    """Per-class Hit@{1,2,5,10,20} and row counts of the top-K lists of every batch, the table behind the
+    class-averaged Hit@k (``class_summary``) that zero-shot results on ImageNet are usually compared by (e.g. Xian et
+    al., TPAMI 2018): the reference's test loader holds one class per batch, so its image-weighted Hit@k
+    (main.py:135-148) is dominated by the most populous classes.  Holds the counters ``[n_sets, n_nodes,
+    HGR_NUM_HITS + 1]``; ``update`` counts a batch on the device (``ops.class_hits``) with no host synchronisation.
+    ``n_sets`` > 1 counts ``[n_sets, B, K]`` lists of several test splits (``SplitEval``).  ``counts``: the counters to
+    own (default: new ones)."""
+
+    def __init__(self, model, n_sets: int = 1, K: int = 20, counts: Optional[torch.Tensor] = None):
+        self.n_nodes = len(model.nodes)
+        self.n_sets, self.K = n_sets, K
+        self.counts = ops.new_class_counts(model.device, self.n_nodes, n_sets) if counts is None else counts
+
+    def update(self, idx: torch.Tensor, targets: torch.Tensor, node_splits: Optional[torch.Tensor] = None,
+               counts: Optional[torch.Tensor] = None):
+        """Count a batch: ``idx`` int32 node ids ``[B, K]`` (or ``[n_sets, B, K]`` with ``node_splits``), ``targets``
+        [B] node ids, one per row (-1 padding counts nowhere).  Into ``counts`` (default: the object's own)."""
+        ops.class_hits(idx, targets.to(torch.int32), self.counts if counts is None else counts, node_splits=node_splits)
+
+    def table(self) -> torch.Tensor:
+        """The host int64 table so far (synchronises): ``[n_nodes, 6]``, or ``[n_sets, n_nodes, 6]`` for several sets."""
+        t = self.counts.cpu()
+        return t[0] if self.n_sets == 1 else t
+
+    def summary(self):
+        """``class_summary`` of every set (synchronises): a dict, or a list of dicts for several sets."""
+        out = [class_summary(t) for t in self.counts.cpu()]
+        return out[0] if self.n_sets == 1 else out
+
+
 _BANK_SEED = 0x48475221   # the seed of tree_model's test-bank permutation (head.py)
 
 
@@ -257,15 +314,18 @@ def split_groups(splits, n_nodes: int):
     return names, np.concatenate(rows), group_end, masks, node_splits
 
 
-def split_line(name, hits, rows, hier=None, mistakes=None):
+def split_line(name, hits, rows, hier=None, mistakes=None, classes=None):
     """The reference's ``test()`` line of one split (``count_acc`` + TOR / POR), prefixed with the split's name.
-    ``hier``: ``(hits, point, path, path_rows)`` sums or None; ``mistakes``: the split's ``mistake_summary`` or None."""
+    ``hier``: ``(hits, point, path, path_rows)`` sums or None; ``mistakes``: the split's ``mistake_summary`` or None;
+    ``classes``: the split's ``class_summary`` or None."""
     out_str, _ = count_acc(dict(zip(HIT_CUTS, hits)), rows)
     if hier is not None:
         tor, point, path, path_rows = hier
         out_str += hier_line(tor / rows * 100.0, path / path_rows * 100.0 if path_rows else 0.0, point / rows * 100.0)
     if mistakes is not None:
         out_str += mistake_line(mistakes)
+    if classes is not None:
+        out_str += class_line(classes)
     return "{}: {}".format(name, out_str)
 
 
@@ -276,16 +336,28 @@ class EvalCounters:
     length); with ``mistakes`` ``mistake_counts [n, HGR_MISTAKE_COUNTERS]`` -- n = S, or 1 without splits.  The
     kernels increment the views in place, so nothing is zeroed per batch and a stream mirrors everything to the host
     with one copy.  ``read(counters)`` gives the counters the readout reports, in the same layout (default: the
-    buffer itself): a stream synchronises its streams first, a class-sharded stream also sums them over ranks."""
+    buffer itself): a stream synchronises its streams first, a class-sharded stream also sums them over ranks.
 
-    def __init__(self, device, n_splits: int = 0, hier: bool = False, mistakes: bool = False, K: int = 20, read=None):
+    With ``classes`` (the node count) the per-class table ``class_counts [n, classes, HGR_NUM_HITS + 1]``
+    (``ClassHits``) is a buffer of its own, outside ``counters``: at 21,841 nodes it is 1 MB per set, and the streams
+    copy ``counters`` to the host after every step.  It is read only by the readout, through the same ``read``."""
+
+    def __init__(self, device, n_splits: int = 0, hier: bool = False, mistakes: bool = False, K: int = 20, read=None,
+                 classes: int = 0):
         n = max(n_splits, 1)
         self.S, self.K = n_splits, K
         self._shapes = [(ops.HGR_NUM_HITS,), (n_splits, ops.HGR_NUM_HITS + 1),
                         (n if hier else 0, HGR_HIER_MAX_CHAIN + 1, 4), (n if mistakes else 0, HGR_MISTAKE_COUNTERS)]
         self.counters = torch.zeros(sum(int(np.prod(sh)) for sh in self._shapes), dtype=torch.int64, device=device)
         self.hits, self.split_counts, self.hier_counts, self.mistake_counts = self._views(self.counters)
+        self.class_counts = ops.new_class_counts(device, classes, n) if classes else None
         self._read = read
+
+    def zero_(self):
+        """Zero every counter (a stream does so after its warm-up runs)."""
+        self.counters.zero_()
+        if self.class_counts is not None:
+            self.class_counts.zero_()
 
     def _views(self, counters: torch.Tensor):
         parts = torch.split(counters, [int(np.prod(sh)) for sh in self._shapes])
@@ -330,15 +402,34 @@ class EvalCounters:
         self._need("per-split mistake counters", self.mistake_counts is not None and self.S > 0)
         return [mistake_summary(c, self.K) for c in self.read()[3]]
 
+    def class_table(self) -> torch.Tensor:
+        """The per-class table so far as a host int64 tensor: ``[n_nodes, HGR_NUM_HITS + 1]`` without splits,
+        ``[S, n_nodes, HGR_NUM_HITS + 1]`` with them (``hgr_class_hits``'s layout)."""
+        self._need("per-class counters", self.class_counts is not None)
+        t = (self.class_counts if self._read is None else self._read(self.class_counts)).cpu()
+        return t if self.S > 0 else t[0]
+
+    def class_summary(self):
+        """``class_summary`` of the one set without splits."""
+        self._need("per-class counters without splits", self.class_counts is not None and self.S == 0)
+        return class_summary(self.class_table())
+
+    def split_class_summary(self):
+        """Per split ``class_summary`` over the rows whose label is in the split."""
+        self._need("per-split per-class counters", self.class_counts is not None and self.S > 0)
+        return [class_summary(t) for t in self.class_table()]
+
     def split_lines(self, names):
-        """One ``split_line`` per split: Hit@k, plus TOR / POR and the mistake metrics when counted."""
+        """One ``split_line`` per split: Hit@k, plus TOR / POR, the mistake metrics and the class-averaged Hit@k when
+        counted."""
         self._need("splits", self.S > 0)
         _, counts, hier, mist = self.read()
         hier = [None] * self.S if hier is None else [(tor, point, path, rows)
                                                      for rows, tor, point, path in hier_totals(hier).tolist()]
         mist = [None] * self.S if mist is None else [mistake_summary(c, self.K) for c in mist.tolist()]
-        return [split_line(name, c[:ops.HGR_NUM_HITS], max(c[ops.HGR_NUM_HITS], 1), h, m)
-                for name, c, h, m in zip(names, counts.tolist(), hier, mist)]
+        cls = [None] * self.S if self.class_counts is None else self.split_class_summary()
+        return [split_line(name, c[:ops.HGR_NUM_HITS], max(c[ops.HGR_NUM_HITS], 1), h, m, k)
+                for name, c, h, m, k in zip(names, counts.tolist(), hier, mist, cls)]
 
 
 class SplitEval:
@@ -347,10 +438,12 @@ class SplitEval:
     counters of every split stay on the device (``EvalCounters``: ``split_counts``, ``hier_counts``,
     ``mistake_counts``).  With ``hier=True`` the TOR / POR counters of every split follow from one level GEMM per batch
     (``HierMetrics.update_rows`` with ``node_splits``).  With ``mistakes=True`` the mistake severity and LCA
-    distance@k of every split are counted from the ``[S, B, K]`` lists (``MistakeMetrics``, one set per split).
+    distance@k of every split are counted from the ``[S, B, K]`` lists (``MistakeMetrics``, one set per split).  With
+    ``class_metrics=True`` so is the per-class Hit@k table (``ClassHits``, one set per split; ``class_counts``).
     ``lines()`` gives one line per split."""
 
-    def __init__(self, model, splits, hier: bool = True, K: int = 20, mistakes: bool = False):
+    def __init__(self, model, splits, hier: bool = True, K: int = 20, mistakes: bool = False,
+                 class_metrics: bool = False):
         self.model = model
         self.K = K
         dev = model.device
@@ -360,11 +453,14 @@ class SplitEval:
         self._bank_nodes = torch.from_numpy(bank_nodes).to(dev)
         self.col_id = self._bank_nodes.to(torch.int32)
         self.node_splits = torch.from_numpy(node_splits).to(dev)
-        self.tally = EvalCounters(dev, n_splits=self.S, hier=hier, mistakes=mistakes, K=K)
+        self.tally = EvalCounters(dev, n_splits=self.S, hier=hier, mistakes=mistakes, K=K,
+                                  classes=len(model.nodes) if class_metrics else 0)
         self.split_counts, self.hier_counts = self.tally.split_counts, self.tally.hier_counts
         self.mistake_counts = self.tally.mistake_counts
         self.hier = HierMetrics(model) if hier else None
         self.mistakes = MistakeMetrics(model, n_sets=self.S, K=K, counts=self.mistake_counts) if mistakes else None
+        self.class_counts = self.tally.class_counts
+        self.classes = ClassHits(model, n_sets=self.S, K=K, counts=self.class_counts) if class_metrics else None
         self._bank = None
         self._bank_version = None
 
@@ -392,6 +488,8 @@ class SplitEval:
                                   counts=self.hier_counts)
         if self.mistakes is not None:
             self.mistakes.update(out[1], t, node_splits=self.node_splits)
+        if self.classes is not None:
+            self.classes.update(out[1], t, node_splits=self.node_splits)
         return out
 
     def hit_counts(self):
@@ -399,8 +497,8 @@ class SplitEval:
         return self.tally.split_hit_counts()
 
     def lines(self):
-        """One line per split: ``name: Top@1(%):..., ... .`` plus TOR / POR with ``hier`` and the mistake metrics with
-        ``mistakes`` (synchronises)."""
+        """One line per split: ``name: Top@1(%):..., ... .`` plus TOR / POR with ``hier``, the mistake metrics with
+        ``mistakes`` and the class-averaged Hit@k with ``class_metrics`` (synchronises)."""
         return self.tally.split_lines(self.names)
 
 
@@ -411,7 +509,8 @@ def test(opts, model, device, splits=None, loader: Optional[Iterable] = None, lo
     TOR / POR score every row of a batch against the batch's first label, as the reference does with ``targets[0]``
     (main.py:152).  A first label outside the hierarchy is counted nowhere (the reference raises ``IndexError``).
     With ``--hgr_mistake_metrics`` the line also gets the mistake rate, the mistake severity and the LCA distance@k
-    (``MistakeMetrics``), every row against its own label."""
+    (``MistakeMetrics``), every row against its own label.  With ``--hgr_class_metrics`` it also gets the
+    class-averaged Hit@k (``ClassHits``, ``class_line``), every row counted toward its own label."""
     print("out", opts.out_ratio)
     print("in", opts.in_ratio)
     model.eval()
@@ -425,6 +524,7 @@ def test(opts, model, device, splits=None, loader: Optional[Iterable] = None, lo
         return _test_splits(opts, model, device, splits, split_keys, loader, log)
     hier = HierMetrics(model) if getattr(opts, "hgr_hier_metrics", True) else None
     mist = MistakeMetrics(model) if getattr(opts, "hgr_mistake_metrics", False) else None
+    cls = ClassHits(model) if getattr(opts, "hgr_class_metrics", False) else None
     hits = ops.new_hits(model.device)
     num_sample = 0
     out_str = ""
@@ -438,11 +538,13 @@ def test(opts, model, device, splits=None, loader: Optional[Iterable] = None, lo
                 hier.update_rows(x, targets[:1].expand(len(targets)))
             if mist is not None:
                 mist.update(idx, targets)
+            if cls is not None:
+                cls.update(idx, targets)
             if i % opts.print_freq == 0:
-                out_str = _format(hits, num_sample, hier, mist)
+                out_str = _format(hits, num_sample, hier, mist, cls)
                 print(out_str, flush=True)
     print("End of testing.")
-    out_str = _format(hits, num_sample, hier, mist)
+    out_str = _format(hits, num_sample, hier, mist, cls)
     print(out_str, flush=True)
     if log:
         _log(opts, model, out_str)
@@ -455,7 +557,8 @@ def _test_splits(opts, model, device, splits, split_keys, loader, log):
         raise ValueError("--hgr_eval_splits needs the split file's class lists (splits)")
     index = model.hierarchy.index
     se = SplitEval(model, {k: [index[c] for c in splits[k]] for k in split_keys},
-                   hier=getattr(opts, "hgr_hier_metrics", True), mistakes=getattr(opts, "hgr_mistake_metrics", False))
+                   hier=getattr(opts, "hgr_hier_metrics", True), mistakes=getattr(opts, "hgr_mistake_metrics", False),
+                   class_metrics=getattr(opts, "hgr_class_metrics", False))
     with torch.no_grad():
         for i, data in enumerate(loader):
             imgs, targets = data["img"].to(device, non_blocking=True)[0], data["label"].to(device, non_blocking=True)[0]
@@ -479,11 +582,13 @@ def _log(opts, model, out_str):
         f.writelines(method + "\n" + out_str + "\n")
 
 
-def _format(hits, num_sample, hier, mist=None):
+def _format(hits, num_sample, hier, mist=None, cls=None):
     out_str, _ = count_acc(dict(zip(HIT_CUTS, hits.tolist())), num_sample)
     out_str = "\n" + out_str
     if hier is not None:
         out_str += hier_line(*hier.ratios(num_sample))
     if mist is not None:
         out_str += mistake_line(mist.summary())
+    if cls is not None:
+        out_str += class_line(cls.summary())
     return out_str

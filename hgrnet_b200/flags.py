@@ -85,6 +85,9 @@ def build_parser() -> argparse.ArgumentParser:
     g.add_argument("--hgr_mistake_metrics", type=_bool, default=False, choices=[True, False],
                    help="also report the mistake rate, the mistake severity (mean LCA height of the wrong top-1) and "
                         "the LCA distance@k of the top-k during test, per split with --hgr_eval_splits")
+    g.add_argument("--hgr_class_metrics", type=_bool, default=False, choices=[True, False],
+                   help="also report the class-averaged Hit@k (the mean over the classes with test rows of each "
+                        "class's Hit@k / rows) during test, per split with --hgr_eval_splits")
     return p
 
 

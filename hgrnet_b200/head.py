@@ -243,7 +243,7 @@ class tree_model(nn.Module):
 
     def make_eval_stream(self, batch: int, slots: int = 4, streams: int = 2, feat_dtype=torch.float32, K: int = 20,
                          banks=None, host_io: bool = True, hier_metrics: bool = False, eval_splits=None,
-                         mistake_metrics: bool = False):
+                         mistake_metrics: bool = False, class_metrics: bool = False):
         """CUDA-graph replayed eval step over pre-computed image features (hgrnet_b200.stream.EvalStream).
 
         ``hier_metrics=True`` adds TOR / POR (``EvalStream.hier_ratios``), every row scored against its own label.  The
@@ -255,9 +255,16 @@ class tree_model(nn.Module):
         per-split TOR / POR, ``EvalStream.split_ratios``).
 
         ``mistake_metrics=True`` adds the mistake severity and LCA distance@k of every row's top-K against its own label
-        (``EvalStream.mistake_summary``, per split ``EvalStream.split_mistake_summary``)."""
+        (``EvalStream.mistake_summary``, per split ``EvalStream.split_mistake_summary``).
+
+        ``class_metrics=True`` adds the Hit@k of every class, every row counted toward its own label
+        (``EvalStream.class_table``; class-averaged: ``EvalStream.class_summary``, per split
+        ``EvalStream.split_class_summary``)."""
         from .stream import EvalStream
-        hier = splits = mistakes = None
+        hier = splits = mistakes = classes = None
+        if class_metrics:
+            from .evaluate import ClassHits
+            classes = ClassHits(self, K=K)
         if mistake_metrics:
             from .evaluate import MistakeMetrics
             mistakes = MistakeMetrics(self, K=K)
@@ -269,7 +276,7 @@ class tree_model(nn.Module):
             hier = HierMetrics(self)
         return EvalStream(self.bank_test, col_id=self._test_index_i32, batch=batch, feat_dtype=feat_dtype, K=K,
                           slots=slots, streams=streams, banks=banks, host_io=host_io, hier=hier, splits=splits,
-                          mistakes=mistakes)
+                          mistakes=mistakes, classes=classes)
 
     # ------------------------------------------------------------------ training step
     def _schedule(self, training_method, target):

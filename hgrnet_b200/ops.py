@@ -720,6 +720,45 @@ def hier_mistakes(idx: torch.Tensor, targets: torch.Tensor, chain_ptr: torch.Ten
                                       _ptr(counts), _stream()))
 
 
+def new_class_counts(device, n_nodes: int, n_sets: int = 1) -> torch.Tensor:
+    """Zeroed counters of ``class_hits``: int64 ``[n_sets, n_nodes, HGR_NUM_HITS + 1]``, per class
+    ``[Hit@1, Hit@2, Hit@5, Hit@10, Hit@20, rows]`` (see ``hgr_class_hits`` in the header)."""
+    return torch.zeros((n_sets, n_nodes, HGR_NUM_HITS + 1), dtype=torch.int64, device=device)
+
+
+def class_hits(idx: torch.Tensor, targets: torch.Tensor, counts: torch.Tensor,
+               node_splits: Optional[torch.Tensor] = None) -> None:
+    """Per-class Hit@{1,2,5,10,20} and row counters (``hgr_class_hits``) of top-K lists on the device: ``idx`` int32
+    node ids ``[B, K]`` (one set) or ``[S, B, K]`` (one set per test split, with ``node_splits``: list set s counts a
+    row only when bit s of ``node_splits[targets[row]]`` is set).  ``targets`` [B] node ids, row by row; a row whose
+    label is outside ``[0, n_nodes)`` counts nowhere.  ``counts`` (``new_class_counts(device, n_nodes, S)``) is
+    incremented.  No host work depends on the batch: the call can be captured in a CUDA graph."""
+    lib = _cabi.load()
+    if idx.dim() == 2:
+        idx = idx.unsqueeze(0)
+    if idx.dim() != 3 or idx.dtype != torch.int32 or not idx.is_cuda:
+        raise ValueError("idx must be a CUDA int32 [B, K] or [S, B, K] tensor")
+    if not (idx.stride(2) == 1 and idx.stride(1) == idx.shape[2]):
+        idx = idx.contiguous()
+    S, B, K = idx.shape
+    targets = _require(targets, "targets", torch.int32)
+    if not counts.is_cuda or counts.dtype != torch.int64 or counts.dim() != 3 or counts.shape[0] != S \
+            or counts.shape[2] != HGR_NUM_HITS + 1 or not counts.is_contiguous():
+        raise ValueError("counts must be a contiguous CUDA int64 [%d, n_nodes, %d] tensor (new_class_counts)"
+                         % (S, HGR_NUM_HITS + 1))
+    n_nodes = counts.shape[1]
+    if node_splits is not None:
+        node_splits = _require(node_splits, "node_splits", torch.uint8)
+        if node_splits.numel() != n_nodes:
+            raise ValueError("node_splits must have one entry per node")
+    elif S != 1:
+        raise ValueError("%d list sets need node_splits" % S)
+    if targets.numel() != B:
+        raise ValueError("targets must have one entry per list row")
+    _cabi.check(lib.hgr_class_hits(_ptr(idx), B, K, idx.stride(0) if S > 1 else B * K, S, _ptr(targets),
+                                   _ptr(node_splits), n_nodes, _ptr(counts), _stream()))
+
+
 def masked_ce(logits: torch.Tensor, set_ptr: torch.Tensor, set_col: torch.Tensor, label_pos: torch.Tensor,
               weight: torch.Tensor, need_grad: bool = True):
     """Fused masked CE over T class sets (model/clip_tree.py:241-277).  Returns ``(loss [T], dlogits [B,U] | None)``."""

@@ -33,6 +33,11 @@ when the stream is built.
 With ``mistakes`` (an ``evaluate.MistakeMetrics``) each graph also counts the mistake severity and LCA distance@k of
 the slot's top-K lists against its per-row labels (``ops.hier_mistakes``, one warp per row), one counter set per split
 with ``splits``.  These counters too sit in the one device buffer (``mistake_summary`` / ``split_mistake_summary``).
+
+With ``classes`` (an ``evaluate.ClassHits``) each graph also counts Hit@k per class of the slot's top-K lists against
+its per-row labels (``ops.class_hits``, one thread per row), one table per split with ``splits``.  The table
+(``class_counts``, 1 MB per set at 21,841 nodes) is a device buffer of its own: the per-step D2H copy stays the few KB
+of ``counters``, and the table is read only at readout (``class_table`` / ``class_summary`` / ``split_class_summary``).
 """
 from __future__ import annotations
 
@@ -47,7 +52,7 @@ from .evaluate import EvalCounters
 class EvalStream:
     def __init__(self, bank: torch.Tensor, col_id: Optional[torch.Tensor] = None, id_base: int = 0, *, batch: int,
                  feat_dtype=torch.float32, K: int = 20, slots: int = 4, streams: int = 2, banks=None,
-                 host_io: bool = True, hier=None, splits=None, mistakes=None):
+                 host_io: bool = True, hier=None, splits=None, mistakes=None, classes=None):
         """``bank`` [C, D] bf16 on the device.  ``banks``: optional list of bank tensors to rotate over per slot
         (benchmarks use it to keep the working set larger than L2).  ``host_io=False`` skips the H2D / D2H nodes
         (features are then written straight into ``dev_feats`` / ``dev_labels``).  ``hier``: optional
@@ -56,7 +61,9 @@ class EvalStream:
         ``evaluate.SplitEval``; every step then scores against its splits instead of ``bank`` (``val`` / ``idx`` are
         ``[S, B, K]``, ``hit_counts`` stays zero, ``split_hit_counts`` / ``split_ratios`` give the per-split results).
         ``mistakes``: optional ``evaluate.MistakeMetrics`` of the model (its chain table); every step then also counts the
-        mistake severity and LCA distance@k of the slot's lists (``mistake_summary`` / ``split_mistake_summary``)."""
+        mistake severity and LCA distance@k of the slot's lists (``mistake_summary`` / ``split_mistake_summary``).
+        ``classes``: optional ``evaluate.ClassHits`` of the model; every step then also counts the slot's Hit@k per class
+        (``class_table`` / ``class_summary`` / ``split_class_summary``)."""
         self.device = bank.device
         self.K = K
         self.B = batch
@@ -87,10 +94,12 @@ class EvalStream:
         self._mistake_args = mistakes.args() if mistakes is not None else None
         self._node_splits = None if splits is None else splits.node_splits
         self.tally = EvalCounters(self.device, n_splits=0 if splits is None else splits.S, hier=hier is not None,
-                                  mistakes=mistakes is not None, K=K, read=self._read_counters)
+                                  mistakes=mistakes is not None, K=K, read=self._read_counters,
+                                  classes=0 if classes is None else classes.n_nodes)
         self.counters, self.hits = self.tally.counters, self.tally.hits
         self.split_counts, self.hier_counts = self.tally.split_counts, self.tally.hier_counts
         self.mistake_counts = self.tally.mistake_counts
+        self.class_counts = self.tally.class_counts
         if host_io:
             self.host_pack = [torch.zeros(nbytes, dtype=torch.uint8).pin_memory() for _ in range(slots)]
             self.host_feats, self.host_labels = map(list, zip(*[views(p) for p in self.host_pack]))
@@ -123,6 +132,8 @@ class EvalStream:
         if self._mistake_args is not None:                                           # main.py:135-148, hierarchy distance
             ops.hier_mistakes(self.idx[s], self.dev_labels[s], counts=self.mistake_counts, node_splits=self._node_splits,
                               **self._mistake_args)
+        if self.class_counts is not None:                                            # main.py:135-148, per class
+            ops.class_hits(self.idx[s], self.dev_labels[s], self.class_counts, node_splits=self._node_splits)
         if self.host_io:
             self.host_counters.copy_(self.counters, non_blocking=True)
 
@@ -136,7 +147,7 @@ class EvalStream:
                 self._body(s)                             # warm-up: workspace allocation, lazy module loading
         for st in self.streams:
             st.synchronize()
-        self.counters.zero_()
+        self.tally.zero_()
         torch.cuda.synchronize(self.device)
         for s in range(self.slots):
             st = self._stream_of(s)
@@ -204,3 +215,17 @@ class EvalStream:
         """Per split ``evaluate.mistake_summary`` over the rows whose label is in the split, in the order of
         ``splits.names`` (synchronises).  Needs ``mistakes`` and ``splits``."""
         return self.tally.split_mistake_summary()
+
+    def class_table(self) -> torch.Tensor:
+        """The per-class table so far, host int64 ``[n_nodes, 6]`` (``[S, n_nodes, 6]`` with ``splits``): per class
+        ``[Hit@1, @2, @5, @10, @20, rows]`` (synchronises).  Needs ``classes``."""
+        return self.tally.class_table()
+
+    def class_summary(self):
+        """``evaluate.class_summary`` of the rows scored so far (synchronises).  Needs ``classes`` without ``splits``."""
+        return self.tally.class_summary()
+
+    def split_class_summary(self):
+        """Per split ``evaluate.class_summary`` over the rows whose label is in the split, in the order of
+        ``splits.names`` (synchronises).  Needs ``classes`` and ``splits``."""
+        return self.tally.split_class_summary()

@@ -454,6 +454,24 @@ int hgr_hier_mistakes(const int32_t* topk_idx, int64_t B, int K, int64_t set_str
                       int64_t* counts, void* stream);
 
 /*
+ * Per-class Hit@{1,2,5,10,20} of top-K lists already on the device -- the lists of hgr_score_topk /
+ * hgr_score_topk_splits / the certified merges: the reference's Hit@k count (main.py:135-148) kept per label, from
+ * which the class-averaged accuracy (the mean over classes of Hit@k / rows) follows.
+ * A row counts when 0 <= targets[row] < n_nodes: it adds 1 to `rows` of its label and, when the label is at position
+ * pos of its list (first match), 1 to every Hit@k with pos < k (the rule of the hits / counts of hgr_score_topk).
+ *
+ *  topk_idx    n_sets lists [B, K] int32 node ids, list set s at topk_idx + s * set_stride; K <= HGR_TOPK_MAX
+ *  node_splits NULL: n_sets must be 1.  Otherwise [n_nodes] uint8 and n_sets <= 8: list set s counts a row only when
+ *              bit s of node_splits[targets[row]] is set (the rule of hgr_score_topk_splits)
+ *  counts      [n_sets][n_nodes][HGR_NUM_HITS + 1] int64, INCREMENTED; row t of set s holds
+ *              {Hit@1, Hit@2, Hit@5, Hit@10, Hit@20, rows} of the rows labelled t
+ * One thread per row; the rows of a warp with equal labels are combined before they reach global memory (one atomic per
+ * non-zero counter, label and warp).  No allocation, no host work per batch: capturable in a CUDA graph.
+ */
+int hgr_class_hits(const int32_t* topk_idx, int64_t B, int K, int64_t set_stride, int n_sets, const int32_t* targets,
+                   const uint8_t* node_splits, int64_t n_nodes, int64_t* counts, void* stream);
+
+/*
  * Fused masked cross-entropy of the OM training step over T sampled class sets
  * (model/clip_tree.py:241-277 with nn.CrossEntropyLoss, :49,:275).
  *
