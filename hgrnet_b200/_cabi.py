@@ -18,6 +18,8 @@ HGR_F32, HGR_BF16, HGR_F16 = 0, 1, 2
 HGR_IMPL_AUTO, HGR_IMPL_SIMT, HGR_IMPL_TCGEN05 = 0, 1, 2
 HGR_IMPL_TCGEN05_EXACT, HGR_IMPL_TCGEN05_NULL, HGR_IMPL_TCGEN05_SKETCH = 4, 5, 12
 HGR_IMPL_FLAG_NO_MERGE = 0x100
+HGR_IMPL_GRID_SHARE_SHIFT = 12
+HGR_GRID_SHARE_MAX = 8
 HGR_NUM_HITS = 5
 HGR_TOPK_MAX = 32
 HGR_HIER_MAX_CHAIN = 32
@@ -37,6 +39,9 @@ SIGNATURES = {
     "hgr_score_topk_workspace_bytes": (c_size_t, [c_int64, c_int64, c_int64, c_int]),
     "hgr_score_topk_plan": (c_int, [c_int64, c_int64, c_int64, c_int, c_void_p]),
     "hgr_score_topk_footprint": (c_int, [c_int64, c_int64, c_int64, c_int, c_int, c_void_p]),
+    "hgr_score_topk_plan_shared": (c_int, [c_int64, c_int64, c_int64, c_int, c_int, c_void_p]),
+    "hgr_score_topk_grid_share": (c_int, [c_int64, c_int64, c_int64, c_int]),
+    "hgr_score_topk_footprint_shared": (c_int, [c_int64, c_int64, c_int64, c_int, c_int, c_int, c_void_p]),
     "hgr_score_topk": (c_int, [c_void_p, c_void_p, c_void_p, c_int32, c_void_p, c_int64, c_int64, c_int64,
                                c_float, c_int, c_void_p, c_size_t, c_void_p, c_void_p, c_void_p, c_int,
                                c_void_p]),

@@ -187,15 +187,18 @@ int launch_logits_simt(const __nv_bfloat16* X, const __nv_bfloat16* bank, int64_
 
 size_t umma_score_workspace_bytes(int64_t B, int64_t C, int K);
 bool umma_supported(int64_t B, int64_t C, int64_t D, int K);
-void umma_plan(int64_t B, int64_t C, int64_t D, int K, int32_t* plan);
-int umma_footprint(int64_t B, int64_t C, int64_t D, int K, int32_t* out);
+// grid_share: batches meant to run at the same time (HGR_IMPL_GRID_SHARE); 1 = the whole grid
+int umma_grid_share(int64_t B, int64_t C);
+void umma_plan(int64_t B, int64_t C, int64_t D, int K, int grid_share, int32_t* plan);
+int umma_footprint(int64_t B, int64_t C, int64_t D, int K, int grid_share, int32_t* out);
 // C_total > 0 (with scatter->emit_bound): the lists are sized for a row's GLOBAL stream of C_total classes, of which
 // this bank is one shard -- no local certificate / repair, the owner of the row certifies against the global K-th value
 int launch_score_topk_umma(const __nv_bfloat16* X, const __nv_bfloat16* bank, const int32_t* col_id,
                            int32_t id_base, const int32_t* targets, int64_t B, int64_t C, int64_t D,
                            float scale, int K, void* ws, size_t ws_bytes, float* topk_val,
                            int32_t* topk_idx, int64_t* hits, int variant, bool skip_merge,
-                           cudaStream_t stream, const OutScatter* scatter = nullptr, int64_t C_total = 0);
+                           cudaStream_t stream, const OutScatter* scatter = nullptr, int64_t C_total = 0,
+                           int grid_share = 1);
 int umma_global_list_len(int64_t B, int64_t C, int64_t D, int K, int64_t C_total);
 size_t umma_split_workspace_bytes(int64_t B, const Groups& gr, int K);
 // scatter (class shard of the union bank, hgr_score_topk_splits_scatter_bounded): lists sized for each split's GLOBAL

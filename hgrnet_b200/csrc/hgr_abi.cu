@@ -120,7 +120,9 @@ static int score_topk_impl(const void* X, const void* bank, const int32_t* col_i
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   if (C == 0) return merge_zero_lists(B, K, topk_val, topk_idx, scatter, s);   // empty class set
   const bool skip_merge = (impl & HGR_IMPL_FLAG_NO_MERGE) != 0;
-  impl &= ~HGR_IMPL_FLAG_NO_MERGE;
+  const int share = (impl & HGR_IMPL_GRID_SHARE_MASK) >> HGR_IMPL_GRID_SHARE_SHIFT;
+  HGR_CHECK_ARG(share <= HGR_GRID_SHARE_MAX, "hgr_score_topk: grid share %d outside [0, %d]", share, HGR_GRID_SHARE_MAX);
+  impl &= ~(HGR_IMPL_FLAG_NO_MERGE | HGR_IMPL_GRID_SHARE_MASK);
   const int which = pick_impl(impl, B, C, D, K);
   if (which == HGR_IMPL_TCGEN05 || which == HGR_IMPL_TCGEN05_EXACT || which == HGR_IMPL_TCGEN05_NULL ||
       which == HGR_IMPL_TCGEN05_SKETCH) {
@@ -128,7 +130,8 @@ static int score_topk_impl(const void* X, const void* bank, const int32_t* col_i
     const int variant = which - HGR_IMPL_TCGEN05;  // umma::Variant
     return launch_score_topk_umma(static_cast<const __nv_bfloat16*>(X), static_cast<const __nv_bfloat16*>(bank), col_id,
                                   id_base, targets, B, C, D, scale, K, workspace, workspace_bytes, topk_val, topk_idx,
-                                  hits, variant, skip_merge || which == HGR_IMPL_TCGEN05_NULL, s, scatter, C_total);
+                                  hits, variant, skip_merge || which == HGR_IMPL_TCGEN05_NULL, s, scatter, C_total,
+                                  share > 1 ? share : 1);
   }
   if (which == HGR_IMPL_SIMT)
     return launch_score_topk_simt(static_cast<const __nv_bfloat16*>(X), static_cast<const __nv_bfloat16*>(bank), col_id,
@@ -287,20 +290,37 @@ int hgr_score_topk_splits_global_list_len(int64_t B, int64_t C, int64_t D, int K
   return umma_split_global_list_len(B, C, D, K, gr, group_splits, n_splits, split_C_total);
 }
 
-int hgr_score_topk_plan(int64_t B, int64_t C, int64_t D, int K, int32_t* plan) {
+int hgr_score_topk_plan_shared(int64_t B, int64_t C, int64_t D, int K, int grid_share, int32_t* plan) {
   HGR_CHECK_ARG(plan != nullptr, "hgr_score_topk_plan: null plan");
   HGR_CHECK_ARG(K >= 1 && K <= HGR_TOPK_MAX, "hgr_score_topk_plan: K = %d outside [1, %d]", K, HGR_TOPK_MAX);
+  HGR_CHECK_ARG(grid_share >= 0 && grid_share <= HGR_GRID_SHARE_MAX, "hgr_score_topk_plan: grid share %d outside [0, %d]",
+                grid_share, HGR_GRID_SHARE_MAX);
   if (!umma_supported(B, C, D, K)) return set_error(HGR_ERR_UNSUPPORTED, "hgr_score_topk_plan: shape not supported by the tcgen05 kernel");
-  umma_plan(B, C, D, K, plan);
+  umma_plan(B, C, D, K, grid_share > 1 ? grid_share : 1, plan);
   return HGR_OK;
 }
 
-int hgr_score_topk_footprint(int64_t B, int64_t C, int64_t D, int K, int x_dtype, int32_t* out) {
+int hgr_score_topk_plan(int64_t B, int64_t C, int64_t D, int K, int32_t* plan) {
+  return hgr_score_topk_plan_shared(B, C, D, K, 1, plan);
+}
+
+int hgr_score_topk_grid_share(int64_t B, int64_t C, int64_t D, int K) {
+  if (K < 1 || K > HGR_TOPK_MAX || !umma_supported(B, C, D, K)) return 1;
+  return umma_grid_share(B, C);
+}
+
+int hgr_score_topk_footprint_shared(int64_t B, int64_t C, int64_t D, int K, int grid_share, int x_dtype, int32_t* out) {
   HGR_CHECK_ARG(out != nullptr, "hgr_score_topk_footprint: null out");
   HGR_CHECK_ARG(K >= 1 && K <= HGR_TOPK_MAX, "hgr_score_topk_footprint: K = %d outside [1, %d]", K, HGR_TOPK_MAX);
+  HGR_CHECK_ARG(grid_share >= 0 && grid_share <= HGR_GRID_SHARE_MAX,
+                "hgr_score_topk_footprint: grid share %d outside [0, %d]", grid_share, HGR_GRID_SHARE_MAX);
   if (!umma_supported(B, C, D, K)) return set_error(HGR_ERR_UNSUPPORTED, "hgr_score_topk_footprint: shape not supported by the tcgen05 kernel");
   const int rc = normalize_rows_footprint(x_dtype, D, out);
-  return rc != HGR_OK ? rc : umma_footprint(B, C, D, K, out + 4);
+  return rc != HGR_OK ? rc : umma_footprint(B, C, D, K, grid_share > 1 ? grid_share : 1, out + 4);
+}
+
+int hgr_score_topk_footprint(int64_t B, int64_t C, int64_t D, int K, int x_dtype, int32_t* out) {
+  return hgr_score_topk_footprint_shared(B, C, D, K, 1, x_dtype, out);
 }
 
 int hgr_score_topk(const void* X, const void* bank, const int32_t* col_id, int32_t id_base, const int32_t* targets,

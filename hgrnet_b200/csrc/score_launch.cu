@@ -49,6 +49,11 @@ int make_map(CUtensorMap* map, const void* base, int64_t rows, int64_t D, int bo
   return HGR_OK;
 }
 
+// Columns per worker up to which a stream counts as short: per-segment and per-launch costs, not the main loop, decide
+constexpr int64_t kShortStreamCols = 3072;
+// Grid share the streaming evaluator asks for on short streams (umma_grid_share)
+constexpr int kStreamGridShare = 2;
+
 // CTA pairs the persistent kernel runs on
 int usable_sms() {
   const int n = num_sms();
@@ -80,30 +85,40 @@ static double sched_cost(const Sched& s) {
 // Workers: all CTA pairs, unless a slightly smaller count that is a multiple of the row-tile count wins -- then no
 // chunk straddles a row tile (one list per worker, no ragged sub-tiles at both ends; measured at B = 4096:
 // 64 aligned pairs beat 74 for every bank size, e.g. 33.6 vs 39.7 us at C = 2,731).
-Sched pick_sched(int64_t B, int64_t C) {
+//
+// grid_share c > 1: the call is one of c batches meant to run side by side (the streaming evaluator's round-robin
+// streams), so it takes floor(pairs / c) pairs, rounded down to a multiple of the row tiles.  Each worker then streams
+// c times the columns: its fixed costs (set-up, first operands, exposed tail) and the A-operand re-stream of its
+// remainder sub-tile are paid once per longer run, and a row has fewer, longer lists.
+Sched pick_sched(int64_t B, int64_t C, int grid_share = 1) {
   const int most = usable_sms() / 2;
+  if (grid_share > 1) {
+    const int budget = most / grid_share > 0 ? most / grid_share : 1;
+    const int MT = static_cast<int>((B + 2 * kTileM - 1) / (2 * kTileM));
+    return make_sched(B, C, budget >= MT ? budget / MT * MT : budget, 2 * kTileM);
+  }
   Sched best = make_sched(B, C, most, 2 * kTileM);
   if (best.MT > 1 && best.MT <= most && best.G == most) {
     const int aligned = most / best.MT * best.MT;
     if (aligned != most && aligned * 10 >= most * 8) {
       const Sched alt = make_sched(B, C, aligned, 2 * kTileM);
-      // only for short streams (<= 3072 columns per worker): there the per-segment costs decide; on long streams the
-      // fewer, larger lists of the aligned split sit closer to the speculation limit (an expected repair of a
-      // 5,000-column range costs more than the alignment saves -- measured at cfg 5)
+      // only for short streams (<= kShortStreamCols columns per worker): there the per-segment costs decide; on long
+      // streams the fewer, larger lists of the aligned split sit closer to the speculation limit (an expected repair
+      // of a 5,000-column range costs more than the alignment saves -- measured at cfg 5)
       const int64_t cols_per_worker = (alt.T + alt.G - 1) / alt.G * kUnit;
-      if (cols_per_worker <= 3072 && sched_cost(alt) < sched_cost(best)) best = alt;
+      if (cols_per_worker <= kShortStreamCols && sched_cost(alt) < sched_cost(best)) best = alt;
     }
   }
   return best;
 }
 
 int common_setup(const __nv_bfloat16* X, const __nv_bfloat16* bank, int64_t B, int64_t C, int64_t D,
-                 CUtensorMap* mx, CUtensorMap* mb, Params* p) {
+                 CUtensorMap* mx, CUtensorMap* mb, Params* p, int grid_share = 1) {
   int rc = make_map(mx, X, B, D, kTileM);
   if (rc != HGR_OK) return rc;
   rc = make_map(mb, bank, C, D, kBBoxRows);
   if (rc != HGR_OK) return rc;
-  p->sched = pick_sched(B, C);
+  p->sched = pick_sched(B, C, grid_share);
   p->B = B;
   p->C = C;
   p->num_k_blocks = static_cast<int>((D + kBlockK - 1) / kBlockK);
@@ -131,8 +146,9 @@ double max_list_share(const Sched& s) {
 
 // Speculate only while the EXPECTED repair time per call stays below 1.5 % of the call's estimated duration (main
 // loop at 60 % of the bf16 peak).  cfg 2 (37 lists of 590 columns per row, KL = 8): 7e-4 repairs x 0.36 ms = 0.25 us
-// of 24 us -- accepted, and worth it (exact 20-entry lists cost 55 us there).  B = 4096 (4-6 lists per row): 16-entry
-// lists would save ~6 us per call but cost 1-8 us in expected repairs -- rejected, exact lists run in the same
+// of 24 us -- accepted, and worth it (exact 20-entry lists cost 55 us there).  cfg 2 on half the grid (grid share 2: 18
+// lists of 1,216 columns): KL = 8 expects 0.1 repairs per call, KL = 10 5e-4 -- KL = 10.  B = 4096 (4-6 lists per row):
+// 16-entry lists would save ~6 us per call but cost 1-8 us in expected repairs -- rejected, exact lists run in the same
 // deferred-insert mode.
 int pick_list_len(int K, int64_t B, int64_t C, int64_t D, int lists_per_row, double share, bool allow_speculation) {
   const int exact = K <= 8 ? 8 : (K <= 12 ? 12 : (K <= 20 ? 20 : 32));
@@ -192,8 +208,13 @@ bool umma_supported(int64_t B, int64_t C, int64_t D, int K) {
 }
 
 size_t umma_score_workspace_bytes(int64_t B, int64_t C, int K) {
-  // worst case over the list-width policy (exact lists) and the candidate lists of the floor-sketch variant
-  const int p2 = pick_sched(B, C).P;
+  // worst case over the grid shares, the list-width policy (exact lists) and the candidate lists of the floor-sketch
+  // variant (all pairs)
+  int p2 = 1;
+  for (int c = 1; c <= HGR_GRID_SHARE_MAX; ++c) {
+    const int p = pick_sched(B, C, c).P;
+    p2 = p > p2 ? p : p2;
+  }
   const int p4 = make_sched(B, C, usable_sms() / 2, 2 * kTileM).P;
   const int kl = K <= 8 ? 8 : (K <= 12 ? 12 : (K <= 20 ? 20 : 32));
   const size_t lists = static_cast<size_t>(p2) * B * kl * (sizeof(float) + sizeof(int32_t));
@@ -201,9 +222,18 @@ size_t umma_score_workspace_bytes(int64_t B, int64_t C, int K) {
   return (lists > sketch ? lists : sketch) + kWsHeaderBytes;
 }
 
-// The decisions launch_score_topk_umma takes for the production variant, without launching anything.
-void umma_plan(int64_t B, int64_t C, int64_t D, int K, int32_t* plan) {
+// The grid share for a batch that runs beside others (the streaming evaluator): on short streams (<= kShortStreamCols
+// columns per worker on the whole grid) kStreamGridShare, the best of shares 1-4 measured at cfg 2
+// (profiles/r09_concurrent_grid); long streams (every B >= 2048, e.g. cfg 5) keep the schedule of a lone call.
+int umma_grid_share(int64_t B, int64_t C) {
+  if (B >= 2048) return 1;
   const Sched s = pick_sched(B, C);
+  return (s.T + s.G - 1) / s.G * kUnit <= kShortStreamCols ? kStreamGridShare : 1;
+}
+
+// The decisions launch_score_topk_umma takes for the production variant, without launching anything.
+void umma_plan(int64_t B, int64_t C, int64_t D, int K, int grid_share, int32_t* plan) {
+  const Sched s = pick_sched(B, C, grid_share);
   plan[0] = s.G;
   plan[1] = s.MT;
   plan[2] = s.U;
@@ -216,9 +246,9 @@ void umma_plan(int64_t B, int64_t C, int64_t D, int K, int32_t* plan) {
 
 // The production scoring kernel and the merge behind it as launch_score_topk_umma runs them: {threads, registers per
 // thread, static shared memory, dynamic shared memory} of each.
-int umma_footprint(int64_t B, int64_t C, int64_t D, int K, int32_t* out) {
+int umma_footprint(int64_t B, int64_t C, int64_t D, int K, int grid_share, int32_t* out) {
   int32_t plan[8];
-  umma_plan(B, C, D, K, plan);
+  umma_plan(B, C, D, K, grid_share, plan);
   const int rc = pair_kernel_footprint(B, plan[4], out);
   return rc != HGR_OK ? rc : merge_kernel_footprint(plan[3], plan[4], out + 4);
 }
@@ -227,7 +257,7 @@ int launch_score_topk_umma(const __nv_bfloat16* X, const __nv_bfloat16* bank, co
                            int32_t id_base, const int32_t* targets, int64_t B, int64_t C, int64_t D, float scale,
                            int K, void* ws, size_t ws_bytes, float* topk_val, int32_t* topk_idx, int64_t* hits,
                            int variant, bool skip_merge, cudaStream_t stream, const OutScatter* scatter,
-                           int64_t C_total) {
+                           int64_t C_total, int grid_share) {
   // variants: kVarProd   production: deferred-insert lists, speculative (KL < K) when provably cheap
   //           kVarExact  the same kernel with K-entry lists (no speculation)
   //           kVarNull   main loop with a trivial epilogue (ceiling; NOT a top-k) -- diagnostics only
@@ -237,7 +267,7 @@ int launch_score_topk_umma(const __nv_bfloat16* X, const __nv_bfloat16* bank, co
                      umma_score_workspace_bytes(B, C, K));
   CUtensorMap mx, mb;
   Params p{};
-  int rc = common_setup(X, bank, B, C, D, &mx, &mb, &p);
+  int rc = common_setup(X, bank, B, C, D, &mx, &mb, &p, grid_share);
   if (rc != HGR_OK) return rc;
   p.scale = scale;
   p.stats = static_cast<unsigned int*>(ws);                              // header: statistics, timeline stamps

@@ -243,7 +243,7 @@ class tree_model(nn.Module):
 
     def make_eval_stream(self, batch: int, slots: int = 4, streams: int = 2, feat_dtype=torch.float32, K: int = 20,
                          banks=None, host_io: bool = True, hier_metrics: bool = False, eval_splits=None,
-                         mistake_metrics: bool = False, class_metrics: bool = False):
+                         mistake_metrics: bool = False, class_metrics: bool = False, concurrent=None):
         """CUDA-graph replayed eval step over pre-computed image features (hgrnet_b200.stream.EvalStream).
 
         ``hier_metrics=True`` adds TOR / POR (``EvalStream.hier_ratios``), every row scored against its own label.  The
@@ -259,7 +259,10 @@ class tree_model(nn.Module):
 
         ``class_metrics=True`` adds the Hit@k of every class, every row counted toward its own label
         (``EvalStream.class_table``; class-averaged: ``EvalStream.class_summary``, per split
-        ``EvalStream.split_class_summary``)."""
+        ``EvalStream.split_class_summary``).
+
+        ``concurrent``: grid share of the slots' scoring calls (``EvalStream``'s ``concurrent``; default: the library's
+        recommendation for the batch shape)."""
         from .stream import EvalStream
         hier = splits = mistakes = classes = None
         if class_metrics:
@@ -276,7 +279,7 @@ class tree_model(nn.Module):
             hier = HierMetrics(self)
         return EvalStream(self.bank_test, col_id=self._test_index_i32, batch=batch, feat_dtype=feat_dtype, K=K,
                           slots=slots, streams=streams, banks=banks, host_io=host_io, hier=hier, splits=splits,
-                          mistakes=mistakes, classes=classes)
+                          mistakes=mistakes, classes=classes, concurrent=concurrent)
 
     # ------------------------------------------------------------------ training step
     def _schedule(self, training_method, target):

@@ -134,10 +134,13 @@ def normalize_rows_dual(E: torch.Tensor, out: torch.Tensor, dst_map: Optional[to
 def score_topk(X: torch.Tensor, bank: torch.Tensor, *, col_id: Optional[torch.Tensor] = None, id_base: int = 0,
                targets: Optional[torch.Tensor] = None, K: int = 20, scale: float = 1.0,
                hits: Optional[torch.Tensor] = None, impl: int = HGR_IMPL_AUTO,
-               out: Optional[Tuple[torch.Tensor, torch.Tensor]] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+               out: Optional[Tuple[torch.Tensor, torch.Tensor]] = None,
+               grid_share: int = 1) -> Tuple[torch.Tensor, torch.Tensor]:
     """Fused logits + per-row sorted top-K (+ Hit@k accumulation into ``hits``).
 
     model/clip_tree.py:331 + main.py:136-147.  Returns ``(val [B,K] fp32, idx [B,K] int32 node ids)``.
+    ``grid_share`` > 1: the call is one of that many batches meant to run at the same time, and the tcgen05 kernel
+    takes that share of the CTA pairs (``HGR_IMPL_GRID_SHARE``; same results).
     """
     lib = _cabi.load()
     X = _require(X, "X", torch.bfloat16)
@@ -164,6 +167,10 @@ def score_topk(X: torch.Tensor, bank: torch.Tensor, *, col_id: Optional[torch.Te
     else:
         val = torch.empty((B, K), dtype=torch.float32, device=X.device)
         idx = torch.empty((B, K), dtype=torch.int32, device=X.device)
+    if not 1 <= grid_share <= _cabi.HGR_GRID_SHARE_MAX:
+        raise ValueError("grid_share = %d outside [1, %d]" % (grid_share, _cabi.HGR_GRID_SHARE_MAX))
+    if grid_share > 1:
+        impl |= grid_share << _cabi.HGR_IMPL_GRID_SHARE_SHIFT
     nbytes = lib.hgr_score_topk_workspace_bytes(B, C, D, K)
     ws = _workspace(nbytes, X.device)
     _cabi.check(lib.hgr_score_topk(_ptr(X), _ptr(bank), _ptr(col_id), id_base, _ptr(targets), B, C, D,
@@ -229,22 +236,29 @@ def score_topk_splits(X: torch.Tensor, bank: torch.Tensor, group_end, group_spli
     return val, idx
 
 
-def score_topk_plan(B: int, C: int, D: int, K: int = 20) -> dict:
-    """What ``score_topk`` would do for this shape on the tcgen05 path (no launch, works without a GPU)."""
+def score_topk_plan(B: int, C: int, D: int, K: int = 20, grid_share: int = 1) -> dict:
+    """What ``score_topk`` would do for this shape on the tcgen05 path at ``grid_share`` (no launch, works without a
+    GPU)."""
     import ctypes
     plan = (ctypes.c_int32 * 8)()
-    _cabi.check(_cabi.load().hgr_score_topk_plan(B, C, D, K, plan))
+    _cabi.check(_cabi.load().hgr_score_topk_plan_shared(B, C, D, K, grid_share, plan))
     keys = ("workers", "row_tiles", "units_per_row_tile", "lists_per_row", "list_len", "warps_per_quarter",
             "ring_depth", "cols_per_worker")
     return dict(zip(keys, list(plan)))
 
 
-def score_topk_footprint(B: int, C: int, D: int, K: int = 20, x_dtype=torch.bfloat16) -> dict:
-    """What one batch of ``normalize_rows`` + ``score_topk`` asks of an SM, per kernel (``normalize``, ``score``,
-    ``merge``): ``{threads, registers, static_smem, dynamic_smem}`` (registers per thread, bytes).  Needs a device."""
+def score_topk_grid_share(B: int, C: int, D: int, K: int = 20) -> int:
+    """The ``grid_share`` the library recommends for a batch of this shape that runs beside others (host only)."""
+    return int(_cabi.load().hgr_score_topk_grid_share(B, C, D, K))
+
+
+def score_topk_footprint(B: int, C: int, D: int, K: int = 20, x_dtype=torch.bfloat16, grid_share: int = 1) -> dict:
+    """What one batch of ``normalize_rows`` + ``score_topk`` (at ``grid_share``) asks of an SM, per kernel
+    (``normalize``, ``score``, ``merge``): ``{threads, registers, static_smem, dynamic_smem}`` (registers per thread,
+    bytes).  Needs a device."""
     import ctypes
     out = (ctypes.c_int32 * 12)()
-    _cabi.check(_cabi.load().hgr_score_topk_footprint(B, C, D, K, _DTYPE_CODE[x_dtype], out))
+    _cabi.check(_cabi.load().hgr_score_topk_footprint_shared(B, C, D, K, grid_share, _DTYPE_CODE[x_dtype], out))
     keys = ("threads", "registers", "static_smem", "dynamic_smem")
     return {name: dict(zip(keys, list(out)[4 * i:4 * i + 4])) for i, name in enumerate(("normalize", "score", "merge"))}
 

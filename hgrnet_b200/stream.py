@@ -38,6 +38,12 @@ With ``classes`` (an ``evaluate.ClassHits``) each graph also counts Hit@k per cl
 its per-row labels (``ops.class_hits``, one thread per row), one table per split with ``splits``.  The table
 (``class_counts``, 1 MB per set at 21,841 nodes) is a device buffer of its own: the per-step D2H copy stays the few KB
 of ``counters``, and the table is read only at readout (``class_table`` / ``class_summary`` / ``split_class_summary``).
+
+With two or more streams, neighbouring batches' scoring kernels run side by side, so each graph's scoring call asks for
+the grid share the library recommends for the batch shape (``ops.score_topk_grid_share``): on short streams (cfg 2:
+B = 512 against 21,841 classes) each batch takes half the CTA pairs and runs twice as many columns per worker, instead
+of every batch paying the kernel's fixed costs on every SM.  ``grid_share`` / ``plan()`` report what the slots run;
+``concurrent=`` overrides the share.  ``splits`` keeps the whole grid.
 """
 from __future__ import annotations
 
@@ -52,7 +58,8 @@ from .evaluate import EvalCounters
 class EvalStream:
     def __init__(self, bank: torch.Tensor, col_id: Optional[torch.Tensor] = None, id_base: int = 0, *, batch: int,
                  feat_dtype=torch.float32, K: int = 20, slots: int = 4, streams: int = 2, banks=None,
-                 host_io: bool = True, hier=None, splits=None, mistakes=None, classes=None):
+                 host_io: bool = True, hier=None, splits=None, mistakes=None, classes=None,
+                 concurrent: Optional[int] = None):
         """``bank`` [C, D] bf16 on the device.  ``banks``: optional list of bank tensors to rotate over per slot
         (benchmarks use it to keep the working set larger than L2).  ``host_io=False`` skips the H2D / D2H nodes
         (features are then written straight into ``dev_feats`` / ``dev_labels``).  ``hier``: optional
@@ -63,7 +70,9 @@ class EvalStream:
         ``mistakes``: optional ``evaluate.MistakeMetrics`` of the model (its chain table); every step then also counts the
         mistake severity and LCA distance@k of the slot's lists (``mistake_summary`` / ``split_mistake_summary``).
         ``classes``: optional ``evaluate.ClassHits`` of the model; every step then also counts the slot's Hit@k per class
-        (``class_table`` / ``class_summary`` / ``split_class_summary``)."""
+        (``class_table`` / ``class_summary`` / ``split_class_summary``).  ``concurrent``: the grid share of every
+        slot's scoring call (``ops.score_topk(grid_share=...)``, 1 = the whole grid); by default the library's
+        recommendation for the batch shape with two or more streams, else 1."""
         self.device = bank.device
         self.K = K
         self.B = batch
@@ -108,6 +117,14 @@ class EvalStream:
         self.val = [None] * slots
         self.idx = [None] * slots
         self.streams = [torch.cuda.Stream(device=self.device) for _ in range(max(1, min(streams, slots)))]
+        if splits is not None and concurrent not in (None, 1):
+            raise ValueError("concurrent: the grid share applies to the single-bank scoring call, not to splits")
+        if concurrent is not None:
+            self.grid_share = int(concurrent)
+        elif splits is None and len(self.streams) >= 2:
+            self.grid_share = ops.score_topk_grid_share(batch, bank.shape[0], D, K)
+        else:
+            self.grid_share = 1
         self.graphs = []
         self.num_samples = 0
         self._capture()
@@ -119,10 +136,10 @@ class EvalStream:
         if self.host_io:
             self.dev_pack[s].copy_(self.host_pack[s], non_blocking=True)
         x = ops.normalize_rows(self.dev_feats[s])                                    # clip_tree.py:330
-        if self._split_args is None:
+        if self._split_args is None:                                                 # clip_tree.py:331 + main.py:136-147
             self.val[s], self.idx[s] = ops.score_topk(x, self.banks[s % len(self.banks)], col_id=self.col_id,
                                                       id_base=self.id_base, targets=self.dev_labels[s], K=self.K,
-                                                      hits=self.hits)                # clip_tree.py:331 + main.py:136-147
+                                                      hits=self.hits, grid_share=self.grid_share)
         else:                                                                        # the same, once per test split
             self.val[s], self.idx[s] = ops.score_topk_splits(x, targets=self.dev_labels[s], counts=self.split_counts,
                                                              **self._split_args)
@@ -157,6 +174,14 @@ class EvalStream:
                     self._body(s)
                 self.graphs.append(g)
         torch.cuda.synchronize(self.device)
+
+    def plan(self) -> dict:
+        """What every slot's scoring call runs (``ops.score_topk_plan`` at ``grid_share``), with ``grid_share``.  Needs
+        no ``splits``."""
+        if self.splits is not None:
+            raise ValueError("plan(): the slots score against splits (ops.score_topk_splits)")
+        C, D = self.banks[0].shape
+        return dict(ops.score_topk_plan(self.B, C, D, self.K, grid_share=self.grid_share), grid_share=self.grid_share)
 
     # ------------------------------------------------------------------ per-batch API
     def begin(self):

@@ -58,6 +58,15 @@ extern "C" {
 /* OR-ed into `impl`: run only the GEMM + fused top-k kernel and leave the per-CTA partial lists in
  * the workspace (outputs untouched).  Lets bench.py time the dominant kernel alone for the roofline. */
 #define HGR_IMPL_FLAG_NO_MERGE 0x100
+/* OR-ed into `impl`: HGR_IMPL_GRID_SHARE(c) plans the tcgen05 scoring kernel for one of c batches meant to run at the
+ * same time on round-robin streams: floor(CTA pairs / c) pairs, rounded down to a multiple of the row tiles, instead of
+ * all of them (fewer, longer worker streams and lists; same results).  c in [1, HGR_GRID_SHARE_MAX]; 0 and 1 mean the
+ * whole grid.  The floor-sketch variant and the SIMT kernel always use the whole grid.  hgr_score_topk_grid_share gives
+ * the share the library recommends for a shape. */
+#define HGR_IMPL_GRID_SHARE_SHIFT 12
+#define HGR_IMPL_GRID_SHARE_MASK (0xF << HGR_IMPL_GRID_SHARE_SHIFT)
+#define HGR_IMPL_GRID_SHARE(c) ((c) << HGR_IMPL_GRID_SHARE_SHIFT)
+#define HGR_GRID_SHARE_MAX 8
 
 int hgr_version(void);
 const char* hgr_last_error(void);
@@ -123,10 +132,18 @@ size_t hgr_score_topk_workspace_bytes(int64_t B, int64_t C, int64_t D, int K);
  * per row tile, partial lists per row, entries per list (< K: speculative), epilogue warps per TMEM quarter, operand
  * ring depth, bank rows streamed per worker}. */
 int hgr_score_topk_plan(int64_t B, int64_t C, int64_t D, int K, int32_t* plan /* [8] */);
+/* hgr_score_topk_plan for a call with impl | HGR_IMPL_GRID_SHARE(grid_share). */
+int hgr_score_topk_plan_shared(int64_t B, int64_t C, int64_t D, int K, int grid_share, int32_t* plan /* [8] */);
+/* The grid share the library recommends for a batch of this shape that runs beside others (host only): > 1 on short
+ * streams (few bank columns per worker on the whole grid), 1 otherwise and for shapes the tcgen05 kernel does not take. */
+int hgr_score_topk_grid_share(int64_t B, int64_t C, int64_t D, int K);
 /* What one batch of hgr_score_topk asks of an SM, for checking which of its kernels can share one: {threads, registers
  * per thread, static shared memory, dynamic shared memory} of (0) the row normalise of x_dtype [B, D] features into
  * bf16, (1) the tcgen05 scoring kernel, (2) the merge of its partial lists.  Needs a device. */
 int hgr_score_topk_footprint(int64_t B, int64_t C, int64_t D, int K, int x_dtype, int32_t* out /* [12] */);
+/* hgr_score_topk_footprint for a call with impl | HGR_IMPL_GRID_SHARE(grid_share). */
+int hgr_score_topk_footprint_shared(int64_t B, int64_t C, int64_t D, int K, int grid_share, int x_dtype,
+                                    int32_t* out /* [12] */);
 int hgr_score_topk(const void* X, const void* bank, const int32_t* col_id, int32_t id_base,
                    const int32_t* targets, int64_t B, int64_t C, int64_t D, float scale, int K,
                    void* workspace, size_t workspace_bytes, float* topk_val, int32_t* topk_idx,
