@@ -176,6 +176,10 @@ struct SplitCertArgs {
 };
 int launch_topk_split_merge_certified(const SplitCertArgs& args, cudaStream_t stream);
 
+// Bytes at the front of the per-stream scoring workspace that carry state from one tcgen05 scoring call to the next
+// (umma_common.cuh: statistics, the floor-sketch epoch, timeline stamps); every other user of the workspace starts
+// behind them.
+constexpr int kScoreWsHeaderBytes = 64 + 256 * 32 * 8;
 size_t simt_score_workspace_bytes(int64_t B, int64_t C, int K);
 int launch_score_topk_simt(const __nv_bfloat16* X, const __nv_bfloat16* bank, const int32_t* col_id,
                            int32_t id_base, const int32_t* targets, int64_t B, int64_t C, int64_t D,

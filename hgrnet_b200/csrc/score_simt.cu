@@ -89,8 +89,10 @@ int pick_splits(int64_t B, int64_t C) {
 
 }  // namespace
 
+// The partial lists sit behind the header of the scoring workspace, which carries the tcgen05 calls' state between
+// calls (umma_common.cuh: re-scan count, floor-sketch epoch) and is left alone here.
 size_t simt_score_workspace_bytes(int64_t B, int64_t C, int K) {
-  return static_cast<size_t>(pick_splits(B, C)) * B * K * (sizeof(float) + sizeof(int32_t));
+  return static_cast<size_t>(pick_splits(B, C)) * B * K * (sizeof(float) + sizeof(int32_t)) + kScoreWsHeaderBytes;
 }
 
 int launch_score_topk_simt(const __nv_bfloat16* X, const __nv_bfloat16* bank, const int32_t* col_id,
@@ -101,7 +103,7 @@ int launch_score_topk_simt(const __nv_bfloat16* X, const __nv_bfloat16* bank, co
   const size_t need = simt_score_workspace_bytes(B, C, K);
   if (ws_bytes < need || ws == nullptr)
     return set_error(HGR_ERR_WORKSPACE, "hgr_score_topk(simt): workspace %zu < %zu bytes", ws_bytes, need);
-  float* part_val = static_cast<float*>(ws);
+  float* part_val = reinterpret_cast<float*>(static_cast<uint8_t*>(ws) + kScoreWsHeaderBytes);
   int32_t* part_idx = reinterpret_cast<int32_t*>(part_val + static_cast<size_t>(S) * B * K);
   const int D8 = static_cast<int>(D / 8);
   const size_t smem = static_cast<size_t>(kSimtWarps) * D8 * sizeof(uint4);

@@ -57,7 +57,8 @@ struct Params {
 };
 
 constexpr int kTimelineSlots = 32;
-constexpr int kWsHeaderBytes = 64 + 256 * kTimelineSlots * 8;  // statistics + timeline stamps in front of the partial lists
+constexpr int kWsHeaderBytes = kScoreWsHeaderBytes;  // statistics + timeline stamps in front of the partial lists
+static_assert(kWsHeaderBytes >= 64 + 256 * kTimelineSlots * 8, "the header holds the statistics and the timeline stamps");
 
 __device__ __forceinline__ void stamp(const Params& p, int slot) {
   if (p.timeline != nullptr && blockIdx.x < 256) {

@@ -787,7 +787,14 @@ def masked_ce(logits: torch.Tensor, set_ptr: torch.Tensor, set_col: torch.Tensor
     loss = torch.empty((T,), dtype=torch.float32, device=logits.device)
     dl = torch.empty_like(logits) if need_grad else None
     nbytes = lib.hgr_masked_ce_workspace_bytes(B, U, T)
-    ws = _workspace(nbytes, logits.device)
+    # a buffer of its own: the scoring workspace's header carries state between scoring calls (hgr_score_topk)
+    key = ("masked_ce", logits.device.index, _stream())
+    ws = _workspaces.get(key)
+    if ws is None or ws.numel() < nbytes:
+        if ws is not None:
+            _retired.append(ws)
+        ws = torch.empty(nbytes, dtype=torch.uint8, device=logits.device)
+        _workspaces[key] = ws
     _cabi.check(lib.hgr_masked_ce(_ptr(logits), logits.stride(0), B, U, _ptr(set_ptr), _ptr(set_col),
                                   _ptr(label_pos), _ptr(weight), T, _ptr(loss), _ptr(dl), _ptr(ws), ws.numel(),
                                   _stream()))

@@ -123,7 +123,11 @@ int hgr_normalize_rows_dual(const void* E, int e_dtype, int64_t n_rows, int64_t 
  *  topk_idx  [B, K] int32 node ids (col_id applied)
  *  hits      [HGR_NUM_HITS] int64, INCREMENTED by the number of rows whose label is within
  *            the top-{1,2,5,10,20}; NULL to skip.  (k beyond K counts within K.)
- *  workspace at least hgr_score_topk_workspace_bytes(B, C, D, K) bytes, 16-byte aligned
+ *  workspace at least hgr_score_topk_workspace_bytes(B, C, D, K) bytes, 16-byte aligned, ZERO on first use and
+ *            reserved for the scoring family (hgr_score_topk, _scatter, _scatter_bounded, hgr_score_topk_splits,
+ *            _splits_scatter_bounded) between calls: its header carries state from one call to the next (the rows the
+ *            last call re-scanned exactly, in its first word, and the launch epoch of the floor-sketch variant), so it
+ *            is never cleared per batch and no other call may write it
  * If C < K the missing entries are (-inf, -1).
  */
 size_t hgr_score_topk_workspace_bytes(int64_t B, int64_t C, int64_t D, int K);
@@ -175,7 +179,8 @@ int hgr_topk_merge(const float* part_val, const int32_t* part_idx, int64_t P, in
  *                                  process maps it with hgr_peer_open (peer access is enabled on first use).
  * hgr_score_topk_scatter           hgr_score_topk whose final [B, K] lists go, block of rows by block of rows, to
  *                                  val_blocks[g] / idx_blocks[g] (HOST arrays of n_blocks device pointers, local
- *                                  or peer); no hit counting (a hit needs the merged, global rank).
+ *                                  or peer); no hit counting (a hit needs the merged, global rank).  workspace as
+ *                                  hgr_score_topk's (zero on first use, reserved for the scoring family).
  * hgr_peer_signal                  after the scatter: publish this rank's next sequence number (device counter
  *                                  *seq, incremented by the kernel) to flags[g] (one word on every rank g).
  * hgr_peer_wait                    before the merge: increment the consumer's own device counter *seq and spin
@@ -204,7 +209,8 @@ int hgr_score_topk_scatter(const void* X, const void* bank, const int32_t* col_i
  *                                  classes; no local certificate, no local repair.  Next to the final list of a row
  *                                  the producer stores bound_blocks[g][row - g * block_rows] = scale * (the largest
  *                                  last entry of its FULL narrow lists; -inf when no list dropped anything): every
- *                                  candidate the shard did not report is <= that bound.
+ *                                  candidate the shard did not report is <= that bound.  workspace as
+ *                                  hgr_score_topk's (zero on first use, reserved for the scoring family).
  * hgr_topk_merge_certified         hgr_topk_merge of the P = n_shards lists of the owner's rows; a row is certified
  *                                  when its merged K-th value beats every shard's bound STRICTLY.  Otherwise the
  *                                  doubtful shards are re-scanned exactly on the CUDA cores with the row's features
